@@ -2,7 +2,7 @@
 """Benchmark of the signal-packer hot path (BASELINE.json: compress/decompress raw GB/s per packer, CR,
 % HBM roofline).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Headline = BASELINE configs[1]: xdelta_hzr, 12 ch x 3 B x 8192 samples, synthetic ECG-like frames generated on
 the device.  A STEP is one pass of the packer over `--batches` distinct batches of `--frames` frames per GPU
@@ -428,6 +428,32 @@ def measure_packer(R, torch, D, kind, sh, F, nbatch, reps, hbm_peak, e2e_frames,
     return r
 
 
+DUMP_FRAMES = 16          # frames per batch whose compressed bytes are dumped
+DUMP_INDEX_BYTES = 1 << 19  # decode-index bytes dumped per batch
+
+
+def dump_outputs(torch, p, outs, nb, F, out_dir):
+    """What a caller of the timed path received in the last step, as .npy files: the batches still held in
+    `outs` (the step's last two; the outputs alternate between two buffers).  Per batch the frame offsets and
+    plane counts in full, the compressed bytes of a fixed sample of frames and a fixed sample of the decode
+    index.  At most 2 x 16 x max_compressed_size x 4 B of stream plus 4 MB of index: under 64 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(0)
+    frames = np.sort(rng.choice(F, size=min(DUMP_FRAMES, F), replace=False))
+    arrays = {"sample_frames": frames.astype(np.float64)}
+    for i in range(max(0, nb - 2), nb):
+        b = outs[i & 1]
+        offs = b.offsets[: F + 1].cpu().numpy()
+        stream = np.concatenate([b.stream[int(offs[f]):int(offs[f + 1])].cpu().numpy() for f in frames])
+        used = p.sidecar_used_bytes(F, int(offs[F]))
+        pos = np.sort(rng.choice(used, size=min(DUMP_INDEX_BYTES, used), replace=False))
+        index = b.sidecar[torch.from_numpy(pos).to(b.sidecar.device)].cpu().numpy()
+        arrays.update({f"batch{i}_offsets": offs.astype(np.float64), f"batch{i}_frame_nb": b.frame_nb[:F].cpu().numpy().astype(np.float32),
+                       f"batch{i}_stream_sample": stream.astype(np.float32), f"batch{i}_index_sample": index.astype(np.float32)})
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     from rspt_b200 import packer as R
@@ -479,6 +505,8 @@ def run_ours(args):
     ms = D.max(e0.elapsed_time(e1))
     clocks = sampler.stop() if rank == 0 else None
     launches = p.counters()["kernel_launches"] - c0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, p, outs, NB, F, args.dump_outputs)
     raw_step = NB * F * fb
     value = world * args.steps * raw_step / (ms * 1e-3) / 1e9
     b = p.compress_batch(inputs[0], out=outs[0])
@@ -566,7 +594,13 @@ def main():
     ap.add_argument("--cpu-budget", type=float, default=5.0)
     ap.add_argument("--cpu-threads", type=int, default=0)
     ap.add_argument("--cpu-frames-per-thread", type=int, default=64)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a fixed sample of the last step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; --impl reference has none")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)

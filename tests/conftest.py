@@ -42,6 +42,3 @@ def golden_inputs(golden, oracle):
 
 def has_ref():
     return os.path.exists(os.path.join(ROOT, "oracle", "_ref", "libref.so"))
-
-
-needs_ref = pytest.mark.skipif(not has_ref(), reason="oracle/_ref/libref.so not built (no /root/reference)")
