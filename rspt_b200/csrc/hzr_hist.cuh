@@ -1,5 +1,5 @@
 // hzr token histogram for sm_100a: one CTA per hzr block, 16 bytes per lane, 512 bytes per
-// warp-step.  Replaces Histogram (lib_hzr/hzr_encode.c:133-173).  Two launches (k_hzr_hist<1>,
+// warp-step.  Replaces Histogram (lib_hzr/hzr_encode.c:133-173).  Two launches (k_hzr_hist<3> or <1>,
 // k_hzr_hist<2>) split the blocks by a density probe: sparse-looking blocks are tokenised from a
 // sorted list of their non-zero bytes (described at the kernel), dense-looking ones by the scan
 // described here.
@@ -115,7 +115,8 @@ __device__ __forceinline__ void scatter_chunks(const Chunk& c, uint32_t off, uin
 
 // ---- sparse blocks ---------------------------------------------------------------------------
 // A block with few non-zero bytes (<= kListCap, i.e. mostly long zero runs: the upper byte planes
-// of a delta-coded signal) is tokenised from a sorted list of its non-zero bytes:
+// of a delta-coded signal) is tokenised from a sorted list of its non-zero bytes (PART 1; PART 3
+// below does steps 1-2 with fewer instructions):
 //   1. every warp scans a contiguous range of <= 16 steps, keeping per step and lane the 16-bit
 //      non-zero mask and the exclusive count of non-zero bytes before the chunk (no barrier; the
 //      loads of a batch of steps are in flight together);
@@ -128,17 +129,28 @@ constexpr uint32_t kListCap = 5120;                 // entries of a block's spar
 constexpr uint8_t kClassSparse = 0, kClassDense = 1;  // blk_class: which histogram launch (and tree launch) owns the block
 constexpr size_t kHistSmem = (size_t)kListCap * 4;
 constexpr int kHistSteps = kMaxSteps / (kHistThreads / 32);      // steps per warp: 16
+// PART 3 builds the same list in two lighter phases (the sparse planes' non-zero bytes are clustered:
+// ~80 % of the steps hold some, ~4 of 32 chunks each):
+//   1. every warp only COUNTS the non-zero bytes of its range and notes, per lane, which of its <= 16
+//      steps have a non-zero chunk (one bit each); one reduction per warp gives the warp total;
+//   2. after the block scan of the totals, the warp walks its steps that have a non-zero chunk: those
+//      lanes reload their chunk into a 512-byte per-warp slot of shared memory, and the chunks are
+//      served two at a time by half a warp each (lane p of the half reads byte p); a ballot of the
+//      kept bytes gives their order, and a warp-uniform running count gives their list index.
+// No per-step prefix scan and no per-step registers remain, so the kernel fits 32 registers.
+constexpr size_t kHistSmemList = kHistSmem + (size_t)(kHistThreads / 32) * kStepBytes;
 
 // Two independent launches per batch, each over all blocks; the density probe (deterministic, the
 // same in both) assigns every block to exactly one of them and is recorded in blk_class:
-//   PART 1 takes the sparse-looking blocks (list + histogram; if the list overflows after all, the
-//          dense scan runs here too -- rare);
+//   PART 1 or 3 takes the sparse-looking blocks (list + histogram; if the list overflows after all,
+//          the dense scan runs here too -- rare); 3 is the default, 1 the earlier list builder
+//          (RSPT_SPARSE_LIST=0), same list and histogram;
 //   PART 2 takes the dense-looking blocks (dense scan).
 // They run on two streams: the tree build of the dense class (long, latency-bound) then overlaps
-// with PART 1.  The split also lets the dense scan run at 8 CTAs per SM (30 registers) while the
-// sparse part keeps 16 mask/prefix registers per lane.
+// with the sparse part.  The split also lets the dense scan run at 8 CTAs per SM (30 registers) while
+// PART 1 keeps 16 mask/prefix registers per lane.
 template <int PART>
-__global__ void __launch_bounds__(kHistThreads, PART == 2 ? 8 : 5) k_hzr_hist(const uint8_t* __restrict__ planes, Shape s,
+__global__ void __launch_bounds__(kHistThreads, PART == 1 ? 5 : 8) k_hzr_hist(const uint8_t* __restrict__ planes, Shape s,
                                                                const uint8_t* __restrict__ frame_nb,
                                                                uint32_t* __restrict__ hist,
                                                                uint16_t* __restrict__ step_lz,
@@ -174,9 +186,11 @@ __global__ void __launch_bounds__(kHistThreads, PART == 2 ? 8 : 5) k_hzr_hist(co
         if (dense_class != (PART == 2)) return;  // the other launch owns this block
     }
     // ---- sparse path
-    if (PART == 1) {
+    if (PART != 2) {
     do {
-
+        uint32_t* list = s_list;
+        uint32_t m = 0;
+        if (PART == 1) {
         // 1. masks and in-warp prefix counts of every step of my warp's range
         uint32_t pk[kHistSteps];  // nz mask | entries of my warp before this chunk << 16
         uint32_t wrun = 0;
@@ -216,7 +230,7 @@ __global__ void __launch_bounds__(kHistThreads, PART == 2 ? 8 : 5) k_hzr_hist(co
         }
         if (lane == 0) s_wtot[wid] = wrun;
         __syncthreads();
-        uint32_t wbase = 0, m = 0;
+        uint32_t wbase = 0;
         for (uint32_t w = 0; w < nwarps; ++w) {
             const uint32_t t = s_wtot[w];
             if (w < wid) wbase += t;
@@ -225,7 +239,6 @@ __global__ void __launch_bounds__(kHistThreads, PART == 2 ? 8 : 5) k_hzr_hist(co
         if (m > kListCap || m > n / 4u) break;
 
         // 2. scatter the non-zero bytes into the list
-        uint32_t* list = s_list;
 #pragma unroll
         for (int j = 0; j < kHistSteps; ++j) {
             const uint32_t nz = pk[j] & 0xFFFFu;
@@ -237,6 +250,67 @@ __global__ void __launch_bounds__(kHistThreads, PART == 2 ? 8 : 5) k_hzr_hist(co
                 if (nz) c.v = __ldg(reinterpret_cast<const uint4*>(src + off));
                 scatter_chunks(c, off, wbase + (pk[j] >> 16), list);
             }
+        }
+        } else {
+        // 1. count the non-zero bytes of my warp's range; bit j of smask: my chunk of step s_lo + j has some
+        uint32_t cnt = 0, smask = 0;
+#pragma unroll
+        for (int j0 = 0; j0 < kHistSteps; j0 += 4) {
+            uint4 v[4];
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                const uint32_t st = s_lo + j0 + j, off = st * kStepBytes + lane * 16u;
+                v[j] = make_uint4(0, 0, 0, 0);
+                if (st < s_hi && off < n) v[j] = __ldg(reinterpret_cast<const uint4*>(src + off));
+            }
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                if ((v[j].x | v[j].y | v[j].z | v[j].w) != 0u) {
+                    const int valid = (int)n - (int)((s_lo + j0 + j) * kStepBytes + lane * 16u);  // > 0 here
+                    const uint32_t c = __popc(nz_mask16(v[j]) & (valid >= 16 ? 0xFFFFu : (1u << valid) - 1u));
+                    cnt += c;
+                    smask |= (c != 0u ? 1u : 0u) << (j0 + j);
+                }
+            }
+        }
+        const uint32_t wtot = __reduce_add_sync(0xFFFFFFFFu, cnt);
+        if (lane == 0) s_wtot[wid] = wtot;
+        __syncthreads();
+        uint32_t at = 0;  // list index of the next entry of my warp (warp-uniform)
+        for (uint32_t w = 0; w < nwarps; ++w) {
+            const uint32_t t = s_wtot[w];
+            if (w < wid) at += t;
+            m += t;
+        }
+        if (m > kListCap || m > n / 4u) break;
+
+        // 2. scatter: chunks staged in my warp's slot, two per iteration, lane p of a half takes byte p
+        uint4* slot = reinterpret_cast<uint4*>(s_list + kListCap) + wid * 32u;
+        const uint8_t* slot_b = reinterpret_cast<const uint8_t*>(slot);
+        const uint32_t p = lane & 15u, below = (1u << lane) - 1u;
+        for (uint32_t steps = __reduce_or_sync(0xFFFFFFFFu, smask); steps; steps &= steps - 1u) {
+            const uint32_t j = __ffs(steps) - 1u, st_off = (s_lo + j) * kStepBytes;
+            const bool mine = (smask >> j) & 1u;
+            if (mine) slot[lane] = __ldg(reinterpret_cast<const uint4*>(src + st_off + lane * 16u));
+            uint32_t todo = __ballot_sync(0xFFFFFFFFu, mine);
+            __syncwarp();
+            while (todo) {
+                const uint32_t la = __ffs(todo) - 1u;
+                todo &= todo - 1u;
+                uint32_t lb = la;  // odd count: the upper half reads the same chunk and keeps nothing
+                if (todo) {
+                    lb = __ffs(todo) - 1u;
+                    todo &= todo - 1u;
+                }
+                const uint32_t sl = lane < 16 ? la : lb, pos = st_off + sl * 16u + p;
+                const uint32_t x = slot_b[sl * 16u + p];
+                const bool keep = x != 0u && pos < n && (lane < 16 || lb != la);
+                const uint32_t kept = __ballot_sync(0xFFFFFFFFu, keep);
+                if (keep) list[at + __popc(kept & below)] = pos | (x << 16);
+                at += __popc(kept);
+            }
+            __syncwarp();  // the slot is read before the next step overwrites it
+        }
         }
         __syncthreads();
 

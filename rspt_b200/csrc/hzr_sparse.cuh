@@ -47,6 +47,15 @@ struct SparseOut {
     uint32_t* sidecar;    // decode index (may be null), see common.cuh
 };
 
+// Every entry i <= m of the list stands for the tokens between the previous non-zero byte and this
+// one: the zero run (if any), its extra bits, then the literal (entry m: the run up to the block end).
+// The entries' bit offsets are a prefix sum of their bit lengths.
+//   ONE_PASS (default): the CTA takes the entries 256 at a time, one per thread, and places each with a
+//     warp scan plus the warp totals of that round (one barrier per round), so every entry is
+//     classified and looked up once;
+//   !ONE_PASS (RSPT_SPARSE_LIST=0): warp w owns the entries [w * R, (w + 1) * R); pass A adds up the
+//     warp's bits, one block scan, pass B classifies every entry again and places it.
+template <bool ONE_PASS>
 __global__ void __launch_bounds__(kSpThreads, 6) k_hzr_encode_sparse(Shape s, const uint8_t* __restrict__ frame_nb,
                                                                      const BlkInfo* __restrict__ info,
                                                                      const uint32_t* __restrict__ codes,
@@ -57,7 +66,7 @@ __global__ void __launch_bounds__(kSpThreads, 6) k_hzr_encode_sparse(Shape s, co
 {
     extern __shared__ __align__(16) uint32_t s_dyn[];  // the list, then the payload staging
     __shared__ uint32_t s_codes[kSymStride];
-    __shared__ uint32_t s_wtot[kSpThreads / 32];
+    __shared__ uint32_t s_wtot[2][kSpThreads / 32];
     uint32_t f, k, b;
     const uint32_t blk = blockIdx.x;
     const uint32_t m = list_n[blk];
@@ -92,11 +101,13 @@ __global__ void __launch_bounds__(kSpThreads, 6) k_hzr_encode_sparse(Shape s, co
     asm volatile("cp.async.wait_group 0;" ::: "memory");
     __syncthreads();
 
-    // bit packing: warp w owns the entries [w * R, (w + 1) * R), one entry per lane and pass;
-    // pass A adds up the warp's bits, one block scan, pass B places every entry's <= 3 slots
-    // (run code, run extra bits, literal) with a warp scan of the entry bit lengths
+    // bit packing: every entry's <= 3 slots (run code, run extra bits, literal) are placed with a warp
+    // scan of the entry bit lengths
+    uint32_t base = bi.tree_nbits, e_lo = 0, e_hi = m + 1u;
+    if (!ONE_PASS) {
     const uint32_t R = ((m + 1u + blockDim.x - 1u) / blockDim.x) * 32u;
-    const uint32_t e_lo = min(m + 1u, wid * R), e_hi = min(m + 1u, e_lo + R);
+    e_lo = min(m + 1u, wid * R);
+    e_hi = min(m + 1u, e_lo + R);
     uint32_t wbits = 0;
     for (uint32_t i = e_lo + lane; i < e_hi; i += 32) {
         const uint32_t e = i < m ? list[i] : n;
@@ -114,12 +125,13 @@ __global__ void __launch_bounds__(kSpThreads, 6) k_hzr_encode_sparse(Shape s, co
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) wbits += __shfl_xor_sync(0xFFFFFFFFu, wbits, o);
-    if (lane == 0) s_wtot[wid] = wbits;
-    __syncthreads();  // also: staging initialised
-    uint32_t base = bi.tree_nbits;
-    for (uint32_t w = 0; w < wid; ++w) base += s_wtot[w];
-    for (uint32_t i0 = e_lo; i0 < e_hi; i0 += 32) {
-        const uint32_t i = i0 + lane;
+    if (lane == 0) s_wtot[0][wid] = wbits;
+    __syncthreads();
+    for (uint32_t w = 0; w < wid; ++w) base += s_wtot[0][w];
+    }
+    // ONE_PASS: the trip count depends on m alone, so every warp reaches the barrier of every round
+    for (uint32_t i0 = e_lo, r = 0; i0 < e_hi; i0 += ONE_PASS ? blockDim.x : 32u, r ^= 1u) {
+        const uint32_t i = i0 + (ONE_PASS ? tid : lane);
         const bool live = i < e_hi;
         uint32_t bits = 0, gap = 0, cur = 0, rs = 0, c_run = 0, c_ext = 0, c_lit = 0;
         if (live) {
@@ -145,8 +157,19 @@ __global__ void __launch_bounds__(kSpThreads, 6) k_hzr_encode_sparse(Shape s, co
             const uint32_t y = __shfl_up_sync(0xFFFFFFFFu, inc, o);
             if (lane >= (uint32_t)o) inc += y;
         }
-        const uint32_t o0 = base + inc - bits;
-        base += __shfl_sync(0xFFFFFFFFu, inc, 31);
+        uint32_t o0;
+        if (ONE_PASS) {
+            // warp totals of this round (double-buffered: a warp may start the next round before the
+            // others have read this one)
+            if (lane == 31) s_wtot[r][wid] = inc;
+            __syncthreads();
+            const uint32_t t = lane < (blockDim.x >> 5) ? s_wtot[r][lane] : 0u;
+            o0 = base + __reduce_add_sync(0xFFFFFFFFu, lane < wid ? t : 0u) + inc - bits;
+            base += __reduce_add_sync(0xFFFFFFFFu, t);
+        } else {
+            o0 = base + inc - bits;
+            base += __shfl_sync(0xFFFFFFFFu, inc, 31);
+        }
         if (live) {
             if (bits > 64u || gap > kRunCap) {
                 EmitSink es{s_codes, pay, 0ull, o0 & 31u, o0 >> 5, true};

@@ -84,6 +84,7 @@ struct rspt_gpu_packer {
     int front_grid;        // persistent CTAs of k_front (SMs x resident CTAs)
     size_t front_smem;
     uint32_t sp_stage;     // payload limit of k_hzr_encode_sparse (kSpStageBytes; lower only under RSPT_SPARSE_STAGE_BYTES)
+    bool sparse_list;      // sparse class: k_hzr_hist<3> + one-pass k_hzr_encode_sparse; false (RSPT_SPARSE_LIST=0) = the earlier kernels
     // transform constants (dct twiddles)
     double2* d_twiddle;
     double2* d_post;

@@ -432,6 +432,7 @@ extern "C" int rspt_gpu_create(int kind, size_t bps, size_t ch, size_t ns, size_
     if (e == cudaSuccess) e = allow_smem(k_hzr_encode<2>, kEncodeSmem);
     if (e == cudaSuccess) e = allow_smem(k_hzr_encode<3>, kEncodeSmem);
     if (e == cudaSuccess) e = allow_smem(k_hzr_hist<1>, kHistSmem);
+    if (e == cudaSuccess) e = allow_smem(k_hzr_hist<3>, kHistSmemList);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&p->side, cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&p->place, cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p->ev_place, cudaEventDisableTiming);
@@ -441,13 +442,17 @@ extern "C" int rspt_gpu_create(int kind, size_t bps, size_t ch, size_t ns, size_
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p->ev_join, cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p->ev_fork2, cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p->ev_join2, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = allow_smem(k_hzr_encode_sparse, kSparseSmem);
+    if (e == cudaSuccess) e = allow_smem(k_hzr_encode_sparse<true>, kSparseSmem);
+    if (e == cudaSuccess) e = allow_smem(k_hzr_encode_sparse<false>, kSparseSmem);
     if (e == cudaSuccess) e = front_setup(p);
     {
         // test hook: a smaller staging limit sends listed blocks down the hand-over path to k_hzr_encode
         const char* ev = getenv("RSPT_SPARSE_STAGE_BYTES");
         const long v = ev ? atol(ev) : (long)kSpStageBytes;
         p->sp_stage = (uint32_t)(v < 1 ? 1 : (v > (long)kSpStageBytes ? (long)kSpStageBytes : v));
+        // A/B switch, per handle so that one process can alternate the two builds of the sparse class
+        const char* el = getenv("RSPT_SPARSE_LIST");
+        p->sparse_list = !(el && atoi(el) == 0);
     }
     if (e == cudaSuccess) e = allow_smem(k_hzr_decode, kDecodeSmem);
     if (e == cudaSuccess) e = allow_smem(k_hzr_verify, kDecodeSmem);
@@ -664,6 +669,16 @@ static int encode_ctas_per_sm(const Shape& s)
     return (s.kind == RSPT_XDELTA_HZR || s.kind == RSPT_HADAMARD) ? 3 : 2;
 }
 
+// histogram + list of the sparse-looking blocks: k_hzr_hist<3>, or the earlier list builder k_hzr_hist<1> under
+// RSPT_SPARSE_LIST=0 (same list and histogram)
+static void launch_sparse_hist(rspt_gpu_packer* p, const uint8_t* planes, const Shape& s, uint32_t nblocks, cudaStream_t st)
+{
+    if (p->sparse_list)
+        k_hzr_hist<3><<<nblocks, kHistThreads, kHistSmemList, st>>>(planes, s, p->d_frame_nb, p->d_hist, p->d_step_lz, p->d_lists, p->d_list_n, p->d_blk_class);
+    else
+        k_hzr_hist<1><<<nblocks, kHistThreads, kHistSmem, st>>>(planes, s, p->d_frame_nb, p->d_hist, p->d_step_lz, p->d_lists, p->d_list_n, p->d_blk_class);
+}
+
 // RSPT_TREE_LS=W (2..32): trees per CTA of the lock-step tree kernel; 0 = one warp per tree (k_hzr_tree)
 static uint32_t tree_lockstep_warps()
 {
@@ -739,7 +754,7 @@ extern "C" int rspt_gpu_compress_batch(rspt_gpu_packer* p, const uint8_t* d_src,
         // histogram, RSPT_STAGE_TREE everything from there to the join.
         RSPT_CUDA_CHECK(cudaEventRecord(p->ev_fork, p->stream));
         RSPT_CUDA_CHECK(cudaStreamWaitEvent(p->side, p->ev_fork, 0));
-        k_hzr_hist<1><<<nblocks, kHistThreads, kHistSmem, p->side>>>(p->d_planes, s, p->d_frame_nb, p->d_hist, p->d_step_lz, p->d_lists, p->d_list_n, p->d_blk_class);
+        launch_sparse_hist(p, p->d_planes, s, nblocks, p->side);
         if (const uint32_t W = tree_lockstep_warps())
             k_hzr_tree_ls<<<(nblocks + W - 1) / W, 32 * W, W * sizeof(TreeWarpSmem), p->side>>>(p->d_hist, s, p->d_frame_nb, p->d_blk_class, kClassSparse, nblocks, p->d_codes, p->d_tree, p->d_info, p->d_ctr);
         else
@@ -772,8 +787,12 @@ extern "C" int rspt_gpu_compress_batch(rspt_gpu_packer* p, const uint8_t* d_src,
         const SparseOut so{d_dst, d_offsets, p->d_blk_off, p->sp_stage, p->d_headers, sidecar};
         RSPT_CUDA_CHECK(cudaEventRecord(p->ev_fork2, p->stream));
         RSPT_CUDA_CHECK(cudaStreamWaitEvent(p->side, p->ev_fork2, 0));
-        k_hzr_encode_sparse<<<nblocks, kSpThreads, kSparseSmem, p->side>>>(s, p->d_frame_nb, p->d_info, p->d_codes, p->d_tree, p->d_lists,
-                                                                           p->d_list_n, p->d_crc, so);
+        if (p->sparse_list)
+            k_hzr_encode_sparse<true><<<nblocks, kSpThreads, kSparseSmem, p->side>>>(s, p->d_frame_nb, p->d_info, p->d_codes, p->d_tree, p->d_lists,
+                                                                                     p->d_list_n, p->d_crc, so);
+        else
+            k_hzr_encode_sparse<false><<<nblocks, kSpThreads, kSparseSmem, p->side>>>(s, p->d_frame_nb, p->d_info, p->d_codes, p->d_tree, p->d_lists,
+                                                                                      p->d_list_n, p->d_crc, so);
         RSPT_CUDA_CHECK(cudaEventRecord(p->ev_join2, p->side));
         if (encode_ctas_per_sm(s) == 3)
             k_hzr_encode<3><<<nblocks, kEncThreads, p->enc_smem, p->stream>>>(p->d_planes, s, p->d_frame_nb, p->d_info, p->d_blk_off,
@@ -1527,7 +1546,7 @@ extern "C" int rspt_gpu_debug_hzr_tables(rspt_gpu_packer* p, const uint8_t* d_bl
     DeviceGuard dg(p->device);
     Shape s = p->s;
     s.N = (uint32_t)n; s.nblk = 1; s.nb_alloc = 1; s.plane_stride = (uint32_t)((n + 15) & ~(size_t)15);
-    k_hzr_hist<1><<<1, kHistThreads, kHistSmem, p->stream>>>(d_block, s, p->d_frame_nb, p->d_hist, p->d_step_lz, p->d_lists, p->d_list_n, p->d_blk_class);
+    launch_sparse_hist(p, d_block, s, 1, p->stream);
     k_hzr_hist<2><<<1, kHistThreads, 0, p->stream>>>(d_block, s, p->d_frame_nb, p->d_hist, p->d_step_lz, p->d_lists, p->d_list_n, p->d_blk_class);
     k_hzr_tree<<<1, 32 * kTreeWarps, 0, p->stream>>>(p->d_hist, s, p->d_frame_nb, p->d_blk_class, kClassSparse, 1, p->d_codes, p->d_tree, p->d_info, p->d_ctr);
     k_hzr_tree<<<1, 32 * kTreeWarps, 0, p->stream>>>(p->d_hist, s, p->d_frame_nb, p->d_blk_class, kClassDense, 1, p->d_codes, p->d_tree, p->d_info, p->d_ctr);
