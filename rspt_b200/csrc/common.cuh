@@ -122,6 +122,14 @@ __device__ __forceinline__ uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel)
 }
 __device__ __forceinline__ void reds_or(uint32_t a, uint32_t v) { asm volatile("red.shared.or.b32 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
 
+// double -> int32 as the reference's x86-64 build does it (cvttsd2si): toward zero, and the
+// "integer indefinite" 0x80000000 for NaN and for values outside the int32 range (CUDA's own
+// conversion would saturate instead).
+__device__ __forceinline__ int32_t to_i32_x86(double v)
+{
+    return (v >= 2147483648.0 || v <= -2147483649.0 || v != v) ? (int32_t)0x80000000 : (int32_t)v;
+}
+
 // Extra bits carried by the zero-run symbols 256..260 (hzr_internal.h:117-121).
 __device__ __forceinline__ uint32_t sym_extra_bits(uint32_t sym)
 {

@@ -20,14 +20,6 @@
 
 namespace rspt {
 
-// double -> int32 as the reference's x86-64 build does it (cvttsd2si): toward zero, and the
-// "integer indefinite" 0x80000000 for NaN and for values outside the int32 range (CUDA's own
-// conversion would saturate instead).
-__device__ __forceinline__ int32_t to_i32_x86(double v)
-{
-    return (v >= 2147483648.0 || v <= -2147483649.0 || v != v) ? (int32_t)0x80000000 : (int32_t)v;
-}
-
 struct IirCoef {
     double n[5], d[5];
     int nc;          // 2..5 coefficients

@@ -650,8 +650,8 @@ __global__ void __launch_bounds__(256, 4) k_dct_inv_half(int32_t* __restrict__ w
     const double scale = sqrt(2.0 / (double)(int)n) * 128.0;  // dct.cpp:97
     for (uint32_t p = threadIdx.x; p < M; p += blockDim.x) {
         const double2 z = xs[fpad(p)];
-        w[makhoul_src(2u * p, n)] = (int32_t)((uint32_t)(int32_t)(z.x * scale) + (uint32_t)mean);
-        w[makhoul_src(2u * p + 1u, n)] = (int32_t)((uint32_t)(int32_t)(z.y * scale) + (uint32_t)mean);
+        w[makhoul_src(2u * p, n)] = (int32_t)((uint32_t)to_i32_x86(z.x * scale) + (uint32_t)mean);
+        w[makhoul_src(2u * p + 1u, n)] = (int32_t)((uint32_t)to_i32_x86(z.y * scale) + (uint32_t)mean);
     }
 }
 
@@ -704,7 +704,7 @@ __global__ void __launch_bounds__(256) k_dct_inv_fast(int32_t* __restrict__ word
     for (uint32_t m = threadIdx.x; m < n; m += blockDim.x) {
         const uint32_t j = m < (n >> 1) ? 2 * m : 2 * (n - 1 - m) + 1;
         const double sum = xs[m].x * scale;
-        w[j] = (int32_t)((uint32_t)(int32_t)sum + (uint32_t)mean);
+        w[j] = (int32_t)((uint32_t)to_i32_x86(sum) + (uint32_t)mean);
     }
 }
 
@@ -726,7 +726,7 @@ __global__ void __launch_bounds__(256) k_dct_inv_direct(int32_t* __restrict__ wo
         const float* rowp = cosT + (size_t)i * n;
         for (uint32_t x = 0; x < n; ++x) sum += (double)__fmul_rn(tf[x], __ldg(rowp + x));
         sum *= scale;
-        w[i] = (int32_t)((uint32_t)(int32_t)sum + (uint32_t)mean);
+        w[i] = (int32_t)((uint32_t)to_i32_x86(sum) + (uint32_t)mean);  // out of int32 range: 0x80000000 + mean
     }
 }
 
@@ -1050,9 +1050,11 @@ inline int launch_inverse_transform(rspt_gpu_packer* p, uint8_t* d_dst, size_t F
             }
             p->launches += 1;
         } else {
-            // coefficient words (BPS unused for word output)
-            const size_t smw = (size_t)2 * ((uint32_t)s.ns / kInvPiece) * s.ch * 4;
-            if ((s.ns % (int)kInvPiece) == 0 && smw <= 200 * 1024) {
+            // coefficient words (BPS unused for word output); the fast kernel walks a frame's 128-element
+            // pieces four at a time, so their number must be a multiple of 4
+            const uint32_t npf = ((uint32_t)s.ns / kInvPiece) * (uint32_t)s.ch;
+            const size_t smw = (size_t)2 * npf * 4;
+            if ((s.ns % (int)kInvPiece) == 0 && (npf & 3u) == 0 && smw <= 200 * 1024) {
                 RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_planes_to_samples_fast<4, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smw));
                 k_planes_to_samples_fast<4, true, true><<<gf, inverse_threads(), smw, p->stream>>>(p->d_planes, s, p->d_dec_nb, 1, nullptr,
                                                                                              inverse_seg_xor(p), p->segs_per_plane, p->d_words);

@@ -627,24 +627,36 @@ def test_dct_fast_path_tolerance(R, oracle, bps, ch, ns, nfr):
     assert n_bad <= max(1, int(n_all * (1.0 - DCT_EQUAL_FRACTION))), (n_bad, n_all)
 
 
+DCT_DIRECT_CASES = [(4, 3, 512), (3, 2, 300), (4, 2, 4096), (1, 3, 2), (1, 2, 3), (1, 4, 5), (1, 3, 77), (3, 2, 77),
+                    (1, 2, 1000), (4, 3, 1000), (1, 2, 4095), (3, 2, 4095), (1, 1, 8192), (4, 12, 4096)]
+
+
 def test_dct_direct_path_bit_exact(R, oracle):
-    """dct, O(n^2) path with the reference's float-product / double-accumulate arithmetic."""
-    os.environ["RSPT_DCT_DIRECT"] = "1"
-    try:
-        for bps, ch, ns in ((4, 3, 512), (3, 2, 300), (4, 2, 4096)):
-            raws = oracle.synth_ecg(1, 2, bps, ch, ns)
-            p = R.SignalPacker.new_dct(bps, ch, ns, max_batch_frames=2)
-            batch = p.compress_batch(to_dev(raws))
-            dec = p.decompress_batch(batch).cpu().numpy().reshape(2, -1)
-            offs = batch.offsets.cpu().numpy()
-            stream = batch.stream.cpu().numpy()
-            o = oracle.OraclePacker("dct", bps, ch, ns)
-            for i in range(2):
-                want = o.compress(raws[i])
-                assert stream[offs[i]:offs[i + 1]].tobytes() == want, (bps, ch, ns, i)
-                assert dec[i].tobytes() == o.decompress(want)[0]
-    finally:
-        os.environ.pop("RSPT_DCT_DIRECT", None)
+    """dct, O(n^2) path with the reference's float-product / double-accumulate arithmetic: two synthetic ECG
+    and two full-range noise frames per shape, lengths 2 to 8192 (powers of two through set_dct_exact).
+    Full-range 3- and 4-byte noise decodes to inverse sums outside int32, which the reference converts to
+    0x80000000."""
+    for bps, ch, ns in DCT_DIRECT_CASES:
+        lo, hi = -(1 << (8 * bps - 1)), 1 << (8 * bps - 1)
+        noise = [np.random.default_rng(seed).integers(lo, hi, (ns, ch)).astype("<i4").view(np.uint8).reshape(ns, ch, 4)[:, :, :bps]
+                 for seed in (1, 2)]
+        raws = np.concatenate([oracle.synth_ecg(1, 2, bps, ch, ns, amplitude=100 if bps == 1 else 20000),
+                               np.stack([x.reshape(-1) for x in noise])])
+        nfr = len(raws)
+        p = R.SignalPacker.new_dct(bps, ch, ns, max_batch_frames=nfr)
+        p.set_dct_exact(True)
+        batch = p.compress_batch(to_dev(raws))
+        dec = p.decompress_batch(batch).cpu().numpy().reshape(nfr, -1)
+        offs = batch.offsets.cpu().numpy()
+        stream = batch.stream.cpu().numpy()
+        p.close()
+        o = oracle.OraclePacker("dct", bps, ch, ns)
+        for i in range(nfr):
+            want = o.compress(raws[i])
+            assert stream[offs[i]:offs[i + 1]].tobytes() == want, (bps, ch, ns, i)
+            wd = np.frombuffer(o.decompress(want)[0], np.uint8)
+            n_diff = int((dec[i] != wd).reshape(-1, bps).any(axis=1).sum())
+            assert n_diff == 0, (bps, ch, ns, i, f"{n_diff} decoded samples differ")
 
 
 def test_prdn_kernel(R, oracle):
