@@ -285,38 +285,6 @@ __device__ __forceinline__ void chain_long_codes(const uint32_t* cw_tab, T* lut,
     }
 }
 
-// xor of the bytes of every 128-byte segment of a block this CTA has just written (the lines are still in L2):
-// a segment per thread-pass, read past L1 since other threads wrote them
-constexpr uint32_t kXorSeg = 128;
-__device__ __forceinline__ void block_segment_xor(const uint8_t* out, uint32_t n, uint8_t* seg)
-{
-    // eight lanes per segment, one 16-byte chunk each (consecutive lanes read consecutive chunks), folded with
-    // three shuffles; the loop bound is warp-uniform so that the shuffles see the whole warp
-    const uint32_t nchunk = (n + 15u) >> 4;
-    const uint4* p4 = reinterpret_cast<const uint4*>(out);
-    for (uint32_t c0 = (threadIdx.x & ~31u); c0 < nchunk; c0 += blockDim.x) {
-        const uint32_t c = c0 + (threadIdx.x & 31u);
-        uint32_t x = 0;
-        if (c < nchunk) {
-            uint4 v = __ldcg(p4 + c);
-            const uint32_t left = n - 16u * c;   // bytes of the block in this chunk (>= 1)
-            if (left < 16u) {
-                if (left <= 12u) v.w = 0; else v.w &= (1u << (8u * (left - 12u))) - 1u;
-                if (left <= 8u) v.z = 0; else if (left < 12u) v.z &= (1u << (8u * (left - 8u))) - 1u;
-                if (left <= 4u) v.y = 0; else if (left < 8u) v.y &= (1u << (8u * (left - 4u))) - 1u;
-                if (left < 4u) v.x &= (1u << (8u * left)) - 1u;
-            }
-            x = v.x ^ v.y ^ v.z ^ v.w;
-        }
-        x ^= __shfl_xor_sync(0xFFFFFFFFu, x, 4);
-        x ^= __shfl_xor_sync(0xFFFFFFFFu, x, 2);
-        x ^= __shfl_xor_sync(0xFFFFFFFFu, x, 1);
-        x ^= x >> 16;
-        x ^= x >> 8;
-        if ((threadIdx.x & 7u) == 0u && c < nchunk) seg[c >> 3] = (uint8_t)x;
-    }
-}
-
 // One CTA per hzr block.  The payload is staged in shared memory with ONE bulk asynchronous copy (the
 // 16-byte chunks of the stream that hold it, unshifted; the bit reader starts 8 * (address mod 16) bits
 // later) that lands while the tables are built; the code table comes from k_hzr_recover_codes; a 12-bit
@@ -329,8 +297,7 @@ __global__ void __launch_bounds__(kDecodeThreads, 3) k_hzr_decode(const uint8_t*
                                                                    const uint32_t* __restrict__ sidecar,
                                                                    const uint32_t* __restrict__ codes,
                                                                    uint8_t* __restrict__ planes, int32_t* __restrict__ status,
-                                                                   uint32_t pair_max_bits, uint32_t small_class,
-                                                                   uint8_t* __restrict__ seg_xor, uint32_t segs_per_plane, uint32_t blk0)
+                                                                   uint32_t pair_max_bits, uint32_t small_class)
 {
     extern __shared__ __align__(16) uint32_t payw[];  // payload words (+ zero slack)
     // 8 KB of look-up table in one of two shapes, chosen per block:
@@ -358,17 +325,10 @@ __global__ void __launch_bounds__(kDecodeThreads, 3) k_hzr_decode(const uint8_t*
     uint4* out4 = reinterpret_cast<uint4*>(out);
     const uint32_t n = d.out_n, nq = (n + 15u) >> 4;
     const uint8_t* pay = src + d.payload_off;
-    // xor of the bytes of every 128-byte output segment, for the inverse transform's first scan
-    // (k_planes_to_samples_fast: a segment is one of its pieces), so that it need not read the planes for it
-    uint8_t* my_xor = seg_xor ? seg_xor + ((size_t)f * s.nb_alloc + k) * segs_per_plane + (size_t)b * (kBlock / kXorSeg) : nullptr;
-    const uint32_t nseg_all = (n + kXorSeg - 1) / kXorSeg;
 
     if (d.mode == MODE_FILL || d.mode == kModeZero) {
         const uint32_t v = d.mode == MODE_FILL ? pay[0] * 0x01010101u : 0u;  // memset (dec:362-370)
         for (uint32_t i = tid; i < nq; i += blockDim.x) out4[i] = make_uint4(v, v, v, v);
-        if (my_xor)
-            for (uint32_t i = tid; i < nseg_all; i += blockDim.x)
-                my_xor[i] = (uint8_t)((min((uint32_t)kXorSeg, n - i * kXorSeg) & 1u) ? (v & 0xFFu) : 0u);
         return;
     }
     const uintptr_t pa = (uintptr_t)pay;
@@ -376,8 +336,6 @@ __global__ void __launch_bounds__(kDecodeThreads, 3) k_hzr_decode(const uint8_t*
         if (d.payload_len != n) {  // "Encoded / decoded size mismatch (COPY)" dec:351-355
             if (tid == 0) status[f] = -4;
             for (uint32_t i = tid; i < nq; i += blockDim.x) out4[i] = make_uint4(0, 0, 0, 0);
-            if (my_xor)
-                for (uint32_t i = tid; i < nseg_all; i += blockDim.x) my_xor[i] = 0;
             return;
         }
         const uint32_t* aw = reinterpret_cast<const uint32_t*>(pa & ~(uintptr_t)3);
@@ -387,10 +345,6 @@ __global__ void __launch_bounds__(kDecodeThreads, 3) k_hzr_decode(const uint8_t*
         for (uint32_t i = tid; i < nw; i += blockDim.x) {
             const uint32_t lo = __ldg(aw + i), hi = (i + 1 < naw) ? __ldg(aw + i + 1) : 0u;
             out32[i] = __funnelshift_r(lo, hi, sh);
-        }
-        if (my_xor) {
-            __syncthreads();
-            block_segment_xor(out, n, my_xor);
         }
         return;
     }
@@ -455,7 +409,7 @@ __global__ void __launch_bounds__(kDecodeThreads, 3) k_hzr_decode(const uint8_t*
 
     const IdxGeom ig = idx_geom(plen);
     const uint32_t limit = plen * 8u, nint = ig.n;
-    const uint32_t* my_idx = sidecar + idx_slot_base(d.payload_off - offsets[0], blk0 + blk);   // blk0: a launch over part of a batch
+    const uint32_t* my_idx = sidecar + idx_slot_base(d.payload_off - offsets[0], blk);
     uint32_t my_err = 0;
     if (tid < nint) {
         const uint32_t e0 = my_idx[tid];
@@ -594,10 +548,6 @@ __global__ void __launch_bounds__(kDecodeThreads, 3) k_hzr_decode(const uint8_t*
         }
     }
     if (my_err) status[f] = -4;
-    if (my_xor) {
-        __syncthreads();   // the block is complete (this CTA wrote all of it)
-        block_segment_xor(out, n, my_xor);
-    }
 }
 
 // ------------------------------------------------------------------------------------------

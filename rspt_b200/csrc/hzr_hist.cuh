@@ -1,5 +1,5 @@
 // hzr token histogram for sm_100a: one CTA per hzr block, 16 bytes per lane, 512 bytes per
-// warp-step.  Replaces Histogram (lib_hzr/hzr_encode.c:133-173).  Two launches (k_hzr_hist<3> or <1>,
+// warp-step.  Replaces Histogram (lib_hzr/hzr_encode.c:133-173).  Two launches (k_hzr_hist<3>,
 // k_hzr_hist<2>) split the blocks by a density probe: sparse-looking blocks are tokenised from a
 // sorted list of their non-zero bytes (described at the kernel), dense-looking ones by the scan
 // described here.
@@ -87,70 +87,37 @@ __device__ __forceinline__ void hist_run(uint32_t z, uint32_t* run)
     atomicAdd(&run[idx], 1u);
 }
 
-// Append the non-zero bytes of every lane's chunk to the list, lane by lane in position order
-// (`at` = list index of the lane's first entry).  Non-zero bytes come in bursts, so instead of
-// every lane looping over its own bytes, the chunks that have any are served two at a time by
-// half a warp each: lane p of the half writes byte p.
-__device__ __forceinline__ void scatter_chunks(const Chunk& c, uint32_t off, uint32_t at, uint32_t* list)
-{
-    uint32_t todo = __ballot_sync(0xFFFFFFFFu, c.nz != 0u);
-    const uint32_t lane = lane_id(), p = lane & 15u;
-    while (todo) {
-        const uint32_t la = __ffs(todo) - 1u;
-        todo &= todo - 1u;
-        uint32_t lb = la;  // odd count: the upper half repeats the same chunk, harmlessly
-        if (todo) {
-            lb = __ffs(todo) - 1u;
-            todo &= todo - 1u;
-        }
-        const uint32_t sl = lane < 16 ? la : lb;
-        const uint32_t nz = __shfl_sync(0xFFFFFFFFu, c.nz, sl), a0 = __shfl_sync(0xFFFFFFFFu, at, sl);
-        const uint32_t o0 = __shfl_sync(0xFFFFFFFFu, off, sl);
-        const uint32_t x0 = __shfl_sync(0xFFFFFFFFu, c.v.x, sl), x1 = __shfl_sync(0xFFFFFFFFu, c.v.y, sl);
-        const uint32_t x2 = __shfl_sync(0xFFFFFFFFu, c.v.z, sl), x3 = __shfl_sync(0xFFFFFFFFu, c.v.w, sl);
-        const uint32_t x = p < 8 ? (p < 4 ? x0 : x1) : (p < 12 ? x2 : x3);
-        if ((nz >> p) & 1u) list[a0 + __popc(nz & ((1u << p) - 1u))] = (o0 + p) | (((x >> (8u * (p & 3u))) & 0xFFu) << 16);
-    }
-}
-
 // ---- sparse blocks ---------------------------------------------------------------------------
 // A block with few non-zero bytes (<= kListCap, i.e. mostly long zero runs: the upper byte planes
-// of a delta-coded signal) is tokenised from a sorted list of its non-zero bytes (PART 1; PART 3
-// below does steps 1-2 with fewer instructions):
-//   1. every warp scans a contiguous range of <= 16 steps, keeping per step and lane the 16-bit
-//      non-zero mask and the exclusive count of non-zero bytes before the chunk (no barrier; the
-//      loads of a batch of steps are in flight together);
-//   2. one block scan of the warp totals, then the non-zero bytes are scattered into the list
-//      (position | value << 16) in shared memory;
+// of a delta-coded signal) is tokenised from a sorted list of its non-zero bytes.  Those bytes are
+// clustered (~80 % of the steps hold some, ~4 of 32 chunks each), so the list is built in two light phases:
+//   1. every warp only COUNTS the non-zero bytes of its contiguous range of <= 16 steps and notes, per
+//      lane, which of its steps have a non-zero chunk (one bit each); one reduction per warp gives the
+//      warp total;
+//   2. after the block scan of the totals, the warp walks its steps that have a non-zero chunk: those
+//      lanes reload their chunk into a 512-byte per-warp slot of shared memory, and the chunks are
+//      served two at a time by half a warp each (lane p of the half reads byte p); a ballot of the
+//      kept bytes gives their order, and a warp-uniform running count gives their list index
+//      (position | value << 16, in shared memory);
 //   3. token histogram from the list: a literal per entry, a zero run per gap.
+// No per-step prefix scan and no per-step registers are needed, so the kernel fits 32 registers.
 // The list goes to global memory for k_hzr_encode_sparse, which packs the block's payload without
 // reading the plane again.  Blocks that are too dense for the list take the dense scan below.
 constexpr uint32_t kListCap = 5120;                 // entries of a block's sparse list
 constexpr uint8_t kClassSparse = 0, kClassDense = 1;  // blk_class: which histogram launch (and tree launch) owns the block
 constexpr size_t kHistSmem = (size_t)kListCap * 4;
 constexpr int kHistSteps = kMaxSteps / (kHistThreads / 32);      // steps per warp: 16
-// PART 3 builds the same list in two lighter phases (the sparse planes' non-zero bytes are clustered:
-// ~80 % of the steps hold some, ~4 of 32 chunks each):
-//   1. every warp only COUNTS the non-zero bytes of its range and notes, per lane, which of its <= 16
-//      steps have a non-zero chunk (one bit each); one reduction per warp gives the warp total;
-//   2. after the block scan of the totals, the warp walks its steps that have a non-zero chunk: those
-//      lanes reload their chunk into a 512-byte per-warp slot of shared memory, and the chunks are
-//      served two at a time by half a warp each (lane p of the half reads byte p); a ballot of the
-//      kept bytes gives their order, and a warp-uniform running count gives their list index.
-// No per-step prefix scan and no per-step registers remain, so the kernel fits 32 registers.
 constexpr size_t kHistSmemList = kHistSmem + (size_t)(kHistThreads / 32) * kStepBytes;
 
 // Two independent launches per batch, each over all blocks; the density probe (deterministic, the
 // same in both) assigns every block to exactly one of them and is recorded in blk_class:
-//   PART 1 or 3 takes the sparse-looking blocks (list + histogram; if the list overflows after all,
-//          the dense scan runs here too -- rare); 3 is the default, 1 the earlier list builder
-//          (RSPT_SPARSE_LIST=0), same list and histogram;
+//   PART 3 takes the sparse-looking blocks (list + histogram; if the list overflows after all, the
+//          dense scan runs here too -- rare);
 //   PART 2 takes the dense-looking blocks (dense scan).
 // They run on two streams: the tree build of the dense class (long, latency-bound) then overlaps
-// with the sparse part.  The split also lets the dense scan run at 8 CTAs per SM (30 registers) while
-// PART 1 keeps 16 mask/prefix registers per lane.
+// with the sparse part.
 template <int PART>
-__global__ void __launch_bounds__(kHistThreads, PART == 1 ? 5 : 8) k_hzr_hist(const uint8_t* __restrict__ planes, Shape s,
+__global__ void __launch_bounds__(kHistThreads, 8) k_hzr_hist(const uint8_t* __restrict__ planes, Shape s,
                                                                const uint8_t* __restrict__ frame_nb,
                                                                uint32_t* __restrict__ hist,
                                                                uint16_t* __restrict__ step_lz,
@@ -190,68 +157,6 @@ __global__ void __launch_bounds__(kHistThreads, PART == 1 ? 5 : 8) k_hzr_hist(co
     do {
         uint32_t* list = s_list;
         uint32_t m = 0;
-        if (PART == 1) {
-        // 1. masks and in-warp prefix counts of every step of my warp's range
-        uint32_t pk[kHistSteps];  // nz mask | entries of my warp before this chunk << 16
-        uint32_t wrun = 0;
-#pragma unroll
-        for (int j0 = 0; j0 < kHistSteps; j0 += 4) {
-            uint4 v[4];
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                const uint32_t st = s_lo + j0 + j, off = st * kStepBytes + lane * 16u;
-                v[j] = make_uint4(0, 0, 0, 0);
-                if (st < s_hi && off < n) v[j] = __ldg(reinterpret_cast<const uint4*>(src + off));
-            }
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                const uint32_t st = s_lo + j0 + j, off = st * kStepBytes + lane * 16u;
-                uint32_t nz = 0;
-                if ((v[j].x | v[j].y | v[j].z | v[j].w) != 0u) {
-                    const int valid = (int)n - (int)off;  // > 0 here; rows are zero-padded only up to 16
-                    nz = nz_mask16(v[j]) & (valid >= 16 ? 0xFFFFu : (1u << valid) - 1u);
-                }
-                uint32_t inc = 0;
-                if (__any_sync(0xFFFFFFFFu, nz != 0u)) {
-                    const uint32_t cnt = __popc(nz);
-                    inc = cnt;
-#pragma unroll
-                    for (int o = 1; o < 32; o <<= 1) {
-                        const uint32_t y = __shfl_up_sync(0xFFFFFFFFu, inc, o);
-                        if (lane >= (uint32_t)o) inc += y;
-                    }
-                    const uint32_t tot = __shfl_sync(0xFFFFFFFFu, inc, 31);
-                    inc = wrun + inc - cnt;
-                    wrun += tot;
-                }
-                pk[j0 + j] = nz | (inc << 16);
-                (void)st;
-            }
-        }
-        if (lane == 0) s_wtot[wid] = wrun;
-        __syncthreads();
-        uint32_t wbase = 0;
-        for (uint32_t w = 0; w < nwarps; ++w) {
-            const uint32_t t = s_wtot[w];
-            if (w < wid) wbase += t;
-            m += t;
-        }
-        if (m > kListCap || m > n / 4u) break;
-
-        // 2. scatter the non-zero bytes into the list
-#pragma unroll
-        for (int j = 0; j < kHistSteps; ++j) {
-            const uint32_t nz = pk[j] & 0xFFFFu;
-            if (__any_sync(0xFFFFFFFFu, nz != 0u)) {
-                const uint32_t off = (s_lo + j) * kStepBytes + lane * 16u;
-                Chunk c;
-                c.nz = nz;
-                c.v = make_uint4(0, 0, 0, 0);
-                if (nz) c.v = __ldg(reinterpret_cast<const uint4*>(src + off));
-                scatter_chunks(c, off, wbase + (pk[j] >> 16), list);
-            }
-        }
-        } else {
         // 1. count the non-zero bytes of my warp's range; bit j of smask: my chunk of step s_lo + j has some
         uint32_t cnt = 0, smask = 0;
 #pragma unroll
@@ -310,7 +215,6 @@ __global__ void __launch_bounds__(kHistThreads, PART == 1 ? 5 : 8) k_hzr_hist(co
                 at += __popc(kept);
             }
             __syncwarp();  // the slot is read before the next step overwrites it
-        }
         }
         __syncthreads();
 

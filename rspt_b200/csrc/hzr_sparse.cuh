@@ -49,13 +49,9 @@ struct SparseOut {
 
 // Every entry i <= m of the list stands for the tokens between the previous non-zero byte and this
 // one: the zero run (if any), its extra bits, then the literal (entry m: the run up to the block end).
-// The entries' bit offsets are a prefix sum of their bit lengths.
-//   ONE_PASS (default): the CTA takes the entries 256 at a time, one per thread, and places each with a
-//     warp scan plus the warp totals of that round (one barrier per round), so every entry is
-//     classified and looked up once;
-//   !ONE_PASS (RSPT_SPARSE_LIST=0): warp w owns the entries [w * R, (w + 1) * R); pass A adds up the
-//     warp's bits, one block scan, pass B classifies every entry again and places it.
-template <bool ONE_PASS>
+// The entries' bit offsets are a prefix sum of their bit lengths: the CTA takes the entries 256 at a
+// time, one per thread, and places each with a warp scan plus the warp totals of that round (one
+// barrier per round), so every entry is classified and looked up once.
 __global__ void __launch_bounds__(kSpThreads, 6) k_hzr_encode_sparse(Shape s, const uint8_t* __restrict__ frame_nb,
                                                                      const BlkInfo* __restrict__ info,
                                                                      const uint32_t* __restrict__ codes,
@@ -103,36 +99,12 @@ __global__ void __launch_bounds__(kSpThreads, 6) k_hzr_encode_sparse(Shape s, co
 
     // bit packing: every entry's <= 3 slots (run code, run extra bits, literal) are placed with a warp
     // scan of the entry bit lengths
-    uint32_t base = bi.tree_nbits, e_lo = 0, e_hi = m + 1u;
-    if (!ONE_PASS) {
-    const uint32_t R = ((m + 1u + blockDim.x - 1u) / blockDim.x) * 32u;
-    e_lo = min(m + 1u, wid * R);
-    e_hi = min(m + 1u, e_lo + R);
-    uint32_t wbits = 0;
-    for (uint32_t i = e_lo + lane; i < e_hi; i += 32) {
-        const uint32_t e = i < m ? list[i] : n;
-        const uint32_t cur = i < m ? e & 0xFFFFu : n;
-        const uint32_t rs = i ? (list[i - 1] & 0xFFFFu) + 1u : 0u;
-        const uint32_t gap = cur - rs;
-        if (gap > kRunCap) {
-            wbits += run_bits(gap, s_codes);
-        } else {
-            uint32_t sym, ev, eb;
-            run_token(gap, sym, ev, eb);  // gap 0 classifies as a run of 1; masked out below
-            wbits += gap ? (s_codes[sym] >> 27) + eb : 0u;
-        }
-        if (i < m) wbits += s_codes[e >> 16] >> 27;
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) wbits += __shfl_xor_sync(0xFFFFFFFFu, wbits, o);
-    if (lane == 0) s_wtot[0][wid] = wbits;
-    __syncthreads();
-    for (uint32_t w = 0; w < wid; ++w) base += s_wtot[0][w];
-    }
-    // ONE_PASS: the trip count depends on m alone, so every warp reaches the barrier of every round
-    for (uint32_t i0 = e_lo, r = 0; i0 < e_hi; i0 += ONE_PASS ? blockDim.x : 32u, r ^= 1u) {
-        const uint32_t i = i0 + (ONE_PASS ? tid : lane);
-        const bool live = i < e_hi;
+    uint32_t base = bi.tree_nbits;
+    const uint32_t ne = m + 1u;  // entries, the run up to the block end included
+    // the trip count depends on m alone, so every warp reaches the barrier of every round
+    for (uint32_t i0 = 0, r = 0; i0 < ne; i0 += blockDim.x, r ^= 1u) {
+        const uint32_t i = i0 + tid;
+        const bool live = i < ne;
         uint32_t bits = 0, gap = 0, cur = 0, rs = 0, c_run = 0, c_ext = 0, c_lit = 0;
         if (live) {
             const uint32_t e = i < m ? list[i] : n;
@@ -157,19 +129,13 @@ __global__ void __launch_bounds__(kSpThreads, 6) k_hzr_encode_sparse(Shape s, co
             const uint32_t y = __shfl_up_sync(0xFFFFFFFFu, inc, o);
             if (lane >= (uint32_t)o) inc += y;
         }
-        uint32_t o0;
-        if (ONE_PASS) {
-            // warp totals of this round (double-buffered: a warp may start the next round before the
-            // others have read this one)
-            if (lane == 31) s_wtot[r][wid] = inc;
-            __syncthreads();
-            const uint32_t t = lane < (blockDim.x >> 5) ? s_wtot[r][lane] : 0u;
-            o0 = base + __reduce_add_sync(0xFFFFFFFFu, lane < wid ? t : 0u) + inc - bits;
-            base += __reduce_add_sync(0xFFFFFFFFu, t);
-        } else {
-            o0 = base + inc - bits;
-            base += __shfl_sync(0xFFFFFFFFu, inc, 31);
-        }
+        // warp totals of this round (double-buffered: a warp may start the next round before the
+        // others have read this one)
+        if (lane == 31) s_wtot[r][wid] = inc;
+        __syncthreads();
+        const uint32_t t = lane < (blockDim.x >> 5) ? s_wtot[r][lane] : 0u;
+        const uint32_t o0 = base + __reduce_add_sync(0xFFFFFFFFu, lane < wid ? t : 0u) + inc - bits;
+        base += __reduce_add_sync(0xFFFFFFFFu, t);
         if (live) {
             if (bits > 64u || gap > kRunCap) {
                 EmitSink es{s_codes, pay, 0ull, o0 & 31u, o0 >> 5, true};

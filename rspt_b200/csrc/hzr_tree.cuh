@@ -33,10 +33,10 @@ struct TreeWarpSmem {
     uint32_t key[264];         // sorted leaf keys
     uint32_t icnt[260];        // B: internal node weight (| bit 31: next node has equal weight); C: node code
     uint32_t child[260];       // child_a | child_b << 10 | leaves below << 20; ids < 512 are leaf ranks, 512 + j internal node j
-    uint32_t ninfo[260];       // C: depth | pre-order bit offset << 8.  Before the build, ninfo and the first words of
-    uint32_t tree[kTreeWords]; //    tree hold the 264-word token histogram of a listed block that comes from k_front (list_hist)
+    uint32_t ninfo[260];       // C: depth | pre-order bit offset << 8
+    uint32_t tree[kTreeWords];
     uint16_t front[2][264];    // C: breadth-first frontiers (internal node indices)
-    uint32_t pad;              // odd word stride: the lanes of a lock-step merge (k_hzr_tree_ls) start in different banks
+    uint32_t pad;              // odd word stride between the warps' trees; part of the measured shared-memory footprint
 };
 
 struct Counters {
@@ -332,34 +332,7 @@ __device__ __forceinline__ void count_block_mode(Counters* ctr, uint32_t mode)
     atomicAdd(mode == MODE_FILL ? &ctr->blocks_fill : (mode == MODE_COPY ? &ctr->blocks_copy : &ctr->blocks_huff), 1ull);
 }
 
-// Token histogram of a block from the sorted list of its non-zero bytes (position | value << 16): one
-// literal per entry, one zero run per gap (hzr_encode.c:140-170).  h[0] = runs of one, h[1..255] literals,
-// h[256..260] the longer run classes.  One warp; h must be zeroed.
-__device__ __forceinline__ void warp_hist_from_list(const uint32_t* __restrict__ list, uint32_t m, uint32_t n, uint32_t* h)
-{
-    for (uint32_t i = lane_id(); i <= m; i += 32) {
-        const uint32_t rs = i ? (list[i - 1] & 0xFFFFu) + 1u : 0u;
-        uint32_t cur = n;
-        if (i < m) {
-            const uint32_t e = list[i];
-            cur = e & 0xFFFFu;
-            atomicAdd(&h[e >> 16], 1u);
-        }
-        uint32_t z = cur > rs ? cur - rs : 0u;
-        while (z > kRunCap) {
-            atomicAdd(&h[260], 1u);
-            z -= kRunCap;
-        }
-        if (z) {
-            const uint32_t idx = (z >= 2u) + (z >= 3u) + (z >= 7u) + (z >= 23u) + (z >= 279u);
-            atomicAdd(&h[idx ? 255u + idx : 0u], 1u);
-        }
-    }
-}
-
-// One warp per block of the class `cls` (blk_class is written by the histogram launches; null = every block).
-// Behind k_front (sub_n given) a listed block first gets its list: the sub-lists of the channel rows it spans,
-// concatenated (they are sorted and block-relative already), and its token histogram from that list.
+// One warp per block of the class `cls` (blk_class is written by the histogram launches).
 __global__ void __launch_bounds__(kTreeWarps * 32) k_hzr_tree(const uint32_t* __restrict__ hist, Shape s,
                                                                const uint8_t* __restrict__ frame_nb,
                                                                const uint8_t* __restrict__ blk_class, uint32_t cls,
@@ -367,12 +340,7 @@ __global__ void __launch_bounds__(kTreeWarps * 32) k_hzr_tree(const uint32_t* __
                                                                uint32_t* __restrict__ codes,
                                                                uint32_t* __restrict__ tree,
                                                                BlkInfo* __restrict__ info,
-                                                               Counters* __restrict__ ctr,
-                                                               const uint32_t* __restrict__ list_n = nullptr, uint32_t sparse_stage = 0,
-                                                               uint8_t* __restrict__ redo = nullptr,
-                                                               const uint32_t* __restrict__ sub_n = nullptr,
-                                                               const uint8_t* __restrict__ planes = nullptr,
-                                                               uint32_t* __restrict__ lists = nullptr, uint32_t list_cap = 0)
+                                                               Counters* __restrict__ ctr)
 {
     __shared__ TreeWarpSmem s_all[kTreeWarps];
     TreeWarpSmem& S = s_all[warp_id()];
@@ -380,75 +348,10 @@ __global__ void __launch_bounds__(kTreeWarps * 32) k_hzr_tree(const uint32_t* __
     if (blk >= total_blocks) return;
     uint32_t f, k, b;
     blk_decode(s, blk, f, k, b);
-    if (k >= frame_nb[f] || (blk_class && blk_class[blk] != cls)) return;
+    if (k >= frame_nb[f] || blk_class[blk] != cls) return;
     const uint32_t n = blk_len(s, b);
-    const uint32_t* h = hist + (size_t)blk * kSymStride;
-    if (sub_n && list_n[blk] != kNoList) {
-        const uint32_t lane = lane_id();
-        const uint32_t ns = (uint32_t)s.ns, c0 = (b * kBlock) / ns, c1 = (b * kBlock + n) / ns;
-        uint32_t* dst = lists + (size_t)blk * list_cap;
-        uint32_t at = 0;
-        for (uint32_t c = c0; c < c1; ++c) {
-            const uint32_t nc = sub_n[((size_t)f * s.nb_alloc + k) * s.ch + c];
-            const uint32_t* sub = reinterpret_cast<const uint32_t*>(planes + ((size_t)f * s.nb_alloc + k) * s.plane_stride + (size_t)c * ns);
-            for (uint32_t i = lane; i < nc; i += 32) dst[at + i] = sub[i];
-            at += nc;
-        }
-        uint32_t* list_hist = S.ninfo;   // 264 words: dead before tree_prepare clears S.tree and tree_assign writes ninfo
-        static_assert(kTreeWords >= 4, "the histogram of a listed block spans ninfo[260] and tree[0..3]");
-        for (uint32_t i = lane; i < (uint32_t)kSymStride; i += 32) list_hist[i] = 0;
-        __syncwarp();
-        warp_hist_from_list(dst, at, n, list_hist);
-        __syncwarp();
-        h = list_hist;
-    }
-    const BlkInfo bi = warp_build_tree(S, h, n, codes + (size_t)blk * kSymStride, tree + (size_t)blk * kTreeWords);
+    const BlkInfo bi = warp_build_tree(S, hist + (size_t)blk * kSymStride, n, codes + (size_t)blk * kSymStride, tree + (size_t)blk * kTreeWords);
     if (lane_id() == 0) {
-        info[blk] = bi;
-        count_block_mode(ctr, bi.mode);
-        // behind k_front a listed block has no plane bytes in memory: if it turns out not to be one the list
-        // encoder packs (COPY, or a payload beyond that kernel's staging) the frame runs through k_front again
-        if (redo && bi.mode != MODE_FILL && list_n[blk] != kNoList && !sparse_block_is_packed_from_list(list_n[blk], bi, sparse_stage))
-            redo[f] = 1;
-    }
-}
-
-// The same, with the serial part shared: a CTA of W warps prepares W trees (one per warp, as above), then the
-// lanes 0..W-1 of warp 0 run the W two-queue merges in lock step -- one tree per LANE instead of one per warp, so
-// the merge's warp-instructions (65 % of k_hzr_tree's, issued with one active lane) are paid once per CTA -- and
-// every warp finishes its own tree.  Dynamic shared memory: W TreeWarpSmem.
-__global__ void __launch_bounds__(1024) k_hzr_tree_ls(const uint32_t* __restrict__ hist, Shape s,
-                                                      const uint8_t* __restrict__ frame_nb,
-                                                      const uint8_t* __restrict__ blk_class, uint32_t cls,
-                                                      uint32_t total_blocks,
-                                                      uint32_t* __restrict__ codes,
-                                                      uint32_t* __restrict__ tree,
-                                                      BlkInfo* __restrict__ info,
-                                                      Counters* __restrict__ ctr)
-{
-    extern __shared__ __align__(16) uint8_t s_tree_raw[];
-    TreeWarpSmem* s_all = reinterpret_cast<TreeWarpSmem*>(s_tree_raw);
-    __shared__ uint32_t s_L[32];
-    const uint32_t W = blockDim.x >> 5, wid = warp_id(), lane = lane_id();
-    TreeWarpSmem& S = s_all[wid];
-    const uint32_t blk = blockIdx.x * W + wid;
-    uint32_t f = 0, k = 0, b = 0, n = 0, L = 0;
-    bool live = blk < total_blocks, merge = false;
-    BlkInfo bi;
-    if (live) {
-        blk_decode(s, blk, f, k, b);
-        live = k < frame_nb[f] && !(blk_class && blk_class[blk] != cls);
-    }
-    if (live) {
-        n = blk_len(s, b);
-        merge = !tree_prepare(S, hist + (size_t)blk * kSymStride, codes + (size_t)blk * kSymStride, L, bi);
-    }
-    if (lane == 0) s_L[wid] = merge ? L : 0u;
-    __syncthreads();
-    if (wid == 0 && lane < W && s_L[lane]) tree_merge(s_all[lane], s_L[lane]);
-    __syncthreads();
-    if (merge) bi = tree_assign(S, L, n, codes + (size_t)blk * kSymStride, tree + (size_t)blk * kTreeWords);
-    if (live && lane == 0) {
         info[blk] = bi;
         count_block_mode(ctr, bi.mode);
     }

@@ -68,23 +68,11 @@ struct rspt_gpu_packer {
     void* d_dec;           // block descriptors
     uint8_t* d_dec_nb;     // per-frame plane count used by the last decompress
     int32_t* d_status_tmp;
-    uint8_t* d_seg_xor;    // per 128-byte segment of every decoded plane: xor of its bytes (k_hzr_decode -> inverse transform)
-    uint32_t segs_per_plane;
     void* d_auto_index;    // decode index built here for streams that came without one
-    uint32_t* d_inv_tot;   // one-pass inverse, chained form: per (frame, round, CTA, channel) totals
-    uint32_t* d_inv_flag;  // ... and the release flags (epoch of the launch that wrote them)
-    uint32_t inv_epoch;
     double* d_fir;         // FIR kernel coefficients of the last rspt_gpu_prefilter_fir call (lazy)
     size_t fir_cap;
     int32_t* d_words2;     // second word buffer (FIR is out of place), lazy
-    uint8_t* d_redo;       // per frame: k_front flagged a sparse-mode plane as too dense (the frame runs again, forced dense)
-    uint8_t* d_redo2;      // per frame: the tree kernel found a listed block the list encoder cannot take (same remedy)
-    uint32_t* d_sub_n;     // k_front: entries in every (frame, plane, channel) sub-list
-    bool front_ok;         // shape is eligible for the fused front end (k_front)
-    int front_grid;        // persistent CTAs of k_front (SMs x resident CTAs)
-    size_t front_smem;
     uint32_t sp_stage;     // payload limit of k_hzr_encode_sparse (kSpStageBytes; lower only under RSPT_SPARSE_STAGE_BYTES)
-    bool sparse_list;      // sparse class: k_hzr_hist<3> + one-pass k_hzr_encode_sparse; false (RSPT_SPARSE_LIST=0) = the earlier kernels
     // transform constants (dct twiddles)
     double2* d_twiddle;
     double2* d_post;

@@ -14,7 +14,7 @@
 
 #include "packer.cuh"
 #include "transforms.cuh"
-#include "front.cuh"
+#include "xdelta_tma.cuh"
 #include "hzr_decode.cuh"
 #include "spectral.cuh"
 #include "filters.cuh"
@@ -160,87 +160,14 @@ bool xdelta_fast_tile(const Shape& s, const uint8_t* d_src, uint32_t& tsq, size_
 }
 
 
-// ---- fused front end (front.cuh) ----------------------------------------------------------------
-#define RSPT_FRONT_SHAPES(X) X(2, 4) X(2, 8) X(2, 12) X(3, 4) X(3, 8) X(3, 12) X(4, 4) X(4, 8) X(4, 12)
+#define RSPT_TMA_SHAPES(X) X(2, 4) X(2, 8) X(2, 12) X(3, 4) X(3, 8) X(3, 12) X(4, 4) X(4, 8) X(4, 12)
 
-// shapes k_xdelta_planes_tma is compiled for (RSPT_FRONT_SHAPES), whole tiles of 128 quads, 16-byte aligned input;
-// RSPT_TMA_TRANSFORM=0 keeps k_xdelta_planes_fast (A/B runs)
+// shapes k_xdelta_planes_tma is compiled for (RSPT_TMA_SHAPES), whole tiles of 128 quads, 16-byte aligned input
 bool tma_transform_ok(const Shape& s, const uint8_t* d_src)
 {
-    static const bool off = [] {
-        const char* e = getenv("RSPT_TMA_TRANSFORM");
-        return e && atoi(e) == 0;
-    }();
-    if (off || ((uintptr_t)d_src & 15)) return false;
+    if ((uintptr_t)d_src & 15) return false;
     if (s.bps < 2 || s.bps > 4 || (s.ch != 4 && s.ch != 8 && s.ch != 12)) return false;
-    return s.ns % (4 * kFrontQuads) == 0 && s.ns >= 4 * kFrontQuads;
-}
-
-bool front_shape_ok(const Shape& s)
-{
-    if (s.kind != RSPT_XDELTA_HZR && s.kind != RSPT_HZR) return false;
-    if (s.bps < 2 || s.bps > 4 || (s.ch != 4 && s.ch != 8 && s.ch != 12)) return false;
-    if (s.ns % kStepBytes != 0 || (uint32_t)s.ns / kStepBytes > kFrontMaxTiles) return false;
-    if (s.nb_alloc < 2 || s.nb_alloc * s.nblk > kFrontMaxHist) return false;
-    if (s.N > kBlock && kBlock % (uint32_t)s.ns != 0) return false;  // hzr blocks must start on channel rows
-    // measured (profiles/r02_front_*.txt): 1.22 ms per 4096 shape-A frames against 0.49 + 0.99 ms for the three
-    // kernels it replaces when those overlap with the tree build -- no gain yet, so it is opt-in
-    if (const char* e = getenv("RSPT_FRONT")) return atoi(e) != 0;
-    return false;
-}
-
-template <int B, int C>
-cudaError_t front_prepare(bool stencil, size_t smem, int* ctas_per_sm)
-{
-    cudaError_t e;
-    if (stencil) {
-        e = cudaFuncSetAttribute(k_front<B, C, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, k_front<B, C, true>, kFrontThreads, smem);
-    } else {
-        e = cudaFuncSetAttribute(k_front<B, C, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, k_front<B, C, false>, kFrontThreads, smem);
-    }
-    return e;
-}
-
-// decides whether the handle uses k_front and sizes its launch (called once, from rspt_gpu_create)
-cudaError_t front_setup(rspt_gpu_packer* p)
-{
-    const Shape& s = p->s;
-    p->front_ok = false;
-    if (p->can_escalate || !front_shape_ok(s)) return cudaSuccess;
-    p->front_smem = front_smem_bytes(s.bps, s.ch, s.nb_alloc, s.nblk, (uint32_t)s.ns / kStepBytes);
-    if (p->front_smem > 200 * 1024) return cudaSuccess;
-    int per_sm = 0, sms = 0;
-    cudaError_t e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, p->device);
-    if (e != cudaSuccess) return e;
-    const bool st = s.kind == RSPT_XDELTA_HZR;
-#define X(B, C) if (s.bps == B && s.ch == C) e = front_prepare<B, C>(st, p->front_smem, &per_sm);
-    RSPT_FRONT_SHAPES(X)
-#undef X
-    if (e != cudaSuccess) return e;
-    if (per_sm < 1) return cudaSuccess;
-    p->front_grid = sms * per_sm;
-    p->front_ok = true;
-    return cudaSuccess;
-}
-
-// pass 0: every frame; pass 1 / 2: the frames flagged in d_redo / d_redo2, every plane forced dense
-void front_launch(rspt_gpu_packer* p, const uint8_t* d_src, size_t F, int pass)
-{
-    const Shape& s = p->s;
-    const FrontOut o{p->d_planes, p->d_hist, p->d_step_lz, p->d_sub_n, p->d_list_n, p->d_redo, p->d_redo2};
-    const unsigned grid = (unsigned)(F < (size_t)p->front_grid ? F : (size_t)p->front_grid);
-    const bool st = s.kind == RSPT_XDELTA_HZR;
-    const uint8_t* only = pass == 0 ? nullptr : (pass == 1 ? p->d_redo : p->d_redo2);
-    const int force = pass != 0;
-#define X(B, C)                                                                                               \
-    if (s.bps == B && s.ch == C) {                                                                            \
-        if (st) k_front<B, C, true><<<grid, kFrontThreads, p->front_smem, p->stream>>>(d_src, s, (uint32_t)F, o, only, force);  \
-        else k_front<B, C, false><<<grid, kFrontThreads, p->front_smem, p->stream>>>(d_src, s, (uint32_t)F, o, only, force);    \
-    }
-    RSPT_FRONT_SHAPES(X)
-#undef X
+    return s.ns % (4 * kTmaQuads) == 0 && s.ns >= 4 * kTmaQuads;
 }
 
 }  // namespace
@@ -395,9 +322,6 @@ extern "C" int rspt_gpu_create(int kind, size_t bps, size_t ch, size_t ns, size_
     A(dalloc(p->d_info, nblocks));
     A(dalloc(p->d_frame_nb, F));
     A(dalloc(p->d_need, F));
-    A(dalloc(p->d_redo, F));
-    A(dalloc(p->d_redo2, F));
-    A(dalloc(p->d_sub_n, F * s.nb_alloc * ch));
     A(dalloc(p->d_nb_state, 4));
     A(dalloc(p->d_all_totals, 64));
     A(dalloc(p->d_sizes, F));
@@ -407,11 +331,6 @@ extern "C" int rspt_gpu_create(int kind, size_t bps, size_t ch, size_t ns, size_
     A(dalloc(p->d_status_tmp, F));
     A(dalloc(p->d_dec_nb, F));
     A(cudaMalloc(&p->d_dec, nblocks * sizeof(DecBlk) + 64));
-    p->segs_per_plane = s.nblk * (kBlock / kXorSeg);
-    A(dalloc(p->d_seg_xor, F * s.nb_alloc * (size_t)p->segs_per_plane));
-    A(dalloc(p->d_inv_tot, F * 2 * 32 * (ch < 32 ? 32 : ch)));
-    A(dalloc(p->d_inv_flag, F * 2 * 32));
-    if (e == cudaSuccess) e = cudaMemsetAsync(p->d_inv_flag, 0, F * 2 * 32 * sizeof(uint32_t), p->stream);
     A(cudaMalloc(&p->d_auto_index, ((F * (1 + s.hdr_bytes + (size_t)s.nb_alloc * (4 + hzr_max(s.N))) >> 6) + nblocks + 2) * sizeof(uint32_t) + 64));
     if (kind == RSPT_HADAMARD || kind == RSPT_DCT) {
         A(dalloc(p->d_words, F * (size_t)s.N));
@@ -431,7 +350,6 @@ extern "C" int rspt_gpu_create(int kind, size_t bps, size_t ch, size_t ns, size_
     if (e == cudaSuccess) e = cudaMemcpyAsync(p->d_nb_state, &s.nb_init, 4, cudaMemcpyHostToDevice, p->stream);
     if (e == cudaSuccess) e = allow_smem(k_hzr_encode<2>, kEncodeSmem);
     if (e == cudaSuccess) e = allow_smem(k_hzr_encode<3>, kEncodeSmem);
-    if (e == cudaSuccess) e = allow_smem(k_hzr_hist<1>, kHistSmem);
     if (e == cudaSuccess) e = allow_smem(k_hzr_hist<3>, kHistSmemList);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&p->side, cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&p->place, cudaStreamNonBlocking);
@@ -442,17 +360,12 @@ extern "C" int rspt_gpu_create(int kind, size_t bps, size_t ch, size_t ns, size_
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p->ev_join, cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p->ev_fork2, cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p->ev_join2, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = allow_smem(k_hzr_encode_sparse<true>, kSparseSmem);
-    if (e == cudaSuccess) e = allow_smem(k_hzr_encode_sparse<false>, kSparseSmem);
-    if (e == cudaSuccess) e = front_setup(p);
+    if (e == cudaSuccess) e = allow_smem(k_hzr_encode_sparse, kSparseSmem);
     {
         // test hook: a smaller staging limit sends listed blocks down the hand-over path to k_hzr_encode
         const char* ev = getenv("RSPT_SPARSE_STAGE_BYTES");
         const long v = ev ? atol(ev) : (long)kSpStageBytes;
         p->sp_stage = (uint32_t)(v < 1 ? 1 : (v > (long)kSpStageBytes ? (long)kSpStageBytes : v));
-        // A/B switch, per handle so that one process can alternate the two builds of the sparse class
-        const char* el = getenv("RSPT_SPARSE_LIST");
-        p->sparse_list = !(el && atoi(el) == 0);
     }
     if (e == cudaSuccess) e = allow_smem(k_hzr_decode, kDecodeSmem);
     if (e == cudaSuccess) e = allow_smem(k_hzr_verify, kDecodeSmem);
@@ -476,7 +389,7 @@ extern "C" int rspt_gpu_destroy(rspt_gpu_packer* p)
     void* ptrs[] = {p->d_planes, p->d_hist, p->d_codes, p->d_tree, p->d_step_lz, p->d_lists, p->d_list_n, p->d_blk_class, p->d_info, p->d_frame_nb,
                     p->d_need, p->d_nb_state, p->d_sizes, p->d_blk_off, p->d_headers, p->d_words, p->d_sums, p->d_ctr,
                     p->d_dec, p->d_dec_nb, p->d_status_tmp, p->d_twiddle, p->d_post, p->d_cos, p->d_one_src, p->d_one_dst,
-                    p->d_one_off, p->d_redo, p->d_redo2, p->d_sub_n, p->d_hb_src, p->d_hb_dst, p->d_hb_off, p->d_auto_index, p->d_fir, p->d_words2, p->d_inv_tot, p->d_inv_flag, p->d_all_totals, p->d_seg_xor};
+                    p->d_one_off, p->d_hb_src, p->d_hb_dst, p->d_hb_off, p->d_auto_index, p->d_fir, p->d_words2, p->d_all_totals};
     for (void* q : ptrs)
         if (q) cudaFree(q);
     if (p->h_pin) cudaFreeHost(p->h_pin);
@@ -571,30 +484,30 @@ extern "C" int rspt_gpu_get_counters(rspt_gpu_packer* p, rspt_gpu_counters* out)
 namespace {
 
 // stage 1: samples -> byte planes (+ header, + need flags)
-int launch_forward_transform(rspt_gpu_packer* p, const uint8_t* d_src, size_t F, const uint8_t* only = nullptr)
+int launch_forward_transform(rspt_gpu_packer* p, const uint8_t* d_src, size_t F)
 {
     const Shape& s = p->s;
     if (s.kind == RSPT_XDELTA_HZR || s.kind == RSPT_HZR) {
         uint32_t* need = p->can_escalate ? p->d_need : nullptr;
         if (need) RSPT_CUDA_CHECK(cudaMemsetAsync(need, 0, F * sizeof(uint32_t), p->stream));
         const bool st = s.kind == RSPT_XDELTA_HZR;
-        // TMA-fed tile kernel (front.cuh: k_xdelta_planes_tma) for the shapes it is compiled for; it has no
-        // plane-count probe (need) and no frame filter (only): those cases keep k_xdelta_planes_fast
-        if (!need && !only && tma_transform_ok(s, d_src)) {
-            const uint32_t tiles = (uint32_t)s.ns / (4u * kFrontQuads);
-            const size_t tsm = (size_t)(kFrontQuads + 2) * 4u * s.ch * s.bps;
+        // TMA-fed tile kernel (xdelta_tma.cuh: k_xdelta_planes_tma) for the shapes it is compiled for; it has no
+        // plane-count probe (need): that case keeps k_xdelta_planes_fast
+        if (!need && tma_transform_ok(s, d_src)) {
+            const uint32_t tiles = (uint32_t)s.ns / (4u * kTmaQuads);
+            const size_t tsm = (size_t)(kTmaQuads + 2) * 4u * s.ch * s.bps;
             const dim3 grid((unsigned)(F * tiles));
 #define X(B, C)                                                                                                          \
     if (s.bps == B && s.ch == C) {                                                                                       \
         if (st) {                                                                                                        \
             RSPT_CUDA_CHECK(allow_smem(k_xdelta_planes_tma<B, C, true>, tsm));                                           \
-            k_xdelta_planes_tma<B, C, true><<<grid, kFrontThreads, tsm, p->stream>>>(d_src, s, tiles, p->d_planes);       \
+            k_xdelta_planes_tma<B, C, true><<<grid, kTmaThreads, tsm, p->stream>>>(d_src, s, tiles, p->d_planes);       \
         } else {                                                                                                         \
             RSPT_CUDA_CHECK(allow_smem(k_xdelta_planes_tma<B, C, false>, tsm));                                          \
-            k_xdelta_planes_tma<B, C, false><<<grid, kFrontThreads, tsm, p->stream>>>(d_src, s, tiles, p->d_planes);      \
+            k_xdelta_planes_tma<B, C, false><<<grid, kTmaThreads, tsm, p->stream>>>(d_src, s, tiles, p->d_planes);      \
         }                                                                                                                \
     }
-            RSPT_FRONT_SHAPES(X)
+            RSPT_TMA_SHAPES(X)
 #undef X
             p->launches += 1;
             RSPT_CUDA_CHECK(cudaGetLastError());
@@ -608,7 +521,7 @@ int launch_forward_transform(rspt_gpu_packer* p, const uint8_t* d_src, size_t F,
 #define LAUNCH_F(B, ST)                                                                                   \
     do {                                                                                                  \
         RSPT_CUDA_CHECK(allow_smem(k_xdelta_planes_fast<B, ST>, fsmem));                                  \
-        k_xdelta_planes_fast<B, ST><<<grid, 128, fsmem, p->stream>>>(d_src, s, tsq, tiles, p->d_planes, need, only); \
+        k_xdelta_planes_fast<B, ST><<<grid, 128, fsmem, p->stream>>>(d_src, s, tsq, tiles, p->d_planes, need);       \
     } while (0)
             switch (s.bps) {
             case 1: if (st) LAUNCH_F(1, true); else LAUNCH_F(1, false); break;
@@ -658,39 +571,10 @@ int launch_frame_nb(rspt_gpu_packer* p, size_t F)
 
 // Dense-encoder CTAs per SM the kernel is compiled for.  Measured per 4096-frame batch: xdelta_hzr 1.075 -> 1.051 ms
 // and hadamard 1.121 -> 1.090 ms with 3 (more warps to cover the barriers), hzr 2.344 -> 2.369 and dct
-// 0.848 -> 0.890 with 3 (their planes take the spilled slow path more often).  RSPT_ENC_CTAS=2|3 overrides.
+// 0.848 -> 0.890 with 3 (their planes take the spilled slow path more often).
 static int encode_ctas_per_sm(const Shape& s)
 {
-    static const int forced = [] {
-        const char* e = getenv("RSPT_ENC_CTAS");
-        return e ? atoi(e) : 0;
-    }();
-    if (forced == 2 || forced == 3) return forced;
     return (s.kind == RSPT_XDELTA_HZR || s.kind == RSPT_HADAMARD) ? 3 : 2;
-}
-
-// histogram + list of the sparse-looking blocks: k_hzr_hist<3>, or the earlier list builder k_hzr_hist<1> under
-// RSPT_SPARSE_LIST=0 (same list and histogram)
-static void launch_sparse_hist(rspt_gpu_packer* p, const uint8_t* planes, const Shape& s, uint32_t nblocks, cudaStream_t st)
-{
-    if (p->sparse_list)
-        k_hzr_hist<3><<<nblocks, kHistThreads, kHistSmemList, st>>>(planes, s, p->d_frame_nb, p->d_hist, p->d_step_lz, p->d_lists, p->d_list_n, p->d_blk_class);
-    else
-        k_hzr_hist<1><<<nblocks, kHistThreads, kHistSmem, st>>>(planes, s, p->d_frame_nb, p->d_hist, p->d_step_lz, p->d_lists, p->d_list_n, p->d_blk_class);
-}
-
-// RSPT_TREE_LS=W (2..32): trees per CTA of the lock-step tree kernel; 0 = one warp per tree (k_hzr_tree)
-static uint32_t tree_lockstep_warps()
-{
-    static const uint32_t v = [] {
-        const char* e = getenv("RSPT_TREE_LS");
-        uint32_t w = e ? (uint32_t)atoi(e) : 0u;
-        if (w > 32u) w = 32u;
-        if (w == 1u) w = 0u;
-        if (w) cudaFuncSetAttribute(k_hzr_tree_ls, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(w * sizeof(TreeWarpSmem)));
-        return w;
-    }();
-    return v;
 }
 
 // A compress that rewrites an offsets array must not overtake a placement still rebasing it.
@@ -720,26 +604,6 @@ extern "C" int rspt_gpu_compress_batch(rspt_gpu_packer* p, const uint8_t* d_src,
     if (rc) return rc;
     uint32_t* sidecar = reinterpret_cast<uint32_t*>(d_sidecar);
     const unsigned tgrid = (nblocks + kTreeWarps - 1) / kTreeWarps;
-    if (p->front_ok && !((uintptr_t)d_src & 15)) {
-        // fused front end: transform + token histograms + sparse lists in one pass over the raw frames
-        // (front.cuh); a frame whose sparse-looking plane turned out dense gets its planes from the
-        // stand-alone transform kernel afterwards (flag per frame, normally no CTA does any work)
-        {
-            StageTimer t(p, RSPT_STAGE_TRANSFORM);
-            front_launch(p, d_src, F, 0);
-            front_launch(p, d_src, F, 1);   // frames whose sub-lists overflowed (normally none: the CTAs read a flag each and leave)
-            p->launches += 2;
-            RSPT_CUDA_CHECK(cudaGetLastError());
-        }
-        {
-            StageTimer t(p, RSPT_STAGE_TREE);
-            k_hzr_tree<<<tgrid, 32 * kTreeWarps, 0, p->stream>>>(p->d_hist, s, p->d_frame_nb, nullptr, 0, nblocks, p->d_codes, p->d_tree, p->d_info, p->d_ctr,
-                                                                 p->d_list_n, p->sp_stage, p->d_redo2, p->d_sub_n, p->d_planes, p->d_lists, kListCap);
-            front_launch(p, d_src, F, 2);   // frames with a listed block the list encoder cannot take
-            p->launches += 2;
-            RSPT_CUDA_CHECK(cudaGetLastError());
-        }
-    } else {
     {
         StageTimer t(p, RSPT_STAGE_TRANSFORM);
         rc = launch_forward_transform(p, d_src, F);
@@ -754,10 +618,7 @@ extern "C" int rspt_gpu_compress_batch(rspt_gpu_packer* p, const uint8_t* d_src,
         // histogram, RSPT_STAGE_TREE everything from there to the join.
         RSPT_CUDA_CHECK(cudaEventRecord(p->ev_fork, p->stream));
         RSPT_CUDA_CHECK(cudaStreamWaitEvent(p->side, p->ev_fork, 0));
-        launch_sparse_hist(p, p->d_planes, s, nblocks, p->side);
-        if (const uint32_t W = tree_lockstep_warps())
-            k_hzr_tree_ls<<<(nblocks + W - 1) / W, 32 * W, W * sizeof(TreeWarpSmem), p->side>>>(p->d_hist, s, p->d_frame_nb, p->d_blk_class, kClassSparse, nblocks, p->d_codes, p->d_tree, p->d_info, p->d_ctr);
-        else
+        k_hzr_hist<3><<<nblocks, kHistThreads, kHistSmemList, p->side>>>(p->d_planes, s, p->d_frame_nb, p->d_hist, p->d_step_lz, p->d_lists, p->d_list_n, p->d_blk_class);
         k_hzr_tree<<<tgrid, 32 * kTreeWarps, 0, p->side>>>(p->d_hist, s, p->d_frame_nb, p->d_blk_class, kClassSparse, nblocks, p->d_codes, p->d_tree, p->d_info, p->d_ctr);
         RSPT_CUDA_CHECK(cudaEventRecord(p->ev_join, p->side));
         {
@@ -766,14 +627,10 @@ extern "C" int rspt_gpu_compress_batch(rspt_gpu_packer* p, const uint8_t* d_src,
         }
         {
             StageTimer t(p, RSPT_STAGE_TREE);
-            if (const uint32_t W = tree_lockstep_warps())
-                k_hzr_tree_ls<<<(nblocks + W - 1) / W, 32 * W, W * sizeof(TreeWarpSmem), p->stream>>>(p->d_hist, s, p->d_frame_nb, p->d_blk_class, kClassDense, nblocks, p->d_codes, p->d_tree, p->d_info, p->d_ctr);
-            else
             k_hzr_tree<<<tgrid, 32 * kTreeWarps, 0, p->stream>>>(p->d_hist, s, p->d_frame_nb, p->d_blk_class, kClassDense, nblocks, p->d_codes, p->d_tree, p->d_info, p->d_ctr);
             RSPT_CUDA_CHECK(cudaStreamWaitEvent(p->stream, p->ev_join, 0));
         }
         p->launches += 4;
-    }
     }
     {
         StageTimer t(p, RSPT_STAGE_LAYOUT);
@@ -787,12 +644,8 @@ extern "C" int rspt_gpu_compress_batch(rspt_gpu_packer* p, const uint8_t* d_src,
         const SparseOut so{d_dst, d_offsets, p->d_blk_off, p->sp_stage, p->d_headers, sidecar};
         RSPT_CUDA_CHECK(cudaEventRecord(p->ev_fork2, p->stream));
         RSPT_CUDA_CHECK(cudaStreamWaitEvent(p->side, p->ev_fork2, 0));
-        if (p->sparse_list)
-            k_hzr_encode_sparse<true><<<nblocks, kSpThreads, kSparseSmem, p->side>>>(s, p->d_frame_nb, p->d_info, p->d_codes, p->d_tree, p->d_lists,
-                                                                                     p->d_list_n, p->d_crc, so);
-        else
-            k_hzr_encode_sparse<false><<<nblocks, kSpThreads, kSparseSmem, p->side>>>(s, p->d_frame_nb, p->d_info, p->d_codes, p->d_tree, p->d_lists,
-                                                                                      p->d_list_n, p->d_crc, so);
+        k_hzr_encode_sparse<<<nblocks, kSpThreads, kSparseSmem, p->side>>>(s, p->d_frame_nb, p->d_info, p->d_codes, p->d_tree, p->d_lists,
+                                                                           p->d_list_n, p->d_crc, so);
         RSPT_CUDA_CHECK(cudaEventRecord(p->ev_join2, p->side));
         if (encode_ctas_per_sm(s) == 3)
             k_hzr_encode<3><<<nblocks, kEncThreads, p->enc_smem, p->stream>>>(p->d_planes, s, p->d_frame_nb, p->d_info, p->d_blk_off,
@@ -852,16 +705,8 @@ extern "C" int rspt_gpu_build_index(rspt_gpu_packer* p, const uint8_t* d_src, co
     return launch_parse_and_index(p, d_src, d_offsets, n_frames, d_frame_nb, d_sidecar, d_status ? d_status : p->d_status_tmp);
 }
 
-// payload bits per output byte up to which k_hzr_decode uses its two-literals-per-look-up table (measured: 4;
-// RSPT_PAIR_MAX_BITS overrides it for experiments)
-static uint32_t decode_pair_max_bits()
-{
-    static const uint32_t v = [] {
-        const char* e = getenv("RSPT_PAIR_MAX_BITS");
-        return e ? (uint32_t)atoi(e) & 255u : 4u;
-    }();
-    return v;
-}
+// payload bits per output byte up to which k_hzr_decode uses its two-literals-per-look-up table (measured)
+constexpr uint32_t kDecodePairMaxBits = 4;
 
 extern "C" int rspt_gpu_decompress_batch(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets,
                                          size_t n_frames, const uint8_t* d_frame_nb, const void* d_sidecar,
@@ -886,68 +731,30 @@ extern "C" int rspt_gpu_decompress_batch(rspt_gpu_packer* p, const uint8_t* d_sr
     }
     int rc = launch_parse_and_index(p, d_src, d_offsets, F, d_frame_nb, own_index, status);
     if (rc) return rc;
-    // Decode and inverse transform can run chunk by chunk (RSPT_DECODE_CHUNK_FRAMES), so that the planes a chunk's
-    // decode writes are still in the L2 when its inverse transform reads them.  Measured on B200 (profiles/
-    // r02_decode_chunks.txt): no gain at any chunk size -- the smaller grids' tails cost more than the L2 hits
-    // save -- so the default is the whole batch at once.
-    static const size_t chunk_env = [] {
-        const char* e = getenv("RSPT_DECODE_CHUNK_FRAMES");
-        return e ? (size_t)atol(e) : (size_t)0;
-    }();
-    size_t chunk = chunk_env ? chunk_env : F;
-    if (chunk > F) chunk = F;
     const uint32_t* sc = reinterpret_cast<const uint32_t*>(d_sidecar);
     const uint32_t maxn = s.N < kBlock ? s.N : kBlock;
-    // per-segment xor of the decoded planes for the inverse transform's first scan: measured a wash (it
-    // takes 0.25 ms off k_planes_to_samples_fast and puts 0.25 ms onto this kernel), so off unless asked for
-    static const bool want_sxor = getenv("RSPT_DECODE_SEG_XOR") != nullptr;
-    uint8_t* sxor_all = (want_sxor && (s.kind == RSPT_XDELTA_HZR || s.kind == RSPT_DCT)) ? p->d_seg_xor : nullptr;
-    struct Saved { uint8_t* planes; uint8_t* dec_nb; uint8_t* headers; int32_t* words; uint8_t* seg_xor; long long* sums; } sv =
-        {p->d_planes, p->d_dec_nb, p->d_headers, p->d_words, p->d_seg_xor, p->d_sums};
-    int rc_all = RSPT_OK;
-    for (size_t f0 = 0; f0 < F && rc_all == RSPT_OK; f0 += chunk) {
-        const size_t nf = F - f0 < chunk ? F - f0 : chunk;
-        const uint32_t blk0 = total_blocks(p, f0), nblk_c = total_blocks(p, nf);
-        // the handle's per-frame scratch, shifted to the chunk
-        p->d_planes = sv.planes + f0 * s.nb_alloc * (size_t)s.plane_stride;
-        p->d_dec_nb = sv.dec_nb + f0;
-        p->d_headers = sv.headers + f0 * (s.hdr_bytes ? s.hdr_bytes : 1);
-        if (sv.words) p->d_words = sv.words + f0 * (size_t)s.N;
-        if (sv.sums) p->d_sums = sv.sums + f0 * (size_t)s.ch;
-        p->d_seg_xor = sv.seg_xor + f0 * s.nb_alloc * (size_t)p->segs_per_plane;
-        uint8_t* sxor = sxor_all ? p->d_seg_xor : nullptr;
-        const DecBlk* dec_c = dec + blk0;
-        const uint32_t* codes_c = p->d_codes + (size_t)blk0 * kSymStride;
-        int32_t* status_c = status + f0;
-        {
-            // the classes with short payloads (few busy threads per CTA, latency-bound) run on the side stream
-            // beside the full-size blocks
-            StageTimer t(p, RSPT_STAGE_DECODE);
-            cudaEventRecord(p->ev_fork, p->stream);
-            cudaStreamWaitEvent(p->side, p->ev_fork, 0);
-            k_hzr_decode<<<nblk_c, decode_class_threads(kSmallPayload), decode_class_smem(kSmallPayload), p->side>>>(
-                d_src, s, dec_c, d_offsets, sc, codes_c, p->d_planes, status_c, decode_pair_max_bits() | (s.kind <= RSPT_HZR ? 256u : 0u), 1u, sxor, p->segs_per_plane, blk0);
-            if (maxn > kSmallPayload) {
-                k_hzr_decode<<<nblk_c, decode_class_threads(kMediumPayload), decode_class_smem(kMediumPayload), p->side>>>(
-                    d_src, s, dec_c, d_offsets, sc, codes_c, p->d_planes, status_c, decode_pair_max_bits() | (s.kind <= RSPT_HZR ? 256u : 0u), 2u, sxor, p->segs_per_plane, blk0);
-                p->launches += 1;
-            }
-            cudaEventRecord(p->ev_join, p->side);
-            k_hzr_decode<<<nblk_c, kDecodeThreads, p->dec_smem, p->stream>>>(d_src, s, dec_c, d_offsets, sc, codes_c, p->d_planes, status_c,
-                                                                             decode_pair_max_bits() | (s.kind <= RSPT_HZR ? 256u : 0u), 0u, sxor, p->segs_per_plane, blk0);
-            cudaStreamWaitEvent(p->stream, p->ev_join, 0);
-            p->launches += 2;
+    const uint32_t flags = kDecodePairMaxBits | (s.kind <= RSPT_HZR ? 256u : 0u);
+    {
+        // the classes with short payloads (few busy threads per CTA, latency-bound) run on the side stream
+        // beside the full-size blocks
+        StageTimer t(p, RSPT_STAGE_DECODE);
+        cudaEventRecord(p->ev_fork, p->stream);
+        cudaStreamWaitEvent(p->side, p->ev_fork, 0);
+        k_hzr_decode<<<nblocks, decode_class_threads(kSmallPayload), decode_class_smem(kSmallPayload), p->side>>>(
+            d_src, s, dec, d_offsets, sc, p->d_codes, p->d_planes, status, flags, 1u);
+        if (maxn > kSmallPayload) {
+            k_hzr_decode<<<nblocks, decode_class_threads(kMediumPayload), decode_class_smem(kMediumPayload), p->side>>>(
+                d_src, s, dec, d_offsets, sc, p->d_codes, p->d_planes, status, flags, 2u);
+            p->launches += 1;
         }
-        if (cudaGetLastError() != cudaSuccess) rc_all = RSPT_E_CUDA;
-        {
-            StageTimer t(p, RSPT_STAGE_INVERSE);
-            const int rc2 = launch_inverse_transform(p, d_dst + f0 * (size_t)s.frame_bytes, nf);
-            if (rc2) rc_all = rc2;
-        }
+        cudaEventRecord(p->ev_join, p->side);
+        k_hzr_decode<<<nblocks, kDecodeThreads, p->dec_smem, p->stream>>>(d_src, s, dec, d_offsets, sc, p->d_codes, p->d_planes, status, flags, 0u);
+        cudaStreamWaitEvent(p->stream, p->ev_join, 0);
+        p->launches += 2;
     }
-    p->d_planes = sv.planes; p->d_dec_nb = sv.dec_nb; p->d_headers = sv.headers; p->d_words = sv.words; p->d_seg_xor = sv.seg_xor; p->d_sums = sv.sums;
-    if (rc_all == RSPT_E_CUDA) return fail_cuda(p, cudaErrorUnknown, "decode launch");
-    return rc_all;
+    RSPT_CUDA_CHECK(cudaGetLastError());
+    StageTimer t(p, RSPT_STAGE_INVERSE);
+    return launch_inverse_transform(p, d_dst, F);
 }
 
 extern "C" int rspt_gpu_verify_batch(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets, size_t n_frames,
@@ -1546,7 +1353,7 @@ extern "C" int rspt_gpu_debug_hzr_tables(rspt_gpu_packer* p, const uint8_t* d_bl
     DeviceGuard dg(p->device);
     Shape s = p->s;
     s.N = (uint32_t)n; s.nblk = 1; s.nb_alloc = 1; s.plane_stride = (uint32_t)((n + 15) & ~(size_t)15);
-    launch_sparse_hist(p, d_block, s, 1, p->stream);
+    k_hzr_hist<3><<<1, kHistThreads, kHistSmemList, p->stream>>>(d_block, s, p->d_frame_nb, p->d_hist, p->d_step_lz, p->d_lists, p->d_list_n, p->d_blk_class);
     k_hzr_hist<2><<<1, kHistThreads, 0, p->stream>>>(d_block, s, p->d_frame_nb, p->d_hist, p->d_step_lz, p->d_lists, p->d_list_n, p->d_blk_class);
     k_hzr_tree<<<1, 32 * kTreeWarps, 0, p->stream>>>(p->d_hist, s, p->d_frame_nb, p->d_blk_class, kClassSparse, 1, p->d_codes, p->d_tree, p->d_info, p->d_ctr);
     k_hzr_tree<<<1, 32 * kTreeWarps, 0, p->stream>>>(p->d_hist, s, p->d_frame_nb, p->d_blk_class, kClassDense, 1, p->d_codes, p->d_tree, p->d_info, p->d_ctr);

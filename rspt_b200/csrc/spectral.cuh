@@ -20,7 +20,6 @@
 
 #include "packer.cuh"
 #include "transforms.cuh"
-#include "inverse.cuh"
 
 namespace rspt {
 
@@ -787,15 +786,13 @@ inline cudaError_t dct_build_tables(rspt_gpu_packer* p)
 // 16-byte aligned frames
 inline bool fwht_raw_ok(const Shape& s, const void* d_raw)
 {
-    return s.kind == 2 && (s.ch & 3) == 0 && fwht_fast_len(s.ns) && ((uintptr_t)d_raw & 15) == 0 && (s.frame_bytes & 15) == 0 &&
-           getenv("RSPT_FWHT_UNFUSED") == nullptr;
+    return s.kind == 2 && (s.ch & 3) == 0 && fwht_fast_len(s.ns) && ((uintptr_t)d_raw & 15) == 0 && (s.frame_bytes & 15) == 0;
 }
 
 // the four-channel-group word kernels apply (a warp's 32 sample quads stay inside one channel group)
 inline bool words_g4_ok(const Shape& s, const void* d_raw)
 {
-    return (s.ch & 3) == 0 && (s.ns % 1024) == 0 && ((uintptr_t)d_raw & 15) == 0 && (s.frame_bytes & 15) == 0 &&
-           getenv("RSPT_WORDS_TILED") == nullptr;
+    return (s.ch & 3) == 0 && (s.ns % 1024) == 0 && ((uintptr_t)d_raw & 15) == 0 && (s.frame_bytes & 15) == 0;
 }
 
 #define FWHT_RAW_LAUNCH(KERNEL, ...)                                                                              \
@@ -882,30 +879,6 @@ inline int spectral_forward(rspt_gpu_packer* p, const uint8_t* d_src, size_t F)
 }
 
 // planes (decoded) -> samples, all four packers
-// RSPT_INV_MODE: 0 = three-pass kernel (k_planes_to_samples_fast), 1 = one pass, a cluster per frame (DSMEM),
-// 2 = one pass, chained CTAs (totals through global memory)
-inline int inverse_mode()
-{
-    static const int v = [] {
-        const char* e = getenv("RSPT_INV_MODE");
-        return e ? atoi(e) : 0;
-    }();
-    return v;
-}
-inline bool inverse_cluster_enabled() { return inverse_mode() != 0; }
-// threads per CTA (= per frame) of the three-pass inverse kernel; the registers allow 1024 threads per SM, so this
-// sets how many frames an SM has in flight (RSPT_INV_THREADS: 256 / 512 / 1024)
-inline unsigned inverse_threads()
-{
-    static const unsigned v = [] {
-        const char* e = getenv("RSPT_INV_THREADS");
-        const unsigned t = e ? (unsigned)atoi(e) : (unsigned)kInvThreads;
-        return (t == 256u || t == 512u || t == 1024u) ? t : (unsigned)kInvThreads;
-    }();
-    return v;
-}
-inline const uint8_t* inverse_seg_xor(const rspt_gpu_packer* p) { return getenv("RSPT_DECODE_SEG_XOR") ? p->d_seg_xor : nullptr; }
-
 inline int launch_inverse_transform(rspt_gpu_packer* p, uint8_t* d_dst, size_t F)
 {
     const Shape& s = p->s;
@@ -914,71 +887,6 @@ inline int launch_inverse_transform(rspt_gpu_packer* p, uint8_t* d_dst, size_t F
     const size_t sm_inv = (size_t)2 * np * 4 + tile_bytes;
     if (sm_inv > 200 * 1024 || tile_bytes > 200 * 1024) return fail_arg(p, "frame too large for the inverse kernel");
     const dim3 gf((unsigned)F);
-    // one pass over the planes: a cluster of CTAs per frame, each with a sample range of every channel (inverse.cuh)
-    if ((s.kind == 0 || s.kind == 1) && inverse_cluster_enabled() && s.bps >= 2 && (s.ch & 3) == 0 && s.ch <= (int)kInvMaxCh &&
-        (s.ns & 127) == 0 && ((uintptr_t)d_dst & 15) == 0) {
-        // S = ns / C samples per CTA, a multiple of 128; warps = (ch / 4) * (S / 128) <= 24.  Cluster form: the
-        // largest CTA that fits (C <= 8 CTAs per cluster).  Chained form: CTAs of about `want` warps (RSPT_INV_CHAIN_WARPS),
-        // up to 32 per frame.
-        const uint32_t G = (uint32_t)s.ch >> 2;
-        const bool chained_sel = inverse_mode() == 2;
-        static const uint32_t want = [] {
-            const char* e = getenv("RSPT_INV_CHAIN_WARPS");
-            return e ? (uint32_t)atoi(e) : 12u;
-        }();
-        uint32_t C = 0, S = 0;
-        for (uint32_t cc = 1; cc <= (chained_sel ? 32u : 8u); cc <<= 1) {
-            if ((uint32_t)s.ns % (cc * 128u)) break;
-            const uint32_t s2 = (uint32_t)s.ns / cc, w2 = G * (s2 >> 7);
-            if (w2 <= 24u && (uint32_t)s.ch * cc <= kInvMaxSeg && inverse_cluster_smem(s.bps, s.ch, s2) <= 100 * 1024) {
-                C = cc;
-                S = s2;
-                if (!chained_sel || w2 <= want) break;
-            }
-        }
-        if (C) {
-            const size_t smc = inverse_cluster_smem(s.bps, s.ch, S);
-            const bool chained = inverse_mode() == 2;
-            cudaLaunchConfig_t cfg = {};
-            cfg.gridDim = dim3((unsigned)(F * C));
-            cfg.blockDim = dim3(32u * G * (S >> 7));
-            cfg.dynamicSmemBytes = smc;
-            cfg.stream = p->stream;
-            cudaLaunchAttribute at[1];
-            at[0].id = cudaLaunchAttributeClusterDimension;
-            at[0].val.clusterDim.x = C;
-            at[0].val.clusterDim.y = 1;
-            at[0].val.clusterDim.z = 1;
-            cfg.attrs = at;
-            cfg.numAttrs = chained ? 0 : 1;
-            const int scan = s.kind == 0 ? 1 : 0;
-            InvChain chain = {p->d_inv_tot, p->d_inv_flag, ++p->inv_epoch, C};
-            cudaError_t e = cudaErrorInvalidValue;
-#define INVC(B, NT, CH)                                                                                                 \
-    do {                                                                                                                \
-        e = cudaFuncSetAttribute(k_inverse_cluster<B, NT, CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smc);  \
-        if (e == cudaSuccess)                                                                                           \
-            e = cudaLaunchKernelEx(&cfg, k_inverse_cluster<B, NT, CH>, (const uint8_t*)p->d_planes, s, (const uint8_t*)p->d_dec_nb, d_dst, scan, S, chain); \
-    } while (0)
-#define INVC_B(B)                                                   \
-    do {                                                            \
-        if (chained) { if (s.nb_alloc <= 3) INVC(B, 3, true); else INVC(B, 4, true); }   \
-        else { if (s.nb_alloc <= 3) INVC(B, 3, false); else INVC(B, 4, false); }         \
-    } while (0)
-            switch (s.bps) {
-            case 2: INVC_B(2); break;
-            case 3: INVC_B(3); break;
-            default: INVC_B(4); break;
-            }
-#undef INVC_B
-#undef INVC
-            if (e == cudaSuccess) {
-                p->launches += 1;
-                return 0;
-            }
-            (void)cudaGetLastError();  // cluster launch not possible here: the three-pass kernel below
-        }
-    }
     // fast path: 4-channel groups, 128-sample pieces, PRMT packing (transforms.cuh)
     if ((s.kind == 0 || s.kind == 1) && (s.ch & 3) == 0 && (s.ns % (int)kInvPiece) == 0 && ((uintptr_t)d_dst & 15) == 0) {
         const size_t row = (size_t)s.ch * s.bps;
@@ -993,8 +901,7 @@ inline int launch_inverse_transform(rspt_gpu_packer* p, uint8_t* d_dst, size_t F
 #define INVF_LAUNCH(B, SC)                                                                                            \
     do {                                                                                                              \
         RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_planes_to_samples_fast<B, SC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smf)); \
-        k_planes_to_samples_fast<B, SC><<<gf, inverse_threads(), smf, p->stream>>>(p->d_planes, s, p->d_dec_nb, tpg, d_dst,    \
-                                                                       inverse_seg_xor(p), p->segs_per_plane); \
+        k_planes_to_samples_fast<B, SC><<<gf, kInvThreads, smf, p->stream>>>(p->d_planes, s, p->d_dec_nb, tpg, d_dst);        \
     } while (0)
             const bool sc = s.kind == 0;
             switch (s.bps) {
@@ -1056,8 +963,7 @@ inline int launch_inverse_transform(rspt_gpu_packer* p, uint8_t* d_dst, size_t F
             const size_t smw = (size_t)2 * npf * 4;
             if ((s.ns % (int)kInvPiece) == 0 && (npf & 3u) == 0 && smw <= 200 * 1024) {
                 RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_planes_to_samples_fast<4, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smw));
-                k_planes_to_samples_fast<4, true, true><<<gf, inverse_threads(), smw, p->stream>>>(p->d_planes, s, p->d_dec_nb, 1, nullptr,
-                                                                                             inverse_seg_xor(p), p->segs_per_plane, p->d_words);
+                k_planes_to_samples_fast<4, true, true><<<gf, kInvThreads, smw, p->stream>>>(p->d_planes, s, p->d_dec_nb, 1, nullptr, p->d_words);
             } else {
                 INV_LAUNCH(4, true, false);
             }

@@ -156,11 +156,10 @@ __device__ __forceinline__ void unpack4(const uint32_t* w, uint32_t (&x)[4])
 template <int BPS, bool STENCIL>
 __global__ void __launch_bounds__(128) k_xdelta_planes_fast(const uint8_t* __restrict__ src, Shape s, uint32_t tsq,
                                                              uint32_t tiles_per_frame, uint8_t* __restrict__ planes,
-                                                             uint32_t* __restrict__ need, const uint8_t* __restrict__ only = nullptr)
+                                                             uint32_t* __restrict__ need)
 {
     extern __shared__ __align__(16) uint32_t smw[];
     const uint32_t f = blockIdx.x / tiles_per_frame, tile = blockIdx.x % tiles_per_frame;
-    if (only && !only[f]) return;                    // second pass behind k_front: flagged frames only
     const uint32_t row = (uint32_t)s.ch * BPS;       // bytes per sample row == words per quad
     const uint32_t qstride = row + 1;                // words
     const uint32_t cpq = row >> 2;                   // 16-byte chunks per quad
@@ -502,7 +501,6 @@ __global__ void __launch_bounds__(1024, 1) k_planes_to_samples_fast(const uint8_
                                                                             const uint8_t* __restrict__ dec_nb,
                                                                             uint32_t tiles_per_group,
                                                                             uint8_t* __restrict__ dst_raw,
-                                                                            const uint8_t* __restrict__ seg_xor, uint32_t segs_per_plane,
                                                                             int32_t* __restrict__ dst_words = nullptr)
 {
     extern __shared__ __align__(16) uint32_t sm32[];
@@ -541,16 +539,7 @@ __global__ void __launch_bounds__(1024, 1) k_planes_to_samples_fast(const uint8_
         q[3] = nba > 3 ? __ldg(a + 3 * pstride4) : make_uint4(0, 0, 0, 0);
     };
     if (SCAN) {
-        // pass 1: xor of all words of a piece = byte-wise fold of the plane words.  k_hzr_decode leaves
-        // exactly that per 128-byte segment (= piece) of every plane, so the planes are not read here.
-        if (seg_xor) {
-            const uint8_t* sx = seg_xor + (size_t)f * s.nb_alloc * segs_per_plane;
-            for (uint32_t p = threadIdx.x; p < np; p += blockDim.x) {
-                uint32_t x = 0;
-                for (uint32_t k = 0; k < nb; ++k) x |= (uint32_t)sx[(size_t)k * segs_per_plane + p] << (8 * k);
-                pxor[p] = (uint32_t)((int32_t)(x << sext) >> sext);
-            }
-        } else
+        // pass 1: xor of all words of a piece = byte-wise fold of the plane words
         // (passes 1 and 2 walk the planes in runs of four pieces: a lane takes 16 consecutive elements with one
         // 128-bit load per plane, eight lanes make a piece, and the warp-level steps are shared by four pieces)
         for (uint32_t P0 = wid * UB; P0 < nbig; P0 += nwarps * UB) {

@@ -1,18 +1,14 @@
-"""The two builds of the sparse class (RSPT_SPARSE_LIST=1: k_hzr_hist<3> + one-pass k_hzr_encode_sparse, the
-default; RSPT_SPARSE_LIST=0: the earlier k_hzr_hist<1> + two-pass encoder) against the oracle: whole streams over
-the plane shapes of the parity suite, and single blocks at the edges of the list builder (list capacity, the n/4
-density limit, chunk and step boundaries, ragged block ends).  The switch is read when a handle is created; each
-value runs in a child process, which gets its inputs and returns its results through files.  Needs a B200."""
-import os
-import subprocess
-import sys
-
+"""The sparse class (k_hzr_hist<3> builds a block's list of non-zero bytes, k_hzr_encode_sparse packs the block
+from it) against the oracle: whole streams over the plane shapes of the parity suite, and single blocks at the
+edges of the list builder (list capacity, the n/4 density limit, chunk and step boundaries, ragged block ends).
+Needs a B200."""
 import numpy as np
 import pytest
 
 pytestmark = [pytest.mark.gpu, pytest.mark.timeout(900)]
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+torch = pytest.importorskip("torch")
+
 LIST_CAP = 5120
 
 # the xdelta_hzr / hzr / hadamard shapes of test_gpu_parity.PLANE_CASES, plus a single-channel hzr plane of
@@ -28,37 +24,13 @@ STREAM_CASES = [
     ("hadamard", 3, 5, 4096, 3), ("hadamard", 2, 1, 4096, 3),
 ]
 
-CHILD = r"""
-import sys, numpy as np, torch
-sys.path.insert(0, sys.argv[1])
-from rspt_b200 import packer as R
-z = np.load(sys.argv[2])
-out = {}
-for c, (kind, (bps, ch, ns, nb)) in enumerate(zip(z["kinds"].tolist(), z["dims"].tolist())):
-    x = z["raw%d" % c]
-    n = x.shape[0]
-    p = R.SignalPacker(kind, bps, ch, ns, nb, max_batch_frames=n)
-    b = p.compress_batch(torch.from_numpy(x.reshape(-1).copy()).cuda())
-    torch.cuda.synchronize()
-    offs = b.offsets.cpu().numpy()
-    out["stream%d" % c] = b.stream[: int(offs[n])].cpu().numpy()
-    out["offs%d" % c] = offs[: n + 1].astype(np.int64)
-    p.close()
-p = R.SignalPacker.new_hzr(1, 1, 65536, max_batch_frames=1)
-for j in range(int(z["nblocks"])):
-    hist, codes, info = p.debug_hzr_tables(z["blk%d" % j])
-    out["hist%d" % j], out["info%d" % j] = hist, info
-np.savez(sys.argv[3], **out)
-"""
 
-
-def _run_child(tmp_path, inputs, env_extra):
-    src, dst = str(tmp_path / "in.npz"), str(tmp_path / ("out_%s.npz" % "_".join(env_extra.values())))
-    np.savez(src, **inputs)
-    env = dict(os.environ, **env_extra)
-    r = subprocess.run([sys.executable, "-c", CHILD, ROOT, src, dst], env=env, capture_output=True, text=True, timeout=800)
-    assert r.returncode == 0, r.stderr[-3000:]
-    return np.load(dst)
+@pytest.fixture(scope="module")
+def R():
+    import rspt_b200
+    from rspt_b200 import packer
+    assert torch.cuda.is_available(), "GPU tests need a CUDA device"
+    return packer
 
 
 def _adversarial_blocks(rng):
@@ -101,11 +73,10 @@ def _adversarial_blocks(rng):
     return out
 
 
-@pytest.mark.parametrize("switch", ["1", "0"])
-def test_sparse_list_streams_and_tables_match_oracle(switch, oracle, tmp_path):
+def _inputs(oracle):
+    """The frames of every STREAM_CASES shape and the single blocks, drawn in one fixed order from one seed."""
     rng = np.random.default_rng(1234)
-    inputs = {"kinds": np.array([c[0] for c in STREAM_CASES]), "dims": np.array([c[1:] for c in STREAM_CASES])}
-    want = []
+    frames = []
     for c, (kind, bps, ch, ns, nb) in enumerate(STREAM_CASES):
         nfr = 3
         raws = np.array(oracle.synth_ecg(50 + c, nfr, bps, ch, ns), np.uint8).reshape(nfr, -1)
@@ -115,34 +86,31 @@ def test_sparse_list_streams_and_tables_match_oracle(switch, oracle, tmp_path):
                 idx = rng.choice(70001, 900, replace=False)
                 r[idx] = rng.integers(1, 256, 900)
         raws[nfr - 1][:] = 0   # a frame of FILL blocks
-        inputs["raw%d" % c] = raws
-        cpu = oracle.OraclePacker(kind, bps, ch, ns, nb)
-        want.append([cpu.compress(r) for r in raws])
-    blocks = _adversarial_blocks(rng)
-    inputs["nblocks"] = np.array(len(blocks))
-    for j, (_, b) in enumerate(blocks):
-        inputs["blk%d" % j] = b
-    got = _run_child(tmp_path, inputs, {"RSPT_SPARSE_LIST": switch})
-    for c, case in enumerate(STREAM_CASES):
-        st, offs = got["stream%d" % c], got["offs%d" % c]
-        for i, w in enumerate(want[c]):
-            assert st[offs[i]:offs[i + 1]].tobytes() == w, (case, i)
-    for j, (name, b) in enumerate(blocks):
-        assert np.array_equal(got["hist%d" % j], oracle.hzr_histogram(b)), name
-        mode, plen = oracle.hzr_block_plan(b)
-        assert (int(got["info%d" % j][0]), int(got["info%d" % j][1])) == (mode, plen), name
+        frames.append(raws)
+    return frames, _adversarial_blocks(rng)
 
 
-@pytest.mark.parametrize("switch", ["1", "0"])
-def test_sparse_list_hand_over_to_general_encoder(switch, oracle, tmp_path):
-    """RSPT_SPARSE_STAGE_BYTES=300: listed blocks whose payload exceeds the list encoder's staging go to
-    k_hzr_encode, which rebuilds the per-step leading-zero counts from the list."""
-    bps, ch, ns, nfr = 3, 12, 8192, 4
-    raws = np.array(oracle.synth_ecg(40, nfr, bps, ch, ns), np.uint8).reshape(nfr, -1)
-    raws[nfr - 1][:] = 0
-    inputs = {"kinds": np.array(["xdelta_hzr"]), "dims": np.array([[bps, ch, ns, 3]]), "raw0": raws, "nblocks": np.array(0)}
-    got = _run_child(tmp_path, inputs, {"RSPT_SPARSE_LIST": switch, "RSPT_SPARSE_STAGE_BYTES": "300"})
-    cpu = oracle.OraclePacker("xdelta_hzr", bps, ch, ns, 3)
-    st, offs = got["stream0"], got["offs0"]
-    for i in range(nfr):
-        assert st[offs[i]:offs[i + 1]].tobytes() == cpu.compress(raws[i]), i
+@pytest.mark.parametrize("part", ["streams", "tables"])
+def test_sparse_list_streams_and_tables_match_oracle(R, oracle, part):
+    """streams: whole batches of every STREAM_CASES shape; tables: histogram and plan of the single blocks."""
+    frames, blocks = _inputs(oracle)
+    if part == "streams":
+        for (kind, bps, ch, ns, nb), raws in zip(STREAM_CASES, frames):
+            nfr = raws.shape[0]
+            cpu = oracle.OraclePacker(kind, bps, ch, ns, nb)
+            p = R.SignalPacker(kind, bps, ch, ns, nb, max_batch_frames=nfr)
+            b = p.compress_batch(torch.from_numpy(raws.reshape(-1).copy()).cuda())
+            torch.cuda.synchronize()
+            offs = b.offsets.cpu().numpy()
+            st = b.stream[: int(offs[nfr])].cpu().numpy()
+            for i, r in enumerate(raws):
+                assert st[offs[i]:offs[i + 1]].tobytes() == cpu.compress(r), ((kind, bps, ch, ns, nb), i)
+            p.close()
+    else:
+        p = R.SignalPacker.new_hzr(1, 1, 65536, max_batch_frames=1)
+        for name, b in blocks:
+            hist, codes, info = p.debug_hzr_tables(b)
+            assert np.array_equal(hist, oracle.hzr_histogram(b)), name
+            mode, plen = oracle.hzr_block_plan(b)
+            assert (int(info[0]), int(info[1])) == (mode, plen), name
+

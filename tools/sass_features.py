@@ -49,7 +49,5 @@ def excerpt(name_part, needle, before, after, title):
 excerpt("k_hzr_decode", "UBLKCP", 14, 4, "payload staging of the decoder: mbarrier init, expect_tx, one bulk copy global -> shared")
 excerpt("k_hzr_decode", "SYNCS.PHASECHK", 2, 6, "... and the wait on it (mbarrier.try_wait.parity loop)")
 excerpt("k_hzr_encodeILi3", "UBLKCP", 10, 4, "dense encoder: header + payload leave the staging with one bulk store shared -> global (default path of xdelta_hzr and hadamard)")
-excerpt("k_inverse_clusterILi3ELi3ELb0", "UCGABAR_ARV", 6, 6, "one-pass inverse, cluster variant: cluster barrier around the DSMEM exchange of the per-CTA totals")
-excerpt("k_frontILi3ELi12ELb1", "UBLKCP.S.G", 4, 3, "fused front end: plane tile leaves shared memory with a bulk store")
 open(sys.argv[1], "w").write("\n".join(out) + "\n")
 print("\n".join(out[:12]))
