@@ -100,6 +100,21 @@ int rspt_gpu_decompress_batch(rspt_gpu_packer* p, const uint8_t* d_src, const ui
                               size_t n_frames, const uint8_t* d_frame_nb, const void* d_sidecar,
                               uint8_t* d_dst, int32_t* d_status);
 
+/* The same two calls with the samples as int32 words [n_frames][ch][ns] (flat channel-major: the reference's
+ * own int32 matrix, convert_native_to_i32) instead of interleaved native bytes.  Frame format, handle state,
+ * counters (raw bytes count bps * ch * ns per frame) and stage timers are shared with the native calls: the
+ * xdelta_hzr plane count carries across batches whichever entry point compressed them.
+ *   compress    only the low 8 * bps bits of a word are the sample, higher bits are ignored.  Stream,
+ *               offsets, frame_nb and sidecar equal what rspt_gpu_compress_batch writes for the native frame
+ *               holding the low bps bytes of every word, for all four packers (and both dct paths).
+ *   decompress  every word is the sample rspt_gpu_decompress_batch writes, sign-extended from 8 * bps bits
+ *               (for every stream, including ones from the CPU reference).
+ * d_src / d_dst (the word side) must be 4-byte aligned, else RSPT_E_ARG; 16-byte alignment is faster. */
+int rspt_gpu_compress_batch_i32(rspt_gpu_packer* p, const int32_t* d_src, size_t n_frames, uint8_t* d_dst,
+                                size_t dst_capacity, uint64_t* d_offsets, uint8_t* d_frame_nb, void* d_sidecar);
+int rspt_gpu_decompress_batch_i32(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets, size_t n_frames,
+                                  const uint8_t* d_frame_nb, const void* d_sidecar, int32_t* d_dst, int32_t* d_status);
+
 /* Integrity check without decoding: replaces hzr_verify (lib_hzr/hzr_decode.c:569-624) applied to
  * every hzr stream of `n_frames` frames -- frame / chunk / block headers are walked as in
  * decompress, and the CRC-32C of every block payload is compared with the block header.

@@ -558,6 +558,29 @@ int launch_forward_transform(rspt_gpu_packer* p, const uint8_t* d_src, size_t F)
     return spectral_forward(p, d_src, F);
 }
 
+// stage 1 from int32 [ch][ns] words (rspt_gpu_compress_batch_i32): the same planes, header and need flags
+int launch_forward_transform_i32(rspt_gpu_packer* p, const int32_t* d_src, size_t F)
+{
+    const Shape& s = p->s;
+    if (s.kind == RSPT_HADAMARD || s.kind == RSPT_DCT) return spectral_forward_i32(p, d_src, F);
+    uint32_t* need = p->can_escalate ? p->d_need : nullptr;
+    if (need) RSPT_CUDA_CHECK(cudaMemsetAsync(need, 0, F * sizeof(uint32_t), p->stream));
+    const bool st = s.kind == RSPT_XDELTA_HZR;
+    const uint32_t chunks = (s.N + kI32Chunk - 1) / kI32Chunk;
+    const dim3 grid((unsigned)(F * chunks));
+#define LAUNCH_I(B, ST) k_xdelta_planes_i32<B, ST><<<grid, 256, 0, p->stream>>>(d_src, s, chunks, p->d_planes, need)
+    switch (s.bps) {
+    case 1: if (st) LAUNCH_I(1, true); else LAUNCH_I(1, false); break;
+    case 2: if (st) LAUNCH_I(2, true); else LAUNCH_I(2, false); break;
+    case 3: if (st) LAUNCH_I(3, true); else LAUNCH_I(3, false); break;
+    default: if (st) LAUNCH_I(4, true); else LAUNCH_I(4, false); break;
+    }
+#undef LAUNCH_I
+    p->launches += 1;
+    RSPT_CUDA_CHECK(cudaGetLastError());
+    return RSPT_OK;
+}
+
 int launch_frame_nb(rspt_gpu_packer* p, size_t F)
 {
     if (!p->can_escalate) return RSPT_OK;
@@ -588,10 +611,18 @@ static int wait_for_placement_of(rspt_gpu_packer* p, const void* d_offsets)
     return RSPT_OK;
 }
 
-extern "C" int rspt_gpu_compress_batch(rspt_gpu_packer* p, const uint8_t* d_src, size_t n_frames, uint8_t* d_dst,
-                                       size_t dst_capacity, uint64_t* d_offsets, uint8_t* d_frame_nb, void* d_sidecar)
+namespace {
+
+// The sample side of a batch call: interleaved native samples or int32 [ch][ns] words (exactly one is set).
+// Only the first stage of compress and the last of decompress depend on it.
+struct Samples {
+    const uint8_t* raw;
+    const int32_t* words;
+};
+
+int compress_batch(rspt_gpu_packer* p, Samples src, size_t n_frames, uint8_t* d_dst, size_t dst_capacity,
+                   uint64_t* d_offsets, uint8_t* d_frame_nb, void* d_sidecar)
 {
-    if (!p || !d_src || !d_dst || !d_offsets) return RSPT_E_ARG;
     if (n_frames == 0) return RSPT_OK;
     if (n_frames > p->max_batch) return fail_arg(p, "n_frames exceeds max_batch_frames"), RSPT_E_CAPACITY;
     if (dst_capacity < n_frames * rspt_gpu_max_compressed_size(p))
@@ -606,7 +637,7 @@ extern "C" int rspt_gpu_compress_batch(rspt_gpu_packer* p, const uint8_t* d_src,
     const unsigned tgrid = (nblocks + kTreeWarps - 1) / kTreeWarps;
     {
         StageTimer t(p, RSPT_STAGE_TRANSFORM);
-        rc = launch_forward_transform(p, d_src, F);
+        rc = src.words ? launch_forward_transform_i32(p, src.words, F) : launch_forward_transform(p, src.raw, F);
         if (rc) return rc;
         rc = launch_frame_nb(p, F);
         if (rc) return rc;
@@ -663,6 +694,22 @@ extern "C" int rspt_gpu_compress_batch(rspt_gpu_packer* p, const uint8_t* d_src,
     return RSPT_OK;
 }
 
+}  // namespace
+
+extern "C" int rspt_gpu_compress_batch(rspt_gpu_packer* p, const uint8_t* d_src, size_t n_frames, uint8_t* d_dst,
+                                       size_t dst_capacity, uint64_t* d_offsets, uint8_t* d_frame_nb, void* d_sidecar)
+{
+    if (!p || !d_src || !d_dst || !d_offsets) return RSPT_E_ARG;
+    return compress_batch(p, Samples{d_src, nullptr}, n_frames, d_dst, dst_capacity, d_offsets, d_frame_nb, d_sidecar);
+}
+
+extern "C" int rspt_gpu_compress_batch_i32(rspt_gpu_packer* p, const int32_t* d_src, size_t n_frames, uint8_t* d_dst,
+                                           size_t dst_capacity, uint64_t* d_offsets, uint8_t* d_frame_nb, void* d_sidecar)
+{
+    if (!p || !d_src || !d_dst || !d_offsets || ((uintptr_t)d_src & 3)) return RSPT_E_ARG;
+    return compress_batch(p, Samples{nullptr, d_src}, n_frames, d_dst, dst_capacity, d_offsets, d_frame_nb, d_sidecar);
+}
+
 // ---------------------------------------------------------------------------------------------
 // decompress
 // ---------------------------------------------------------------------------------------------
@@ -708,11 +755,17 @@ extern "C" int rspt_gpu_build_index(rspt_gpu_packer* p, const uint8_t* d_src, co
 // payload bits per output byte up to which k_hzr_decode uses its two-literals-per-look-up table (measured)
 constexpr uint32_t kDecodePairMaxBits = 4;
 
-extern "C" int rspt_gpu_decompress_batch(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets,
-                                         size_t n_frames, const uint8_t* d_frame_nb, const void* d_sidecar,
-                                         uint8_t* d_dst, int32_t* d_status)
+namespace {
+
+// the decoded samples go to out.raw (interleaved native) or out.words (int32 [ch][ns]); exactly one is set
+struct SamplesOut {
+    uint8_t* raw;
+    int32_t* words;
+};
+
+int decompress_batch(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets, size_t n_frames,
+                     const uint8_t* d_frame_nb, const void* d_sidecar, SamplesOut out, int32_t* d_status)
 {
-    if (!p || !d_src || !d_offsets || !d_dst) return RSPT_E_ARG;
     if (n_frames == 0) return RSPT_OK;
     if (n_frames > p->max_batch) return fail_arg(p, "n_frames exceeds max_batch_frames"), RSPT_E_CAPACITY;
     DeviceGuard dg(p->device);
@@ -754,7 +807,25 @@ extern "C" int rspt_gpu_decompress_batch(rspt_gpu_packer* p, const uint8_t* d_sr
     }
     RSPT_CUDA_CHECK(cudaGetLastError());
     StageTimer t(p, RSPT_STAGE_INVERSE);
-    return launch_inverse_transform(p, d_dst, F);
+    return out.words ? launch_inverse_transform_i32(p, out.words, F) : launch_inverse_transform(p, out.raw, F);
+}
+
+}  // namespace
+
+extern "C" int rspt_gpu_decompress_batch(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets,
+                                         size_t n_frames, const uint8_t* d_frame_nb, const void* d_sidecar,
+                                         uint8_t* d_dst, int32_t* d_status)
+{
+    if (!p || !d_src || !d_offsets || !d_dst) return RSPT_E_ARG;
+    return decompress_batch(p, d_src, d_offsets, n_frames, d_frame_nb, d_sidecar, SamplesOut{d_dst, nullptr}, d_status);
+}
+
+extern "C" int rspt_gpu_decompress_batch_i32(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets,
+                                             size_t n_frames, const uint8_t* d_frame_nb, const void* d_sidecar,
+                                             int32_t* d_dst, int32_t* d_status)
+{
+    if (!p || !d_src || !d_offsets || !d_dst || ((uintptr_t)d_dst & 3)) return RSPT_E_ARG;
+    return decompress_batch(p, d_src, d_offsets, n_frames, d_frame_nb, d_sidecar, SamplesOut{nullptr, d_dst}, d_status);
 }
 
 extern "C" int rspt_gpu_verify_batch(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets, size_t n_frames,

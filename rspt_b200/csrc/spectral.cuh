@@ -816,6 +816,45 @@ inline bool words_g4_ok(const Shape& s, const void* d_raw)
         }                                                                                                         \
     } while (0)
 
+// hadamard / dct: the word matrix in d_words (+ its per-channel sums in d_sums) -> planes + header
+inline int spectral_words_forward(rspt_gpu_packer* p, size_t F)
+{
+    const Shape& s = p->s;
+    const dim3 g2((unsigned)(F * s.ch));
+    if (s.kind == 2 /*RSPT_HADAMARD*/) {
+        const size_t sm = (size_t)s.ns * 4;
+        if (s.ns == 4096) {
+            k_fwht_fast_fwd<12><<<g2, 256, 0, p->stream>>>(p->d_words, p->d_sums, s, p->d_planes, p->d_headers);
+        } else if (s.ns == 8192) {
+            k_fwht_fast_fwd<13><<<g2, 512, 0, p->stream>>>(p->d_words, p->d_sums, s, p->d_planes, p->d_headers);
+        } else {
+            RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_fwht_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+            k_fwht_fwd<<<g2, 256, sm, p->stream>>>(p->d_words, p->d_sums, s, p->d_planes, p->d_headers);
+        }
+        p->launches += 1;
+    } else {
+        if (dct_use_direct(p)) {
+            const size_t sm = (size_t)s.ns * 4;
+            RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_dct_fwd_direct, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+            k_dct_fwd_direct<<<g2, 256, sm, p->stream>>>(p->d_words, p->d_sums, s, p->d_cos, p->d_headers);
+        } else {
+            if (s.ns >= 16) {
+                const size_t sm = (size_t)fpad_host((uint32_t)s.ns / 2) * 16;
+                RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_dct_fwd_half, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+                k_dct_fwd_half<<<g2, 256, sm, p->stream>>>(p->d_words, p->d_sums, s, p->d_twiddle, p->d_post, p->d_headers);
+            } else {
+                const size_t sm = (size_t)s.ns * 16;
+                k_dct_fwd_fast<<<g2, 256, sm, p->stream>>>(p->d_words, p->d_sums, s, p->d_twiddle, p->d_post, p->d_headers);
+            }
+        }
+        const uint32_t chunks = (s.N + 1023) / 1024;
+        k_words_stencil_planes<<<(unsigned)(F * chunks), 256, 0, p->stream>>>(p->d_words, s, chunks, p->d_planes);
+        p->launches += 2;
+    }
+    RSPT_CUDA_CHECK(cudaGetLastError());
+    return 0;
+}
+
 // hadamard / dct: samples -> planes + header
 inline int spectral_forward(rspt_gpu_packer* p, const uint8_t* d_src, size_t F)
 {
@@ -843,37 +882,70 @@ inline int spectral_forward(rspt_gpu_packer* p, const uint8_t* d_src, size_t F)
     } else {
         SPECTRAL_BPS_SWITCH(k_raw_to_words, <<<g1, 256, tile_smem, p->stream>>>(d_src, s, tiles, p->d_words, p->d_sums));
     }
-    const dim3 g2((unsigned)(F * s.ch));
-    if (s.kind == 2 /*RSPT_HADAMARD*/) {
+    p->launches += 1;
+    return spectral_words_forward(p, F);
+}
+
+// hadamard / dct from int32 [ch][ns] words: their low 8*bps bits into the word matrix, then the same word path.
+// The dct kernels transform d_words in place, so the caller's buffer is only read.
+inline int spectral_forward_i32(rspt_gpu_packer* p, const int32_t* d_src, size_t F)
+{
+    const Shape& s = p->s;
+    const uint32_t tiles = ((uint32_t)s.ns + 1023) / 1024;
+    RSPT_CUDA_CHECK(cudaMemsetAsync(p->d_sums, 0, F * s.ch * sizeof(long long), p->stream));
+    SPECTRAL_BPS_SWITCH(k_i32_to_words, <<<(unsigned)(F * s.ch * tiles), 256, 0, p->stream>>>(d_src, s, tiles, p->d_words, p->d_sums));
+    p->launches += 1;
+    return spectral_words_forward(p, F);
+}
+
+// planes (decoded) -> the samples as int32 words in `words`, hadamard / dct.  The dct kernels work in place on
+// the coefficient words, so for dct `words` is also their scratch.
+inline int spectral_inverse_words(rspt_gpu_packer* p, size_t F, int32_t* words)
+{
+    const Shape& s = p->s;
+    const dim3 gf((unsigned)F), g2((unsigned)(F * s.ch));
+    if (s.kind == 2) {
         const size_t sm = (size_t)s.ns * 4;
         if (s.ns == 4096) {
-            k_fwht_fast_fwd<12><<<g2, 256, 0, p->stream>>>(p->d_words, p->d_sums, s, p->d_planes, p->d_headers);
+            k_fwht_fast_inv<12><<<g2, 256, 0, p->stream>>>(p->d_planes, p->d_headers, p->d_dec_nb, s, words);
         } else if (s.ns == 8192) {
-            k_fwht_fast_fwd<13><<<g2, 512, 0, p->stream>>>(p->d_words, p->d_sums, s, p->d_planes, p->d_headers);
+            k_fwht_fast_inv<13><<<g2, 512, 0, p->stream>>>(p->d_planes, p->d_headers, p->d_dec_nb, s, words);
         } else {
-            RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_fwht_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-            k_fwht_fwd<<<g2, 256, sm, p->stream>>>(p->d_words, p->d_sums, s, p->d_planes, p->d_headers);
+            RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_fwht_inv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+            k_fwht_inv<<<g2, 256, sm, p->stream>>>(p->d_planes, p->d_headers, p->d_dec_nb, s, words);
         }
-        p->launches += 2;
-    } else {
-        if (dct_use_direct(p)) {
-            const size_t sm = (size_t)s.ns * 4;
-            RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_dct_fwd_direct, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-            k_dct_fwd_direct<<<g2, 256, sm, p->stream>>>(p->d_words, p->d_sums, s, p->d_cos, p->d_headers);
-        } else {
-            if (s.ns >= 16) {
-                const size_t sm = (size_t)fpad_host((uint32_t)s.ns / 2) * 16;
-                RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_dct_fwd_half, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-                k_dct_fwd_half<<<g2, 256, sm, p->stream>>>(p->d_words, p->d_sums, s, p->d_twiddle, p->d_post, p->d_headers);
-            } else {
-                const size_t sm = (size_t)s.ns * 16;
-                k_dct_fwd_fast<<<g2, 256, sm, p->stream>>>(p->d_words, p->d_sums, s, p->d_twiddle, p->d_post, p->d_headers);
-            }
-        }
-        const uint32_t chunks = (s.N + 1023) / 1024;
-        k_words_stencil_planes<<<(unsigned)(F * chunks), 256, 0, p->stream>>>(p->d_words, s, chunks, p->d_planes);
-        p->launches += 3;
+        p->launches += 1;
+        RSPT_CUDA_CHECK(cudaGetLastError());
+        return 0;
     }
+    // coefficient words (BPS unused for word output); the fast kernel walks a frame's 128-element
+    // pieces four at a time, so their number must be a multiple of 4
+    const uint32_t npf = ((uint32_t)s.ns / kInvPiece) * (uint32_t)s.ch;
+    const size_t smw = (size_t)2 * npf * 4;
+    if ((s.ns % (int)kInvPiece) == 0 && (npf & 3u) == 0 && smw <= 200 * 1024) {
+        RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_planes_to_samples_fast<4, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smw));
+        k_planes_to_samples_fast<4, true, true><<<gf, kInvThreads, smw, p->stream>>>(p->d_planes, s, p->d_dec_nb, 1, nullptr, words);
+    } else {
+        const uint32_t np = (((uint32_t)s.ns + kPiece - 1) / kPiece) * (uint32_t)s.ch;
+        const size_t sm_inv = (size_t)2 * np * 4 + (size_t)kPiece * s.ch * s.bps + 48;
+        RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_planes_to_samples<4, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_inv));
+        k_planes_to_samples<4, true, false><<<gf, 512, sm_inv, p->stream>>>(p->d_planes, s, p->d_dec_nb, nullptr, words);
+    }
+    if (dct_use_direct(p)) {
+        const size_t sm = (size_t)s.ns * 4;
+        RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_dct_inv_direct, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+        k_dct_inv_direct<<<g2, 256, sm, p->stream>>>(words, p->d_headers, s, p->d_cos);
+    } else {
+        if (s.ns >= 16) {
+            const size_t sm = (size_t)fpad_host((uint32_t)s.ns / 2) * 16;
+            RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_dct_inv_half, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+            k_dct_inv_half<<<g2, 256, sm, p->stream>>>(words, p->d_headers, s, p->d_twiddle, p->d_post);
+        } else {
+            const size_t sm = (size_t)s.ns * 16;
+            k_dct_inv_fast<<<g2, 256, sm, p->stream>>>(words, p->d_headers, s, p->d_twiddle, p->d_post);
+        }
+    }
+    p->launches += 2;
     RSPT_CUDA_CHECK(cudaGetLastError());
     return 0;
 }
@@ -938,51 +1010,14 @@ inline int launch_inverse_transform(rspt_gpu_packer* p, uint8_t* d_dst, size_t F
         }
         p->launches += 1;
     } else {
-        const dim3 g2((unsigned)(F * s.ch));
         if (fwht_raw_ok(s, d_dst)) {
             FWHT_RAW_LAUNCH(k_fwht_raw_inv, p->d_planes, p->d_headers, p->d_dec_nb, s, d_dst);
             p->launches += 1;
             RSPT_CUDA_CHECK(cudaGetLastError());
             return 0;
         }
-        if (s.kind == 2) {
-            const size_t sm = (size_t)s.ns * 4;
-            if (s.ns == 4096) {
-                k_fwht_fast_inv<12><<<g2, 256, 0, p->stream>>>(p->d_planes, p->d_headers, p->d_dec_nb, s, p->d_words);
-            } else if (s.ns == 8192) {
-                k_fwht_fast_inv<13><<<g2, 512, 0, p->stream>>>(p->d_planes, p->d_headers, p->d_dec_nb, s, p->d_words);
-            } else {
-                RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_fwht_inv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-                k_fwht_inv<<<g2, 256, sm, p->stream>>>(p->d_planes, p->d_headers, p->d_dec_nb, s, p->d_words);
-            }
-            p->launches += 1;
-        } else {
-            // coefficient words (BPS unused for word output); the fast kernel walks a frame's 128-element
-            // pieces four at a time, so their number must be a multiple of 4
-            const uint32_t npf = ((uint32_t)s.ns / kInvPiece) * (uint32_t)s.ch;
-            const size_t smw = (size_t)2 * npf * 4;
-            if ((s.ns % (int)kInvPiece) == 0 && (npf & 3u) == 0 && smw <= 200 * 1024) {
-                RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_planes_to_samples_fast<4, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smw));
-                k_planes_to_samples_fast<4, true, true><<<gf, kInvThreads, smw, p->stream>>>(p->d_planes, s, p->d_dec_nb, 1, nullptr, p->d_words);
-            } else {
-                INV_LAUNCH(4, true, false);
-            }
-            if (dct_use_direct(p)) {
-                const size_t sm = (size_t)s.ns * 4;
-                RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_dct_inv_direct, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-                k_dct_inv_direct<<<g2, 256, sm, p->stream>>>(p->d_words, p->d_headers, s, p->d_cos);
-            } else {
-                if (s.ns >= 16) {
-                    const size_t sm = (size_t)fpad_host((uint32_t)s.ns / 2) * 16;
-                    RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_dct_inv_half, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-                    k_dct_inv_half<<<g2, 256, sm, p->stream>>>(p->d_words, p->d_headers, s, p->d_twiddle, p->d_post);
-                } else {
-                    const size_t sm = (size_t)s.ns * 16;
-                    k_dct_inv_fast<<<g2, 256, sm, p->stream>>>(p->d_words, p->d_headers, s, p->d_twiddle, p->d_post);
-                }
-            }
-            p->launches += 2;
-        }
+        const int rc = spectral_inverse_words(p, F, p->d_words);
+        if (rc) return rc;
         const uint32_t tiles = ppc;
         switch (s.bps) {
         case 1: RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_words_to_raw<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_bytes)); break;
@@ -999,6 +1034,66 @@ inline int launch_inverse_transform(rspt_gpu_packer* p, uint8_t* d_dst, size_t F
         p->launches += 1;
     }
 #undef INV_LAUNCH
+    RSPT_CUDA_CHECK(cudaGetLastError());
+    return 0;
+}
+
+// planes (decoded) -> int32 [ch][ns] words, sign-extended from 8*bps bits (rspt_gpu_decompress_batch_i32).
+// d_dst only needs 4-byte alignment; 16 bytes let the fast sample kernel store it directly.
+inline int launch_inverse_transform_i32(rspt_gpu_packer* p, int32_t* d_dst, size_t F)
+{
+    const Shape& s = p->s;
+    if (s.kind == 2 || s.kind == 3) {
+        // hadamard's inverse kernels only write their output, so 4-byte samples go straight to the caller;
+        // dct transforms its coefficient words in place and keeps the handle's scratch
+        int32_t* words = (s.kind == 2 && s.bps == 4) ? d_dst : p->d_words;
+        const int rc = spectral_inverse_words(p, F, words);
+        if (rc) return rc;
+        if (words != d_dst) {
+            const size_t n = F * (size_t)s.N;
+            const unsigned grid = (unsigned)((n + 1023) / 1024);
+            SPECTRAL_BPS_SWITCH(k_words_sext, <<<grid, 256, 0, p->stream>>>(words, n, d_dst));
+            p->launches += 1;
+        }
+        RSPT_CUDA_CHECK(cudaGetLastError());
+        return 0;
+    }
+    const dim3 gf((unsigned)F);
+    const bool sc = s.kind == 0;
+    // the fast kernel walks a frame's 128-element pieces four at a time (their number must be a multiple of 4)
+    // and stores 128-bit words
+    const uint32_t npf = ((uint32_t)s.ns / kInvPiece) * (uint32_t)s.ch;
+    const size_t smw = (size_t)2 * npf * 4;
+    if ((s.ns % (int)kInvPiece) == 0 && (npf & 3u) == 0 && smw <= 200 * 1024 && ((uintptr_t)d_dst & 15) == 0) {
+#define INVW_LAUNCH(B, SC)                                                                                                  \
+    do {                                                                                                                    \
+        RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_planes_to_samples_fast<B, SC, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smw)); \
+        k_planes_to_samples_fast<B, SC, true><<<gf, kInvThreads, smw, p->stream>>>(p->d_planes, s, p->d_dec_nb, 1, nullptr, d_dst); \
+    } while (0)
+        switch (s.bps) {
+        case 1: if (sc) INVW_LAUNCH(1, true); else INVW_LAUNCH(1, false); break;
+        case 2: if (sc) INVW_LAUNCH(2, true); else INVW_LAUNCH(2, false); break;
+        case 3: if (sc) INVW_LAUNCH(3, true); else INVW_LAUNCH(3, false); break;
+        default: if (sc) INVW_LAUNCH(4, true); else INVW_LAUNCH(4, false); break;
+        }
+#undef INVW_LAUNCH
+    } else {
+        const uint32_t np = (((uint32_t)s.ns + kPiece - 1) / kPiece) * (uint32_t)s.ch;
+        const size_t sm = (size_t)2 * np * 4;
+#define INVG_LAUNCH(B, SC)                                                                                                  \
+    do {                                                                                                                    \
+        RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_planes_to_samples<B, SC, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm)); \
+        k_planes_to_samples<B, SC, false><<<gf, 512, sm, p->stream>>>(p->d_planes, s, p->d_dec_nb, nullptr, d_dst);      \
+    } while (0)
+        switch (s.bps) {
+        case 1: if (sc) INVG_LAUNCH(1, true); else INVG_LAUNCH(1, false); break;
+        case 2: if (sc) INVG_LAUNCH(2, true); else INVG_LAUNCH(2, false); break;
+        case 3: if (sc) INVG_LAUNCH(3, true); else INVG_LAUNCH(3, false); break;
+        default: if (sc) INVG_LAUNCH(4, true); else INVG_LAUNCH(4, false); break;
+        }
+#undef INVG_LAUNCH
+    }
+    p->launches += 1;
     RSPT_CUDA_CHECK(cudaGetLastError());
     return 0;
 }

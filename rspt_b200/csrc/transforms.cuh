@@ -256,6 +256,85 @@ __global__ void __launch_bounds__(128) k_xdelta_planes_fast(const uint8_t* __res
 }
 
 // ------------------------------------------------------------------------------------------
+// int32 [ch][ns] input (rspt_gpu_compress_batch_i32): the word matrix the interleaved samples are
+// converted into (convert_native_to_i32, utils.cpp:123-191).  In flat order the stencil's
+// predecessors are simply the two previous words, so every shape takes this kernel.  A thread owns
+// kI32Groups groups of 4 consecutive words, 1024 words apart (one 128-bit load per group where the
+// group is 16-byte aligned, scalar loads otherwise), keeps the low 8*BPS bits of each word sign-
+// extended, and after the 4 x 4 byte transpose stores one 32-bit word per plane.  A CTA covers
+// kI32Chunk words of one frame, so a warp never spans two frames (one atomicMax per warp for `need`).
+// ------------------------------------------------------------------------------------------
+constexpr int kI32Groups = 2;
+constexpr uint32_t kI32Chunk = 1024u * kI32Groups;
+
+// the low 8*BPS bits of w as a sign-extended word (identity for BPS = 4)
+template <int BPS>
+__device__ __forceinline__ uint32_t sext_bps(uint32_t w)
+{
+    return (uint32_t)((int32_t)(w << (32 - 8 * BPS)) >> (32 - 8 * BPS));
+}
+
+template <int BPS, bool STENCIL>
+__global__ void __launch_bounds__(256) k_xdelta_planes_i32(const int32_t* __restrict__ src, Shape s, uint32_t chunks,
+                                                            uint8_t* __restrict__ planes, uint32_t* __restrict__ need)
+{
+    const uint32_t f = blockIdx.x / chunks, i0 = (blockIdx.x % chunks) * kI32Chunk + threadIdx.x * 4u;
+    const uint32_t* w = reinterpret_cast<const uint32_t*>(src) + (size_t)f * s.N;
+    uint32_t x[kI32Groups][4], cnt[kI32Groups];
+#pragma unroll
+    for (int g = 0; g < kI32Groups; ++g) {
+        const uint32_t i = i0 + 1024u * g;
+        cnt[g] = i < s.N ? min(4u, s.N - i) : 0u;
+        if (cnt[g] == 4 && ((uintptr_t)(w + i) & 15u) == 0) {
+            const uint4 v = __ldg(reinterpret_cast<const uint4*>(w + i));
+            x[g][0] = v.x; x[g][1] = v.y; x[g][2] = v.z; x[g][3] = v.w;
+        } else {
+#pragma unroll
+            for (int k = 0; k < 4; ++k) x[g][k] = (uint32_t)k < cnt[g] ? __ldg(w + i + k) : 0u;
+        }
+    }
+    uint32_t my_need = 1;
+#pragma unroll
+    for (int g = 0; g < kI32Groups; ++g) {
+        const uint32_t i = i0 + 1024u * g;
+        uint32_t y[4];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) y[k] = sext_bps<BPS>(x[g][k]);
+        if (STENCIL) {
+            // x[-2], x[-1] of the frame are 0; the very first word has no predecessor delta: y[0] = x[0] - 128
+            const bool pred = i && cnt[g];  // groups past the frame's end load nothing
+            const uint32_t xm2 = pred ? sext_bps<BPS>(__ldg(w + i - 2)) : 0u, xm1 = pred ? sext_bps<BPS>(__ldg(w + i - 1)) : 0u;
+            const uint32_t dm = i ? xm1 - xm2 - 128u : 0u;
+            const uint32_t d0 = y[0] - xm1 - 128u, d1 = y[1] - y[0] - 128u, d2 = y[2] - y[1] - 128u, d3 = y[3] - y[2] - 128u;
+            y[0] = d0 ^ dm; y[1] = d1 ^ d0; y[2] = d2 ^ d1; y[3] = d3 ^ d2;
+            if (need) {
+#pragma unroll
+                for (int k = 0; k < 4; ++k)
+                    if ((uint32_t)k < cnt[g]) my_need = max(my_need, planes_needed(y[k], BPS));
+            }
+        }
+        uint8_t* out = planes + (size_t)f * s.nb_alloc * s.plane_stride + i;
+        if (cnt[g] == 4) {
+            const uint32_t t01 = prmt(y[0], y[1], 0x5140u), t23 = prmt(y[2], y[3], 0x5140u);
+            const uint32_t u01 = prmt(y[0], y[1], 0x7362u), u23 = prmt(y[2], y[3], 0x7362u);
+            *reinterpret_cast<uint32_t*>(out) = prmt(t01, t23, 0x5410u);
+            if (s.nb_alloc > 1) *reinterpret_cast<uint32_t*>(out + s.plane_stride) = prmt(t01, t23, 0x7632u);
+            if (s.nb_alloc > 2) *reinterpret_cast<uint32_t*>(out + 2 * (size_t)s.plane_stride) = prmt(u01, u23, 0x5410u);
+            if (s.nb_alloc > 3) *reinterpret_cast<uint32_t*>(out + 3 * (size_t)s.plane_stride) = prmt(u01, u23, 0x7632u);
+        } else {
+#pragma unroll
+            for (int k = 0; k < 4; ++k)
+                if ((uint32_t)k < cnt[g])
+                    for (uint32_t b = 0; b < s.nb_alloc; ++b) out[(size_t)b * s.plane_stride + k] = (uint8_t)(y[k] >> (8 * b));
+        }
+    }
+    if (STENCIL && need) {
+        my_need = __reduce_max_sync(0xFFFFFFFFu, my_need);
+        if (lane_id() == 0 && my_need > 1) atomicMax(&need[f], my_need);
+    }
+}
+
+// ------------------------------------------------------------------------------------------
 // planes -> samples.  One CTA per frame.  The decode-side chains are two scans over the flat
 // [ch*ns] order that cross channel rows: d = prefix-xor(y) (xor_decode_32, utils.cpp:232-236),
 // x = prefix-sum(d + 128) (offset_32(+128) and delta_decode, :204-219).  The frame is cut into
@@ -263,7 +342,8 @@ __global__ void __launch_bounds__(128) k_xdelta_planes_fast(const uint8_t* __res
 // are scanned in shared memory: pass 1 xor totals, pass 2 sums of d + 128, pass 3 the samples.
 // OUT_RAW: pass 3 walks sample tiles, transposes through shared memory and stores interleaved
 // little-endian samples (convert_i32_to_native, utils.cpp:51-121) with coalesced writes;
-// otherwise the int32 words are stored in flat order (input of the inverse DCT).
+// otherwise the int32 words are stored in flat order (input of the inverse DCT, or the samples of
+// rspt_gpu_decompress_batch_i32).
 // ------------------------------------------------------------------------------------------
 constexpr int kPiece = 256;
 
@@ -431,10 +511,11 @@ __global__ void __launch_bounds__(512) k_planes_to_samples(const uint8_t* __rest
                         for (int bb = 0; bb < BPS; ++bb) q[bb] = (uint8_t)(y[i] >> (8 * bb));
                     }
             } else {
+                // sample words are sign-extended from 8*BPS bits (the dct's coefficient words use BPS = 4)
                 int32_t* w = dst_words + (size_t)f * s.N + (size_t)c * ns + s0;
 #pragma unroll
                 for (int i = 0; i < 8; ++i)
-                    if ((uint32_t)i < cnt) w[i] = (int32_t)y[i];
+                    if ((uint32_t)i < cnt) w[i] = (int32_t)sext_bps<BPS>(y[i]);
             }
         }
         if (OUT_RAW) {
@@ -455,7 +536,8 @@ __global__ void __launch_bounds__(512) k_planes_to_samples(const uint8_t* __rest
 //           the four channels' samples are packed row-wise with PRMT into a shared-memory tile
 //           (quad stride row + 1 words, conflict-free) that the CTA then copies out coalesced.
 // SCAN = false is the plain hzr packer (no chain).  WORDS = true stops after the scans and stores
-// the int32 words in flat order (the coefficient words of the inverse DCT): pass 3 then walks the
+// the int32 words in flat order, sign-extended from 8*BPS bits (the coefficient words of the inverse
+// DCT with BPS = 4, or the samples of rspt_gpu_decompress_batch_i32): pass 3 then walks the
 // pieces like pass 2 and every lane writes its 4 consecutive words with one 128-bit store.
 // ------------------------------------------------------------------------------------------
 constexpr int kInvThreads = 256;
@@ -663,8 +745,8 @@ __global__ void __launch_bounds__(1024, 1) k_planes_to_samples_fast(const uint8_
                     for (int i = 0; i < 8; ++i) y[i] += base;
                 }
                 uint4* w2 = wout + (size_t)(P0 + u) * 64u + 2u * lane;
-                w2[0] = make_uint4(y[0], y[1], y[2], y[3]);
-                w2[1] = make_uint4(y[4], y[5], y[6], y[7]);
+                w2[0] = make_uint4(sext_bps<BPS>(y[0]), sext_bps<BPS>(y[1]), sext_bps<BPS>(y[2]), sext_bps<BPS>(y[3]));
+                w2[1] = make_uint4(sext_bps<BPS>(y[4]), sext_bps<BPS>(y[5]), sext_bps<BPS>(y[6]), sext_bps<BPS>(y[7]));
             }
         }
         return;
@@ -959,6 +1041,70 @@ __global__ void __launch_bounds__(256) k_raw_to_words_g4(const uint8_t* __restri
         if (lane_id() == 0)
             atomicAdd(reinterpret_cast<unsigned long long*>(sums + f * s.ch + 4 * g + cc),
                       (unsigned long long)((long long)hi * 65536ll + (long long)lo));
+    }
+}
+
+// int32 [ch][ns] input of rspt_gpu_compress_batch_i32 -> the word matrix (low 8*BPS bits, sign-extended) +
+// per-channel sums, what k_raw_to_words makes of interleaved samples.  One CTA per (frame, channel,
+// 1024-sample tile), 4 consecutive words per thread: a warp stays in one channel row, so its partial sum
+// goes out with one 64-bit atomic.  128-bit accesses where the address allows, scalar ones otherwise.
+template <int BPS>
+__global__ void __launch_bounds__(256) k_i32_to_words(const int32_t* __restrict__ src, Shape s, uint32_t tiles,
+                                                      int32_t* __restrict__ words, long long* __restrict__ sums)
+{
+    const uint32_t fc = blockIdx.x / tiles, s0 = (blockIdx.x % tiles) * 1024u + threadIdx.x * 4u;
+    const uint32_t ns = (uint32_t)s.ns, cnt = s0 < ns ? min(4u, ns - s0) : 0u;
+    const size_t e = (size_t)fc * ns + s0;  // frames are [ch][ns] blocks, so (frame, channel) rows are consecutive
+    const uint32_t* in = reinterpret_cast<const uint32_t*>(src) + e;
+    uint32_t* out = reinterpret_cast<uint32_t*>(words) + e;
+    uint32_t x[4];
+    if (cnt == 4 && ((uintptr_t)in & 15u) == 0) {
+        const uint4 v = __ldg(reinterpret_cast<const uint4*>(in));
+        x[0] = v.x; x[1] = v.y; x[2] = v.z; x[3] = v.w;
+    } else {
+#pragma unroll
+        for (int k = 0; k < 4; ++k) x[k] = (uint32_t)k < cnt ? __ldg(in + k) : 0u;
+    }
+#pragma unroll
+    for (int k = 0; k < 4; ++k) x[k] = sext_bps<BPS>(x[k]);
+    if (cnt == 4 && ((uintptr_t)out & 15u) == 0) {
+        *reinterpret_cast<uint4*>(out) = make_uint4(x[0], x[1], x[2], x[3]);
+    } else {
+#pragma unroll
+        for (int k = 0; k < 4; ++k)
+            if ((uint32_t)k < cnt) out[k] = x[k];
+    }
+    // 64-bit channel sum from two 32-bit warp reductions (as k_raw_to_words_g4); words past the row are 0
+    int hi = 0;
+    uint32_t lo = 0;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        hi += (int32_t)x[k] >> 16;
+        lo += x[k] & 0xFFFFu;
+    }
+    hi = __reduce_add_sync(0xFFFFFFFFu, hi);
+    lo = __reduce_add_sync(0xFFFFFFFFu, lo);
+    if (lane_id() == 0 && cnt)
+        atomicAdd(reinterpret_cast<unsigned long long*>(sums + fc), (unsigned long long)((long long)hi * 65536ll + (long long)lo));
+}
+
+// decoded word matrix -> int32 output of rspt_gpu_decompress_batch_i32: the low 8*BPS bits, sign-extended
+// (the sample convert_i32_to_native keeps).  4 words per thread over the flat batch.
+template <int BPS>
+__global__ void __launch_bounds__(256) k_words_sext(const int32_t* __restrict__ words, size_t n, int32_t* __restrict__ dst)
+{
+    const size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) * 4u;
+    if (i >= n) return;
+    const uint32_t cnt = n - i < 4 ? (uint32_t)(n - i) : 4u;
+    const uint32_t* in = reinterpret_cast<const uint32_t*>(words) + i;
+    uint32_t* out = reinterpret_cast<uint32_t*>(dst) + i;
+    if (cnt == 4 && ((uintptr_t)out & 15u) == 0) {
+        const uint4 v = __ldg(reinterpret_cast<const uint4*>(in));
+        *reinterpret_cast<uint4*>(out) = make_uint4(sext_bps<BPS>(v.x), sext_bps<BPS>(v.y), sext_bps<BPS>(v.z), sext_bps<BPS>(v.w));
+    } else {
+#pragma unroll
+        for (int k = 0; k < 4; ++k)
+            if ((uint32_t)k < cnt) out[k] = sext_bps<BPS>(__ldg(in + k));
     }
 }
 

@@ -180,6 +180,23 @@ class SignalPacker:
         n = frames.numel() // self.frame_bytes
         if n * self.frame_bytes != frames.numel():
             raise ValueError("frames is not a whole number of frames")
+        return self._compress(self.L.rspt_gpu_compress_batch, frames, n, out, sidecar)
+
+    def compress_tensor(self, x: torch.Tensor, out: CompressedBatch | None = None, sidecar: bool = True) -> CompressedBatch:
+        """x: contiguous int32 CUDA tensor [n, ch, ns] on the handle's device, the samples in the low 8 * bps bits of
+        each word (higher bits are ignored).  The batch equals what compress_batch writes for the same samples in
+        the native layout; both calls share the handle's state.  Asynchronous on torch's current stream."""
+        self._check_words(x)
+        return self._compress(self.L.rspt_gpu_compress_batch_i32, x, x.shape[0], out, sidecar)
+
+    def _check_words(self, x, n: int | None = None) -> None:
+        shape = (x.shape[0] if n is None else n, self.ch, self.ns) if isinstance(x, torch.Tensor) and x.dim() == 3 else None
+        if not (isinstance(x, torch.Tensor) and x.dtype == torch.int32 and x.is_cuda and x.device.index == self.device
+                and tuple(x.shape) == shape and x.is_contiguous()):
+            want = f"[{'n' if n is None else n}, {self.ch}, {self.ns}]"
+            raise ValueError(f"expected a contiguous torch.int32 tensor {want} on cuda:{self.device}")
+
+    def _compress(self, fn, src: torch.Tensor, n: int, out: CompressedBatch | None, sidecar: bool) -> CompressedBatch:
         if out is None:
             out = self.alloc_output(n, sidecar)
         if out.offsets.numel() < n + 1 or out.frame_nb.numel() < n or out.stream.numel() < n * self.max_compressed_size:
@@ -188,9 +205,9 @@ class SignalPacker:
             raise ValueError("the output batch's sidecar is too small for these frames")
         self._bind_stream()
         sc = out.sidecar.data_ptr() if out.sidecar is not None else None
-        rc = self.L.rspt_gpu_compress_batch(self.h, frames.data_ptr(), n, out.stream.data_ptr(), out.stream.numel(),
-                                            out.offsets.data_ptr(), out.frame_nb.data_ptr(), sc)
-        check(rc, self.h, "rspt_gpu_compress_batch")
+        rc = fn(self.h, src.data_ptr(), n, out.stream.data_ptr(), out.stream.numel(), out.offsets.data_ptr(),
+                out.frame_nb.data_ptr(), sc)
+        check(rc, self.h, fn.__name__)
         out.n_frames = n
         return out
 
@@ -199,12 +216,27 @@ class SignalPacker:
         n = batch.n_frames
         if out is None:
             out = torch.empty(n * self.frame_bytes, dtype=torch.uint8, device=self._dev())
+        return self._decompress(self.L.rspt_gpu_decompress_batch, batch, out, status, use_sidecar)
+
+    def decompress_tensor(self, batch: CompressedBatch, out: torch.Tensor | None = None, status: torch.Tensor | None = None,
+                          use_sidecar: bool = True) -> torch.Tensor:
+        """The batch's samples as an int32 tensor [n, ch, ns]: every word is the sample decompress_batch writes,
+        sign-extended from 8 * bps bits.  `out`, when given, must be a contiguous int32 tensor of that shape on the
+        handle's device."""
+        n = batch.n_frames
+        if out is None:
+            out = torch.empty((n, self.ch, self.ns), dtype=torch.int32, device=self._dev())
+        self._check_words(out, n)
+        return self._decompress(self.L.rspt_gpu_decompress_batch_i32, batch, out, status, use_sidecar)
+
+    def _decompress(self, fn, batch: CompressedBatch, out: torch.Tensor, status: torch.Tensor | None,
+                    use_sidecar: bool) -> torch.Tensor:
         sc = batch.sidecar.data_ptr() if (use_sidecar and batch.sidecar is not None) else None
         nbp = batch.frame_nb.data_ptr() if batch.frame_nb is not None else None
         self._bind_stream()
-        rc = self.L.rspt_gpu_decompress_batch(self.h, batch.stream.data_ptr(), batch.offsets.data_ptr(), n, nbp, sc,
-                                              out.data_ptr(), status.data_ptr() if status is not None else None)
-        check(rc, self.h, "rspt_gpu_decompress_batch")
+        rc = fn(self.h, batch.stream.data_ptr(), batch.offsets.data_ptr(), batch.n_frames, nbp, sc,
+                out.data_ptr(), status.data_ptr() if status is not None else None)
+        check(rc, self.h, fn.__name__)
         return out
 
     def prefilter_iir(self, frames: torch.Tensor, n, d, init_nr_samples: int) -> torch.Tensor:
