@@ -6,6 +6,9 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <mutex>
+#include <type_traits>
+#include <utility>
 #include <vector>
 
 #include "common.cuh"
@@ -26,7 +29,6 @@ struct rspt_gpu_packer {
     rspt::Shape s;
     int device;
     cudaStream_t stream;
-    bool own_stream;
     size_t max_batch;
     size_t enc_smem;       // dynamic shared memory of k_hzr_encode (staging of the largest block)
     size_t dec_smem;       // dynamic shared memory of k_hzr_decode (payload of the largest block)
@@ -83,11 +85,6 @@ struct rspt_gpu_packer {
     uint64_t* d_one_off;
     uint8_t* h_pin;
     size_t h_pin_bytes;
-    // host batch API staging (grown on demand)
-    uint8_t* d_hb_src;
-    uint8_t* d_hb_dst;
-    uint64_t* d_hb_off;
-    size_t hb_frames;
     HostPipe pipe;
 
     unsigned long long launches;
@@ -113,6 +110,56 @@ inline int fail_arg(rspt_gpu_packer* p, const char* what)
 {
     if (p) snprintf(p->err, sizeof(p->err), "%s", what);
     return -1;  // RSPT_E_ARG
+}
+
+// f(std::integral_constant<int, bps>{}) for bps 1..4 (anything above as 4): names a kernel template's
+// instantiation from a run-time value.  f returns a status.  The return type is int, not deduced, so that
+// the kernels f names are instantiated at the end of the translation unit: the order in which it first names
+// its kernels orders their extern shared-memory declarations, which decides where k_hzr_hist<3>'s dynamic
+// shared memory starts.
+template <class F>
+int with_bps(int bps, F&& f)
+{
+    switch (bps) {
+    case 1: return f(std::integral_constant<int, 1>{});
+    case 2: return f(std::integral_constant<int, 2>{});
+    case 3: return f(std::integral_constant<int, 3>{});
+    default: return f(std::integral_constant<int, 4>{});
+    }
+}
+
+template <class F>
+int with_flag(bool b, F&& f)
+{
+    return b ? f(std::true_type{}) : f(std::false_type{});
+}
+
+// The dynamic shared-memory limit belongs to the kernel, for the whole process and device, not to a handle.
+// It only ever goes up, to what some launch needed, so that no handle can lower it under another handle's
+// launch; the check and the raise hold one process mutex.
+template <class K>
+cudaError_t raise_smem_limit(K* kernel, size_t bytes)
+{
+    static std::mutex mu;
+    std::lock_guard<std::mutex> lk(mu);
+    cudaFuncAttributes a;
+    cudaError_t e = cudaFuncGetAttributes(&a, kernel);
+    if (e == cudaSuccess && (size_t)a.maxDynamicSharedSizeBytes < bytes)
+        e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    return e;
+}
+
+// kernel<<<grid, block, smem>>>(args...) on the handle's stream, counted in p->launches.  48 KB, static
+// included, need no raised limit; the kernels launched here with dynamic shared memory declare at most an
+// mbarrier's worth of static shared memory, and ask for far less or far more than 48 KB.
+template <class... P, class... A>
+int launch(rspt_gpu_packer* p, void (*kernel)(P...), dim3 grid, dim3 block, size_t smem, A&&... args)
+{
+    if (smem > 48 * 1024) RSPT_CUDA_CHECK(raise_smem_limit(kernel, smem));
+    kernel<<<grid, block, smem, p->stream>>>(std::forward<A>(args)...);
+    p->launches += 1;
+    RSPT_CUDA_CHECK(cudaGetLastError());
+    return 0;
 }
 
 }  // namespace rspt

@@ -13,10 +13,8 @@
 #include <vector>
 
 #include "packer.cuh"
-#include "transforms.cuh"
-#include "xdelta_tma.cuh"
 #include "hzr_decode.cuh"
-#include "spectral.cuh"
+#include "sample_stages.cuh"
 #include "filters.cuh"
 
 using namespace rspt;
@@ -129,47 +127,6 @@ void destroy_host_pipe(rspt_gpu_packer* p);
 
 uint32_t total_blocks(const rspt_gpu_packer* p, size_t frames) { return (uint32_t)(frames * p->s.nb_alloc * p->s.nblk); }
 
-// tile height (samples) of k_xdelta_planes and the dynamic shared memory it needs
-bool xdelta_tile(const Shape& s, uint32_t& ts, size_t& smem)
-{
-    const size_t row = (size_t)s.ch * s.bps, per = row + 4 * (size_t)s.ch;
-    const size_t budget = 96 * 1024;
-    size_t t = (budget - 64 - 8 * (size_t)s.ch) / per;
-    t = t > 512 ? 512 : (t & ~(size_t)31);
-    if (t < 32) return false;
-    const size_t need_t = ((size_t)s.ns + 31) & ~(size_t)31;
-    if (t > need_t) t = need_t;
-    ts = (uint32_t)t;
-    smem = ((t * row + 31) & ~(size_t)15) + (size_t)s.ch * (t + 2) * 4;
-    return true;
-}
-
-// quads per tile and dynamic shared memory of k_xdelta_planes_fast; false = shape not eligible
-bool xdelta_fast_tile(const Shape& s, const uint8_t* d_src, uint32_t& tsq, size_t& smem)
-{
-    if ((s.ch & 3) || (s.ns & 3) || s.ns < 4 || ((uintptr_t)d_src & 15)) return false;
-    const size_t row = (size_t)s.ch * s.bps;
-    for (uint32_t t = 128; t >= 32; t >>= 1) {
-        smem = (size_t)(t + 1) * (row + 1) * 4;
-        if (smem <= 56 * 1024) {
-            tsq = t;
-            return true;
-        }
-    }
-    return false;
-}
-
-
-#define RSPT_TMA_SHAPES(X) X(2, 4) X(2, 8) X(2, 12) X(3, 4) X(3, 8) X(3, 12) X(4, 4) X(4, 8) X(4, 12)
-
-// shapes k_xdelta_planes_tma is compiled for (RSPT_TMA_SHAPES), whole tiles of 128 quads, 16-byte aligned input
-bool tma_transform_ok(const Shape& s, const uint8_t* d_src)
-{
-    if ((uintptr_t)d_src & 15) return false;
-    if (s.bps < 2 || s.bps > 4 || (s.ch != 4 && s.ch != 8 && s.ch != 12)) return false;
-    return s.ns % (4 * kTmaQuads) == 0 && s.ns >= 4 * kTmaQuads;
-}
-
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------
@@ -266,17 +223,11 @@ extern "C" int rspt_gpu_create(int kind, size_t bps, size_t ch, size_t ns, size_
     if (kind == RSPT_XDELTA_HZR && (nb < 1 || nb > 4)) return RSPT_E_ARG;
     if (kind == RSPT_HADAMARD && ((ns & (ns - 1)) || ns < 2 || ns > kFwhtMaxN)) return RSPT_E_ARG;  // needs 2^k (fwht.c)
     if (kind == RSPT_DCT && (ns < 2 || ns > kDctMaxN)) return RSPT_E_ARG;
-    // A shape that the tile kernels cannot stage in shared memory is refused here, not at the first call:
-    // the generic forward tile (xdelta_tile / kPiece sample rows), the inverse kernel's carries + tile.
+    // A shape that the tile kernels cannot stage in shared memory is refused here, not at the first call.
     {
         Shape t{};
         t.kind = kind; t.bps = (int)bps; t.ch = (int)ch; t.ns = (int)ns;
-        uint32_t ts;
-        size_t smem;
-        if ((kind == RSPT_XDELTA_HZR || kind == RSPT_HZR) && !xdelta_tile(t, ts, smem)) return RSPT_E_ARG;
-        const size_t tile_bytes = (size_t)kPiece * ch * bps + 48;
-        const size_t pieces = ((ns + kPiece - 1) / kPiece) * ch;
-        if (tile_bytes > 200 * 1024 || 2 * pieces * 4 + tile_bytes > 200 * 1024) return RSPT_E_ARG;
+        if (!sample_tiles_fit(t)) return RSPT_E_ARG;
     }
     DeviceGuard dg(device);
     int rc = ensure_device_constants(device);
@@ -307,7 +258,6 @@ extern "C" int rspt_gpu_create(int kind, size_t bps, size_t ch, size_t ns, size_
     p->enc_smem = (size_t)(12 + (maxn + 3) / 4 + 8) * 4;  // staging of the largest block: header + payload at an offset of <= 38 bytes, + slack
     p->dec_smem = ((size_t)(maxn + 30) / 16 + 2) * 16;   // the 16-byte chunks that hold the largest payload (any alignment) + zero slack
     p->stream = (cudaStream_t)stream;  // NULL = the CUDA default stream
-    p->own_stream = false;
     const size_t F = max_batch_frames, nblocks = F * s.nb_alloc * s.nblk;
     cudaError_t e = cudaSuccess;
     auto A = [&](cudaError_t r) { if (e == cudaSuccess) e = r; };
@@ -389,7 +339,7 @@ extern "C" int rspt_gpu_destroy(rspt_gpu_packer* p)
     void* ptrs[] = {p->d_planes, p->d_hist, p->d_codes, p->d_tree, p->d_step_lz, p->d_lists, p->d_list_n, p->d_blk_class, p->d_info, p->d_frame_nb,
                     p->d_need, p->d_nb_state, p->d_sizes, p->d_blk_off, p->d_headers, p->d_words, p->d_sums, p->d_ctr,
                     p->d_dec, p->d_dec_nb, p->d_status_tmp, p->d_twiddle, p->d_post, p->d_cos, p->d_one_src, p->d_one_dst,
-                    p->d_one_off, p->d_hb_src, p->d_hb_dst, p->d_hb_off, p->d_auto_index, p->d_fir, p->d_words2, p->d_all_totals};
+                    p->d_one_off, p->d_auto_index, p->d_fir, p->d_words2, p->d_all_totals};
     for (void* q : ptrs)
         if (q) cudaFree(q);
     if (p->h_pin) cudaFreeHost(p->h_pin);
@@ -408,7 +358,6 @@ extern "C" int rspt_gpu_destroy(rspt_gpu_packer* p)
     if (p->ev_join) cudaEventDestroy(p->ev_join);
     if (p->ev_fork2) cudaEventDestroy(p->ev_fork2);
     if (p->ev_join2) cudaEventDestroy(p->ev_join2);
-    if (p->own_stream) cudaStreamDestroy(p->stream);
     delete p;
     return RSPT_OK;
 }
@@ -482,104 +431,6 @@ extern "C" int rspt_gpu_get_counters(rspt_gpu_packer* p, rspt_gpu_counters* out)
 // compress
 // ---------------------------------------------------------------------------------------------
 namespace {
-
-// stage 1: samples -> byte planes (+ header, + need flags)
-int launch_forward_transform(rspt_gpu_packer* p, const uint8_t* d_src, size_t F)
-{
-    const Shape& s = p->s;
-    if (s.kind == RSPT_XDELTA_HZR || s.kind == RSPT_HZR) {
-        uint32_t* need = p->can_escalate ? p->d_need : nullptr;
-        if (need) RSPT_CUDA_CHECK(cudaMemsetAsync(need, 0, F * sizeof(uint32_t), p->stream));
-        const bool st = s.kind == RSPT_XDELTA_HZR;
-        // TMA-fed tile kernel (xdelta_tma.cuh: k_xdelta_planes_tma) for the shapes it is compiled for; it has no
-        // plane-count probe (need): that case keeps k_xdelta_planes_fast
-        if (!need && tma_transform_ok(s, d_src)) {
-            const uint32_t tiles = (uint32_t)s.ns / (4u * kTmaQuads);
-            const size_t tsm = (size_t)(kTmaQuads + 2) * 4u * s.ch * s.bps;
-            const dim3 grid((unsigned)(F * tiles));
-#define X(B, C)                                                                                                          \
-    if (s.bps == B && s.ch == C) {                                                                                       \
-        if (st) {                                                                                                        \
-            RSPT_CUDA_CHECK(allow_smem(k_xdelta_planes_tma<B, C, true>, tsm));                                           \
-            k_xdelta_planes_tma<B, C, true><<<grid, kTmaThreads, tsm, p->stream>>>(d_src, s, tiles, p->d_planes);       \
-        } else {                                                                                                         \
-            RSPT_CUDA_CHECK(allow_smem(k_xdelta_planes_tma<B, C, false>, tsm));                                          \
-            k_xdelta_planes_tma<B, C, false><<<grid, kTmaThreads, tsm, p->stream>>>(d_src, s, tiles, p->d_planes);      \
-        }                                                                                                                \
-    }
-            RSPT_TMA_SHAPES(X)
-#undef X
-            p->launches += 1;
-            RSPT_CUDA_CHECK(cudaGetLastError());
-            return RSPT_OK;
-        }
-        uint32_t tsq;
-        size_t fsmem;
-        if (xdelta_fast_tile(s, d_src, tsq, fsmem)) {
-            const uint32_t nq = (uint32_t)s.ns >> 2, tiles = (nq + tsq - 1) / tsq;
-            const dim3 grid((unsigned)(F * tiles));
-#define LAUNCH_F(B, ST)                                                                                   \
-    do {                                                                                                  \
-        RSPT_CUDA_CHECK(allow_smem(k_xdelta_planes_fast<B, ST>, fsmem));                                  \
-        k_xdelta_planes_fast<B, ST><<<grid, 128, fsmem, p->stream>>>(d_src, s, tsq, tiles, p->d_planes, need);       \
-    } while (0)
-            switch (s.bps) {
-            case 1: if (st) LAUNCH_F(1, true); else LAUNCH_F(1, false); break;
-            case 2: if (st) LAUNCH_F(2, true); else LAUNCH_F(2, false); break;
-            case 3: if (st) LAUNCH_F(3, true); else LAUNCH_F(3, false); break;
-            default: if (st) LAUNCH_F(4, true); else LAUNCH_F(4, false); break;
-            }
-#undef LAUNCH_F
-            p->launches += 1;
-            RSPT_CUDA_CHECK(cudaGetLastError());
-            return RSPT_OK;
-        }
-        uint32_t ts;
-        size_t smem;
-        if (!xdelta_tile(s, ts, smem)) return fail_arg(p, "too many channels for the tile kernel");
-        const uint32_t tiles = ((uint32_t)s.ns + ts - 1) / ts;
-        const dim3 grid((unsigned)(F * tiles));
-#define LAUNCH_X(B, ST)                                                                              \
-    do {                                                                                             \
-        RSPT_CUDA_CHECK(allow_smem(k_xdelta_planes<B, ST>, smem));                                   \
-        k_xdelta_planes<B, ST><<<grid, 256, smem, p->stream>>>(d_src, s, ts, tiles, p->d_planes, need); \
-    } while (0)
-        switch (s.bps) {
-        case 1: if (st) LAUNCH_X(1, true); else LAUNCH_X(1, false); break;
-        case 2: if (st) LAUNCH_X(2, true); else LAUNCH_X(2, false); break;
-        case 3: if (st) LAUNCH_X(3, true); else LAUNCH_X(3, false); break;
-        default: if (st) LAUNCH_X(4, true); else LAUNCH_X(4, false); break;
-        }
-#undef LAUNCH_X
-        p->launches += 1;
-        RSPT_CUDA_CHECK(cudaGetLastError());
-        return RSPT_OK;
-    }
-    return spectral_forward(p, d_src, F);
-}
-
-// stage 1 from int32 [ch][ns] words (rspt_gpu_compress_batch_i32): the same planes, header and need flags
-int launch_forward_transform_i32(rspt_gpu_packer* p, const int32_t* d_src, size_t F)
-{
-    const Shape& s = p->s;
-    if (s.kind == RSPT_HADAMARD || s.kind == RSPT_DCT) return spectral_forward_i32(p, d_src, F);
-    uint32_t* need = p->can_escalate ? p->d_need : nullptr;
-    if (need) RSPT_CUDA_CHECK(cudaMemsetAsync(need, 0, F * sizeof(uint32_t), p->stream));
-    const bool st = s.kind == RSPT_XDELTA_HZR;
-    const uint32_t chunks = (s.N + kI32Chunk - 1) / kI32Chunk;
-    const dim3 grid((unsigned)(F * chunks));
-#define LAUNCH_I(B, ST) k_xdelta_planes_i32<B, ST><<<grid, 256, 0, p->stream>>>(d_src, s, chunks, p->d_planes, need)
-    switch (s.bps) {
-    case 1: if (st) LAUNCH_I(1, true); else LAUNCH_I(1, false); break;
-    case 2: if (st) LAUNCH_I(2, true); else LAUNCH_I(2, false); break;
-    case 3: if (st) LAUNCH_I(3, true); else LAUNCH_I(3, false); break;
-    default: if (st) LAUNCH_I(4, true); else LAUNCH_I(4, false); break;
-    }
-#undef LAUNCH_I
-    p->launches += 1;
-    RSPT_CUDA_CHECK(cudaGetLastError());
-    return RSPT_OK;
-}
 
 int launch_frame_nb(rspt_gpu_packer* p, size_t F)
 {
@@ -1084,42 +935,6 @@ int ensure_words(rspt_gpu_packer* p)
     return RSPT_OK;
 }
 
-int launch_words_to_raw(rspt_gpu_packer* p, const int32_t* d_words, uint8_t* d_dst, size_t F)
-{
-    const Shape& s = p->s;
-    const uint32_t tiles = ((uint32_t)s.ns + kPiece - 1) / kPiece;
-    const size_t tile_bytes = (size_t)kPiece * s.ch * s.bps + 48;
-    if (tile_bytes > 200 * 1024) return fail_arg(p, "too many channels");
-    switch (s.bps) {
-    case 1: RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_words_to_raw<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_bytes)); break;
-    case 2: RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_words_to_raw<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_bytes)); break;
-    case 3: RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_words_to_raw<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_bytes)); break;
-    default: RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_words_to_raw<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_bytes)); break;
-    }
-    SPECTRAL_BPS_SWITCH(k_words_to_raw, <<<(unsigned)(F * tiles), 256, tile_bytes, p->stream>>>(d_words, s, tiles, d_dst));
-    p->launches += 1;
-    RSPT_CUDA_CHECK(cudaGetLastError());
-    return RSPT_OK;
-}
-
-int launch_raw_to_words(rspt_gpu_packer* p, const uint8_t* d_src, size_t F)
-{
-    const Shape& s = p->s;
-    const uint32_t tiles = ((uint32_t)s.ns + kPiece - 1) / kPiece;
-    const size_t tile_smem = (size_t)kPiece * s.ch * s.bps + 48;
-    if (tile_smem > 200 * 1024) return fail_arg(p, "too many channels");
-    switch (s.bps) {
-    case 1: RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_raw_to_words<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_smem)); break;
-    case 2: RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_raw_to_words<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_smem)); break;
-    case 3: RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_raw_to_words<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_smem)); break;
-    default: RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_raw_to_words<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_smem)); break;
-    }
-    SPECTRAL_BPS_SWITCH(k_raw_to_words, <<<(unsigned)(F * tiles), 256, tile_smem, p->stream>>>(d_src, s, tiles, p->d_words, p->d_sums));
-    p->launches += 1;
-    RSPT_CUDA_CHECK(cudaGetLastError());
-    return RSPT_OK;
-}
-
 }  // namespace
 
 extern "C" int rspt_gpu_prefilter_iir(rspt_gpu_packer* p, uint8_t* d_frames, size_t n_frames, const double* n, const double* d,
@@ -1144,15 +959,11 @@ extern "C" int rspt_gpu_prefilter_iir(rspt_gpu_packer* p, uint8_t* d_frames, siz
         c.n[i] = n[i];
         c.d[i] = d[i];
     }
-    const unsigned grid = (unsigned)((F + 31) / 32);
-    switch (nr_coefficients) {
-    case 2: k_iir_frames<2><<<grid, 32, 0, p->stream>>>(p->d_words, s, (uint32_t)F, c); break;
-    case 3: k_iir_frames<3><<<grid, 32, 0, p->stream>>>(p->d_words, s, (uint32_t)F, c); break;
-    case 4: k_iir_frames<4><<<grid, 32, 0, p->stream>>>(p->d_words, s, (uint32_t)F, c); break;
-    default: k_iir_frames<5><<<grid, 32, 0, p->stream>>>(p->d_words, s, (uint32_t)F, c); break;
-    }
-    p->launches += 1;
-    RSPT_CUDA_CHECK(cudaGetLastError());
+    // 2..5 coefficients: with_bps spans 1..4
+    rc = with_bps(nr_coefficients - 1, [&](auto B) {
+        return launch(p, k_iir_frames<B + 1>, (unsigned)((F + 31) / 32), 32, 0, p->d_words, s, (uint32_t)F, c);
+    });
+    if (rc) return rc;
     return launch_words_to_raw(p, p->d_words, d_frames, F);
 }
 
@@ -1178,11 +989,9 @@ extern "C" int rspt_gpu_prefilter_fir(rspt_gpu_packer* p, uint8_t* d_frames, siz
     if (rc) return rc;
     const size_t sm = (size_t)(2 * kernel_size + kFirTile) * sizeof(double);
     if (sm > 200 * 1024) return fail_arg(p, "fir kernel too long for the shared-memory tile");
-    RSPT_CUDA_CHECK(allow_smem(k_fir_words, sm));
     const uint32_t tiles = ((uint32_t)s.ns + kFirTile - 1) / kFirTile;
-    k_fir_words<<<(unsigned)(F * s.ch * tiles), kFirTile, sm, p->stream>>>(p->d_words, s, tiles, p->d_fir, kernel_size, p->d_words2);
-    p->launches += 1;
-    RSPT_CUDA_CHECK(cudaGetLastError());
+    rc = launch(p, k_fir_words, (unsigned)(F * s.ch * tiles), kFirTile, sm, p->d_words, s, tiles, p->d_fir, kernel_size, p->d_words2);
+    if (rc) return rc;
     return launch_words_to_raw(p, p->d_words2, d_frames, F);
 }
 
@@ -1552,13 +1361,10 @@ extern "C" int rspt_gpu_synth_ecg(uint8_t* d_dst, uint64_t first_frame, size_t n
     const uint32_t tiles = ((uint32_t)ns + 255u) / 256u;
     const dim3 grid((unsigned)(n_frames * tiles));
     cudaStream_t st = (cudaStream_t)stream;
-    switch (bps) {
-    case 1: k_synth<1><<<grid, 256, 0, st>>>(d_dst, first_frame, (uint32_t)n_frames, ch, ns, prm, g_synth_tab[dev]); break;
-    case 2: k_synth<2><<<grid, 256, 0, st>>>(d_dst, first_frame, (uint32_t)n_frames, ch, ns, prm, g_synth_tab[dev]); break;
-    case 3: k_synth<3><<<grid, 256, 0, st>>>(d_dst, first_frame, (uint32_t)n_frames, ch, ns, prm, g_synth_tab[dev]); break;
-    default: k_synth<4><<<grid, 256, 0, st>>>(d_dst, first_frame, (uint32_t)n_frames, ch, ns, prm, g_synth_tab[dev]); break;
-    }
-    return cudaGetLastError() == cudaSuccess ? RSPT_OK : RSPT_E_CUDA;
+    return with_bps(bps, [&](auto B) {
+        k_synth<B><<<grid, 256, 0, st>>>(d_dst, first_frame, (uint32_t)n_frames, ch, ns, prm, g_synth_tab[dev]);
+        return cudaGetLastError() == cudaSuccess ? RSPT_OK : RSPT_E_CUDA;
+    });
 }
 
 extern "C" int rspt_gpu_prdn_terms(const uint8_t* d_orig, const uint8_t* d_dec, size_t n_frames, int bps, int ch, int ns,
@@ -1573,12 +1379,10 @@ extern "C" int rspt_gpu_prdn_terms(const uint8_t* d_orig, const uint8_t* d_dec, 
     cudaStream_t st = (cudaStream_t)stream;
     cudaMemsetAsync(d_out, 0, 16, st);
     const dim3 grid((unsigned)(n_frames * ch));
-    switch (bps) {
-    case 1: k_prdn<1><<<grid, 256, 0, st>>>(d_orig, d_dec, (uint32_t)n_frames, ch, ns, d_out); break;
-    case 2: k_prdn<2><<<grid, 256, 0, st>>>(d_orig, d_dec, (uint32_t)n_frames, ch, ns, d_out); break;
-    case 3: k_prdn<3><<<grid, 256, 0, st>>>(d_orig, d_dec, (uint32_t)n_frames, ch, ns, d_out); break;
-    default: k_prdn<4><<<grid, 256, 0, st>>>(d_orig, d_dec, (uint32_t)n_frames, ch, ns, d_out); break;
-    }
+    with_bps(bps, [&](auto B) {
+        k_prdn<B><<<grid, 256, 0, st>>>(d_orig, d_dec, (uint32_t)n_frames, ch, ns, d_out);
+        return RSPT_OK;
+    });
     cudaError_t e = cudaMemcpyAsync(h_out, d_out, 16, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     return e == cudaSuccess ? RSPT_OK : RSPT_E_CUDA;

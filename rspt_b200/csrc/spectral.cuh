@@ -110,7 +110,6 @@ __global__ void __launch_bounds__(256) k_fwht_inv(const uint8_t* __restrict__ pl
 // which keeps the stride-16 accesses of pass 3 conflict-free.  Butterfly order is irrelevant mod
 // 2^32, so the result is the reference's natural-order transform (fwht.c:15-25).
 __device__ __forceinline__ uint32_t fwht_phys(uint32_t i) { return i + (i >> 5); }
-inline bool fwht_fast_len(int ns) { return ns == 4096 || ns == 8192; }
 
 __device__ __forceinline__ void radix16(uint32_t (&r)[16])
 {
@@ -729,9 +728,7 @@ __global__ void __launch_bounds__(256) k_dct_inv_direct(int32_t* __restrict__ wo
     }
 }
 
-// ---- host side ----------------------------------------------------------------------------
-inline uint32_t fpad_host(uint32_t m) { return m + (m >> 3) + (m >> 6) + 2; }
-inline bool dct_use_direct(const rspt_gpu_packer* p) { return p->dct_direct; }
+// ---- dct tables (host) ----------------------------------------------------------------------------
 
 // decided once, when the handle is created: non-power-of-two lengths need the direct path,
 // RSPT_DCT_DIRECT=1 requests it
@@ -761,7 +758,7 @@ inline cudaError_t dct_build_tables(rspt_gpu_packer* p)
         if (e == cudaSuccess) e = cudaMemcpy(p->d_twiddle, tw.data(), sizeof(double2) * (n / 2), cudaMemcpyHostToDevice);
         if (e == cudaSuccess) e = cudaMemcpy(p->d_post, post.data(), sizeof(double2) * n, cudaMemcpyHostToDevice);
     }
-    if (e == cudaSuccess && dct_use_direct(p)) {
+    if (e == cudaSuccess && p->dct_direct) {
         // COSINES[i][j] = (float)cos(((i << 1) * j + j) * PI / (2n))  (dct.cpp:60-68); the same
         // symmetric-in-role table serves the forward ([x][i]) and inverse ([i][x]) sums
         std::vector<float> t((size_t)n * n);
@@ -772,330 +769,6 @@ inline cudaError_t dct_build_tables(rspt_gpu_packer* p)
         if (e == cudaSuccess) e = cudaMemcpy(p->d_cos, t.data(), sizeof(float) * (size_t)n * n, cudaMemcpyHostToDevice);
     }
     return e;
-}
-
-#define SPECTRAL_BPS_SWITCH(KERNEL, ...)                     \
-    switch (s.bps) {                                         \
-    case 1: KERNEL<1> __VA_ARGS__; break;                    \
-    case 2: KERNEL<2> __VA_ARGS__; break;                    \
-    case 3: KERNEL<3> __VA_ARGS__; break;                    \
-    default: KERNEL<4> __VA_ARGS__; break;                   \
-    }
-
-// the fused hadamard kernels apply: four-channel groups, a transform length with a register path,
-// 16-byte aligned frames
-inline bool fwht_raw_ok(const Shape& s, const void* d_raw)
-{
-    return s.kind == 2 && (s.ch & 3) == 0 && fwht_fast_len(s.ns) && ((uintptr_t)d_raw & 15) == 0 && (s.frame_bytes & 15) == 0;
-}
-
-// the four-channel-group word kernels apply (a warp's 32 sample quads stay inside one channel group)
-inline bool words_g4_ok(const Shape& s, const void* d_raw)
-{
-    return (s.ch & 3) == 0 && (s.ns % 1024) == 0 && ((uintptr_t)d_raw & 15) == 0 && (s.frame_bytes & 15) == 0;
-}
-
-#define FWHT_RAW_LAUNCH(KERNEL, ...)                                                                              \
-    do {                                                                                                          \
-        const size_t smr = (size_t)4 * ((size_t)s.ns + s.ns / 32) * 4;                                            \
-        const unsigned gr = (unsigned)(F * (s.ch >> 2));                                                          \
-        if (s.ns == 4096) {                                                                                       \
-            switch (s.bps) {                                                                                      \
-            case 1: RSPT_CUDA_CHECK(cudaFuncSetAttribute(KERNEL<12, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smr)); KERNEL<12, 1><<<gr, 256, smr, p->stream>>>(__VA_ARGS__); break; \
-            case 2: RSPT_CUDA_CHECK(cudaFuncSetAttribute(KERNEL<12, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smr)); KERNEL<12, 2><<<gr, 256, smr, p->stream>>>(__VA_ARGS__); break; \
-            case 3: RSPT_CUDA_CHECK(cudaFuncSetAttribute(KERNEL<12, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smr)); KERNEL<12, 3><<<gr, 256, smr, p->stream>>>(__VA_ARGS__); break; \
-            default: RSPT_CUDA_CHECK(cudaFuncSetAttribute(KERNEL<12, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smr)); KERNEL<12, 4><<<gr, 256, smr, p->stream>>>(__VA_ARGS__); break; \
-            }                                                                                                     \
-        } else {                                                                                                  \
-            switch (s.bps) {                                                                                      \
-            case 1: RSPT_CUDA_CHECK(cudaFuncSetAttribute(KERNEL<13, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smr)); KERNEL<13, 1><<<gr, 512, smr, p->stream>>>(__VA_ARGS__); break; \
-            case 2: RSPT_CUDA_CHECK(cudaFuncSetAttribute(KERNEL<13, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smr)); KERNEL<13, 2><<<gr, 512, smr, p->stream>>>(__VA_ARGS__); break; \
-            case 3: RSPT_CUDA_CHECK(cudaFuncSetAttribute(KERNEL<13, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smr)); KERNEL<13, 3><<<gr, 512, smr, p->stream>>>(__VA_ARGS__); break; \
-            default: RSPT_CUDA_CHECK(cudaFuncSetAttribute(KERNEL<13, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smr)); KERNEL<13, 4><<<gr, 512, smr, p->stream>>>(__VA_ARGS__); break; \
-            }                                                                                                     \
-        }                                                                                                         \
-    } while (0)
-
-// hadamard / dct: the word matrix in d_words (+ its per-channel sums in d_sums) -> planes + header
-inline int spectral_words_forward(rspt_gpu_packer* p, size_t F)
-{
-    const Shape& s = p->s;
-    const dim3 g2((unsigned)(F * s.ch));
-    if (s.kind == 2 /*RSPT_HADAMARD*/) {
-        const size_t sm = (size_t)s.ns * 4;
-        if (s.ns == 4096) {
-            k_fwht_fast_fwd<12><<<g2, 256, 0, p->stream>>>(p->d_words, p->d_sums, s, p->d_planes, p->d_headers);
-        } else if (s.ns == 8192) {
-            k_fwht_fast_fwd<13><<<g2, 512, 0, p->stream>>>(p->d_words, p->d_sums, s, p->d_planes, p->d_headers);
-        } else {
-            RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_fwht_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-            k_fwht_fwd<<<g2, 256, sm, p->stream>>>(p->d_words, p->d_sums, s, p->d_planes, p->d_headers);
-        }
-        p->launches += 1;
-    } else {
-        if (dct_use_direct(p)) {
-            const size_t sm = (size_t)s.ns * 4;
-            RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_dct_fwd_direct, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-            k_dct_fwd_direct<<<g2, 256, sm, p->stream>>>(p->d_words, p->d_sums, s, p->d_cos, p->d_headers);
-        } else {
-            if (s.ns >= 16) {
-                const size_t sm = (size_t)fpad_host((uint32_t)s.ns / 2) * 16;
-                RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_dct_fwd_half, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-                k_dct_fwd_half<<<g2, 256, sm, p->stream>>>(p->d_words, p->d_sums, s, p->d_twiddle, p->d_post, p->d_headers);
-            } else {
-                const size_t sm = (size_t)s.ns * 16;
-                k_dct_fwd_fast<<<g2, 256, sm, p->stream>>>(p->d_words, p->d_sums, s, p->d_twiddle, p->d_post, p->d_headers);
-            }
-        }
-        const uint32_t chunks = (s.N + 1023) / 1024;
-        k_words_stencil_planes<<<(unsigned)(F * chunks), 256, 0, p->stream>>>(p->d_words, s, chunks, p->d_planes);
-        p->launches += 2;
-    }
-    RSPT_CUDA_CHECK(cudaGetLastError());
-    return 0;
-}
-
-// hadamard / dct: samples -> planes + header
-inline int spectral_forward(rspt_gpu_packer* p, const uint8_t* d_src, size_t F)
-{
-    const Shape& s = p->s;
-    if (fwht_raw_ok(s, d_src)) {
-        FWHT_RAW_LAUNCH(k_fwht_raw_fwd, d_src, s, p->d_planes, p->d_headers);
-        p->launches += 1;
-        RSPT_CUDA_CHECK(cudaGetLastError());
-        return 0;
-    }
-    const uint32_t tiles = ((uint32_t)s.ns + kPiece - 1) / kPiece;
-    const size_t tile_smem = (size_t)kPiece * s.ch * s.bps + 48;
-    if (tile_smem > 200 * 1024) return fail_arg(p, "too many channels");
-    RSPT_CUDA_CHECK(cudaMemsetAsync(p->d_sums, 0, F * s.ch * sizeof(long long), p->stream));
-    const dim3 g1((unsigned)(F * tiles));
-    switch (s.bps) {
-    case 1: RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_raw_to_words<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_smem)); break;
-    case 2: RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_raw_to_words<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_smem)); break;
-    case 3: RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_raw_to_words<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_smem)); break;
-    default: RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_raw_to_words<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_smem)); break;
-    }
-    if (words_g4_ok(s, d_src)) {
-        const unsigned gb = (unsigned)(F * (s.ch >> 2) * (size_t)(s.ns >> 2) / 256);
-        SPECTRAL_BPS_SWITCH(k_raw_to_words_g4, <<<gb, 256, 0, p->stream>>>(d_src, s, p->d_words, p->d_sums));
-    } else {
-        SPECTRAL_BPS_SWITCH(k_raw_to_words, <<<g1, 256, tile_smem, p->stream>>>(d_src, s, tiles, p->d_words, p->d_sums));
-    }
-    p->launches += 1;
-    return spectral_words_forward(p, F);
-}
-
-// hadamard / dct from int32 [ch][ns] words: their low 8*bps bits into the word matrix, then the same word path.
-// The dct kernels transform d_words in place, so the caller's buffer is only read.
-inline int spectral_forward_i32(rspt_gpu_packer* p, const int32_t* d_src, size_t F)
-{
-    const Shape& s = p->s;
-    const uint32_t tiles = ((uint32_t)s.ns + 1023) / 1024;
-    RSPT_CUDA_CHECK(cudaMemsetAsync(p->d_sums, 0, F * s.ch * sizeof(long long), p->stream));
-    SPECTRAL_BPS_SWITCH(k_i32_to_words, <<<(unsigned)(F * s.ch * tiles), 256, 0, p->stream>>>(d_src, s, tiles, p->d_words, p->d_sums));
-    p->launches += 1;
-    return spectral_words_forward(p, F);
-}
-
-// planes (decoded) -> the samples as int32 words in `words`, hadamard / dct.  The dct kernels work in place on
-// the coefficient words, so for dct `words` is also their scratch.
-inline int spectral_inverse_words(rspt_gpu_packer* p, size_t F, int32_t* words)
-{
-    const Shape& s = p->s;
-    const dim3 gf((unsigned)F), g2((unsigned)(F * s.ch));
-    if (s.kind == 2) {
-        const size_t sm = (size_t)s.ns * 4;
-        if (s.ns == 4096) {
-            k_fwht_fast_inv<12><<<g2, 256, 0, p->stream>>>(p->d_planes, p->d_headers, p->d_dec_nb, s, words);
-        } else if (s.ns == 8192) {
-            k_fwht_fast_inv<13><<<g2, 512, 0, p->stream>>>(p->d_planes, p->d_headers, p->d_dec_nb, s, words);
-        } else {
-            RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_fwht_inv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-            k_fwht_inv<<<g2, 256, sm, p->stream>>>(p->d_planes, p->d_headers, p->d_dec_nb, s, words);
-        }
-        p->launches += 1;
-        RSPT_CUDA_CHECK(cudaGetLastError());
-        return 0;
-    }
-    // coefficient words (BPS unused for word output); the fast kernel walks a frame's 128-element
-    // pieces four at a time, so their number must be a multiple of 4
-    const uint32_t npf = ((uint32_t)s.ns / kInvPiece) * (uint32_t)s.ch;
-    const size_t smw = (size_t)2 * npf * 4;
-    if ((s.ns % (int)kInvPiece) == 0 && (npf & 3u) == 0 && smw <= 200 * 1024) {
-        RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_planes_to_samples_fast<4, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smw));
-        k_planes_to_samples_fast<4, true, true><<<gf, kInvThreads, smw, p->stream>>>(p->d_planes, s, p->d_dec_nb, 1, nullptr, words);
-    } else {
-        const uint32_t np = (((uint32_t)s.ns + kPiece - 1) / kPiece) * (uint32_t)s.ch;
-        const size_t sm_inv = (size_t)2 * np * 4 + (size_t)kPiece * s.ch * s.bps + 48;
-        RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_planes_to_samples<4, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_inv));
-        k_planes_to_samples<4, true, false><<<gf, 512, sm_inv, p->stream>>>(p->d_planes, s, p->d_dec_nb, nullptr, words);
-    }
-    if (dct_use_direct(p)) {
-        const size_t sm = (size_t)s.ns * 4;
-        RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_dct_inv_direct, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-        k_dct_inv_direct<<<g2, 256, sm, p->stream>>>(words, p->d_headers, s, p->d_cos);
-    } else {
-        if (s.ns >= 16) {
-            const size_t sm = (size_t)fpad_host((uint32_t)s.ns / 2) * 16;
-            RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_dct_inv_half, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-            k_dct_inv_half<<<g2, 256, sm, p->stream>>>(words, p->d_headers, s, p->d_twiddle, p->d_post);
-        } else {
-            const size_t sm = (size_t)s.ns * 16;
-            k_dct_inv_fast<<<g2, 256, sm, p->stream>>>(words, p->d_headers, s, p->d_twiddle, p->d_post);
-        }
-    }
-    p->launches += 2;
-    RSPT_CUDA_CHECK(cudaGetLastError());
-    return 0;
-}
-
-// planes (decoded) -> samples, all four packers
-inline int launch_inverse_transform(rspt_gpu_packer* p, uint8_t* d_dst, size_t F)
-{
-    const Shape& s = p->s;
-    const uint32_t ppc = ((uint32_t)s.ns + kPiece - 1) / kPiece, np = ppc * (uint32_t)s.ch;
-    const size_t tile_bytes = (size_t)kPiece * s.ch * s.bps + 48;
-    const size_t sm_inv = (size_t)2 * np * 4 + tile_bytes;
-    if (sm_inv > 200 * 1024 || tile_bytes > 200 * 1024) return fail_arg(p, "frame too large for the inverse kernel");
-    const dim3 gf((unsigned)F);
-    // fast path: 4-channel groups, 128-sample pieces, PRMT packing (transforms.cuh)
-    if ((s.kind == 0 || s.kind == 1) && (s.ch & 3) == 0 && (s.ns % (int)kInvPiece) == 0 && ((uintptr_t)d_dst & 15) == 0) {
-        const size_t row = (size_t)s.ch * s.bps;
-        const size_t npf = (size_t)((uint32_t)s.ns / kInvPiece) * s.ch;  // 128-element pieces per frame
-        uint32_t tpg = 8;  // sample tiles per output group, sized to keep 4 CTAs per SM
-        size_t smf = 0;
-        for (; tpg >= 1; tpg >>= 1) {
-            smf = 2 * npf * 4 + (size_t)tpg * 32 * (row + 1) * 4 + (size_t)tpg * 4;   // + one pad word per 32 quads
-            if (smf <= 54 * 1024) break;
-        }
-        if (tpg >= 1) {
-#define INVF_LAUNCH(B, SC)                                                                                            \
-    do {                                                                                                              \
-        RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_planes_to_samples_fast<B, SC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smf)); \
-        k_planes_to_samples_fast<B, SC><<<gf, kInvThreads, smf, p->stream>>>(p->d_planes, s, p->d_dec_nb, tpg, d_dst);        \
-    } while (0)
-            const bool sc = s.kind == 0;
-            switch (s.bps) {
-            case 1: if (sc) INVF_LAUNCH(1, true); else INVF_LAUNCH(1, false); break;
-            case 2: if (sc) INVF_LAUNCH(2, true); else INVF_LAUNCH(2, false); break;
-            case 3: if (sc) INVF_LAUNCH(3, true); else INVF_LAUNCH(3, false); break;
-            default: if (sc) INVF_LAUNCH(4, true); else INVF_LAUNCH(4, false); break;
-            }
-#undef INVF_LAUNCH
-            p->launches += 1;
-            RSPT_CUDA_CHECK(cudaGetLastError());
-            return 0;
-        }
-    }
-#define INV_LAUNCH(B, SC, RAW)                                                                                   \
-    do {                                                                                                         \
-        RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_planes_to_samples<B, SC, RAW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_inv)); \
-        k_planes_to_samples<B, SC, RAW><<<gf, 512, sm_inv, p->stream>>>(p->d_planes, s, p->d_dec_nb, d_dst, p->d_words);  \
-    } while (0)
-    if (s.kind == 0 /*xdelta_hzr*/) {
-        switch (s.bps) {
-        case 1: INV_LAUNCH(1, true, true); break;
-        case 2: INV_LAUNCH(2, true, true); break;
-        case 3: INV_LAUNCH(3, true, true); break;
-        default: INV_LAUNCH(4, true, true); break;
-        }
-        p->launches += 1;
-    } else if (s.kind == 1 /*hzr*/) {
-        switch (s.bps) {
-        case 1: INV_LAUNCH(1, false, true); break;
-        case 2: INV_LAUNCH(2, false, true); break;
-        case 3: INV_LAUNCH(3, false, true); break;
-        default: INV_LAUNCH(4, false, true); break;
-        }
-        p->launches += 1;
-    } else {
-        if (fwht_raw_ok(s, d_dst)) {
-            FWHT_RAW_LAUNCH(k_fwht_raw_inv, p->d_planes, p->d_headers, p->d_dec_nb, s, d_dst);
-            p->launches += 1;
-            RSPT_CUDA_CHECK(cudaGetLastError());
-            return 0;
-        }
-        const int rc = spectral_inverse_words(p, F, p->d_words);
-        if (rc) return rc;
-        const uint32_t tiles = ppc;
-        switch (s.bps) {
-        case 1: RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_words_to_raw<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_bytes)); break;
-        case 2: RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_words_to_raw<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_bytes)); break;
-        case 3: RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_words_to_raw<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_bytes)); break;
-        default: RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_words_to_raw<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_bytes)); break;
-        }
-        if (words_g4_ok(s, d_dst)) {
-            const unsigned gb = (unsigned)(F * (s.ch >> 2) * (size_t)(s.ns >> 2) / 256);
-            SPECTRAL_BPS_SWITCH(k_words_to_raw_g4, <<<gb, 256, 0, p->stream>>>(p->d_words, s, d_dst));
-        } else {
-            SPECTRAL_BPS_SWITCH(k_words_to_raw, <<<(unsigned)(F * tiles), 256, tile_bytes, p->stream>>>(p->d_words, s, tiles, d_dst));
-        }
-        p->launches += 1;
-    }
-#undef INV_LAUNCH
-    RSPT_CUDA_CHECK(cudaGetLastError());
-    return 0;
-}
-
-// planes (decoded) -> int32 [ch][ns] words, sign-extended from 8*bps bits (rspt_gpu_decompress_batch_i32).
-// d_dst only needs 4-byte alignment; 16 bytes let the fast sample kernel store it directly.
-inline int launch_inverse_transform_i32(rspt_gpu_packer* p, int32_t* d_dst, size_t F)
-{
-    const Shape& s = p->s;
-    if (s.kind == 2 || s.kind == 3) {
-        // hadamard's inverse kernels only write their output, so 4-byte samples go straight to the caller;
-        // dct transforms its coefficient words in place and keeps the handle's scratch
-        int32_t* words = (s.kind == 2 && s.bps == 4) ? d_dst : p->d_words;
-        const int rc = spectral_inverse_words(p, F, words);
-        if (rc) return rc;
-        if (words != d_dst) {
-            const size_t n = F * (size_t)s.N;
-            const unsigned grid = (unsigned)((n + 1023) / 1024);
-            SPECTRAL_BPS_SWITCH(k_words_sext, <<<grid, 256, 0, p->stream>>>(words, n, d_dst));
-            p->launches += 1;
-        }
-        RSPT_CUDA_CHECK(cudaGetLastError());
-        return 0;
-    }
-    const dim3 gf((unsigned)F);
-    const bool sc = s.kind == 0;
-    // the fast kernel walks a frame's 128-element pieces four at a time (their number must be a multiple of 4)
-    // and stores 128-bit words
-    const uint32_t npf = ((uint32_t)s.ns / kInvPiece) * (uint32_t)s.ch;
-    const size_t smw = (size_t)2 * npf * 4;
-    if ((s.ns % (int)kInvPiece) == 0 && (npf & 3u) == 0 && smw <= 200 * 1024 && ((uintptr_t)d_dst & 15) == 0) {
-#define INVW_LAUNCH(B, SC)                                                                                                  \
-    do {                                                                                                                    \
-        RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_planes_to_samples_fast<B, SC, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smw)); \
-        k_planes_to_samples_fast<B, SC, true><<<gf, kInvThreads, smw, p->stream>>>(p->d_planes, s, p->d_dec_nb, 1, nullptr, d_dst); \
-    } while (0)
-        switch (s.bps) {
-        case 1: if (sc) INVW_LAUNCH(1, true); else INVW_LAUNCH(1, false); break;
-        case 2: if (sc) INVW_LAUNCH(2, true); else INVW_LAUNCH(2, false); break;
-        case 3: if (sc) INVW_LAUNCH(3, true); else INVW_LAUNCH(3, false); break;
-        default: if (sc) INVW_LAUNCH(4, true); else INVW_LAUNCH(4, false); break;
-        }
-#undef INVW_LAUNCH
-    } else {
-        const uint32_t np = (((uint32_t)s.ns + kPiece - 1) / kPiece) * (uint32_t)s.ch;
-        const size_t sm = (size_t)2 * np * 4;
-#define INVG_LAUNCH(B, SC)                                                                                                  \
-    do {                                                                                                                    \
-        RSPT_CUDA_CHECK(cudaFuncSetAttribute(k_planes_to_samples<B, SC, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm)); \
-        k_planes_to_samples<B, SC, false><<<gf, 512, sm, p->stream>>>(p->d_planes, s, p->d_dec_nb, nullptr, d_dst);      \
-    } while (0)
-        switch (s.bps) {
-        case 1: if (sc) INVG_LAUNCH(1, true); else INVG_LAUNCH(1, false); break;
-        case 2: if (sc) INVG_LAUNCH(2, true); else INVG_LAUNCH(2, false); break;
-        case 3: if (sc) INVG_LAUNCH(3, true); else INVG_LAUNCH(3, false); break;
-        default: if (sc) INVG_LAUNCH(4, true); else INVG_LAUNCH(4, false); break;
-        }
-#undef INVG_LAUNCH
-    }
-    p->launches += 1;
-    RSPT_CUDA_CHECK(cudaGetLastError());
-    return 0;
 }
 
 }  // namespace rspt

@@ -2,7 +2,7 @@
 // asynchronous copy global -> shared per tile of raw samples, completion on an mbarrier, then de-interleave +
 // sign-extend (convert_native_to_i32, utils.cpp:123-191), the delta / offset / xor stencil (utils.cpp:193-230,
 // flat chain crossing channel rows) and the byte-plane split (signal_packer_base.cpp:40-68).
-// Compiled for ch in {4, 8, 12} (RSPT_TMA_SHAPES in rspt_gpu.cu); k_xdelta_planes_fast serves the other shapes.
+// Compiled for the RSPT_TMA_SHAPES below (bps 2..4, ch in {4, 8, 12}); k_xdelta_planes_fast serves the other shapes.
 #pragma once
 
 #include <type_traits>
@@ -57,6 +57,9 @@ __device__ __forceinline__ uint32_t unpack_at(const uint32_t* w)
 // About 9 instructions per sample against 25 in k_xdelta_planes_fast (whose staging loop, padded layout and 32-bit
 // shared-memory loads are gone).  Same bytes as k_xdelta_planes (tests: STREAM_CASES, test_transform_planes_bit_exact).
 // ------------------------------------------------------------------------------------------
+// (bps, ch) of the instantiations; sample_stages.cuh launches these, and only these, for eligible shapes
+#define RSPT_TMA_SHAPES(X) X(2, 4) X(2, 8) X(2, 12) X(3, 4) X(3, 8) X(3, 12) X(4, 4) X(4, 8) X(4, 12)
+
 template <int BPS, int CH, bool STENCIL>
 __global__ void __launch_bounds__(kTmaThreads, 4) k_xdelta_planes_tma(const uint8_t* __restrict__ src, Shape s, uint32_t tiles_per_frame,
                                                                         uint8_t* __restrict__ planes)
