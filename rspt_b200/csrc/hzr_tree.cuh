@@ -11,8 +11,8 @@
 //
 // Phases (all 32 lanes unless noted):
 //   A  load the 261 counts, classify (FILL?), compact the used symbols into sort keys
-//      count << 9 | (511 - symbol), sort ascending (register bitonic network for <= 32 symbols,
-//      shared-memory bitonic network otherwise)
+//      count << 9 | (511 - symbol), sort ascending in registers (one key per lane and
+//      shuffles for <= 32 symbols; otherwise K keys per lane over 32 * K >= L slots)
 //   B  lane 0: two-queue merge (sorted leaves / internal nodes in creation order).  Internal
 //      nodes win ties against leaves; inside a run of equal-weight internal nodes the most
 //      recently created one is taken first -- exactly MakeTree's tie-break.  Also counts the
@@ -28,11 +28,14 @@
 namespace rspt {
 
 constexpr int kTreeWarps = 2;  // trees per CTA (5.6 KB of shared memory each: 40 trees per SM)
+constexpr uint32_t kLeafSlots = 264;       // node[0, kLeafSlots): leaves by rank; internal node j is node[kLeafSlots + j]
+constexpr uint32_t kNodeInf = 0x7FFFFFFFu; // an internal slot not filled yet: heavier than any leaf
 
 struct TreeWarpSmem {
-    uint32_t key[264];         // sorted leaf keys
-    uint32_t icnt[260];        // B: internal node weight (| bit 31: next node has equal weight); C: node code
-    uint32_t child[260];       // child_a | child_b << 10 | leaves below << 20; ids < 512 are leaf ranks, 512 + j internal node j
+    // leaf r: its sort key (+inf from L on).  Internal node j, phase B: weight << 9 | leaves below;
+    // phase C: its code.  A node's id is its slot.
+    uint32_t node[kLeafSlots + 260];
+    uint32_t child[260];       // internal node j: child_a id | child_b id << 10
     uint32_t ninfo[260];       // C: depth | pre-order bit offset << 8
     uint32_t tree[kTreeWords];
     uint16_t front[2][264];    // C: breadth-first frontiers (internal node indices)
@@ -64,6 +67,61 @@ __device__ __forceinline__ const uint8_t* blk_ptr(const uint8_t* planes, const S
 // too few warps to hide the latency of the cooperative parts).  h = the block's 261 token counts (global or shared memory), n = block length.
 // tree_prepare and tree_assign are warp-cooperative; tree_merge is ONE thread's job.
 
+// Bitonic sort of key[0..L), L <= 32 * K, with K keys per lane in registers: slot lane * K + r,
+// slots from L on +inf.  The network is in its all-ascending form (the first step of every merge
+// pairs slot i with its mirror image i ^ (kk - 1)), so no compare depends on a direction: strides
+// below K are min/max pairs inside a lane, strides >= K one shuffle and one min-or-max per key.
+// Writes every slot below kLeafSlots back (+inf from L on).
+template <int K>
+__device__ __forceinline__ void warp_sort_regs(uint32_t* key, const uint32_t L)
+{
+    const uint32_t lane = lane_id();
+    uint32_t v[K];
+#pragma unroll
+    for (int r = 0; r < K; ++r) v[r] = lane * K + r < L ? key[lane * K + r] : 0xFFFFFFFFu;
+    auto cas = [&](int r, int q) {  // r < q
+        const uint32_t a = v[r], b = v[q];
+        v[r] = min(a, b);
+        v[q] = max(a, b);
+    };
+#pragma unroll
+    for (int kk = 2; kk <= 32 * K; kk <<= 1) {
+        if (kk <= K) {
+#pragma unroll
+            for (int r = 0; r < K; ++r)
+                if (!(r & (kk >> 1))) cas(r, r ^ (kk - 1));
+        } else {
+            // mirror step across lanes: lane ^ (kk / K - 1), key K - 1 - r
+            const bool lower = (lane & (kk / K / 2)) == 0;
+#pragma unroll
+            for (int r = 0; r < K / 2; ++r) {
+                const uint32_t o0 = __shfl_xor_sync(0xFFFFFFFFu, v[K - 1 - r], kk / K - 1);
+                const uint32_t o1 = __shfl_xor_sync(0xFFFFFFFFu, v[r], kk / K - 1);
+                v[r] = lower ? min(v[r], o0) : max(v[r], o0);
+                v[K - 1 - r] = lower ? min(v[K - 1 - r], o1) : max(v[K - 1 - r], o1);
+            }
+        }
+#pragma unroll
+        for (int j = kk >> 2; j > 0; j >>= 1) {
+            if (j >= K) {
+                const bool lower = (lane & (j / K)) == 0;
+#pragma unroll
+                for (int r = 0; r < K; ++r) {
+                    const uint32_t o = __shfl_xor_sync(0xFFFFFFFFu, v[r], j / K);
+                    v[r] = lower ? min(v[r], o) : max(v[r], o);
+                }
+            } else {
+#pragma unroll
+                for (int r = 0; r < K; ++r)
+                    if (!(r & j)) cas(r, r | j);
+            }
+        }
+    }
+#pragma unroll
+    for (int r = 0; r < K; ++r)
+        if (lane * K + r < kLeafSlots) key[lane * K + r] = v[r];
+}
+
 // Part 1: classify (FILL?), compact the used symbols into sort keys, sort.  Returns true when the
 // block is a FILL (bi is final then).  Unused symbols get code table entry 0.
 __device__ __forceinline__ bool tree_prepare(TreeWarpSmem& S, const uint32_t* h, uint32_t* codes_out, uint32_t& L_out, BlkInfo& bi)
@@ -79,7 +137,7 @@ __device__ __forceinline__ bool tree_prepare(TreeWarpSmem& S, const uint32_t* h,
         const bool used = c != 0;
         const uint32_t m = __ballot_sync(0xFFFFFFFFu, used);
         const uint32_t pos = L + __popc(m & ((1u << lane) - 1u));
-        if (used) S.key[pos] = (c << 9) | (511u - sym);
+        if (used) S.node[pos] = (c << 9) | (511u - sym);
         else if (sym < (uint32_t)kSymStride) codes_out[sym] = 0;  // 0 = symbol has no code
         L += __popc(m);
         if (r == 0) {
@@ -104,7 +162,7 @@ __device__ __forceinline__ bool tree_prepare(TreeWarpSmem& S, const uint32_t* h,
     __syncwarp();
     if (L <= 32) {
         // one key per lane, bitonic network over the warp
-        mykey = lane < L ? S.key[lane] : 0xFFFFFFFFu;
+        mykey = lane < L ? S.node[lane] : 0xFFFFFFFFu;
 #pragma unroll
         for (uint32_t kk = 2; kk <= 32; kk <<= 1)
 #pragma unroll
@@ -113,116 +171,72 @@ __device__ __forceinline__ bool tree_prepare(TreeWarpSmem& S, const uint32_t* h,
                 const bool up = (lane & kk) == 0, lower = (lane & j) == 0;
                 mykey = (lower == up) ? min(mykey, other) : max(mykey, other);
             }
-        S.key[lane] = mykey;
+        S.node[lane] = mykey;
+    } else if (L <= 64) {
+        warp_sort_regs<2>(S.node, L);
+    } else if (L <= 128) {
+        warp_sort_regs<4>(S.node, L);
+    } else if (L <= 256) {
+        warp_sort_regs<8>(S.node, L);
     } else {
-        // bitonic network in its all-ascending form (the first step of every merge mirrors the
-        // upper half), so the slots from L up to the next power of two are virtual +infinity
-        // and need no storage: a compare whose upper partner is >= L is a no-op
-        uint32_t P = 64;
-        while (P < L) P <<= 1;
-        for (uint32_t kk = 2; kk <= P; kk <<= 1) {
-            for (uint32_t j = kk >> 1; j > 0; j >>= 1) {
-                const bool mirror = j == (kk >> 1);
-                for (uint32_t idx = lane; idx < (P >> 1); idx += 32) {
-                    const uint32_t i = ((idx & ~(j - 1)) << 1) | (idx & (j - 1));
-                    const uint32_t ixj = mirror ? i ^ (kk - 1u) : i | j;
-                    if (ixj < L) {
-                        const uint32_t a = S.key[i], c2 = S.key[ixj];
-                        if (a > c2) {
-                            S.key[i] = c2;
-                            S.key[ixj] = a;
-                        }
-                    }
-                }
-                __syncwarp();
-            }
-        }
+        warp_sort_regs<16>(S.node, L);
     }
     for (uint32_t i = lane; i < kTreeWords; i += 32) S.tree[i] = 0;
+    for (uint32_t i = lane; i < 260; i += 32) S.node[kLeafSlots + i] = kNodeInf;
     __syncwarp();
 
     L_out = L;
     return false;
 }
 
-// Part 2 (one thread): two-queue merge.
-// Phase B: two-queue merge.  Registers hold both queue heads; an internal node's
-// weight word carries a flag "the node created right after me has the same weight", so the
-// common pick (a run of one) needs no look-ahead load.
+// Part 2 (one thread): two-queue merge.  Internal nodes are kept in pick order: weights never
+// decrease, and a run of equal weights goes latest first, so a node as heavy as the one before it
+// takes the first slot of that run and the run moves up one slot.  A run is complete before its
+// first node is taken (a node made later is heavier) and no node of it has a parent yet, so the
+// move renames nothing.  Registers hold both queue heads: the leaf head as lc = key | 511 for the
+// compare (an internal node of equal weight compares <= it: internal nodes win ties; its word is
+// lc - 510), the internal head as ic = its word.  Words are weight << 9 | leaves below, so a new node's
+// word is the sum of its children's.  A pick loads the next head of the queue it took from,
+// node[id + 1]: +inf past the last leaf and in internal slots not filled yet.
 __device__ __forceinline__ void tree_merge(TreeWarpSmem& S, const uint32_t L)
 {
-    constexpr uint32_t kInf = 0x7FFFFFFFu, kEqNext = 0x80000000u;
-    uint32_t li = 0, lc = S.key[0] >> 9;          // leaf queue head
-    uint32_t fr = 0, ni = 0, ic = kInf;           // internal queue: head index, count, head weight
-    uint32_t icf = 0;                             // head has an equal-weight successor (flag bit)
-    uint32_t last_w = kInf;
-    // one pick: the lighter head; ties go to the internal node.  Branch-free unless the
-    // internal head starts a run of equal weights (then the latest of the run goes first).
-    uint32_t top = 0, run_end = 0;
-    bool in_run = false;
-    auto pick = [&](uint32_t& id, uint32_t& wt, uint32_t& lv) {
-        const bool take_int = ic <= lc;
-        if (take_int && (in_run || icf)) {
-            uint32_t pk;
-            bool advance;
-            if (!in_run) {
-                top = fr + 1;
-                while (top < ni && (S.icnt[top] & kInf) == ic) ++top;
-                run_end = top;
-                in_run = true;
-                pk = --top;
-                advance = false;  // a flagged run has >= 2 nodes
-            } else {
-                pk = --top;
-                advance = top == fr;
-            }
-            id = 512u + pk;
-            wt = ic;
-            lv = S.child[pk] >> 20;
-            if (advance) {
-                in_run = false;
-                fr = run_end;
-                const uint32_t raw = fr < ni ? S.icnt[fr] : kInf;
-                ic = raw & kInf;
-                icf = raw & kEqNext;
-            }
-            return;
-        }
-        // heads after this pick, loaded unconditionally (indices stay inside the arrays)
-        const uint32_t nfr = fr + (take_int ? 1u : 0u), nli = li + (take_int ? 0u : 1u);
-        const uint32_t raw = S.icnt[nfr], nk = S.key[nli], ch = S.child[fr];
-        id = take_int ? 512u + fr : li;
-        wt = take_int ? ic : lc;
-        lv = take_int ? ch >> 20 : 1u;
-        if (take_int) {
-            ic = nfr < ni ? raw & kInf : kInf;
-            icf = nfr < ni ? raw & kEqNext : 0u;
-        } else {
-            lc = nli < L ? nk >> 9 : kInf;
-        }
-        fr = nfr;
-        li = nli;
+    uint32_t* node = S.node;
+    node[L] = 0xFFFFFFFFu;  // the slot after the last leaf (the sorts leave it unwritten when L = 32 * K)
+    uint32_t hl = 0, lc = node[0] | 511u;
+    uint32_t hi = kLeafSlots, ic = kNodeInf;
+    uint32_t last = 0, run = kLeafSlots;  // weight field of the newest node | 511; first slot of its run
+    auto pick = [&](uint32_t& id, uint32_t& v) {
+        const bool take = ic <= lc;
+        id = take ? hi : hl;
+        v = take ? ic : lc - 510u;  // a leaf's word: count << 9 | 1
+        const uint32_t raw = node[id + 1];
+        hi += take;
+        hl += !take;
+        if (take) ic = raw;
+        else lc = raw | 511u;
     };
-    for (uint32_t round = 0; round + 1 < L; ++round) {
-        uint32_t id0, id1, w0, w1, lv0, lv1;
-        pick(id0, w0, lv0);
-        pick(id1, w1, lv1);
-        const uint32_t w = w0 + w1;
-        if (w == last_w) {
-            S.icnt[ni - 1] = w | kEqNext;
-            if (ni - 1 == fr) icf = kEqNext;
+    for (uint32_t n = kLeafSlots; n < kLeafSlots + L - 1; ++n) {
+        uint32_t a, b, va, vb;
+        pick(a, va);
+        pick(b, vb);
+        const uint32_t w = va + vb, ch = a | (b << 10);
+        uint32_t at = n;
+        if (w <= last) {
+#pragma unroll 1
+            for (; at > run; --at) {
+                node[at] = node[at - 1];
+                S.child[at - kLeafSlots] = S.child[at - 1 - kLeafSlots];
+            }
+        } else {
+            run = n;
         }
-        if (fr == ni) {
-            ic = w;
-            icf = 0;
-        }
-        S.icnt[ni] = w;
-        S.child[ni] = id0 | (id1 << 10) | ((lv0 + lv1) << 20);
-        last_w = w;
-        ++ni;
+        node[at] = w;
+        S.child[at - kLeafSlots] = ch;
+        if (hi == at) ic = w;  // the new node is the internal head
+        last = w | 511u;
     }
     // root = last internal node: depth 0, code 0, pre-order offset 0
-    S.icnt[L - 2] = 0;
+    node[kLeafSlots + L - 2] = 0;
     S.ninfo[L - 2] = 0;
     S.front[0][0] = (uint16_t)(L - 2);
 }
@@ -238,7 +252,7 @@ __device__ __forceinline__ BlkInfo tree_assign(TreeWarpSmem& S, const uint32_t L
     uint32_t token_bits = 0, maxlen = 0, ntok = 0;
     {
         auto leaf = [&](uint32_t rank, uint32_t code, uint32_t depth, uint32_t off) {
-            const uint32_t kv = S.key[rank];
+            const uint32_t kv = S.node[rank];
             const uint32_t sym = 511u - (kv & 511u), cnt = kv >> 9;
             codes_out[sym] = code | (depth << 27);
             token_bits += cnt * (depth + sym_extra_bits(sym));
@@ -258,31 +272,32 @@ __device__ __forceinline__ BlkInfo tree_assign(TreeWarpSmem& S, const uint32_t L
                 uint32_t a = 0, bb = 0;
                 if (act) {
                     const uint32_t j = S.front[cur][i];
-                    const uint32_t ch = S.child[j], code = S.icnt[j], inf = S.ninfo[j];
+                    const uint32_t ch = S.child[j], code = S.node[kLeafSlots + j], inf = S.ninfo[j];
                     const uint32_t depth = inf & 255u, off = inf >> 8;
                     a = ch & 1023u;
-                    bb = (ch >> 10) & 1023u;
+                    bb = ch >> 10;
                     uint32_t bits_a = 10;
-                    if (a < 512u) {
+                    if (a < kLeafSlots) {
                         leaf(a, code, depth + 1u, off + 1u);
                     } else {
-                        bits_a = 11u * (S.child[a - 512u] >> 20) - 1u;
-                        S.icnt[a - 512u] = code;
-                        S.ninfo[a - 512u] = (depth + 1u) | ((off + 1u) << 8);
+                        // node[a] still holds the merge's word: leaves below it in the low 9 bits
+                        bits_a = 11u * (S.node[a] & 511u) - 1u;
+                        S.node[a] = code;
+                        S.ninfo[a - kLeafSlots] = (depth + 1u) | ((off + 1u) << 8);
                     }
                     const uint32_t code_b = code | (1u << depth), off_b = off + 1u + bits_a;
-                    if (bb < 512u) {
+                    if (bb < kLeafSlots) {
                         leaf(bb, code_b, depth + 1u, off_b);
                     } else {
-                        S.icnt[bb - 512u] = code_b;
-                        S.ninfo[bb - 512u] = (depth + 1u) | (off_b << 8);
+                        S.node[bb] = code_b;
+                        S.ninfo[bb - kLeafSlots] = (depth + 1u) | (off_b << 8);
                     }
                 }
-                const bool ia = act && a >= 512u, ib = act && bb >= 512u;
+                const bool ia = act && a >= kLeafSlots, ib = act && bb >= kLeafSlots;
                 const uint32_t ma = __ballot_sync(0xFFFFFFFFu, ia), mb = __ballot_sync(0xFFFFFFFFu, ib);
-                if (ia) S.front[cur ^ 1][nn + __popc(ma & lt)] = (uint16_t)(a - 512u);
+                if (ia) S.front[cur ^ 1][nn + __popc(ma & lt)] = (uint16_t)(a - kLeafSlots);
                 nn += __popc(ma);
-                if (ib) S.front[cur ^ 1][nn + __popc(mb & lt)] = (uint16_t)(bb - 512u);
+                if (ib) S.front[cur ^ 1][nn + __popc(mb & lt)] = (uint16_t)(bb - kLeafSlots);
                 nn += __popc(mb);
             }
             __syncwarp();
@@ -332,8 +347,9 @@ __device__ __forceinline__ void count_block_mode(Counters* ctr, uint32_t mode)
     atomicAdd(mode == MODE_FILL ? &ctr->blocks_fill : (mode == MODE_COPY ? &ctr->blocks_copy : &ctr->blocks_huff), 1ull);
 }
 
-// One warp per block of the class `cls` (blk_class is written by the histogram launches).
-__global__ void __launch_bounds__(kTreeWarps * 32) k_hzr_tree(const uint32_t* __restrict__ hist, Shape s,
+// One warp per block of the class `cls` (blk_class is written by the histogram launches).  20 CTAs per SM
+// keep 40 trees resident (as the shared memory allows), which caps the registers at 48.
+__global__ void __launch_bounds__(kTreeWarps * 32, 20) k_hzr_tree(const uint32_t* __restrict__ hist, Shape s,
                                                                const uint8_t* __restrict__ frame_nb,
                                                                const uint8_t* __restrict__ blk_class, uint32_t cls,
                                                                uint32_t total_blocks,
