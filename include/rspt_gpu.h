@@ -115,6 +115,34 @@ int rspt_gpu_compress_batch_i32(rspt_gpu_packer* p, const int32_t* d_src, size_t
 int rspt_gpu_decompress_batch_i32(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets, size_t n_frames,
                                   const uint8_t* d_frame_nb, const void* d_sidecar, int32_t* d_dst, int32_t* d_status);
 
+/* Decode any list of frames of a stored batch (seek in a recording, a random minibatch of a dataset kept
+ * compressed in HBM).  Output slot j receives stored frame d_frame_ids[j]: its bytes (words) equal row
+ * d_frame_ids[j] of what rspt_gpu_decompress_batch (_i32) writes for the whole stored batch.  Ids may come in
+ * any order and repeat.
+ *   d_src, d_offsets [n_stored + 1], d_frame_nb [n_stored], d_sidecar
+ *              the stored batch exactly as compress_batch produced it: d_offsets is the batch's full array, not
+ *              a slice; d_frame_nb is indexed by stored id (NULL = the handle's current plane count for every
+ *              frame); d_sidecar needs only its used prefix (rspt_gpu_sidecar_used_bytes(p, n_stored, ...)).
+ *              d_sidecar NULL: an index is built for the selected frames only, in scratch owned by the handle
+ *              (the cost follows n_frames, not n_stored).
+ *   d_frame_ids [n_frames] int64 stored ids, on the device.  An id < 0 or >= n_stored gives d_status[j] =
+ *              RSPT_E_ARG: nothing is read for it and the slot is written like a frame that fails to parse.
+ *   d_dst      [n_frames][frame_bytes] (_i32: [n_frames][ch][ns] words, aligned as for decompress_batch_i32)
+ *   d_status   [n_frames] per output slot, as for decompress_batch; may be NULL
+ * n_frames <= max_batch_frames, else RSPT_E_CAPACITY; n_stored is not limited by the handle, but a stored batch
+ * of more than 2^32 - 1 blocks (n_stored * planes * blocks per plane) is refused with RSPT_E_ARG, and a block
+ * whose index entries would lie at or beyond word 2^32 of the index fails its frame with RSPT_E_STREAM.  A
+ * malformed frame or a wrong index entry costs only the slots that name that frame.  Asynchronous on the
+ * handle's stream; counters (frames_decompressed += n_frames) and the PARSE / DECODE / INVERSE stage timers
+ * as for decompress_batch.  The decode index of a stored batch depends on the largest plane count of the
+ * handle that wrote it: it is valid for any handle of the same kind, shape and `nb` argument. */
+int rspt_gpu_decompress_frames(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets, size_t n_stored,
+                               const uint8_t* d_frame_nb, const void* d_sidecar, const int64_t* d_frame_ids,
+                               size_t n_frames, uint8_t* d_dst, int32_t* d_status);
+int rspt_gpu_decompress_frames_i32(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets, size_t n_stored,
+                                   const uint8_t* d_frame_nb, const void* d_sidecar, const int64_t* d_frame_ids,
+                                   size_t n_frames, int32_t* d_dst, int32_t* d_status);
+
 /* Integrity check without decoding: replaces hzr_verify (lib_hzr/hzr_decode.c:569-624) applied to
  * every hzr stream of `n_frames` frames -- frame / chunk / block headers are walked as in
  * decompress, and the CRC-32C of every block payload is compared with the block header.

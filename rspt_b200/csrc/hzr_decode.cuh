@@ -37,7 +37,7 @@ struct DecBlk {
     uint32_t payload_len;
     uint32_t out_n;
     uint32_t mode;
-    uint32_t pad;
+    uint32_t idx_slot;               // word of the block's first decode-index entry (k_frame_parse)
 };
 
 __device__ __forceinline__ uint32_t decode_class(const DecBlk& d)
@@ -51,10 +51,29 @@ __device__ __forceinline__ uint32_t ld_le32(const uint8_t* p)
     return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24);
 }
 
-// one thread per frame: method byte, header, nb chunks, block headers
+// Which stored frame every output slot decodes.  The batch calls decode stored frame f into slot f
+// (GATHER = false: ids, n_stored and slot_region are unused).  The gather calls read the stored id of
+// slot j from ids[j]; an id outside [0, n_stored) fails the slot with RSPT_E_ARG and reads nothing.
+// Decode-index addressing (common.cuh), decided here once per block:
+//   slot_region == 0  the stored batch's own index: word ((payload_off - offsets[0]) >> 6) + ordinal of the
+//                     block (stored frame, plane, block) in the stored batch
+//   slot_region != 0  an index built for this call only: slot j owns words [j * slot_region, (j + 1) * slot_region)
+//                     and addresses them as a one-frame batch ((payload_off - offsets[g]) >> 6) + ordinal in the
+//                     frame.  A frame that parses is at most rspt_gpu_max_compressed_size bytes long, so
+//                     (max_compressed_size >> 6) + nb_alloc * nblk + 1 words hold it.
+// A HUFF block whose entries would not fit below 2^32 fails its frame (RSPT_E_STREAM).
+struct FrameSel {
+    const int64_t* ids;
+    unsigned long long n_stored;
+    unsigned long long slot_region;
+};
+
+// one thread per output slot: method byte, header, nb chunks, block headers
+template <bool GATHER>
 __global__ void __launch_bounds__(128) k_frame_parse(const uint8_t* __restrict__ src, const uint64_t* __restrict__ offsets,
                                                       Shape s, const uint8_t* __restrict__ frame_nb_in,
                                                       const uint32_t* __restrict__ nb_state, uint32_t n_frames,
+                                                      FrameSel sel,
                                                       DecBlk* __restrict__ dec, uint8_t* __restrict__ headers,
                                                       uint8_t* __restrict__ dec_nb, int32_t* __restrict__ status,
                                                       Counters* __restrict__ ctr)
@@ -62,9 +81,21 @@ __global__ void __launch_bounds__(128) k_frame_parse(const uint8_t* __restrict__
     const uint32_t f = blockIdx.x * blockDim.x + threadIdx.x;
     if (f == 0) atomicAdd(&ctr->frames_decompressed, (unsigned long long)n_frames);
     if (f >= n_frames) return;
-    const unsigned long long base = offsets[f], end = offsets[f + 1];
-    uint32_t nb = frame_nb_in ? frame_nb_in[f] : *nb_state;
-    int err = 0;
+    unsigned long long g = f;  // stored frame
+    bool bad_id = false;
+    if (GATHER) {
+        const int64_t id = sel.ids[f];
+        bad_id = id < 0 || (unsigned long long)id >= sel.n_stored;
+        g = bad_id ? 0ull : (unsigned long long)id;
+    }
+    // a bad id reads nothing of the stored batch: its slot is written like a frame that fails to parse
+    const unsigned long long base = bad_id ? 0ull : offsets[g], end = bad_id ? 0ull : offsets[g + 1];
+    // index words of this frame's blocks: slot_org + ((payload_off - slot_off) >> 6) + ordinal
+    const bool local = GATHER && sel.slot_region != 0;
+    const unsigned long long slot_org = local ? f * sel.slot_region : 0ull, slot_off = (local || bad_id) ? base : offsets[0];
+    const unsigned long long ord0 = local ? 0ull : g * s.nb_alloc * s.nblk;
+    uint32_t nb = bad_id ? s.nb_init : frame_nb_in ? frame_nb_in[g] : *nb_state;
+    int err = bad_id;
     if (nb < 1 || nb > s.nb_alloc) {
         err = 1;
         nb = nb < 1 ? 1 : s.nb_alloc;
@@ -82,7 +113,7 @@ __global__ void __launch_bounds__(128) k_frame_parse(const uint8_t* __restrict__
     for (uint32_t k = 0; k < s.nb_alloc; ++k) {
         for (uint32_t b = 0; b < s.nblk; ++b) {
             DecBlk d;
-            d.payload_off = 0; d.payload_len = 0; d.out_n = blk_len(s, b); d.pad = 0;
+            d.payload_off = 0; d.payload_len = 0; d.out_n = blk_len(s, b); d.idx_slot = 0;
             d.mode = k < nb ? kModeZero : kModeInactive;
             row[k * s.nblk + b] = d;
         }
@@ -105,10 +136,13 @@ __global__ void __launch_bounds__(128) k_frame_parse(const uint8_t* __restrict__
             // largest legitimate payload.
             const uint32_t bl = blk_len(s, b);
             if ((mode == MODE_HUFF && plen > bl) || (mode == MODE_COPY && plen != bl) || (mode == MODE_FILL && plen != 1u)) { err = 1; break; }
+            const unsigned long long slot = slot_org + ((q + 7 - slot_off) >> 6) + ord0 + k * s.nblk + b;
+            if (mode == MODE_HUFF && slot + idx_geom(plen).n > 0xFFFFFFFFull) { err = 1; break; }
             DecBlk& d = row[k * s.nblk + b];
             d.payload_off = q + 7;
             d.payload_len = plen;
             d.mode = mode;
+            d.idx_slot = (uint32_t)slot;
             q += 7 + plen;
         }
         if (!err && q != cend) err = 1;
@@ -120,7 +154,7 @@ __global__ void __launch_bounds__(128) k_frame_parse(const uint8_t* __restrict__
             for (uint32_t b = 0; b < s.nblk; ++b) row[k * s.nblk + b].mode = kModeZero;
     }
     dec_nb[f] = (uint8_t)nb;
-    status[f] = err ? -4 : 0;
+    status[f] = bad_id ? -1 : (err ? -4 : 0);
 }
 
 // sequential bit reader over the payload staged in shared memory (word 0 = payload bytes 0..3),
@@ -293,7 +327,6 @@ __device__ __forceinline__ void chain_long_codes(const uint32_t* cw_tab, T* lut,
 // decode index (common.cuh) and writes the bytes they produce.
 __global__ void __launch_bounds__(kDecodeThreads, 3) k_hzr_decode(const uint8_t* __restrict__ src, Shape s,
                                                                    const DecBlk* __restrict__ dec,
-                                                                   const uint64_t* __restrict__ offsets,
                                                                    const uint32_t* __restrict__ sidecar,
                                                                    const uint32_t* __restrict__ codes,
                                                                    uint8_t* __restrict__ planes, int32_t* __restrict__ status,
@@ -409,7 +442,7 @@ __global__ void __launch_bounds__(kDecodeThreads, 3) k_hzr_decode(const uint8_t*
 
     const IdxGeom ig = idx_geom(plen);
     const uint32_t limit = plen * 8u, nint = ig.n;
-    const uint32_t* my_idx = sidecar + idx_slot_base(d.payload_off - offsets[0], blk);
+    const uint32_t* my_idx = sidecar + d.idx_slot;
     uint32_t my_err = 0;
     if (tid < nint) {
         const uint32_t e0 = my_idx[tid];
@@ -605,7 +638,6 @@ struct TokenDecoder {
 
 __global__ void __launch_bounds__(kIndexThreads, 2) k_hzr_build_index(const uint8_t* __restrict__ src, Shape s,
                                                                        const DecBlk* __restrict__ dec,
-                                                                       const uint64_t* __restrict__ offsets,
                                                                        const uint32_t* __restrict__ codes,
                                                                        uint32_t* __restrict__ sidecar,
                                                                        int32_t* __restrict__ status)
@@ -625,7 +657,7 @@ __global__ void __launch_bounds__(kIndexThreads, 2) k_hzr_build_index(const uint
     uint32_t f, k, b;
     blk_decode(s, blk, f, k, b);
     const uint32_t n = d.out_n;
-    uint32_t* my_idx = sidecar + idx_slot_base(d.payload_off - offsets[0], blk);
+    uint32_t* my_idx = sidecar + d.idx_slot;
     const uint8_t* pay = src + d.payload_off;
     const uintptr_t pa = (uintptr_t)pay;
     const uint32_t* aw = reinterpret_cast<const uint32_t*>(pa & ~(uintptr_t)3);

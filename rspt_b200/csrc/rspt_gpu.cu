@@ -281,7 +281,9 @@ extern "C" int rspt_gpu_create(int kind, size_t bps, size_t ch, size_t ns, size_
     A(dalloc(p->d_status_tmp, F));
     A(dalloc(p->d_dec_nb, F));
     A(cudaMalloc(&p->d_dec, nblocks * sizeof(DecBlk) + 64));
-    A(cudaMalloc(&p->d_auto_index, ((F * (1 + s.hdr_bytes + (size_t)s.nb_alloc * (4 + hzr_max(s.N))) >> 6) + nblocks + 2) * sizeof(uint32_t) + 64));
+    // the batch addressing needs ((F * max_compressed_size) >> 6) + nblocks + 2 words, a gather call's per-slot
+    // regions (gather_slot_region) F * ((max_compressed_size >> 6) + nb_alloc * nblk + 1): F more cover both
+    A(cudaMalloc(&p->d_auto_index, ((F * (1 + s.hdr_bytes + (size_t)s.nb_alloc * (4 + hzr_max(s.N))) >> 6) + nblocks + F + 2) * sizeof(uint32_t) + 64));
     if (kind == RSPT_HADAMARD || kind == RSPT_DCT) {
         A(dalloc(p->d_words, F * (size_t)s.N));
         A(dalloc(p->d_sums, F * (size_t)s.ch));
@@ -566,29 +568,42 @@ extern "C" int rspt_gpu_compress_batch_i32(rspt_gpu_packer* p, const int32_t* d_
 // ---------------------------------------------------------------------------------------------
 namespace {
 
-// frame / block header walk + (for streams without a decode index) the index itself
+// frame / block header walk + (for streams without a decode index) the index itself.  sel.ids = NULL: slot f
+// decodes stored frame f (the batch calls); else slot j decodes stored frame sel.ids[j] (k_frame_parse).
 int launch_parse_and_index(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets, size_t F,
-                           const uint8_t* d_frame_nb, void* d_sidecar_out, int32_t* status)
+                           const uint8_t* d_frame_nb, void* d_sidecar_out, int32_t* status, FrameSel sel)
 {
     const Shape& s = p->s;
     const uint32_t nblocks = total_blocks(p, F);
     DecBlk* dec = reinterpret_cast<DecBlk*>(p->d_dec);
     {
         StageTimer t(p, RSPT_STAGE_PARSE);
-        k_frame_parse<<<(unsigned)((F + 127) / 128), 128, 0, p->stream>>>(d_src, d_offsets, s, d_frame_nb, p->d_nb_state,
-                                                                          (uint32_t)F, dec, p->d_headers, p->d_dec_nb, status, p->d_ctr);
+        const unsigned pgrid = (unsigned)((F + 127) / 128);
+        if (sel.ids)
+            k_frame_parse<true><<<pgrid, 128, 0, p->stream>>>(d_src, d_offsets, s, d_frame_nb, p->d_nb_state, (uint32_t)F, sel,
+                                                              dec, p->d_headers, p->d_dec_nb, status, p->d_ctr);
+        else
+            k_frame_parse<false><<<pgrid, 128, 0, p->stream>>>(d_src, d_offsets, s, d_frame_nb, p->d_nb_state, (uint32_t)F, sel,
+                                                               dec, p->d_headers, p->d_dec_nb, status, p->d_ctr);
         // code tables of the HUFF blocks from their in-stream trees (unused symbols stay 0)
         RSPT_CUDA_CHECK(cudaMemsetAsync(p->d_codes, 0, (size_t)nblocks * kSymStride * sizeof(uint32_t), p->stream));
         k_hzr_recover_codes<<<(nblocks + kRecoverThreads - 1) / kRecoverThreads, kRecoverThreads, 0, p->stream>>>(d_src, nblocks, dec, p->d_codes, s, status);
         p->launches += 2;
         if (d_sidecar_out) {
-            k_hzr_build_index<<<nblocks, kIndexThreads, p->dec_smem, p->stream>>>(d_src, s, dec, d_offsets, p->d_codes,
+            k_hzr_build_index<<<nblocks, kIndexThreads, p->dec_smem, p->stream>>>(d_src, s, dec, p->d_codes,
                                                                                   reinterpret_cast<uint32_t*>(d_sidecar_out), status);
             p->launches += 1;
         }
     }
     RSPT_CUDA_CHECK(cudaGetLastError());
     return RSPT_OK;
+}
+
+// words of the handle's decode-index scratch that one output slot of a gather call owns when the call builds its
+// own index (k_frame_parse: FrameSel::slot_region)
+size_t gather_slot_region(const rspt_gpu_packer* p)
+{
+    return (rspt_gpu_max_compressed_size(p) >> 6) + (size_t)p->s.nb_alloc * p->s.nblk + 1;
 }
 
 }  // namespace
@@ -600,7 +615,8 @@ extern "C" int rspt_gpu_build_index(rspt_gpu_packer* p, const uint8_t* d_src, co
     if (n_frames == 0) return RSPT_OK;
     if (n_frames > p->max_batch) return fail_arg(p, "n_frames exceeds max_batch_frames"), RSPT_E_CAPACITY;
     DeviceGuard dg(p->device);
-    return launch_parse_and_index(p, d_src, d_offsets, n_frames, d_frame_nb, d_sidecar, d_status ? d_status : p->d_status_tmp);
+    return launch_parse_and_index(p, d_src, d_offsets, n_frames, d_frame_nb, d_sidecar, d_status ? d_status : p->d_status_tmp,
+                                  FrameSel{nullptr, 0, 0});
 }
 
 // payload bits per output byte up to which k_hzr_decode uses its two-literals-per-look-up table (measured)
@@ -614,13 +630,19 @@ struct SamplesOut {
     int32_t* words;
 };
 
+// Slot f of the output decodes stored frame f (ids = NULL: the batch calls) or stored frame ids[f] of the
+// n_stored frames that d_offsets / d_frame_nb / d_sidecar describe (the gather calls).
 int decompress_batch(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets, size_t n_frames,
-                     const uint8_t* d_frame_nb, const void* d_sidecar, SamplesOut out, int32_t* d_status)
+                     const uint8_t* d_frame_nb, const void* d_sidecar, SamplesOut out, int32_t* d_status,
+                     const int64_t* ids = nullptr, size_t n_stored = 0)
 {
     if (n_frames == 0) return RSPT_OK;
     if (n_frames > p->max_batch) return fail_arg(p, "n_frames exceeds max_batch_frames"), RSPT_E_CAPACITY;
-    DeviceGuard dg(p->device);
     const Shape& s = p->s;
+    // the parse keeps the ordinal of a stored block in 32 bits
+    if (ids && n_stored > 0xFFFFFFFFull / ((uint64_t)s.nb_alloc * s.nblk))
+        return fail_arg(p, "n_stored: the stored batch has more blocks than 32-bit ordinals can number"), RSPT_E_ARG;
+    DeviceGuard dg(p->device);
     const size_t F = n_frames;
     const uint32_t nblocks = total_blocks(p, F);
     int32_t* status = d_status ? d_status : p->d_status_tmp;
@@ -629,11 +651,13 @@ int decompress_batch(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d
     // as the reference's decompress does (signal_packer_xdelta_hzr.cpp:77).
     void* own_index = nullptr;
     if (!d_sidecar) {
-        // stream from the CPU reference: build the decode index here first (handle-owned scratch)
+        // stream from the CPU reference: build the decode index here first (handle-owned scratch); a gather call
+        // indexes the selected frames only, each in a region of its own
         own_index = p->d_auto_index;
         d_sidecar = own_index;
     }
-    int rc = launch_parse_and_index(p, d_src, d_offsets, F, d_frame_nb, own_index, status);
+    const FrameSel sel{ids, n_stored, (ids && own_index) ? gather_slot_region(p) : 0};
+    int rc = launch_parse_and_index(p, d_src, d_offsets, F, d_frame_nb, own_index, status, sel);
     if (rc) return rc;
     const uint32_t* sc = reinterpret_cast<const uint32_t*>(d_sidecar);
     const uint32_t maxn = s.N < kBlock ? s.N : kBlock;
@@ -645,14 +669,14 @@ int decompress_batch(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d
         cudaEventRecord(p->ev_fork, p->stream);
         cudaStreamWaitEvent(p->side, p->ev_fork, 0);
         k_hzr_decode<<<nblocks, decode_class_threads(kSmallPayload), decode_class_smem(kSmallPayload), p->side>>>(
-            d_src, s, dec, d_offsets, sc, p->d_codes, p->d_planes, status, flags, 1u);
+            d_src, s, dec, sc, p->d_codes, p->d_planes, status, flags, 1u);
         if (maxn > kSmallPayload) {
             k_hzr_decode<<<nblocks, decode_class_threads(kMediumPayload), decode_class_smem(kMediumPayload), p->side>>>(
-                d_src, s, dec, d_offsets, sc, p->d_codes, p->d_planes, status, flags, 2u);
+                d_src, s, dec, sc, p->d_codes, p->d_planes, status, flags, 2u);
             p->launches += 1;
         }
         cudaEventRecord(p->ev_join, p->side);
-        k_hzr_decode<<<nblocks, kDecodeThreads, p->dec_smem, p->stream>>>(d_src, s, dec, d_offsets, sc, p->d_codes, p->d_planes, status, flags, 0u);
+        k_hzr_decode<<<nblocks, kDecodeThreads, p->dec_smem, p->stream>>>(d_src, s, dec, sc, p->d_codes, p->d_planes, status, flags, 0u);
         cudaStreamWaitEvent(p->stream, p->ev_join, 0);
         p->launches += 2;
     }
@@ -679,6 +703,24 @@ extern "C" int rspt_gpu_decompress_batch_i32(rspt_gpu_packer* p, const uint8_t* 
     return decompress_batch(p, d_src, d_offsets, n_frames, d_frame_nb, d_sidecar, SamplesOut{nullptr, d_dst}, d_status);
 }
 
+extern "C" int rspt_gpu_decompress_frames(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets, size_t n_stored,
+                                          const uint8_t* d_frame_nb, const void* d_sidecar, const int64_t* d_frame_ids,
+                                          size_t n_frames, uint8_t* d_dst, int32_t* d_status)
+{
+    if (!p || !d_src || !d_offsets || !d_frame_ids || !d_dst) return RSPT_E_ARG;
+    return decompress_batch(p, d_src, d_offsets, n_frames, d_frame_nb, d_sidecar, SamplesOut{d_dst, nullptr}, d_status,
+                            d_frame_ids, n_stored);
+}
+
+extern "C" int rspt_gpu_decompress_frames_i32(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets, size_t n_stored,
+                                              const uint8_t* d_frame_nb, const void* d_sidecar, const int64_t* d_frame_ids,
+                                              size_t n_frames, int32_t* d_dst, int32_t* d_status)
+{
+    if (!p || !d_src || !d_offsets || !d_frame_ids || !d_dst || ((uintptr_t)d_dst & 3)) return RSPT_E_ARG;
+    return decompress_batch(p, d_src, d_offsets, n_frames, d_frame_nb, d_sidecar, SamplesOut{nullptr, d_dst}, d_status,
+                            d_frame_ids, n_stored);
+}
+
 extern "C" int rspt_gpu_verify_batch(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets, size_t n_frames,
                                      const uint8_t* d_frame_nb, int32_t* d_status)
 {
@@ -690,8 +732,9 @@ extern "C" int rspt_gpu_verify_batch(rspt_gpu_packer* p, const uint8_t* d_src, c
     const size_t F = n_frames;
     const uint32_t nblocks = total_blocks(p, F);
     DecBlk* dec = reinterpret_cast<DecBlk*>(p->d_dec);
-    k_frame_parse<<<(unsigned)((F + 127) / 128), 128, 0, p->stream>>>(d_src, d_offsets, s, d_frame_nb, p->d_nb_state, (uint32_t)F, dec,
-                                                                      p->d_headers, p->d_dec_nb, d_status, p->d_ctr);
+    k_frame_parse<false><<<(unsigned)((F + 127) / 128), 128, 0, p->stream>>>(d_src, d_offsets, s, d_frame_nb, p->d_nb_state, (uint32_t)F,
+                                                                             FrameSel{nullptr, 0, 0}, dec, p->d_headers, p->d_dec_nb,
+                                                                             d_status, p->d_ctr);
     k_hzr_verify<<<nblocks, kVerifyThreads, p->dec_smem, p->stream>>>(d_src, s, dec, p->d_crc, d_status, p->d_ctr);
     p->launches += 2;
     RSPT_CUDA_CHECK(cudaGetLastError());

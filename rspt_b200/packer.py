@@ -230,14 +230,48 @@ class SignalPacker:
         return self._decompress(self.L.rspt_gpu_decompress_batch_i32, batch, out, status, use_sidecar)
 
     def _decompress(self, fn, batch: CompressedBatch, out: torch.Tensor, status: torch.Tensor | None,
-                    use_sidecar: bool) -> torch.Tensor:
+                    use_sidecar: bool, ids: torch.Tensor | None = None) -> torch.Tensor:
+        """The whole batch, or (ids given: the gather calls) its frames ids[0], ids[1], ..."""
         sc = batch.sidecar.data_ptr() if (use_sidecar and batch.sidecar is not None) else None
         nbp = batch.frame_nb.data_ptr() if batch.frame_nb is not None else None
+        sel = () if ids is None else (ids.data_ptr(), ids.numel())
         self._bind_stream()
-        rc = fn(self.h, batch.stream.data_ptr(), batch.offsets.data_ptr(), batch.n_frames, nbp, sc,
+        rc = fn(self.h, batch.stream.data_ptr(), batch.offsets.data_ptr(), batch.n_frames, nbp, sc, *sel,
                 out.data_ptr(), status.data_ptr() if status is not None else None)
         check(rc, self.h, fn.__name__)
         return out
+
+    def decompress_frames(self, batch: CompressedBatch, frame_ids, out: torch.Tensor | None = None,
+                          status: torch.Tensor | None = None, use_sidecar: bool = True) -> torch.Tensor:
+        """Stored frames frame_ids[0], frame_ids[1], ... of `batch` (any order, repeats allowed) as native uint8
+        [n * frame_bytes]: row j equals row frame_ids[j] of decompress_batch(batch).  frame_ids: an int64 CUDA
+        tensor on the handle's device, or a sequence / range of ints (copied to one).  An id outside
+        [0, batch.n_frames) gives status -1 in its slot.  The handle's max_batch_frames bounds len(frame_ids),
+        not batch.n_frames.  Asynchronous on torch's current stream."""
+        ids = self._frame_ids(frame_ids)
+        if out is None:
+            out = torch.empty(ids.numel() * self.frame_bytes, dtype=torch.uint8, device=self._dev())
+        if not (out.is_cuda and out.dtype == torch.uint8 and out.is_contiguous() and out.numel() >= ids.numel() * self.frame_bytes):
+            raise ValueError(f"out must be a contiguous uint8 CUDA tensor of at least {ids.numel() * self.frame_bytes} bytes")
+        return self._decompress(self.L.rspt_gpu_decompress_frames, batch, out, status, use_sidecar, ids)
+
+    def decompress_frames_tensor(self, batch: CompressedBatch, frame_ids, out: torch.Tensor | None = None,
+                                 status: torch.Tensor | None = None, use_sidecar: bool = True) -> torch.Tensor:
+        """decompress_frames with the samples as an int32 tensor [n, ch, ns], as decompress_tensor writes them."""
+        ids = self._frame_ids(frame_ids)
+        n = ids.numel()
+        if out is None:
+            out = torch.empty((n, self.ch, self.ns), dtype=torch.int32, device=self._dev())
+        self._check_words(out, n)
+        return self._decompress(self.L.rspt_gpu_decompress_frames_i32, batch, out, status, use_sidecar, ids)
+
+    def _frame_ids(self, frame_ids) -> torch.Tensor:
+        if isinstance(frame_ids, (list, tuple, range)):
+            return torch.tensor(list(frame_ids), dtype=torch.int64, device=self._dev())
+        if not (isinstance(frame_ids, torch.Tensor) and frame_ids.dtype == torch.int64 and frame_ids.is_cuda
+                and frame_ids.device.index == self.device and frame_ids.dim() == 1 and frame_ids.is_contiguous()):
+            raise ValueError(f"frame_ids must be a contiguous 1-D torch.int64 tensor on cuda:{self.device}, or a sequence of ints")
+        return frame_ids
 
     def prefilter_iir(self, frames: torch.Tensor, n, d, init_nr_samples: int) -> torch.Tensor:
         """In place on device frames: the IIR pre-filter step of rspt_test.cpp:116-136 (i_filter::new_iir)."""
