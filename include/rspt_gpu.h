@@ -115,6 +115,37 @@ int rspt_gpu_compress_batch_i32(rspt_gpu_packer* p, const int32_t* d_src, size_t
 int rspt_gpu_decompress_batch_i32(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets, size_t n_frames,
                                   const uint8_t* d_frame_nb, const void* d_sidecar, int32_t* d_dst, int32_t* d_status);
 
+/* Compress n_frames frames and append them to a stored batch (a "store") of n_stored frames / stored_bytes stream
+ * bytes, so that a store can grow far beyond max_batch_frames.  Writes frames n_stored .. n_stored + n_frames - 1
+ * of the store and nothing else of it:
+ *   d_store          the stream from byte stored_bytes on (store_capacity bytes in all)
+ *   d_store_offsets  entries n_stored .. n_stored + n_frames; entry n_stored is (re)written as stored_bytes
+ *   d_store_frame_nb entries n_stored .. n_stored + n_frames - 1 (may be NULL)
+ *   d_store_sidecar  the decode-index entries of the new blocks at their places in the store's index (may be NULL;
+ *                    sidecar_capacity bytes in all)
+ * stored_bytes must equal d_store_offsets[n_stored] as the previous append left it (0 for an empty store); it is
+ * passed from the host so that capacities are checked without a read-back and the call stays asynchronous on the
+ * handle's stream.  Appending B1 .. Bk on one handle writes, byte for byte, the stream [0, total), offsets,
+ * frame_nb and used sidecar prefix that one rspt_gpu_compress_batch over all their frames writes on a fresh handle
+ * of the same arguments: the xdelta_hzr plane count carries across appends as across batches.  Counters add
+ * n_frames and this call's bytes; stage timers as for compress_batch.  Refused before anything is launched:
+ *   n_frames > max_batch_frames                                                    RSPT_E_CAPACITY
+ *   (n_stored + n_frames) * planes * blocks per plane >= 2^32 (block ordinals)     RSPT_E_ARG
+ *   stored_bytes + n_frames * rspt_gpu_max_compressed_size > store_capacity        RSPT_E_CAPACITY
+ *   a sidecar whose index words could reach 2^32 (the limit of the decode calls)   RSPT_E_ARG
+ *   a sidecar with sidecar_capacity < rspt_gpu_sidecar_used_bytes(p, n_stored + n_frames,
+ *                         stored_bytes + n_frames * rspt_gpu_max_compressed_size)  RSPT_E_CAPACITY
+ * rspt_gpu_compress_batch is this call with n_stored = stored_bytes = 0.  _i32: d_src is int32 [n][ch][ns] as for
+ * rspt_gpu_compress_batch_i32 (4-byte aligned, else RSPT_E_ARG); both may be mixed on one store. */
+int rspt_gpu_compress_append(rspt_gpu_packer* p, const uint8_t* d_src, size_t n_frames,
+                             uint8_t* d_store, size_t store_capacity, uint64_t* d_store_offsets,
+                             size_t n_stored, size_t stored_bytes, uint8_t* d_store_frame_nb,
+                             void* d_store_sidecar, size_t sidecar_capacity);
+int rspt_gpu_compress_append_i32(rspt_gpu_packer* p, const int32_t* d_src, size_t n_frames,
+                                 uint8_t* d_store, size_t store_capacity, uint64_t* d_store_offsets,
+                                 size_t n_stored, size_t stored_bytes, uint8_t* d_store_frame_nb,
+                                 void* d_store_sidecar, size_t sidecar_capacity);
+
 /* Decode any list of frames of a stored batch (seek in a recording, a random minibatch of a dataset kept
  * compressed in HBM).  Output slot j receives stored frame d_frame_ids[j]: its bytes (words) equal row
  * d_frame_ids[j] of what rspt_gpu_decompress_batch (_i32) writes for the whole stored batch.  Ids may come in
@@ -174,6 +205,18 @@ size_t rspt_gpu_sidecar_used_bytes(const rspt_gpu_packer* p, size_t n_frames, si
  * next to the stream: build once, decode many times.  d_sidecar: rspt_gpu_sidecar_bytes bytes. */
 int rspt_gpu_build_index(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets,
                          size_t n_frames, const uint8_t* d_frame_nb, void* d_sidecar, int32_t* d_status);
+
+/* rspt_gpu_build_index for the listed frames d_frame_ids[0 .. n_frames) of a stored batch of n_stored frames
+ * (d_offsets [n_stored + 1], d_frame_nb [n_stored] or NULL, as for rspt_gpu_decompress_frames): their entries are
+ * written into the stored batch's own index d_sidecar, at the words a whole-batch build_index would write, so a
+ * store of any length is indexed in pieces of at most max_batch_frames frames.  n_frames > max_batch_frames gives
+ * RSPT_E_CAPACITY; n_stored is not limited by the handle (but by 32-bit block ordinals, RSPT_E_ARG).  Per slot,
+ * d_status[j] (may be NULL): RSPT_E_ARG for an id outside [0, n_stored), RSPT_E_STREAM for a malformed frame or
+ * one whose entries would lie at or beyond byte sidecar_capacity of d_sidecar; such a slot writes nothing.
+ * Asynchronous on the handle's stream. */
+int rspt_gpu_build_index_frames(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets, size_t n_stored,
+                                const uint8_t* d_frame_nb, const int64_t* d_frame_ids, size_t n_frames,
+                                void* d_sidecar, size_t sidecar_capacity, int32_t* d_status);
 
 /* Single-frame convenience with HOST buffers -- the exact shape of the reference calls
  * (signal_packer.h:44,57): stages host<->device, runs the batch path with n_frames = 1 and

@@ -9,7 +9,7 @@ from ._lib import KINDS, RsptError  # noqa: F401
 def __getattr__(name):
     # torch is imported lazily so that `import rspt_b200` (and the symbol-export test) works
     # in processes that never touch the GPU
-    if name in ("SignalPacker", "CompressedBatch", "crc32c", "synth_ecg", "prdn"):
+    if name in ("SignalPacker", "CompressedBatch", "CompressedStore", "crc32c", "synth_ecg", "prdn"):
         from . import packer
         return getattr(packer, name)
     if name in ("shard_range", "allgather_totals", "place_offsets"):

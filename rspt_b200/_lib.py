@@ -18,6 +18,7 @@ EXPORTS = [
     "rspt_gpu_create", "rspt_gpu_destroy", "rspt_gpu_frame_bytes", "rspt_gpu_header_bytes",
     "rspt_gpu_max_compressed_size", "rspt_gpu_nb", "rspt_gpu_compress_batch", "rspt_gpu_decompress_batch",
     "rspt_gpu_compress_batch_i32", "rspt_gpu_decompress_batch_i32",
+    "rspt_gpu_compress_append", "rspt_gpu_compress_append_i32", "rspt_gpu_build_index_frames",
     "rspt_gpu_decompress_frames", "rspt_gpu_decompress_frames_i32",
     "rspt_gpu_sidecar_bytes", "rspt_gpu_sidecar_used_bytes", "rspt_gpu_compress_host", "rspt_gpu_decompress_host",
     "rspt_gpu_compress_batch_host", "rspt_gpu_decompress_batch_host", "rspt_gpu_sync", "rspt_gpu_last_error",
@@ -74,6 +75,11 @@ def lib() -> C.CDLL:
     L.rspt_gpu_compress_batch_i32.argtypes = [vp, vp, sz, vp, sz, vp, vp, vp]
     L.rspt_gpu_decompress_batch_i32.restype = C.c_int
     L.rspt_gpu_decompress_batch_i32.argtypes = [vp, vp, vp, sz, vp, vp, vp, vp]
+    for name in ("rspt_gpu_compress_append", "rspt_gpu_compress_append_i32"):
+        getattr(L, name).restype = C.c_int
+        getattr(L, name).argtypes = [vp, vp, sz, vp, sz, vp, sz, sz, vp, vp, sz]
+    L.rspt_gpu_build_index_frames.restype = C.c_int
+    L.rspt_gpu_build_index_frames.argtypes = [vp, vp, vp, sz, vp, vp, sz, vp, sz, vp]
     for name in ("rspt_gpu_decompress_frames", "rspt_gpu_decompress_frames_i32"):
         getattr(L, name).restype = C.c_int
         getattr(L, name).argtypes = [vp, vp, vp, sz, vp, vp, vp, sz, vp, vp]

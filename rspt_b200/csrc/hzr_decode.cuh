@@ -61,12 +61,16 @@ __device__ __forceinline__ uint32_t ld_le32(const uint8_t* p)
 //                     and addresses them as a one-frame batch ((payload_off - offsets[g]) >> 6) + ordinal in the
 //                     frame.  A frame that parses is at most rspt_gpu_max_compressed_size bytes long, so
 //                     (max_compressed_size >> 6) + nb_alloc * nblk + 1 words hold it.
-// A HUFF block whose entries would not fit below 2^32 fails its frame (RSPT_E_STREAM).
+// A HUFF block whose entries would not all lie below word idx_limit (GATHER = false: below 2^32 - 1) fails its frame
+// (RSPT_E_STREAM): 2^32 - 1 for the decode calls (32-bit index words), the caller's index capacity for
+// rspt_gpu_build_index_frames, whose offsets come from outside the program.
 struct FrameSel {
     const int64_t* ids;
     unsigned long long n_stored;
     unsigned long long slot_region;
+    unsigned long long idx_limit;
 };
+constexpr unsigned long long kIdxWordLimit = 0xFFFFFFFFull;
 
 // one thread per output slot: method byte, header, nb chunks, block headers
 template <bool GATHER>
@@ -137,7 +141,7 @@ __global__ void __launch_bounds__(128) k_frame_parse(const uint8_t* __restrict__
             const uint32_t bl = blk_len(s, b);
             if ((mode == MODE_HUFF && plen > bl) || (mode == MODE_COPY && plen != bl) || (mode == MODE_FILL && plen != 1u)) { err = 1; break; }
             const unsigned long long slot = slot_org + ((q + 7 - slot_off) >> 6) + ord0 + k * s.nblk + b;
-            if (mode == MODE_HUFF && slot + idx_geom(plen).n > 0xFFFFFFFFull) { err = 1; break; }
+            if (mode == MODE_HUFF && slot + idx_geom(plen).n > (GATHER ? sel.idx_limit : kIdxWordLimit)) { err = 1; break; }
             DecBlk& d = row[k * s.nblk + b];
             d.payload_off = q + 7;
             d.payload_len = plen;

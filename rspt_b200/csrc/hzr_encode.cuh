@@ -69,9 +69,10 @@ __global__ void k_frame_sizes(const BlkInfo* __restrict__ info, Shape s, const u
     sizes[f] = sz;
 }
 
+// offsets[f] = base + the sizes of frames 0 .. f - 1 (base: where the batch starts in the stored batch it extends)
 __global__ void __launch_bounds__(1024) k_scan_offsets(const uint32_t* __restrict__ sizes, uint32_t n_frames,
-                                                        uint64_t* __restrict__ offsets, Counters* __restrict__ ctr,
-                                                        uint32_t frame_bytes)
+                                                        unsigned long long base, uint64_t* __restrict__ offsets,
+                                                        Counters* __restrict__ ctr, uint32_t frame_bytes)
 {
     __shared__ unsigned long long s_w[33];
     const uint32_t per = (n_frames + blockDim.x - 1) / blockDim.x;
@@ -96,13 +97,13 @@ __global__ void __launch_bounds__(1024) k_scan_offsets(const uint32_t* __restric
         s_w[32] = run;
     }
     __syncthreads();
-    unsigned long long off = s_w[warp_id()] + inc - sum;
+    unsigned long long off = base + s_w[warp_id()] + inc - sum;
     for (uint32_t f = lo; f < hi; ++f) {
         offsets[f] = off;
         off += sizes[f];
     }
     if (threadIdx.x == 0) {
-        offsets[n_frames] = s_w[32];
+        offsets[n_frames] = base + s_w[32];
         atomicAdd(&ctr->frames_compressed, (unsigned long long)n_frames);
         atomicAdd(&ctr->raw_bytes_in, (unsigned long long)n_frames * frame_bytes);
         atomicAdd(&ctr->compressed_bytes_out, s_w[32]);
@@ -293,8 +294,9 @@ __global__ void __launch_bounds__(kEncThreads, MINB) k_hzr_encode(const uint8_t*
             stg[i] = v;
         }
         for (uint32_t i = (tw4 >> 2) + tid; i < ((pw0 + pw + 3u + 3u) >> 2); i += blockDim.x) reinterpret_cast<uint4*>(stg)[i] = make_uint4(0, 0, 0, 0);
-        // decode index: where this block's entries go (common.cuh)
-        uint32_t* my_idx = sidecar ? sidecar + idx_slot_base(frame_off - offsets[0] + blk_off[blk] + 7u, blk) : nullptr;
+        // decode index: where this block's entries go (common.cuh); offsets are store-relative and `sidecar`
+        // starts at the batch's first block ordinal, so an appended batch lands where one long batch would
+        uint32_t* my_idx = sidecar ? sidecar + idx_slot_base(frame_off + blk_off[blk] + 7u, blk) : nullptr;
         const IdxGeom ig = idx_geom(plen);
         if (my_idx && tid <= idx_interval_of(ig, bi.tree_nbits)) my_idx[tid] = bi.tree_nbits - tid * ig.bits;  // first token, output byte 0
         if (wid == kEncWarps - 1) {

@@ -89,7 +89,7 @@ __global__ void __launch_bounds__(kSpThreads, 6) k_hzr_encode_sparse(Shape s, co
     for (uint32_t i = tid; i < kSymStride; i += blockDim.x) s_codes[i] = __ldg(codes + (size_t)blk * kSymStride + i);
     // decode index: where this block's entries go (common.cuh); the first token starts behind the tree bits
     const unsigned long long frame_off = so.offsets[f];
-    uint32_t* my_idx = so.sidecar ? so.sidecar + idx_slot_base(frame_off - so.offsets[0] + so.blk_off[blk] + 7u, blk) : nullptr;
+    uint32_t* my_idx = so.sidecar ? so.sidecar + idx_slot_base(frame_off + so.blk_off[blk] + 7u, blk) : nullptr;
     const IdxGeom ig = idx_geom(bi.payload_len);
     if (my_idx && tid <= idx_interval_of(ig, bi.tree_nbits)) my_idx[tid] = bi.tree_nbits - tid * ig.bits;
     // staging: tree words, then zeros (the code words are OR-ed in)

@@ -127,6 +127,12 @@ void destroy_host_pipe(rspt_gpu_packer* p);
 
 uint32_t total_blocks(const rspt_gpu_packer* p, size_t frames) { return (uint32_t)(frames * p->s.nb_alloc * p->s.nblk); }
 
+// the header walk keeps the ordinal of a stored block in 32 bits
+bool stored_ordinals_fit(const rspt_gpu_packer* p, size_t n_stored)
+{
+    return n_stored <= 0xFFFFFFFFull / ((uint64_t)p->s.nb_alloc * p->s.nblk);
+}
+
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------
@@ -473,20 +479,37 @@ struct Samples {
     const int32_t* words;
 };
 
-int compress_batch(rspt_gpu_packer* p, Samples src, size_t n_frames, uint8_t* d_dst, size_t dst_capacity,
-                   uint64_t* d_offsets, uint8_t* d_frame_nb, void* d_sidecar)
+// Frames n_stored .. n_stored + n_frames - 1 of a stored batch of n_stored frames and stored_bytes stream bytes
+// (compress_batch: n_stored = stored_bytes = 0).  Offsets are store-relative and index entries are addressed by
+// store-relative payload offset and block ordinal from the store's first frame (common.cuh), so appending batch
+// after batch writes the same bytes as one batch over all their frames.
+int compress_append(rspt_gpu_packer* p, Samples src, size_t n_frames, uint8_t* d_store, size_t store_capacity,
+                    uint64_t* d_store_offsets, size_t n_stored, size_t stored_bytes, uint8_t* d_store_frame_nb,
+                    void* d_store_sidecar, size_t sidecar_capacity)
 {
     if (n_frames == 0) return RSPT_OK;
     if (n_frames > p->max_batch) return fail_arg(p, "n_frames exceeds max_batch_frames"), RSPT_E_CAPACITY;
-    if (dst_capacity < n_frames * rspt_gpu_max_compressed_size(p))
-        return fail_arg(p, "dst_capacity < n_frames * rspt_gpu_max_compressed_size"), RSPT_E_CAPACITY;
+    if (!stored_ordinals_fit(p, n_stored + n_frames))
+        return fail_arg(p, "n_stored + n_frames: the store would have more blocks than 32-bit ordinals can number"), RSPT_E_ARG;
+    const size_t worst = n_frames * rspt_gpu_max_compressed_size(p);
+    if (stored_bytes > store_capacity || store_capacity - stored_bytes < worst)
+        return fail_arg(p, "store_capacity < stored_bytes + n_frames * rspt_gpu_max_compressed_size"), RSPT_E_CAPACITY;
+    if (d_store_sidecar) {
+        const size_t need = rspt_gpu_sidecar_used_bytes(p, n_stored + n_frames, stored_bytes + worst);
+        if (need / sizeof(uint32_t) > kIdxWordLimit)
+            return fail_arg(p, "the store's decode index could reach word 2^32"), RSPT_E_ARG;
+        if (sidecar_capacity < need)
+            return fail_arg(p, "sidecar_capacity < rspt_gpu_sidecar_used_bytes of the store after the append"), RSPT_E_CAPACITY;
+    }
     DeviceGuard dg(p->device);
     const Shape& s = p->s;
     const size_t F = n_frames;
     const uint32_t nblocks = total_blocks(p, F);
-    int rc = wait_for_placement_of(p, d_offsets);
+    int rc = wait_for_placement_of(p, d_store_offsets);
     if (rc) return rc;
-    uint32_t* sidecar = reinterpret_cast<uint32_t*>(d_sidecar);
+    uint64_t* d_offsets = d_store_offsets + n_stored;
+    // the batch's first block has ordinal total_blocks(n_stored) in the store: the encoders count from there
+    uint32_t* sidecar = d_store_sidecar ? reinterpret_cast<uint32_t*>(d_store_sidecar) + (size_t)total_blocks(p, n_stored) : nullptr;
     const unsigned tgrid = (nblocks + kTreeWarps - 1) / kTreeWarps;
     {
         StageTimer t(p, RSPT_STAGE_TRANSFORM);
@@ -519,13 +542,13 @@ int compress_batch(rspt_gpu_packer* p, Samples src, size_t n_frames, uint8_t* d_
     {
         StageTimer t(p, RSPT_STAGE_LAYOUT);
         k_frame_sizes<<<(unsigned)((F + 255) / 256), 256, 0, p->stream>>>(p->d_info, s, p->d_frame_nb, (uint32_t)F, p->d_sizes, p->d_blk_off);
-        k_scan_offsets<<<1, 1024, 0, p->stream>>>(p->d_sizes, (uint32_t)F, d_offsets, p->d_ctr, s.frame_bytes);
+        k_scan_offsets<<<1, 1024, 0, p->stream>>>(p->d_sizes, (uint32_t)F, stored_bytes, d_offsets, p->d_ctr, s.frame_bytes);
     }
     {
         // sparse blocks from their lists (side stream) beside everything else from the planes: both kernels
         // decide with the same predicate which of them writes a block
         StageTimer t(p, RSPT_STAGE_ENCODE);
-        const SparseOut so{d_dst, d_offsets, p->d_blk_off, p->sp_stage, p->d_headers, sidecar};
+        const SparseOut so{d_store, d_offsets, p->d_blk_off, p->sp_stage, p->d_headers, sidecar};
         RSPT_CUDA_CHECK(cudaEventRecord(p->ev_fork2, p->stream));
         RSPT_CUDA_CHECK(cudaStreamWaitEvent(p->side, p->ev_fork2, 0));
         k_hzr_encode_sparse<<<nblocks, kSpThreads, kSparseSmem, p->side>>>(s, p->d_frame_nb, p->d_info, p->d_codes, p->d_tree, p->d_lists,
@@ -534,33 +557,53 @@ int compress_batch(rspt_gpu_packer* p, Samples src, size_t n_frames, uint8_t* d_
         if (encode_ctas_per_sm(s) == 3)
             k_hzr_encode<3><<<nblocks, kEncThreads, p->enc_smem, p->stream>>>(p->d_planes, s, p->d_frame_nb, p->d_info, p->d_blk_off,
                                                                                p->d_codes, p->d_tree, p->d_step_lz, p->d_lists, p->d_list_n, p->sp_stage,
-                                                                               d_offsets, p->d_headers, p->d_crc, d_dst, sidecar);
+                                                                               d_offsets, p->d_headers, p->d_crc, d_store, sidecar);
         else
             k_hzr_encode<2><<<nblocks, kEncThreads, p->enc_smem, p->stream>>>(p->d_planes, s, p->d_frame_nb, p->d_info, p->d_blk_off,
                                                                                p->d_codes, p->d_tree, p->d_step_lz, p->d_lists, p->d_list_n, p->sp_stage,
-                                                                               d_offsets, p->d_headers, p->d_crc, d_dst, sidecar);
+                                                                               d_offsets, p->d_headers, p->d_crc, d_store, sidecar);
         RSPT_CUDA_CHECK(cudaStreamWaitEvent(p->stream, p->ev_join2, 0));
     }
     p->launches += 4;
     RSPT_CUDA_CHECK(cudaGetLastError());
-    if (d_frame_nb) RSPT_CUDA_CHECK(cudaMemcpyAsync(d_frame_nb, p->d_frame_nb, F, cudaMemcpyDeviceToDevice, p->stream));
+    if (d_store_frame_nb)
+        RSPT_CUDA_CHECK(cudaMemcpyAsync(d_store_frame_nb + n_stored, p->d_frame_nb, F, cudaMemcpyDeviceToDevice, p->stream));
     return RSPT_OK;
 }
 
 }  // namespace
 
+// compress_batch is the append to an empty store; its sidecar is sized by rspt_gpu_sidecar_bytes (not passed)
 extern "C" int rspt_gpu_compress_batch(rspt_gpu_packer* p, const uint8_t* d_src, size_t n_frames, uint8_t* d_dst,
                                        size_t dst_capacity, uint64_t* d_offsets, uint8_t* d_frame_nb, void* d_sidecar)
 {
     if (!p || !d_src || !d_dst || !d_offsets) return RSPT_E_ARG;
-    return compress_batch(p, Samples{d_src, nullptr}, n_frames, d_dst, dst_capacity, d_offsets, d_frame_nb, d_sidecar);
+    return compress_append(p, Samples{d_src, nullptr}, n_frames, d_dst, dst_capacity, d_offsets, 0, 0, d_frame_nb, d_sidecar, SIZE_MAX);
 }
 
 extern "C" int rspt_gpu_compress_batch_i32(rspt_gpu_packer* p, const int32_t* d_src, size_t n_frames, uint8_t* d_dst,
                                            size_t dst_capacity, uint64_t* d_offsets, uint8_t* d_frame_nb, void* d_sidecar)
 {
     if (!p || !d_src || !d_dst || !d_offsets || ((uintptr_t)d_src & 3)) return RSPT_E_ARG;
-    return compress_batch(p, Samples{nullptr, d_src}, n_frames, d_dst, dst_capacity, d_offsets, d_frame_nb, d_sidecar);
+    return compress_append(p, Samples{nullptr, d_src}, n_frames, d_dst, dst_capacity, d_offsets, 0, 0, d_frame_nb, d_sidecar, SIZE_MAX);
+}
+
+extern "C" int rspt_gpu_compress_append(rspt_gpu_packer* p, const uint8_t* d_src, size_t n_frames, uint8_t* d_store,
+                                        size_t store_capacity, uint64_t* d_store_offsets, size_t n_stored, size_t stored_bytes,
+                                        uint8_t* d_store_frame_nb, void* d_store_sidecar, size_t sidecar_capacity)
+{
+    if (!p || !d_src || !d_store || !d_store_offsets) return RSPT_E_ARG;
+    return compress_append(p, Samples{d_src, nullptr}, n_frames, d_store, store_capacity, d_store_offsets, n_stored, stored_bytes,
+                           d_store_frame_nb, d_store_sidecar, sidecar_capacity);
+}
+
+extern "C" int rspt_gpu_compress_append_i32(rspt_gpu_packer* p, const int32_t* d_src, size_t n_frames, uint8_t* d_store,
+                                            size_t store_capacity, uint64_t* d_store_offsets, size_t n_stored, size_t stored_bytes,
+                                            uint8_t* d_store_frame_nb, void* d_store_sidecar, size_t sidecar_capacity)
+{
+    if (!p || !d_src || !d_store || !d_store_offsets || ((uintptr_t)d_src & 3)) return RSPT_E_ARG;
+    return compress_append(p, Samples{nullptr, d_src}, n_frames, d_store, store_capacity, d_store_offsets, n_stored, stored_bytes,
+                           d_store_frame_nb, d_store_sidecar, sidecar_capacity);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -616,7 +659,23 @@ extern "C" int rspt_gpu_build_index(rspt_gpu_packer* p, const uint8_t* d_src, co
     if (n_frames > p->max_batch) return fail_arg(p, "n_frames exceeds max_batch_frames"), RSPT_E_CAPACITY;
     DeviceGuard dg(p->device);
     return launch_parse_and_index(p, d_src, d_offsets, n_frames, d_frame_nb, d_sidecar, d_status ? d_status : p->d_status_tmp,
-                                  FrameSel{nullptr, 0, 0});
+                                  FrameSel{nullptr, 0, 0, kIdxWordLimit});
+}
+
+extern "C" int rspt_gpu_build_index_frames(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets, size_t n_stored,
+                                           const uint8_t* d_frame_nb, const int64_t* d_frame_ids, size_t n_frames,
+                                           void* d_sidecar, size_t sidecar_capacity, int32_t* d_status)
+{
+    if (!p || !d_src || !d_offsets || !d_frame_ids || !d_sidecar) return RSPT_E_ARG;
+    if (n_frames == 0) return RSPT_OK;
+    if (n_frames > p->max_batch) return fail_arg(p, "n_frames exceeds max_batch_frames"), RSPT_E_CAPACITY;
+    if (!stored_ordinals_fit(p, n_stored))
+        return fail_arg(p, "n_stored: the stored batch has more blocks than 32-bit ordinals can number"), RSPT_E_ARG;
+    DeviceGuard dg(p->device);
+    // the stored batch's own addressing (slot_region 0); a frame whose entries would reach sidecar_capacity fails
+    const unsigned long long words = sidecar_capacity / sizeof(uint32_t);
+    return launch_parse_and_index(p, d_src, d_offsets, n_frames, d_frame_nb, d_sidecar, d_status ? d_status : p->d_status_tmp,
+                                  FrameSel{d_frame_ids, n_stored, 0, words < kIdxWordLimit ? words : kIdxWordLimit});
 }
 
 // payload bits per output byte up to which k_hzr_decode uses its two-literals-per-look-up table (measured)
@@ -639,8 +698,7 @@ int decompress_batch(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d
     if (n_frames == 0) return RSPT_OK;
     if (n_frames > p->max_batch) return fail_arg(p, "n_frames exceeds max_batch_frames"), RSPT_E_CAPACITY;
     const Shape& s = p->s;
-    // the parse keeps the ordinal of a stored block in 32 bits
-    if (ids && n_stored > 0xFFFFFFFFull / ((uint64_t)s.nb_alloc * s.nblk))
+    if (ids && !stored_ordinals_fit(p, n_stored))
         return fail_arg(p, "n_stored: the stored batch has more blocks than 32-bit ordinals can number"), RSPT_E_ARG;
     DeviceGuard dg(p->device);
     const size_t F = n_frames;
@@ -656,7 +714,7 @@ int decompress_batch(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d
         own_index = p->d_auto_index;
         d_sidecar = own_index;
     }
-    const FrameSel sel{ids, n_stored, (ids && own_index) ? gather_slot_region(p) : 0};
+    const FrameSel sel{ids, n_stored, (ids && own_index) ? gather_slot_region(p) : 0, kIdxWordLimit};
     int rc = launch_parse_and_index(p, d_src, d_offsets, F, d_frame_nb, own_index, status, sel);
     if (rc) return rc;
     const uint32_t* sc = reinterpret_cast<const uint32_t*>(d_sidecar);
@@ -733,7 +791,7 @@ extern "C" int rspt_gpu_verify_batch(rspt_gpu_packer* p, const uint8_t* d_src, c
     const uint32_t nblocks = total_blocks(p, F);
     DecBlk* dec = reinterpret_cast<DecBlk*>(p->d_dec);
     k_frame_parse<false><<<(unsigned)((F + 127) / 128), 128, 0, p->stream>>>(d_src, d_offsets, s, d_frame_nb, p->d_nb_state, (uint32_t)F,
-                                                                             FrameSel{nullptr, 0, 0}, dec, p->d_headers, p->d_dec_nb,
+                                                                             FrameSel{nullptr, 0, 0, kIdxWordLimit}, dec, p->d_headers, p->d_dec_nb,
                                                                              d_status, p->d_ctr);
     k_hzr_verify<<<nblocks, kVerifyThreads, p->dec_smem, p->stream>>>(d_src, s, dec, p->d_crc, d_status, p->d_ctr);
     p->launches += 2;

@@ -10,7 +10,7 @@ torch is used only to own device memory and to name the CUDA stream.
 from __future__ import annotations
 
 import ctypes as C
-from dataclasses import dataclass
+from dataclasses import dataclass, field
 
 import numpy as np
 import torch
@@ -35,6 +35,51 @@ class CompressedBatch:
     def frame(self, i: int) -> bytes:
         off = self.offsets[i:i + 2].cpu().tolist()
         return bytes(self.stream[off[0]:off[1]].cpu().numpy())
+
+
+# bytes behind the last frame that the decoder's 16-byte staging reads may touch (decompress_stream pads the same way)
+STREAM_PAD = 16
+
+
+@dataclass
+class CompressedStore(CompressedBatch):
+    """A stored batch that grows past max_batch_frames by appends (SignalPacker.new_store / append_batch /
+    append_tensor), e.g. a dataset kept compressed in HBM.  Frames [0, n_frames) and stream bytes [0, stored_bytes)
+    are used; the buffers have room behind them.  Offsets are store-relative and the decode index is addressed
+    from the store's start, so the used prefix of every buffer is the whole store: growth copies it and trim()
+    cuts the buffers down to it.  Accepted wherever a CompressedBatch is (decompress_frames(_tensor), frame(),
+    slices for verify_batch)."""
+    stored_bytes: int = 0
+    packer: "SignalPacker | None" = field(default=None, repr=False)
+
+    def total_bytes(self) -> int:
+        return self.stored_bytes
+
+    def sidecar_used_bytes(self) -> int:
+        return self.packer.sidecar_used_bytes(self.n_frames, self.stored_bytes)
+
+    def trim(self) -> "CompressedStore":
+        """Shrink every buffer to what the store uses: the stream to stored_bytes + STREAM_PAD zero bytes, offsets
+        and frame_nb to n_frames + 1 and n_frames entries, the sidecar to sidecar_used_bytes().  Ordered on torch's
+        current stream."""
+        n, used = self.n_frames, self.stored_bytes
+        stream = torch.zeros(used + STREAM_PAD, dtype=torch.uint8, device=self.stream.device)
+        stream[:used].copy_(self.stream[:used])
+        self.stream = stream
+        self.offsets = self.offsets[:n + 1].clone()
+        self.frame_nb = self.frame_nb[:n].clone()
+        if self.sidecar is not None:
+            self.sidecar = self.sidecar[:self.sidecar_used_bytes()].clone()
+        return self
+
+    def index_all(self, p: "SignalPacker", status: torch.Tensor | None = None) -> "CompressedStore":
+        """Build the decode index of every stored frame (e.g. for a store appended without one) with
+        p.index_frames, p.max_batch frames per call.  status: optional int32 [n_frames], as for index_frames."""
+        for a in range(0, self.n_frames, p.max_batch):
+            b = min(self.n_frames, a + p.max_batch)
+            ids = torch.arange(a, b, dtype=torch.int64, device=self.stream.device)
+            p.index_frames(self, ids, status[a:b] if status is not None else None)
+        return self
 
 
 class SignalPacker:
@@ -175,12 +220,15 @@ class SignalPacker:
     def compress_batch(self, frames: torch.Tensor, out: CompressedBatch | None = None, sidecar: bool = True) -> CompressedBatch:
         """frames: uint8 CUDA tensor of n * frame_bytes bytes.  Asynchronous on torch's current stream (the
         handle is re-bound to it when it changed since the last call)."""
+        return self._compress(self.L.rspt_gpu_compress_batch, frames, self._check_frames(frames), out, sidecar)
+
+    def _check_frames(self, frames) -> int:
         if not (frames.is_cuda and frames.dtype == torch.uint8 and frames.is_contiguous()):
             raise ValueError("frames must be a contiguous uint8 CUDA tensor")
         n = frames.numel() // self.frame_bytes
         if n * self.frame_bytes != frames.numel():
             raise ValueError("frames is not a whole number of frames")
-        return self._compress(self.L.rspt_gpu_compress_batch, frames, n, out, sidecar)
+        return n
 
     def compress_tensor(self, x: torch.Tensor, out: CompressedBatch | None = None, sidecar: bool = True) -> CompressedBatch:
         """x: contiguous int32 CUDA tensor [n, ch, ns] on the handle's device, the samples in the low 8 * bps bits of
@@ -210,6 +258,89 @@ class SignalPacker:
         check(rc, self.h, fn.__name__)
         out.n_frames = n
         return out
+
+    # -- stores: batches appended past max_batch_frames ---------------------------------------------
+    def new_store(self, frames_capacity: int, bytes_capacity: int | None = None, sidecar: bool = True) -> CompressedStore:
+        """An empty store with room for frames_capacity frames and bytes_capacity stream bytes (None: the worst case
+        of frames_capacity frames, max_compressed_size each -- raw-sized; pass an estimate for a large store).  The
+        store grows when an append does not fit, so the capacities are only a starting point."""
+        dev = self._dev()
+        if bytes_capacity is None:
+            bytes_capacity = frames_capacity * self.max_compressed_size
+        stream = torch.empty(bytes_capacity + STREAM_PAD, dtype=torch.uint8, device=dev)
+        offsets = torch.zeros(frames_capacity + 1, dtype=torch.int64, device=dev)
+        frame_nb = torch.zeros(frames_capacity, dtype=torch.uint8, device=dev)
+        sc = torch.zeros(self.sidecar_used_bytes(frames_capacity, bytes_capacity), dtype=torch.uint8, device=dev) if sidecar else None
+        return CompressedStore(stream, offsets, frame_nb, sc, 0, 0, self)
+
+    def append_batch(self, store: CompressedStore, frames: torch.Tensor) -> CompressedStore:
+        """Compress frames (as for compress_batch, at most max_batch_frames of them) and append them to the store
+        (rspt_gpu_compress_append): the store then equals what one compress_batch over all its frames writes.  Runs
+        on torch's current stream, then reads the new stream total back (one 8-byte copy and a synchronisation), so
+        that the next append can be checked and placed from the host."""
+        return self._append(self.L.rspt_gpu_compress_append, store, frames, self._check_frames(frames))
+
+    def append_tensor(self, store: CompressedStore, x: torch.Tensor) -> CompressedStore:
+        """append_batch for an int32 tensor [n, ch, ns], as compress_tensor takes it.  Native and int32 appends may be
+        mixed on one store."""
+        self._check_words(x)
+        return self._append(self.L.rspt_gpu_compress_append_i32, store, x, x.shape[0])
+
+    def _append(self, fn, store: CompressedStore, src: torch.Tensor, n: int) -> CompressedStore:
+        if n > self.max_batch:
+            raise ValueError(f"{n} frames in one append: max_batch_frames is {self.max_batch}")
+        if n == 0:
+            return store
+        self._bind_stream()
+        self._reserve(store, store.n_frames + n, store.stored_bytes + n * self.max_compressed_size)
+        sc = store.sidecar
+        rc = fn(self.h, src.data_ptr(), n, store.stream.data_ptr(), store.stream.numel() - STREAM_PAD, store.offsets.data_ptr(),
+                store.n_frames, store.stored_bytes, store.frame_nb.data_ptr(), sc.data_ptr() if sc is not None else None,
+                sc.numel() if sc is not None else 0)
+        check(rc, self.h, fn.__name__)
+        store.n_frames += n
+        store.stored_bytes = int(store.offsets[store.n_frames].item())
+        return store
+
+    def _reserve(self, store: CompressedStore, frames: int, stream_bytes: int) -> None:
+        """Grow the store's buffers (at least doubling a buffer that is too small) so that `frames` frames and
+        `stream_bytes` stream bytes fit; the used prefix of each is copied over."""
+        def grown(t, used, need, zero):
+            if t.numel() >= need:
+                return t
+            new = (torch.zeros if zero else torch.empty)(max(need, 2 * t.numel()), dtype=t.dtype, device=t.device)
+            new[:used].copy_(t[:used])
+            return new
+        n = store.n_frames
+        store.offsets = grown(store.offsets, n + 1, frames + 1, True)
+        store.frame_nb = grown(store.frame_nb, n, frames, True)
+        store.stream = grown(store.stream, store.stored_bytes, stream_bytes + STREAM_PAD, False)
+        if store.sidecar is not None:
+            need = self.sidecar_used_bytes(frames, stream_bytes)
+            if store.sidecar.numel() < need:
+                used = self.sidecar_used_bytes(n, store.stored_bytes)
+                room = self.sidecar_used_bytes(store.offsets.numel() - 1, store.stream.numel() - STREAM_PAD)
+                new = torch.zeros(max(need, room), dtype=torch.uint8, device=store.sidecar.device)
+                new[:used].copy_(store.sidecar[:used])
+                store.sidecar = new
+
+    def index_frames(self, batch: CompressedBatch, frame_ids, status: torch.Tensor | None = None) -> CompressedBatch:
+        """Write the decode-index entries of stored frames frame_ids[0], frame_ids[1], ... (at most max_batch_frames
+        ids, as for decompress_frames) into the batch's own index (rspt_gpu_build_index_frames): indexing a batch
+        in pieces gives the words one build_index over the whole batch gives.  A batch without a sidecar first gets
+        a zeroed one of sidecar_used_bytes(n_frames, total).  status: optional int32 per id, -1 for an id outside
+        the batch, -4 for a malformed frame.  Asynchronous on torch's current stream."""
+        ids = self._frame_ids(frame_ids)
+        if batch.sidecar is None:
+            total = int(batch.offsets[batch.n_frames].item())
+            batch.sidecar = torch.zeros(self.sidecar_used_bytes(batch.n_frames, total), dtype=torch.uint8, device=self._dev())
+        nbp = batch.frame_nb.data_ptr() if batch.frame_nb is not None else None
+        self._bind_stream()
+        rc = self.L.rspt_gpu_build_index_frames(self.h, batch.stream.data_ptr(), batch.offsets.data_ptr(), batch.n_frames, nbp,
+                                                ids.data_ptr(), ids.numel(), batch.sidecar.data_ptr(), batch.sidecar.numel(),
+                                                status.data_ptr() if status is not None else None)
+        check(rc, self.h, "rspt_gpu_build_index_frames")
+        return batch
 
     def decompress_batch(self, batch: CompressedBatch, out: torch.Tensor | None = None, status: torch.Tensor | None = None,
                          use_sidecar: bool = True) -> torch.Tensor:
