@@ -44,7 +44,9 @@ struct rspt_gpu_packer {
     uint32_t* d_list_n;    // per block: entries in d_lists, kNoList = dense block
     uint8_t* d_blk_class;  // per block: kClassSparse / kClassDense (density probe of the histogram launches)
     cudaStream_t side;     // sparse-class histogram + trees run here, beside the dense class on `stream`
-    cudaEvent_t ev_fork, ev_join, ev_fork2, ev_join2;
+    // fork_side / join_side: one pair serves every fork and join of a call, since cudaStreamWaitEvent waits for
+    // the event's last record before the wait was enqueued
+    cudaEvent_t ev_fork, ev_join;
     cudaStream_t place;    // multi-GPU placement (all-gather of totals + offset rebase) runs here, off the compute stream
     cudaEvent_t ev_place;
     // placements possibly still in flight, by the offsets array they rewrite: a later compress into the same
@@ -135,8 +137,8 @@ int with_flag(bool b, F&& f)
 }
 
 // The dynamic shared-memory limit belongs to the kernel, for the whole process and device, not to a handle.
-// It only ever goes up, to what some launch needed, so that no handle can lower it under another handle's
-// launch; the check and the raise hold one process mutex.
+// It only ever goes up, so that no handle can lower it under another handle's launch; the check and the raise
+// hold one process mutex.
 template <class K>
 cudaError_t raise_smem_limit(K* kernel, size_t bytes)
 {
@@ -149,16 +151,49 @@ cudaError_t raise_smem_limit(K* kernel, size_t bytes)
     return e;
 }
 
-// kernel<<<grid, block, smem>>>(args...) on the handle's stream, counted in p->launches.  48 KB, static
-// included, need no raised limit; the kernels launched here with dynamic shared memory declare at most an
-// mbarrier's worth of static shared memory, and ask for far less or far more than 48 KB.
+// kernel<<<grid, block, smem, stream>>>(args...) and the launch's error.  A kernel's dynamic shared-memory limit
+// starts at 48 KB minus its static shared memory.  Above 48 KB this raises the limit to smem.  Below, a kernel
+// with static shared memory of its own can still need a raised limit: rspt_gpu_create raises the hzr kernels
+// (up to 12 544 bytes of static shared memory) to the most any handle launches them with.
+template <class... P, class... A>
+cudaError_t launch(cudaStream_t stream, void (*kernel)(P...), dim3 grid, dim3 block, size_t smem, A&&... args)
+{
+    if (smem > 48 * 1024) {
+        const cudaError_t e = raise_smem_limit(kernel, smem);
+        if (e != cudaSuccess) return e;
+    }
+    kernel<<<grid, block, smem, stream>>>(std::forward<A>(args)...);
+    return cudaGetLastError();
+}
+
+// the same on one of the handle's streams, counted in p->launches
+template <class... P, class... A>
+int launch(rspt_gpu_packer* p, cudaStream_t stream, void (*kernel)(P...), dim3 grid, dim3 block, size_t smem, A&&... args)
+{
+    p->launches += 1;
+    RSPT_CUDA_CHECK(launch(stream, kernel, grid, block, smem, std::forward<A>(args)...));
+    return 0;
+}
+
 template <class... P, class... A>
 int launch(rspt_gpu_packer* p, void (*kernel)(P...), dim3 grid, dim3 block, size_t smem, A&&... args)
 {
-    if (smem > 48 * 1024) RSPT_CUDA_CHECK(raise_smem_limit(kernel, smem));
-    kernel<<<grid, block, smem, p->stream>>>(std::forward<A>(args)...);
-    p->launches += 1;
-    RSPT_CUDA_CHECK(cudaGetLastError());
+    return launch(p, p->stream, kernel, grid, block, smem, std::forward<A>(args)...);
+}
+
+// p->side starts behind the work enqueued on p->stream so far
+inline int fork_side(rspt_gpu_packer* p)
+{
+    RSPT_CUDA_CHECK(cudaEventRecord(p->ev_fork, p->stream));
+    RSPT_CUDA_CHECK(cudaStreamWaitEvent(p->side, p->ev_fork, 0));
+    return 0;
+}
+
+// p->stream continues behind the work enqueued on p->side so far
+inline int join_side(rspt_gpu_packer* p)
+{
+    RSPT_CUDA_CHECK(cudaEventRecord(p->ev_join, p->side));
+    RSPT_CUDA_CHECK(cudaStreamWaitEvent(p->stream, p->ev_join, 0));
     return 0;
 }
 

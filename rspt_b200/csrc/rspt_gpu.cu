@@ -103,12 +103,6 @@ cudaError_t dalloc(T*& ptr, size_t count)
     return cudaMalloc(reinterpret_cast<void**>(&ptr), count * sizeof(T) + 64);
 }
 
-template <class K>
-cudaError_t allow_smem(K kernel, size_t bytes)
-{
-    return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-}
-
 struct DeviceGuard {
     int prev = -1;
     explicit DeviceGuard(int dev)
@@ -306,9 +300,14 @@ extern "C" int rspt_gpu_create(int kind, size_t bps, size_t ch, size_t ns, size_
     if (e == cudaSuccess) e = cudaMemsetAsync(p->d_frame_nb, (int)s.nb_init, F, p->stream);
     if (e == cudaSuccess) e = cudaMemsetAsync(p->d_ctr, 0, sizeof(Counters), p->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(p->d_nb_state, &s.nb_init, 4, cudaMemcpyHostToDevice, p->stream);
-    if (e == cudaSuccess) e = allow_smem(k_hzr_encode<2>, kEncodeSmem);
-    if (e == cudaSuccess) e = allow_smem(k_hzr_encode<3>, kEncodeSmem);
-    if (e == cudaSuccess) e = allow_smem(k_hzr_hist<3>, kHistSmemList);
+    // the hzr kernels go to the most dynamic shared memory any shape launches them with (see launch)
+    if (e == cudaSuccess) e = raise_smem_limit(k_hzr_encode<2>, kEncodeSmem);
+    if (e == cudaSuccess) e = raise_smem_limit(k_hzr_encode<3>, kEncodeSmem);
+    if (e == cudaSuccess) e = raise_smem_limit(k_hzr_hist<3>, kHistSmemList);
+    if (e == cudaSuccess) e = raise_smem_limit(k_hzr_encode_sparse, kSparseSmem);
+    if (e == cudaSuccess) e = raise_smem_limit(k_hzr_decode, kDecodeSmem);
+    if (e == cudaSuccess) e = raise_smem_limit(k_hzr_verify, kDecodeSmem);
+    if (e == cudaSuccess) e = raise_smem_limit(k_hzr_build_index, kDecodeSmem);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&p->side, cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&p->place, cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p->ev_place, cudaEventDisableTiming);
@@ -316,19 +315,12 @@ extern "C" int rspt_gpu_create(int kind, size_t bps, size_t ch, size_t ns, size_
         e = cudaEventCreateWithFlags(&p->ev_placed[k], cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p->ev_fork, cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p->ev_join, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p->ev_fork2, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p->ev_join2, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = allow_smem(k_hzr_encode_sparse, kSparseSmem);
     {
         // test hook: a smaller staging limit sends listed blocks down the hand-over path to k_hzr_encode
         const char* ev = getenv("RSPT_SPARSE_STAGE_BYTES");
         const long v = ev ? atol(ev) : (long)kSpStageBytes;
         p->sp_stage = (uint32_t)(v < 1 ? 1 : (v > (long)kSpStageBytes ? (long)kSpStageBytes : v));
     }
-    if (e == cudaSuccess) e = allow_smem(k_hzr_decode, kDecodeSmem);
-    if (e == cudaSuccess) e = allow_smem(k_hzr_verify, kDecodeSmem);
-    if (e == cudaSuccess) e = allow_smem(k_hzr_build_index, kDecodeSmem);
-    if (e == cudaSuccess) e = allow_smem(k_crc32c, kEncodeSmem);
     if (e == cudaSuccess) e = cudaStreamSynchronize(p->stream);
     if (e != cudaSuccess) {
         fprintf(stderr, "rspt_gpu_create: %s\n", cudaGetErrorString(e));
@@ -364,8 +356,6 @@ extern "C" int rspt_gpu_destroy(rspt_gpu_packer* p)
     for (cudaEvent_t ev : p->ev_placed) if (ev) cudaEventDestroy(ev);
     if (p->ev_fork) cudaEventDestroy(p->ev_fork);
     if (p->ev_join) cudaEventDestroy(p->ev_join);
-    if (p->ev_fork2) cudaEventDestroy(p->ev_fork2);
-    if (p->ev_join2) cudaEventDestroy(p->ev_join2);
     delete p;
     return RSPT_OK;
 }
@@ -438,19 +428,6 @@ extern "C" int rspt_gpu_get_counters(rspt_gpu_packer* p, rspt_gpu_counters* out)
 // ---------------------------------------------------------------------------------------------
 // compress
 // ---------------------------------------------------------------------------------------------
-namespace {
-
-int launch_frame_nb(rspt_gpu_packer* p, size_t F)
-{
-    if (!p->can_escalate) return RSPT_OK;
-    k_frame_nb<<<1, 1024, 0, p->stream>>>(p->d_need, (uint32_t)F, p->d_nb_state, p->d_frame_nb, p->d_ctr);
-    p->launches += 1;
-    RSPT_CUDA_CHECK(cudaGetLastError());
-    return RSPT_OK;
-}
-
-}  // namespace
-
 // Dense-encoder CTAs per SM the kernel is compiled for.  Measured per 4096-frame batch: xdelta_hzr 1.075 -> 1.051 ms
 // and hadamard 1.121 -> 1.090 ms with 3 (more warps to cover the barriers), hzr 2.344 -> 2.369 and dct
 // 0.848 -> 0.890 with 3 (their planes take the spilled slow path more often).
@@ -478,6 +455,33 @@ struct Samples {
     const uint8_t* raw;
     const int32_t* words;
 };
+
+// Histograms and Huffman trees of the nblocks blocks of `planes` that s describes.  Two classes of blocks
+// (density probe): the sparse-looking ones go through histogram + tree on the side stream while this stream
+// does the dense-looking ones, whose tree build is long and latency-bound and overlaps with the sparse
+// histogram.  RSPT_STAGE_HIST times the dense histogram, RSPT_STAGE_TREE everything from there to the join.
+int launch_hist_and_trees(rspt_gpu_packer* p, const uint8_t* planes, const Shape& s, uint32_t nblocks)
+{
+    const unsigned tgrid = (nblocks + kTreeWarps - 1) / kTreeWarps;
+    int rc = fork_side(p);
+    if (!rc)
+        rc = launch(p, p->side, k_hzr_hist<3>, nblocks, kHistThreads, kHistSmemList, planes, s, p->d_frame_nb, p->d_hist,
+                    p->d_step_lz, p->d_lists, p->d_list_n, p->d_blk_class);
+    if (!rc)
+        rc = launch(p, p->side, k_hzr_tree, tgrid, 32 * kTreeWarps, 0, p->d_hist, s, p->d_frame_nb, p->d_blk_class, kClassSparse,
+                    nblocks, p->d_codes, p->d_tree, p->d_info, p->d_ctr);
+    if (rc) return rc;
+    {
+        StageTimer t(p, RSPT_STAGE_HIST);
+        rc = launch(p, k_hzr_hist<2>, nblocks, kHistThreads, 0, planes, s, p->d_frame_nb, p->d_hist, p->d_step_lz, p->d_lists,
+                    p->d_list_n, p->d_blk_class);
+        if (rc) return rc;
+    }
+    StageTimer t(p, RSPT_STAGE_TREE);
+    rc = launch(p, k_hzr_tree, tgrid, 32 * kTreeWarps, 0, p->d_hist, s, p->d_frame_nb, p->d_blk_class, kClassDense, nblocks,
+                p->d_codes, p->d_tree, p->d_info, p->d_ctr);
+    return rc ? rc : join_side(p);
+}
 
 // Frames n_stored .. n_stored + n_frames - 1 of a stored batch of n_stored frames and stored_bytes stream bytes
 // (compress_batch: n_stored = stored_bytes = 0).  Offsets are store-relative and index entries are addressed by
@@ -510,62 +514,38 @@ int compress_append(rspt_gpu_packer* p, Samples src, size_t n_frames, uint8_t* d
     uint64_t* d_offsets = d_store_offsets + n_stored;
     // the batch's first block has ordinal total_blocks(n_stored) in the store: the encoders count from there
     uint32_t* sidecar = d_store_sidecar ? reinterpret_cast<uint32_t*>(d_store_sidecar) + (size_t)total_blocks(p, n_stored) : nullptr;
-    const unsigned tgrid = (nblocks + kTreeWarps - 1) / kTreeWarps;
     {
         StageTimer t(p, RSPT_STAGE_TRANSFORM);
         rc = src.words ? launch_forward_transform_i32(p, src.words, F) : launch_forward_transform(p, src.raw, F);
-        if (rc) return rc;
-        rc = launch_frame_nb(p, F);
+        if (!rc && p->can_escalate)
+            rc = launch(p, k_frame_nb, 1, 1024, 0, p->d_need, (uint32_t)F, p->d_nb_state, p->d_frame_nb, p->d_ctr);
         if (rc) return rc;
     }
-    {
-        // Two classes of blocks (density probe): the sparse-looking ones go through histogram + tree on
-        // the side stream while this stream does the dense-looking ones, whose tree build is long and
-        // latency-bound and overlaps with the sparse histogram.  RSPT_STAGE_HIST times the dense
-        // histogram, RSPT_STAGE_TREE everything from there to the join.
-        RSPT_CUDA_CHECK(cudaEventRecord(p->ev_fork, p->stream));
-        RSPT_CUDA_CHECK(cudaStreamWaitEvent(p->side, p->ev_fork, 0));
-        k_hzr_hist<3><<<nblocks, kHistThreads, kHistSmemList, p->side>>>(p->d_planes, s, p->d_frame_nb, p->d_hist, p->d_step_lz, p->d_lists, p->d_list_n, p->d_blk_class);
-        k_hzr_tree<<<tgrid, 32 * kTreeWarps, 0, p->side>>>(p->d_hist, s, p->d_frame_nb, p->d_blk_class, kClassSparse, nblocks, p->d_codes, p->d_tree, p->d_info, p->d_ctr);
-        RSPT_CUDA_CHECK(cudaEventRecord(p->ev_join, p->side));
-        {
-            StageTimer t(p, RSPT_STAGE_HIST);
-            k_hzr_hist<2><<<nblocks, kHistThreads, 0, p->stream>>>(p->d_planes, s, p->d_frame_nb, p->d_hist, p->d_step_lz, p->d_lists, p->d_list_n, p->d_blk_class);
-        }
-        {
-            StageTimer t(p, RSPT_STAGE_TREE);
-            k_hzr_tree<<<tgrid, 32 * kTreeWarps, 0, p->stream>>>(p->d_hist, s, p->d_frame_nb, p->d_blk_class, kClassDense, nblocks, p->d_codes, p->d_tree, p->d_info, p->d_ctr);
-            RSPT_CUDA_CHECK(cudaStreamWaitEvent(p->stream, p->ev_join, 0));
-        }
-        p->launches += 4;
-    }
+    rc = launch_hist_and_trees(p, p->d_planes, s, nblocks);
+    if (rc) return rc;
     {
         StageTimer t(p, RSPT_STAGE_LAYOUT);
-        k_frame_sizes<<<(unsigned)((F + 255) / 256), 256, 0, p->stream>>>(p->d_info, s, p->d_frame_nb, (uint32_t)F, p->d_sizes, p->d_blk_off);
-        k_scan_offsets<<<1, 1024, 0, p->stream>>>(p->d_sizes, (uint32_t)F, stored_bytes, d_offsets, p->d_ctr, s.frame_bytes);
+        rc = launch(p, k_frame_sizes, (unsigned)((F + 255) / 256), 256, 0, p->d_info, s, p->d_frame_nb, (uint32_t)F, p->d_sizes,
+                    p->d_blk_off);
+        if (!rc) rc = launch(p, k_scan_offsets, 1, 1024, 0, p->d_sizes, (uint32_t)F, stored_bytes, d_offsets, p->d_ctr, s.frame_bytes);
+        if (rc) return rc;
     }
     {
         // sparse blocks from their lists (side stream) beside everything else from the planes: both kernels
         // decide with the same predicate which of them writes a block
         StageTimer t(p, RSPT_STAGE_ENCODE);
         const SparseOut so{d_store, d_offsets, p->d_blk_off, p->sp_stage, p->d_headers, sidecar};
-        RSPT_CUDA_CHECK(cudaEventRecord(p->ev_fork2, p->stream));
-        RSPT_CUDA_CHECK(cudaStreamWaitEvent(p->side, p->ev_fork2, 0));
-        k_hzr_encode_sparse<<<nblocks, kSpThreads, kSparseSmem, p->side>>>(s, p->d_frame_nb, p->d_info, p->d_codes, p->d_tree, p->d_lists,
-                                                                           p->d_list_n, p->d_crc, so);
-        RSPT_CUDA_CHECK(cudaEventRecord(p->ev_join2, p->side));
-        if (encode_ctas_per_sm(s) == 3)
-            k_hzr_encode<3><<<nblocks, kEncThreads, p->enc_smem, p->stream>>>(p->d_planes, s, p->d_frame_nb, p->d_info, p->d_blk_off,
-                                                                               p->d_codes, p->d_tree, p->d_step_lz, p->d_lists, p->d_list_n, p->sp_stage,
-                                                                               d_offsets, p->d_headers, p->d_crc, d_store, sidecar);
-        else
-            k_hzr_encode<2><<<nblocks, kEncThreads, p->enc_smem, p->stream>>>(p->d_planes, s, p->d_frame_nb, p->d_info, p->d_blk_off,
-                                                                               p->d_codes, p->d_tree, p->d_step_lz, p->d_lists, p->d_list_n, p->sp_stage,
-                                                                               d_offsets, p->d_headers, p->d_crc, d_store, sidecar);
-        RSPT_CUDA_CHECK(cudaStreamWaitEvent(p->stream, p->ev_join2, 0));
+        rc = fork_side(p);
+        if (!rc)
+            rc = launch(p, p->side, k_hzr_encode_sparse, nblocks, kSpThreads, kSparseSmem, s, p->d_frame_nb, p->d_info, p->d_codes,
+                        p->d_tree, p->d_lists, p->d_list_n, p->d_crc, so);
+        if (!rc)
+            rc = launch(p, encode_ctas_per_sm(s) == 3 ? k_hzr_encode<3> : k_hzr_encode<2>, nblocks, kEncThreads, p->enc_smem,
+                        p->d_planes, s, p->d_frame_nb, p->d_info, p->d_blk_off, p->d_codes, p->d_tree, p->d_step_lz, p->d_lists,
+                        p->d_list_n, p->sp_stage, d_offsets, p->d_headers, p->d_crc, d_store, sidecar);
+        if (!rc) rc = join_side(p);
+        if (rc) return rc;
     }
-    p->launches += 4;
-    RSPT_CUDA_CHECK(cudaGetLastError());
     if (d_store_frame_nb)
         RSPT_CUDA_CHECK(cudaMemcpyAsync(d_store_frame_nb + n_stored, p->d_frame_nb, F, cudaMemcpyDeviceToDevice, p->stream));
     return RSPT_OK;
@@ -619,27 +599,18 @@ int launch_parse_and_index(rspt_gpu_packer* p, const uint8_t* d_src, const uint6
     const Shape& s = p->s;
     const uint32_t nblocks = total_blocks(p, F);
     DecBlk* dec = reinterpret_cast<DecBlk*>(p->d_dec);
-    {
-        StageTimer t(p, RSPT_STAGE_PARSE);
-        const unsigned pgrid = (unsigned)((F + 127) / 128);
-        if (sel.ids)
-            k_frame_parse<true><<<pgrid, 128, 0, p->stream>>>(d_src, d_offsets, s, d_frame_nb, p->d_nb_state, (uint32_t)F, sel,
-                                                              dec, p->d_headers, p->d_dec_nb, status, p->d_ctr);
-        else
-            k_frame_parse<false><<<pgrid, 128, 0, p->stream>>>(d_src, d_offsets, s, d_frame_nb, p->d_nb_state, (uint32_t)F, sel,
-                                                               dec, p->d_headers, p->d_dec_nb, status, p->d_ctr);
-        // code tables of the HUFF blocks from their in-stream trees (unused symbols stay 0)
-        RSPT_CUDA_CHECK(cudaMemsetAsync(p->d_codes, 0, (size_t)nblocks * kSymStride * sizeof(uint32_t), p->stream));
-        k_hzr_recover_codes<<<(nblocks + kRecoverThreads - 1) / kRecoverThreads, kRecoverThreads, 0, p->stream>>>(d_src, nblocks, dec, p->d_codes, s, status);
-        p->launches += 2;
-        if (d_sidecar_out) {
-            k_hzr_build_index<<<nblocks, kIndexThreads, p->dec_smem, p->stream>>>(d_src, s, dec, p->d_codes,
-                                                                                  reinterpret_cast<uint32_t*>(d_sidecar_out), status);
-            p->launches += 1;
-        }
-    }
-    RSPT_CUDA_CHECK(cudaGetLastError());
-    return RSPT_OK;
+    StageTimer t(p, RSPT_STAGE_PARSE);
+    int rc = launch(p, sel.ids ? k_frame_parse<true> : k_frame_parse<false>, (unsigned)((F + 127) / 128), 128, 0, d_src,
+                    d_offsets, s, d_frame_nb, p->d_nb_state, (uint32_t)F, sel, dec, p->d_headers, p->d_dec_nb, status, p->d_ctr);
+    if (rc) return rc;
+    // code tables of the HUFF blocks from their in-stream trees (unused symbols stay 0)
+    RSPT_CUDA_CHECK(cudaMemsetAsync(p->d_codes, 0, (size_t)nblocks * kSymStride * sizeof(uint32_t), p->stream));
+    rc = launch(p, k_hzr_recover_codes, (nblocks + kRecoverThreads - 1) / kRecoverThreads, kRecoverThreads, 0, d_src, nblocks,
+                dec, p->d_codes, s, status);
+    if (!rc && d_sidecar_out)
+        rc = launch(p, k_hzr_build_index, nblocks, kIndexThreads, p->dec_smem, d_src, s, dec, p->d_codes,
+                    reinterpret_cast<uint32_t*>(d_sidecar_out), status);
+    return rc;
 }
 
 // words of the handle's decode-index scratch that one output slot of a gather call owns when the call builds its
@@ -724,21 +695,19 @@ int decompress_batch(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d
         // the classes with short payloads (few busy threads per CTA, latency-bound) run on the side stream
         // beside the full-size blocks
         StageTimer t(p, RSPT_STAGE_DECODE);
-        cudaEventRecord(p->ev_fork, p->stream);
-        cudaStreamWaitEvent(p->side, p->ev_fork, 0);
-        k_hzr_decode<<<nblocks, decode_class_threads(kSmallPayload), decode_class_smem(kSmallPayload), p->side>>>(
-            d_src, s, dec, sc, p->d_codes, p->d_planes, status, flags, 1u);
-        if (maxn > kSmallPayload) {
-            k_hzr_decode<<<nblocks, decode_class_threads(kMediumPayload), decode_class_smem(kMediumPayload), p->side>>>(
-                d_src, s, dec, sc, p->d_codes, p->d_planes, status, flags, 2u);
-            p->launches += 1;
-        }
-        cudaEventRecord(p->ev_join, p->side);
-        k_hzr_decode<<<nblocks, kDecodeThreads, p->dec_smem, p->stream>>>(d_src, s, dec, sc, p->d_codes, p->d_planes, status, flags, 0u);
-        cudaStreamWaitEvent(p->stream, p->ev_join, 0);
-        p->launches += 2;
+        rc = fork_side(p);
+        if (!rc)
+            rc = launch(p, p->side, k_hzr_decode, nblocks, decode_class_threads(kSmallPayload), decode_class_smem(kSmallPayload),
+                        d_src, s, dec, sc, p->d_codes, p->d_planes, status, flags, 1u);
+        if (!rc && maxn > kSmallPayload)
+            rc = launch(p, p->side, k_hzr_decode, nblocks, decode_class_threads(kMediumPayload), decode_class_smem(kMediumPayload),
+                        d_src, s, dec, sc, p->d_codes, p->d_planes, status, flags, 2u);
+        if (!rc)
+            rc = launch(p, k_hzr_decode, nblocks, kDecodeThreads, p->dec_smem, d_src, s, dec, sc, p->d_codes, p->d_planes, status,
+                        flags, 0u);
+        if (!rc) rc = join_side(p);
+        if (rc) return rc;
     }
-    RSPT_CUDA_CHECK(cudaGetLastError());
     StageTimer t(p, RSPT_STAGE_INVERSE);
     return out.words ? launch_inverse_transform_i32(p, out.words, F) : launch_inverse_transform(p, out.raw, F);
 }
@@ -790,13 +759,10 @@ extern "C" int rspt_gpu_verify_batch(rspt_gpu_packer* p, const uint8_t* d_src, c
     const size_t F = n_frames;
     const uint32_t nblocks = total_blocks(p, F);
     DecBlk* dec = reinterpret_cast<DecBlk*>(p->d_dec);
-    k_frame_parse<false><<<(unsigned)((F + 127) / 128), 128, 0, p->stream>>>(d_src, d_offsets, s, d_frame_nb, p->d_nb_state, (uint32_t)F,
-                                                                             FrameSel{nullptr, 0, 0, kIdxWordLimit}, dec, p->d_headers, p->d_dec_nb,
-                                                                             d_status, p->d_ctr);
-    k_hzr_verify<<<nblocks, kVerifyThreads, p->dec_smem, p->stream>>>(d_src, s, dec, p->d_crc, d_status, p->d_ctr);
-    p->launches += 2;
-    RSPT_CUDA_CHECK(cudaGetLastError());
-    return RSPT_OK;
+    const int rc = launch(p, k_frame_parse<false>, (unsigned)((F + 127) / 128), 128, 0, d_src, d_offsets, s, d_frame_nb,
+                          p->d_nb_state, (uint32_t)F, FrameSel{nullptr, 0, 0, kIdxWordLimit}, dec, p->d_headers, p->d_dec_nb,
+                          d_status, p->d_ctr);
+    return rc ? rc : launch(p, k_hzr_verify, nblocks, kVerifyThreads, p->dec_smem, d_src, s, dec, p->d_crc, d_status, p->d_ctr);
 }
 
 
@@ -1334,12 +1300,8 @@ extern "C" int rspt_gpu_debug_hzr_tables(rspt_gpu_packer* p, const uint8_t* d_bl
     DeviceGuard dg(p->device);
     Shape s = p->s;
     s.N = (uint32_t)n; s.nblk = 1; s.nb_alloc = 1; s.plane_stride = (uint32_t)((n + 15) & ~(size_t)15);
-    k_hzr_hist<3><<<1, kHistThreads, kHistSmemList, p->stream>>>(d_block, s, p->d_frame_nb, p->d_hist, p->d_step_lz, p->d_lists, p->d_list_n, p->d_blk_class);
-    k_hzr_hist<2><<<1, kHistThreads, 0, p->stream>>>(d_block, s, p->d_frame_nb, p->d_hist, p->d_step_lz, p->d_lists, p->d_list_n, p->d_blk_class);
-    k_hzr_tree<<<1, 32 * kTreeWarps, 0, p->stream>>>(p->d_hist, s, p->d_frame_nb, p->d_blk_class, kClassSparse, 1, p->d_codes, p->d_tree, p->d_info, p->d_ctr);
-    k_hzr_tree<<<1, 32 * kTreeWarps, 0, p->stream>>>(p->d_hist, s, p->d_frame_nb, p->d_blk_class, kClassDense, 1, p->d_codes, p->d_tree, p->d_info, p->d_ctr);
-    p->launches += 4;
-    RSPT_CUDA_CHECK(cudaGetLastError());
+    const int rc = launch_hist_and_trees(p, d_block, s, 1);
+    if (rc) return rc;
     if (d_hist) RSPT_CUDA_CHECK(cudaMemcpyAsync(d_hist, p->d_hist, kNumSymbols * 4, cudaMemcpyDeviceToDevice, p->stream));
     if (d_codes) RSPT_CUDA_CHECK(cudaMemcpyAsync(d_codes, p->d_codes, kNumSymbols * 4, cudaMemcpyDeviceToDevice, p->stream));
     if (d_info) {
@@ -1360,10 +1322,10 @@ extern "C" int rspt_gpu_crc32c(const uint8_t* d_data, size_t n, uint32_t* h_crc,
     int rc = ensure_device_constants(dev);
     if (rc) return rc;
     uint32_t* d_out = static_cast<uint32_t*>(result_slot(dev));
-    allow_smem(k_crc32c, kEncodeSmem);
-    k_crc32c<<<1, 1024, kEncodeSmem, (cudaStream_t)stream>>>(d_data, (uint32_t)n, g_crc[dev], 3, d_out);
-    cudaError_t e = cudaMemcpyAsync(h_crc, d_out, 4, cudaMemcpyDeviceToHost, (cudaStream_t)stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize((cudaStream_t)stream);
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t e = launch(st, k_crc32c, 1, 1024, kEncodeSmem, d_data, (uint32_t)n, g_crc[dev], 3, d_out);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(h_crc, d_out, 4, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     return e == cudaSuccess ? RSPT_OK : RSPT_E_CUDA;
 }
 
@@ -1463,8 +1425,8 @@ extern "C" int rspt_gpu_synth_ecg(uint8_t* d_dst, uint64_t first_frame, size_t n
     const dim3 grid((unsigned)(n_frames * tiles));
     cudaStream_t st = (cudaStream_t)stream;
     return with_bps(bps, [&](auto B) {
-        k_synth<B><<<grid, 256, 0, st>>>(d_dst, first_frame, (uint32_t)n_frames, ch, ns, prm, g_synth_tab[dev]);
-        return cudaGetLastError() == cudaSuccess ? RSPT_OK : RSPT_E_CUDA;
+        const cudaError_t e = launch(st, k_synth<B>, grid, 256, 0, d_dst, first_frame, (uint32_t)n_frames, ch, ns, prm, g_synth_tab[dev]);
+        return e == cudaSuccess ? RSPT_OK : RSPT_E_CUDA;
     });
 }
 
@@ -1472,18 +1434,23 @@ extern "C" int rspt_gpu_prdn_terms(const uint8_t* d_orig, const uint8_t* d_dec, 
                                    double* h_out, void* stream)
 {
     if (!d_orig || !d_dec || !h_out || bps < 1 || bps > 4) return RSPT_E_ARG;
+    if (n_frames == 0) {
+        h_out[0] = h_out[1] = 0;
+        return RSPT_OK;
+    }
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess) return RSPT_E_NOGPU;
     int rc = ensure_device_constants(dev);
     if (rc) return rc;
     double* d_out = static_cast<double*>(result_slot(dev));
     cudaStream_t st = (cudaStream_t)stream;
-    cudaMemsetAsync(d_out, 0, 16, st);
+    if (cudaMemsetAsync(d_out, 0, 16, st) != cudaSuccess) return RSPT_E_CUDA;
     const dim3 grid((unsigned)(n_frames * ch));
-    with_bps(bps, [&](auto B) {
-        k_prdn<B><<<grid, 256, 0, st>>>(d_orig, d_dec, (uint32_t)n_frames, ch, ns, d_out);
-        return RSPT_OK;
+    rc = with_bps(bps, [&](auto B) {
+        const cudaError_t e = launch(st, k_prdn<B>, grid, 256, 0, d_orig, d_dec, (uint32_t)n_frames, ch, ns, d_out);
+        return e == cudaSuccess ? RSPT_OK : RSPT_E_CUDA;
     });
+    if (rc) return rc;
     cudaError_t e = cudaMemcpyAsync(h_out, d_out, 16, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     return e == cudaSuccess ? RSPT_OK : RSPT_E_CUDA;
@@ -1493,6 +1460,6 @@ extern "C" int rspt_gpu_rebase_offsets(uint64_t* d_offsets, size_t n, const uint
 {
     if (!d_offsets || !d_all_totals || rank < 0) return RSPT_E_ARG;
     if (n == 0 || rank == 0) return RSPT_OK;
-    k_rebase<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(d_offsets, n, d_all_totals, rank);
-    return cudaGetLastError() == cudaSuccess ? RSPT_OK : RSPT_E_CUDA;
+    const cudaError_t e = launch((cudaStream_t)stream, k_rebase, (unsigned)((n + 255) / 256), 256, 0, d_offsets, n, d_all_totals, rank);
+    return e == cudaSuccess ? RSPT_OK : RSPT_E_CUDA;
 }

@@ -1,10 +1,10 @@
-"""Which kernels each sample-side entry point launches, with grid, block and shared memory, as JSON.
+"""Which kernels each entry point of a handle launches, with grid, block and shared memory, as JSON.
 
 A refactor of kernel selection can change which kernel runs without changing any output.  This drives a fixed
 matrix of calls (every packer, the dct exact path, bps 1..4, several channel counts and lengths, 16-byte-aligned
-and 4-byte-offset buffers, the native / int32 / host / debug / pre-filter entry points) under torch.profiler and
-records, per call, the kernels of the library it launched and the handle's kernel_launches count.  Run it once per
-library, each in its own process, and compare:
+and 4-byte-offset buffers, the native / int32 / host / debug / pre-filter / store / gather / index / verify entry
+points) under torch.profiler and records, per call, the kernels of the library it launched and the handle's
+kernel_launches count.  Run it once per library, each in its own process, and compare:
 
     python tools/launch_trace.py --lib rspt_b200/librspt_gpu.so --out new.json
     python tools/launch_trace.py --lib /path/to/other/librspt_gpu.so --out old.json
@@ -74,9 +74,10 @@ def calls(torch, np, p, rng):
 
     st = {}
 
-    def setup():  # what the decompress calls decode
+    def setup():  # what the decompress calls decode, and a store to append to
         st["batch"] = p.compress_batch(raw_view(0))
         st["one"] = p.compress(one)
+        st["store"] = p.new_store(2 * n)
 
     one = raw[:fb].copy()
     out = [("setup", setup)]
@@ -100,6 +101,13 @@ def calls(torch, np, p, rng):
         ("decompress_host", lambda: p.decompress(st["one"])),
         ("compress_batch_host", lambda: p.compress_batch_host(raw, host_dst, host_off)),
         ("decompress_batch_host", lambda: p.decompress_batch_host(host_dst, host_off, host_out)),
+        ("append_batch", lambda: p.append_batch(st["store"], raw_view(0))),
+        ("index_frames", lambda: p.index_frames(st["store"], [1, 0])),
+        ("decompress_frames", lambda: p.decompress_frames(st["batch"], [1, 1])),
+        ("decompress_frames_no_index", lambda: p.decompress_frames(st["batch"], [1, 1], use_sidecar=False)),
+        ("build_index", lambda: p.build_index(st["batch"])),
+        ("verify_batch", lambda: p.verify_batch(st["batch"])),
+        ("debug_hzr_tables", lambda: p.debug_hzr_tables(raw[:min(fb, 65536)])),
     ]
     return out
 
