@@ -14,96 +14,161 @@
 #include "common.cuh"
 #include "hzr_encode.cuh"
 
+namespace rspt {
+
+struct DecBlk;
+struct DeviceFree { void operator()(void* q) const { cudaFree(q); } };
+struct PinnedFree { void operator()(void* q) const { cudaFreeHost(q); } };
+struct StreamDestroy { void operator()(cudaStream_t s) const { cudaStreamDestroy(s); } };
+struct EventDestroy { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
+
+// Sole owner of one CUDA resource, released by Release when the owner is destroyed or reset.  It converts to the
+// raw handle, so that it is used where the handle is.
+template <class H, class Release>
+class Owned {
+public:
+    Owned() = default;
+    Owned(Owned&& o) noexcept : h_(o.release()) {}
+    Owned& operator=(Owned&& o) noexcept { reset(o.release()); return *this; }
+    ~Owned() { reset(); }
+    operator H() const { return h_; }
+    void reset(H h = nullptr) { if (h_) Release()(h_); h_ = h; }
+    H release() { return std::exchange(h_, nullptr); }
+    // make_raw(&h) creates a resource; only if it succeeds does the owner take it, releasing the one it held
+    template <class Make>
+    cudaError_t make(Make&& make_raw)
+    {
+        H h = nullptr;
+        const cudaError_t e = make_raw(&h);
+        if (e == cudaSuccess) reset(h);
+        return e;
+    }
+
+private:
+    H h_ = nullptr;
+};
+
+template <class T> using DeviceBuf = Owned<T*, DeviceFree>;
+template <class T> using PinnedBuf = Owned<T*, PinnedFree>;
+using Stream = Owned<cudaStream_t, StreamDestroy>;
+using Event = Owned<cudaEvent_t, EventDestroy>;
+
+// count elements and `slack` bytes of device memory
+template <class T>
+cudaError_t dalloc(DeviceBuf<T>& b, size_t count, size_t slack = 64)
+{
+    return b.make([&](T** q) { return cudaMalloc(reinterpret_cast<void**>(q), count * sizeof(T) + slack); });
+}
+
+template <class T>
+cudaError_t palloc(PinnedBuf<T>& b, size_t count)
+{
+    return b.make([&](T** q) { return cudaMallocHost(reinterpret_cast<void**>(q), count * sizeof(T)); });
+}
+
+inline cudaError_t create(Stream& s)
+{
+    return s.make([](cudaStream_t* h) { return cudaStreamCreateWithFlags(h, cudaStreamNonBlocking); });
+}
+
+inline cudaError_t create(Event& ev, unsigned flags = cudaEventDisableTiming)
+{
+    return ev.make([&](cudaEvent_t* h) { return cudaEventCreateWithFlags(h, flags); });
+}
+
+}  // namespace rspt
+
 // streams, events and double buffers of the pipelined host-buffer compress (rspt_gpu_compress_batch_host)
 struct HostPipe {
-    cudaStream_t s_in, s_out;
-    cudaEvent_t ev_in[2], ev_comp[2], ev_off[2], ev_out[2];
-    uint8_t* d_src[2];
-    uint8_t* d_dst[2];
-    uint64_t* d_off[2];
-    uint64_t* h_off[2];
-    size_t chunk;  // frames per chunk; 0 = not set up yet
+    rspt::Stream s_in, s_out;
+    rspt::Event ev_in[2], ev_comp[2], ev_off[2], ev_out[2];
+    rspt::DeviceBuf<uint8_t> d_src[2];
+    rspt::DeviceBuf<uint8_t> d_dst[2];
+    rspt::DeviceBuf<uint64_t> d_off[2];
+    rspt::PinnedBuf<uint64_t> h_off[2];
+    size_t chunk = 0;  // frames per chunk; 0 = not set up yet
 };
 
 struct rspt_gpu_packer {
-    rspt::Shape s;
-    int device;
-    cudaStream_t stream;
-    size_t max_batch;
-    size_t enc_smem;       // dynamic shared memory of k_hzr_encode (staging of the largest block)
-    size_t dec_smem;       // dynamic shared memory of k_hzr_decode (payload of the largest block)
-    bool can_escalate;     // xdelta_hzr with nb < bps
-    bool dct_direct;       // dct: O(n^2) bit-exact path (fixed at create time)
+    rspt::Shape s{};
+    int device = 0;
+    cudaStream_t stream = nullptr;          // the caller's
+    size_t max_batch = 0;
+    size_t enc_smem = 0;                    // dynamic shared memory of k_hzr_encode (staging of the largest block)
+    size_t dec_smem = 0;                    // dynamic shared memory of k_hzr_decode (payload of the largest block)
+    bool can_escalate = false;              // xdelta_hzr with nb < bps
+    bool dct_direct = false;                // dct: O(n^2) bit-exact path; set only while d_cos holds the cosine table
 
     // compress scratch
-    uint8_t* d_planes;
-    uint32_t* d_hist;
-    uint32_t* d_codes;
-    uint32_t* d_tree;
-    uint32_t* d_lists;     // per block: sorted non-zero bytes (position | value << 16) of sparse blocks, kListCap entries
-    uint32_t* d_list_n;    // per block: entries in d_lists, kNoList = dense block
-    uint8_t* d_blk_class;  // per block: kClassSparse / kClassDense (density probe of the histogram launches)
-    cudaStream_t side;     // sparse-class histogram + trees run here, beside the dense class on `stream`
+    rspt::DeviceBuf<uint8_t> d_planes;
+    rspt::DeviceBuf<uint32_t> d_hist;
+    rspt::DeviceBuf<uint32_t> d_codes;
+    rspt::DeviceBuf<uint32_t> d_tree;
+    rspt::DeviceBuf<uint32_t> d_lists;      // per block: sorted non-zero bytes (position | value << 16) of sparse blocks, kListCap entries
+    rspt::DeviceBuf<uint32_t> d_list_n;     // per block: entries in d_lists, kNoList = dense block
+    rspt::DeviceBuf<uint8_t> d_blk_class;   // per block: kClassSparse / kClassDense (density probe of the histogram launches)
+    rspt::Stream side;                      // sparse-class histogram + trees run here, beside the dense class on `stream`
     // fork_side / join_side: one pair serves every fork and join of a call, since cudaStreamWaitEvent waits for
     // the event's last record before the wait was enqueued
-    cudaEvent_t ev_fork, ev_join;
-    cudaStream_t place;    // multi-GPU placement (all-gather of totals + offset rebase) runs here, off the compute stream
-    cudaEvent_t ev_place;
+    rspt::Event ev_fork, ev_join;
+    rspt::Stream place;                     // multi-GPU placement (all-gather of totals + offset rebase) runs here, off the compute stream
+    rspt::Event ev_place;
     // placements possibly still in flight, by the offsets array they rewrite: a later compress into the same
     // array waits for its own entry only (rspt_gpu_place_offsets_async)
     static constexpr int kPlaceRing = 4;
-    cudaEvent_t ev_placed[kPlaceRing];
-    const void* placed_ptr[kPlaceRing];
-    unsigned place_seq;
-    uint64_t* d_all_totals;
-    uint16_t* d_step_lz;   // per 512-byte step of every block: leading zero count (512 = all zero)
-    rspt::BlkInfo* d_info;
-    uint8_t* d_frame_nb;
-    uint32_t* d_need;
-    uint32_t* d_nb_state;
-    uint32_t* d_sizes;
-    uint32_t* d_blk_off;   // per block: offset of its header from the frame start
-    uint8_t* d_headers;
-    int32_t* d_words;      // hadamard / dct: de-interleaved samples, then coefficients
-    long long* d_sums;     // hadamard / dct: per (frame, channel) sample sums
-    rspt::Counters* d_ctr;
-    const rspt::CrcConst* d_crc;
+    rspt::Event ev_placed[kPlaceRing];
+    const void* placed_ptr[kPlaceRing] = {};
+    unsigned place_seq = 0;
+    rspt::DeviceBuf<uint64_t> d_all_totals;
+    rspt::DeviceBuf<uint16_t> d_step_lz;    // per 512-byte step of every block: leading zero count (512 = all zero)
+    rspt::DeviceBuf<rspt::BlkInfo> d_info;
+    rspt::DeviceBuf<uint8_t> d_frame_nb;
+    rspt::DeviceBuf<uint32_t> d_need;
+    rspt::DeviceBuf<uint32_t> d_nb_state;
+    rspt::DeviceBuf<uint32_t> d_sizes;
+    rspt::DeviceBuf<uint32_t> d_blk_off;    // per block: offset of its header from the frame start
+    rspt::DeviceBuf<uint8_t> d_headers;
+    rspt::DeviceBuf<int32_t> d_words;       // hadamard / dct: de-interleaved samples, then coefficients
+    rspt::DeviceBuf<long long> d_sums;      // hadamard / dct: per (frame, channel) sample sums
+    rspt::DeviceBuf<rspt::Counters> d_ctr;
+    const rspt::CrcConst* d_crc = nullptr;  // per device, for the life of the process
     // decompress scratch
-    void* d_dec;           // block descriptors
-    uint8_t* d_dec_nb;     // per-frame plane count used by the last decompress
-    int32_t* d_status_tmp;
-    void* d_auto_index;    // decode index built here for streams that came without one
-    double* d_fir;         // FIR kernel coefficients of the last rspt_gpu_prefilter_fir call (lazy)
-    size_t fir_cap;
-    int32_t* d_words2;     // second word buffer (FIR is out of place), lazy
-    uint32_t sp_stage;     // payload limit of k_hzr_encode_sparse (kSpStageBytes; lower only under RSPT_SPARSE_STAGE_BYTES)
+    rspt::DeviceBuf<rspt::DecBlk> d_dec;    // block descriptors
+    rspt::DeviceBuf<uint8_t> d_dec_nb;      // per-frame plane count used by the last decompress
+    rspt::DeviceBuf<int32_t> d_status_tmp;
+    rspt::DeviceBuf<uint32_t> d_auto_index; // decode index built here for streams that came without one
+    rspt::DeviceBuf<double> d_fir;          // FIR kernel coefficients of the last rspt_gpu_prefilter_fir call (lazy)
+    size_t fir_cap = 0;                     // coefficients d_fir holds room for
+    rspt::DeviceBuf<int32_t> d_words2;      // second word buffer (FIR is out of place), lazy
+    uint32_t sp_stage = 0;                  // payload limit of k_hzr_encode_sparse (kSpStageBytes; lower only under RSPT_SPARSE_STAGE_BYTES)
     // transform constants (dct twiddles)
-    double2* d_twiddle;
-    double2* d_post;
-    float* d_cos;          // dct direct path: the reference's float cosine table
+    rspt::DeviceBuf<double2> d_twiddle;
+    rspt::DeviceBuf<double2> d_post;
+    rspt::DeviceBuf<float> d_cos;           // dct direct path: the reference's float cosine table
     // single-frame host API staging
-    uint8_t* d_one_src;
-    uint8_t* d_one_dst;
-    uint64_t* d_one_off;
-    uint8_t* h_pin;
-    size_t h_pin_bytes;
+    rspt::DeviceBuf<uint8_t> d_one_src;
+    rspt::DeviceBuf<uint8_t> d_one_dst;
+    rspt::DeviceBuf<uint64_t> d_one_off;
+    rspt::PinnedBuf<uint8_t> h_pin;
     HostPipe pipe;
 
-    unsigned long long launches;
+    unsigned long long launches = 0;
     // stage timing
-    bool timing;
-    std::vector<cudaEvent_t>* ev_free;
-    struct Pending { int stage; cudaEvent_t a, b; };
-    std::vector<Pending>* ev_pending;
-    double stage_ms[8];
-    unsigned long long stage_calls[8];
-    char err[256];
+    bool timing = false;
+    std::vector<rspt::Event> ev_free;
+    struct Pending { int stage; rspt::Event a, b; };
+    std::vector<Pending> ev_pending;
+    double stage_ms[8] = {};
+    unsigned long long stage_calls[8] = {};
+    char err[256] = {};
 };
 
 namespace rspt {
 
 inline int fail_cuda(rspt_gpu_packer* p, cudaError_t e, const char* what)
 {
+    // the failed call's error is also the thread's last error: cleared, or the next launch reports it as its own
+    cudaGetLastError();
     if (p) snprintf(p->err, sizeof(p->err), "CUDA error %d (%s) at %s", (int)e, cudaGetErrorString(e), what);
     return -2;  // RSPT_E_CUDA
 }

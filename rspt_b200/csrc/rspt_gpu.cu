@@ -8,6 +8,7 @@
 #include <stdlib.h>
 
 #include <atomic>
+#include <memory>
 #include <mutex>
 #include <new>
 #include <vector>
@@ -79,29 +80,23 @@ int ensure_device_constants(int dev)
         for (int b = 0; b < 4; ++b)
             for (uint32_t v = 0; v < 256; ++v) c.zt32[b][v] = h_multmodp(z, v << (8 * b));
     }
-    CrcConst* d = nullptr;
-    if (cudaMalloc(&d, sizeof(CrcConst)) != cudaSuccess) return RSPT_E_CUDA;
-    if (cudaMemcpy(d, &c, sizeof(CrcConst), cudaMemcpyHostToDevice) != cudaSuccess) return RSPT_E_CUDA;
     std::vector<int32_t> tab(2 * RSPT_SYNTH_TABLE);
     rspt_synth_build_tables(tab.data(), tab.data() + RSPT_SYNTH_TABLE);
-    int32_t* dt = nullptr;
-    if (cudaMalloc(&dt, tab.size() * sizeof(int32_t)) != cudaSuccess) return RSPT_E_CUDA;
-    if (cudaMemcpy(dt, tab.data(), tab.size() * sizeof(int32_t), cudaMemcpyHostToDevice) != cudaSuccess) return RSPT_E_CUDA;
-    uint8_t* ring = nullptr;
-    if (cudaMalloc(&ring, 64 * 16) != cudaSuccess) return RSPT_E_CUDA;
-    g_result_ring[dev] = ring;
-    g_crc[dev] = d;
-    g_synth_tab[dev] = dt;
+    // all three or none: a failed call leaves nothing behind, and the next one starts over
+    DeviceBuf<CrcConst> d;
+    DeviceBuf<int32_t> dt;
+    DeviceBuf<uint8_t> ring;
+    if (dalloc(d, 1, 0) != cudaSuccess || dalloc(dt, tab.size(), 0) != cudaSuccess || dalloc(ring, 64 * 16, 0) != cudaSuccess ||
+        cudaMemcpy(d, &c, sizeof(CrcConst), cudaMemcpyHostToDevice) != cudaSuccess ||
+        cudaMemcpy(dt, tab.data(), tab.size() * sizeof(int32_t), cudaMemcpyHostToDevice) != cudaSuccess)
+        return RSPT_E_CUDA;
+    g_result_ring[dev] = ring.release();
+    g_crc[dev] = d.release();
+    g_synth_tab[dev] = dt.release();
     return RSPT_OK;
 }
 
 size_t hzr_max(size_t n) { return 4 + (n ? ((n + kBlock - 1) / kBlock) * 7 + n : 0); }
-
-template <class T>
-cudaError_t dalloc(T*& ptr, size_t count)
-{
-    return cudaMalloc(reinterpret_cast<void**>(&ptr), count * sizeof(T) + 64);
-}
 
 struct DeviceGuard {
     int prev = -1;
@@ -116,8 +111,6 @@ struct DeviceGuard {
         if (prev >= 0) cudaSetDevice(prev);
     }
 };
-
-void destroy_host_pipe(rspt_gpu_packer* p);
 
 uint32_t total_blocks(const rspt_gpu_packer* p, size_t frames) { return (uint32_t)(frames * p->s.nb_alloc * p->s.nblk); }
 
@@ -134,36 +127,36 @@ bool stored_ordinals_fit(const rspt_gpu_packer* p, size_t n_stored)
 // ---------------------------------------------------------------------------------------------
 namespace {
 
-cudaEvent_t ev_get(rspt_gpu_packer* p)
+Event ev_get(rspt_gpu_packer* p)
 {
-    if (!p->ev_free->empty()) {
-        cudaEvent_t e = p->ev_free->back();
-        p->ev_free->pop_back();
-        return e;
+    Event e;
+    if (p->ev_free.empty()) {
+        create(e, cudaEventDefault);
+    } else {
+        e = std::move(p->ev_free.back());
+        p->ev_free.pop_back();
     }
-    cudaEvent_t e = nullptr;
-    cudaEventCreate(&e);
     return e;
 }
 
 void ev_resolve(rspt_gpu_packer* p)
 {
-    for (auto& q : *p->ev_pending) {
+    for (auto& q : p->ev_pending) {
         float ms = 0;
         if (cudaEventSynchronize(q.b) == cudaSuccess && cudaEventElapsedTime(&ms, q.a, q.b) == cudaSuccess) {
             p->stage_ms[q.stage] += ms;
             p->stage_calls[q.stage] += 1;
         }
-        p->ev_free->push_back(q.a);
-        p->ev_free->push_back(q.b);
+        p->ev_free.push_back(std::move(q.a));
+        p->ev_free.push_back(std::move(q.b));
     }
-    p->ev_pending->clear();
+    p->ev_pending.clear();
 }
 
 struct StageTimer {
     rspt_gpu_packer* p;
     int stage;
-    cudaEvent_t a = nullptr;
+    Event a;
     StageTimer(rspt_gpu_packer* p_, int stage_) : p(p_), stage(stage_)
     {
         if (p->timing) {
@@ -174,10 +167,10 @@ struct StageTimer {
     ~StageTimer()
     {
         if (a) {
-            cudaEvent_t b = ev_get(p);
+            Event b = ev_get(p);
             cudaEventRecord(b, p->stream);
-            p->ev_pending->push_back({stage, a, b});
-            if (p->ev_pending->size() > 4096) ev_resolve(p);
+            p->ev_pending.push_back({stage, std::move(a), std::move(b)});
+            if (p->ev_pending.size() > 4096) ev_resolve(p);
         }
     }
 };
@@ -210,6 +203,67 @@ extern "C" int rspt_gpu_get_stage_times(rspt_gpu_packer* p, double* ms, uint64_t
 // ---------------------------------------------------------------------------------------------
 // create / destroy
 // ---------------------------------------------------------------------------------------------
+// Everything rspt_gpu_create allocates, in order, stopping at the first failure.  Nothing is enqueued on the
+// caller's stream before the last call that can fail to allocate, except the dct table uploads.
+static int alloc_handle(rspt_gpu_packer* p)
+{
+    const Shape& s = p->s;
+    const size_t F = p->max_batch, nblocks = F * s.nb_alloc * s.nblk;
+    RSPT_CUDA_CHECK(dalloc(p->d_planes, F * s.nb_alloc * (size_t)s.plane_stride));
+    RSPT_CUDA_CHECK(dalloc(p->d_hist, nblocks * kSymStride));
+    RSPT_CUDA_CHECK(dalloc(p->d_codes, nblocks * kSymStride));
+    RSPT_CUDA_CHECK(dalloc(p->d_tree, nblocks * kTreeWords));
+    RSPT_CUDA_CHECK(dalloc(p->d_step_lz, nblocks * kMaxSteps));
+    RSPT_CUDA_CHECK(dalloc(p->d_lists, nblocks * (size_t)kListCap));
+    RSPT_CUDA_CHECK(dalloc(p->d_list_n, nblocks));
+    RSPT_CUDA_CHECK(dalloc(p->d_blk_class, nblocks));
+    RSPT_CUDA_CHECK(dalloc(p->d_info, nblocks));
+    RSPT_CUDA_CHECK(dalloc(p->d_frame_nb, F));
+    RSPT_CUDA_CHECK(dalloc(p->d_need, F));
+    RSPT_CUDA_CHECK(dalloc(p->d_nb_state, 4));
+    RSPT_CUDA_CHECK(dalloc(p->d_all_totals, 64));
+    RSPT_CUDA_CHECK(dalloc(p->d_sizes, F));
+    RSPT_CUDA_CHECK(dalloc(p->d_blk_off, nblocks));
+    RSPT_CUDA_CHECK(dalloc(p->d_headers, F * (s.hdr_bytes ? s.hdr_bytes : 1)));
+    RSPT_CUDA_CHECK(dalloc(p->d_ctr, 1));
+    RSPT_CUDA_CHECK(dalloc(p->d_status_tmp, F));
+    RSPT_CUDA_CHECK(dalloc(p->d_dec_nb, F));
+    RSPT_CUDA_CHECK(dalloc(p->d_dec, nblocks));
+    // the batch addressing needs ((F * max_compressed_size) >> 6) + nblocks + 2 words, a gather call's per-slot
+    // regions (gather_slot_region) F * ((max_compressed_size >> 6) + nb_alloc * nblk + 1): F more cover both
+    RSPT_CUDA_CHECK(dalloc(p->d_auto_index, ((F * (1 + s.hdr_bytes + (size_t)s.nb_alloc * (4 + hzr_max(s.N))) >> 6) + nblocks + F + 2)));
+    if (s.kind == RSPT_HADAMARD || s.kind == RSPT_DCT) {
+        RSPT_CUDA_CHECK(dalloc(p->d_words, F * (size_t)s.N));
+        RSPT_CUDA_CHECK(dalloc(p->d_sums, F * (size_t)s.ch));
+    }
+    if (s.kind == RSPT_DCT && (s.ns & (s.ns - 1)) == 0) RSPT_CUDA_CHECK(dct_build_fft_tables(p));
+    if (p->dct_direct) RSPT_CUDA_CHECK(dct_build_cos_table(p));
+    const size_t maxc = rspt_gpu_max_compressed_size(p);
+    RSPT_CUDA_CHECK(dalloc(p->d_one_src, (size_t)s.frame_bytes));
+    RSPT_CUDA_CHECK(dalloc(p->d_one_dst, maxc));
+    RSPT_CUDA_CHECK(dalloc(p->d_one_off, 2));
+    RSPT_CUDA_CHECK(palloc(p->h_pin, (maxc > s.frame_bytes ? maxc : s.frame_bytes) + 64));
+    // the hzr kernels go to the most dynamic shared memory any shape launches them with (see launch)
+    RSPT_CUDA_CHECK(raise_smem_limit(k_hzr_encode<2>, kEncodeSmem));
+    RSPT_CUDA_CHECK(raise_smem_limit(k_hzr_encode<3>, kEncodeSmem));
+    RSPT_CUDA_CHECK(raise_smem_limit(k_hzr_hist<3>, kHistSmemList));
+    RSPT_CUDA_CHECK(raise_smem_limit(k_hzr_encode_sparse, kSparseSmem));
+    RSPT_CUDA_CHECK(raise_smem_limit(k_hzr_decode, kDecodeSmem));
+    RSPT_CUDA_CHECK(raise_smem_limit(k_hzr_verify, kDecodeSmem));
+    RSPT_CUDA_CHECK(raise_smem_limit(k_hzr_build_index, kDecodeSmem));
+    RSPT_CUDA_CHECK(create(p->side));
+    RSPT_CUDA_CHECK(create(p->place));
+    RSPT_CUDA_CHECK(create(p->ev_place));
+    for (Event& ev : p->ev_placed) RSPT_CUDA_CHECK(create(ev));
+    RSPT_CUDA_CHECK(create(p->ev_fork));
+    RSPT_CUDA_CHECK(create(p->ev_join));
+    RSPT_CUDA_CHECK(cudaMemsetAsync(p->d_frame_nb, (int)s.nb_init, F, p->stream));
+    RSPT_CUDA_CHECK(cudaMemsetAsync(p->d_ctr, 0, sizeof(Counters), p->stream));
+    RSPT_CUDA_CHECK(cudaMemcpyAsync(p->d_nb_state, &s.nb_init, 4, cudaMemcpyHostToDevice, p->stream));
+    RSPT_CUDA_CHECK(cudaStreamSynchronize(p->stream));
+    return RSPT_OK;
+}
+
 extern "C" int rspt_gpu_create(int kind, size_t bps, size_t ch, size_t ns, size_t nb, int device, void* stream,
                                size_t max_batch_frames, rspt_gpu_packer** out)
 {
@@ -233,9 +287,8 @@ extern "C" int rspt_gpu_create(int kind, size_t bps, size_t ch, size_t ns, size_
     int rc = ensure_device_constants(device);
     if (rc != RSPT_OK) return rc;
 
-    rspt_gpu_packer* p = new (std::nothrow) rspt_gpu_packer();
+    std::unique_ptr<rspt_gpu_packer> p(new (std::nothrow) rspt_gpu_packer());
     if (!p) return RSPT_E_ARG;
-    memset(p, 0, sizeof(*p));
     Shape& s = p->s;
     s.kind = kind; s.bps = (int)bps; s.ch = (int)ch; s.ns = (int)ns;
     s.N = (uint32_t)(ch * ns);
@@ -249,8 +302,6 @@ extern "C" int rspt_gpu_create(int kind, size_t bps, size_t ch, size_t ns, size_
     s.plane_stride = (s.N + 15u) & ~15u;
     s.frame_bytes = (uint32_t)(bps * ch * ns);
     s.method = kind == RSPT_DCT ? 1u : (kind == RSPT_HADAMARD ? 2u : 0u);
-    p->ev_free = new std::vector<cudaEvent_t>();
-    p->ev_pending = new std::vector<rspt_gpu_packer::Pending>();
     p->device = device;
     p->max_batch = max_batch_frames;
     p->d_crc = g_crc[device];
@@ -258,76 +309,18 @@ extern "C" int rspt_gpu_create(int kind, size_t bps, size_t ch, size_t ns, size_
     p->enc_smem = (size_t)(12 + (maxn + 3) / 4 + 8) * 4;  // staging of the largest block: header + payload at an offset of <= 38 bytes, + slack
     p->dec_smem = ((size_t)(maxn + 30) / 16 + 2) * 16;   // the 16-byte chunks that hold the largest payload (any alignment) + zero slack
     p->stream = (cudaStream_t)stream;  // NULL = the CUDA default stream
-    const size_t F = max_batch_frames, nblocks = F * s.nb_alloc * s.nblk;
-    cudaError_t e = cudaSuccess;
-    auto A = [&](cudaError_t r) { if (e == cudaSuccess) e = r; };
-    A(dalloc(p->d_planes, F * s.nb_alloc * (size_t)s.plane_stride));
-    A(dalloc(p->d_hist, nblocks * kSymStride));
-    A(dalloc(p->d_codes, nblocks * kSymStride));
-    A(dalloc(p->d_tree, nblocks * kTreeWords));
-    A(dalloc(p->d_step_lz, nblocks * kMaxSteps));
-    A(dalloc(p->d_lists, nblocks * (size_t)kListCap));
-    A(dalloc(p->d_list_n, nblocks));
-    A(dalloc(p->d_blk_class, nblocks));
-    A(dalloc(p->d_info, nblocks));
-    A(dalloc(p->d_frame_nb, F));
-    A(dalloc(p->d_need, F));
-    A(dalloc(p->d_nb_state, 4));
-    A(dalloc(p->d_all_totals, 64));
-    A(dalloc(p->d_sizes, F));
-    A(dalloc(p->d_blk_off, nblocks));
-    A(dalloc(p->d_headers, F * (s.hdr_bytes ? s.hdr_bytes : 1)));
-    A(dalloc(p->d_ctr, 1));
-    A(dalloc(p->d_status_tmp, F));
-    A(dalloc(p->d_dec_nb, F));
-    A(cudaMalloc(&p->d_dec, nblocks * sizeof(DecBlk) + 64));
-    // the batch addressing needs ((F * max_compressed_size) >> 6) + nblocks + 2 words, a gather call's per-slot
-    // regions (gather_slot_region) F * ((max_compressed_size >> 6) + nb_alloc * nblk + 1): F more cover both
-    A(cudaMalloc(&p->d_auto_index, ((F * (1 + s.hdr_bytes + (size_t)s.nb_alloc * (4 + hzr_max(s.N))) >> 6) + nblocks + F + 2) * sizeof(uint32_t) + 64));
-    if (kind == RSPT_HADAMARD || kind == RSPT_DCT) {
-        A(dalloc(p->d_words, F * (size_t)s.N));
-        A(dalloc(p->d_sums, F * (size_t)s.ch));
-    }
     p->dct_direct = kind == RSPT_DCT && dct_choose_direct((uint32_t)ns);
-    if (e == cudaSuccess && kind == RSPT_DCT) e = dct_build_tables(p);
-    const size_t maxc = rspt_gpu_max_compressed_size(p);
-    A(dalloc(p->d_one_src, (size_t)s.frame_bytes));
-    A(dalloc(p->d_one_dst, maxc));
-    A(dalloc(p->d_one_off, 2));
-    p->h_pin_bytes = maxc > s.frame_bytes ? maxc : s.frame_bytes;
-    p->h_pin_bytes += 64;
-    if (e == cudaSuccess) e = cudaMallocHost(reinterpret_cast<void**>(&p->h_pin), p->h_pin_bytes);
-    if (e == cudaSuccess) e = cudaMemsetAsync(p->d_frame_nb, (int)s.nb_init, F, p->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(p->d_ctr, 0, sizeof(Counters), p->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(p->d_nb_state, &s.nb_init, 4, cudaMemcpyHostToDevice, p->stream);
-    // the hzr kernels go to the most dynamic shared memory any shape launches them with (see launch)
-    if (e == cudaSuccess) e = raise_smem_limit(k_hzr_encode<2>, kEncodeSmem);
-    if (e == cudaSuccess) e = raise_smem_limit(k_hzr_encode<3>, kEncodeSmem);
-    if (e == cudaSuccess) e = raise_smem_limit(k_hzr_hist<3>, kHistSmemList);
-    if (e == cudaSuccess) e = raise_smem_limit(k_hzr_encode_sparse, kSparseSmem);
-    if (e == cudaSuccess) e = raise_smem_limit(k_hzr_decode, kDecodeSmem);
-    if (e == cudaSuccess) e = raise_smem_limit(k_hzr_verify, kDecodeSmem);
-    if (e == cudaSuccess) e = raise_smem_limit(k_hzr_build_index, kDecodeSmem);
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&p->side, cudaStreamNonBlocking);
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&p->place, cudaStreamNonBlocking);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p->ev_place, cudaEventDisableTiming);
-    for (int k = 0; k < rspt_gpu_packer::kPlaceRing && e == cudaSuccess; ++k)
-        e = cudaEventCreateWithFlags(&p->ev_placed[k], cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p->ev_fork, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p->ev_join, cudaEventDisableTiming);
     {
         // test hook: a smaller staging limit sends listed blocks down the hand-over path to k_hzr_encode
         const char* ev = getenv("RSPT_SPARSE_STAGE_BYTES");
         const long v = ev ? atol(ev) : (long)kSpStageBytes;
         p->sp_stage = (uint32_t)(v < 1 ? 1 : (v > (long)kSpStageBytes ? (long)kSpStageBytes : v));
     }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(p->stream);
-    if (e != cudaSuccess) {
-        fprintf(stderr, "rspt_gpu_create: %s\n", cudaGetErrorString(e));
-        rspt_gpu_destroy(p);
+    if (alloc_handle(p.get()) != RSPT_OK) {
+        fprintf(stderr, "rspt_gpu_create: %s\n", p->err);
         return RSPT_E_CUDA;
     }
-    *out = p;
+    *out = p.release();
     return RSPT_OK;
 }
 
@@ -335,27 +328,10 @@ extern "C" int rspt_gpu_destroy(rspt_gpu_packer* p)
 {
     if (!p) return RSPT_E_ARG;
     DeviceGuard dg(p->device);
+    // work still queued on the caller's stream or the handle's own may use what the handle owns
     cudaStreamSynchronize(p->stream);
-    void* ptrs[] = {p->d_planes, p->d_hist, p->d_codes, p->d_tree, p->d_step_lz, p->d_lists, p->d_list_n, p->d_blk_class, p->d_info, p->d_frame_nb,
-                    p->d_need, p->d_nb_state, p->d_sizes, p->d_blk_off, p->d_headers, p->d_words, p->d_sums, p->d_ctr,
-                    p->d_dec, p->d_dec_nb, p->d_status_tmp, p->d_twiddle, p->d_post, p->d_cos, p->d_one_src, p->d_one_dst,
-                    p->d_one_off, p->d_auto_index, p->d_fir, p->d_words2, p->d_all_totals};
-    for (void* q : ptrs)
-        if (q) cudaFree(q);
-    if (p->h_pin) cudaFreeHost(p->h_pin);
-    destroy_host_pipe(p);
-    if (p->ev_pending) {
-        ev_resolve(p);
-        for (cudaEvent_t e : *p->ev_free) cudaEventDestroy(e);
-        delete p->ev_pending;
-        delete p->ev_free;
-    }
-    if (p->side) cudaStreamDestroy(p->side);
-    if (p->place) cudaStreamDestroy(p->place);
-    if (p->ev_place) cudaEventDestroy(p->ev_place);
-    for (cudaEvent_t ev : p->ev_placed) if (ev) cudaEventDestroy(ev);
-    if (p->ev_fork) cudaEventDestroy(p->ev_fork);
-    if (p->ev_join) cudaEventDestroy(p->ev_join);
+    for (const Stream* st : {&p->side, &p->place, &p->pipe.s_in, &p->pipe.s_out})
+        if (*st) cudaStreamSynchronize(*st);
     delete p;
     return RSPT_OK;
 }
@@ -598,17 +574,16 @@ int launch_parse_and_index(rspt_gpu_packer* p, const uint8_t* d_src, const uint6
 {
     const Shape& s = p->s;
     const uint32_t nblocks = total_blocks(p, F);
-    DecBlk* dec = reinterpret_cast<DecBlk*>(p->d_dec);
     StageTimer t(p, RSPT_STAGE_PARSE);
     int rc = launch(p, sel.ids ? k_frame_parse<true> : k_frame_parse<false>, (unsigned)((F + 127) / 128), 128, 0, d_src,
-                    d_offsets, s, d_frame_nb, p->d_nb_state, (uint32_t)F, sel, dec, p->d_headers, p->d_dec_nb, status, p->d_ctr);
+                    d_offsets, s, d_frame_nb, p->d_nb_state, (uint32_t)F, sel, p->d_dec, p->d_headers, p->d_dec_nb, status, p->d_ctr);
     if (rc) return rc;
     // code tables of the HUFF blocks from their in-stream trees (unused symbols stay 0)
     RSPT_CUDA_CHECK(cudaMemsetAsync(p->d_codes, 0, (size_t)nblocks * kSymStride * sizeof(uint32_t), p->stream));
     rc = launch(p, k_hzr_recover_codes, (nblocks + kRecoverThreads - 1) / kRecoverThreads, kRecoverThreads, 0, d_src, nblocks,
-                dec, p->d_codes, s, status);
+                p->d_dec, p->d_codes, s, status);
     if (!rc && d_sidecar_out)
-        rc = launch(p, k_hzr_build_index, nblocks, kIndexThreads, p->dec_smem, d_src, s, dec, p->d_codes,
+        rc = launch(p, k_hzr_build_index, nblocks, kIndexThreads, p->dec_smem, d_src, s, p->d_dec, p->d_codes,
                     reinterpret_cast<uint32_t*>(d_sidecar_out), status);
     return rc;
 }
@@ -675,7 +650,6 @@ int decompress_batch(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d
     const size_t F = n_frames;
     const uint32_t nblocks = total_blocks(p, F);
     int32_t* status = d_status ? d_status : p->d_status_tmp;
-    DecBlk* dec = reinterpret_cast<DecBlk*>(p->d_dec);
     // Without an explicit per-frame plane count every frame uses the instance's current count,
     // as the reference's decompress does (signal_packer_xdelta_hzr.cpp:77).
     void* own_index = nullptr;
@@ -698,12 +672,12 @@ int decompress_batch(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d
         rc = fork_side(p);
         if (!rc)
             rc = launch(p, p->side, k_hzr_decode, nblocks, decode_class_threads(kSmallPayload), decode_class_smem(kSmallPayload),
-                        d_src, s, dec, sc, p->d_codes, p->d_planes, status, flags, 1u);
+                        d_src, s, p->d_dec, sc, p->d_codes, p->d_planes, status, flags, 1u);
         if (!rc && maxn > kSmallPayload)
             rc = launch(p, p->side, k_hzr_decode, nblocks, decode_class_threads(kMediumPayload), decode_class_smem(kMediumPayload),
-                        d_src, s, dec, sc, p->d_codes, p->d_planes, status, flags, 2u);
+                        d_src, s, p->d_dec, sc, p->d_codes, p->d_planes, status, flags, 2u);
         if (!rc)
-            rc = launch(p, k_hzr_decode, nblocks, kDecodeThreads, p->dec_smem, d_src, s, dec, sc, p->d_codes, p->d_planes, status,
+            rc = launch(p, k_hzr_decode, nblocks, kDecodeThreads, p->dec_smem, d_src, s, p->d_dec, sc, p->d_codes, p->d_planes, status,
                         flags, 0u);
         if (!rc) rc = join_side(p);
         if (rc) return rc;
@@ -758,11 +732,10 @@ extern "C" int rspt_gpu_verify_batch(rspt_gpu_packer* p, const uint8_t* d_src, c
     const Shape& s = p->s;
     const size_t F = n_frames;
     const uint32_t nblocks = total_blocks(p, F);
-    DecBlk* dec = reinterpret_cast<DecBlk*>(p->d_dec);
     const int rc = launch(p, k_frame_parse<false>, (unsigned)((F + 127) / 128), 128, 0, d_src, d_offsets, s, d_frame_nb,
-                          p->d_nb_state, (uint32_t)F, FrameSel{nullptr, 0, 0, kIdxWordLimit}, dec, p->d_headers, p->d_dec_nb,
+                          p->d_nb_state, (uint32_t)F, FrameSel{nullptr, 0, 0, kIdxWordLimit}, p->d_dec, p->d_headers, p->d_dec_nb,
                           d_status, p->d_ctr);
-    return rc ? rc : launch(p, k_hzr_verify, nblocks, kVerifyThreads, p->dec_smem, d_src, s, dec, p->d_crc, d_status, p->d_ctr);
+    return rc ? rc : launch(p, k_hzr_verify, nblocks, kVerifyThreads, p->dec_smem, d_src, s, p->d_dec, p->d_crc, d_status, p->d_ctr);
 }
 
 
@@ -875,16 +848,7 @@ extern "C" int rspt_gpu_set_dct_exact(rspt_gpu_packer* p, int exact)
     if (!p || p->s.kind != RSPT_DCT) return RSPT_E_ARG;
     if (!exact && ((p->s.ns & (p->s.ns - 1)) != 0)) return fail_arg(p, "the FFT path needs a power-of-two length");
     DeviceGuard dg(p->device);
-    if (exact && !p->d_cos) {
-        // the cosine table is built on first use (the twiddles of the FFT path are rebuilt with it)
-        RSPT_CUDA_CHECK(cudaStreamSynchronize(p->stream));
-        if (p->d_twiddle) cudaFree(p->d_twiddle);
-        if (p->d_post) cudaFree(p->d_post);
-        p->d_twiddle = nullptr;
-        p->d_post = nullptr;
-        p->dct_direct = true;
-        RSPT_CUDA_CHECK(dct_build_tables(p));
-    }
+    if (exact && !p->d_cos) RSPT_CUDA_CHECK(dct_build_cos_table(p));  // built on first use
     p->dct_direct = exact != 0;
     return RSPT_OK;
 }
@@ -893,11 +857,11 @@ extern "C" int rspt_gpu_set_dct_exact(rspt_gpu_packer* p, int exact)
 // streaming ingest ring (io_buffer, lib_ring_buffer/ring_buffers.h:150-201, with pinned packets)
 // ---------------------------------------------------------------------------------------------
 struct rspt_gpu_ingest {
-    rspt_gpu_packer* p;
-    size_t packet_bytes, nr_max_packets;
-    uint8_t* buffer;                   // pinned, nr_max_packets * packet_bytes
-    std::atomic<uint8_t>* rw_states;   // 0 free, 1 being filled, 2 filled, 3 consumed
-    size_t it_read, it_write, it_write_last;
+    rspt_gpu_packer* p = nullptr;
+    size_t packet_bytes = 0, nr_max_packets = 0;
+    PinnedBuf<uint8_t> buffer;                          // nr_max_packets * packet_bytes
+    std::unique_ptr<std::atomic<uint8_t>[]> rw_states;  // 0 free, 1 being filled, 2 filled, 3 consumed
+    size_t it_read = 0, it_write = 0, it_write_last = 0;
 };
 
 extern "C" int rspt_gpu_ingest_create(rspt_gpu_packer* p, size_t nr_max_packets, rspt_gpu_ingest** out)
@@ -905,21 +869,11 @@ extern "C" int rspt_gpu_ingest_create(rspt_gpu_packer* p, size_t nr_max_packets,
     if (!p || !out || nr_max_packets < 2) return RSPT_E_ARG;
     *out = nullptr;
     DeviceGuard dg(p->device);
-    rspt_gpu_ingest* g = new (std::nothrow) rspt_gpu_ingest();
+    std::unique_ptr<rspt_gpu_ingest> g(new (std::nothrow) rspt_gpu_ingest{p, p->s.frame_bytes, nr_max_packets});
     if (!g) return RSPT_E_ARG;
-    g->p = p;
-    g->packet_bytes = p->s.frame_bytes;
-    g->nr_max_packets = nr_max_packets;
-    g->it_read = g->it_write = g->it_write_last = 0;
-    g->buffer = nullptr;
-    g->rw_states = new (std::nothrow) std::atomic<uint8_t>[nr_max_packets];
-    if (!g->rw_states || cudaMallocHost(reinterpret_cast<void**>(&g->buffer), nr_max_packets * g->packet_bytes) != cudaSuccess) {
-        delete[] g->rw_states;
-        delete g;
-        return RSPT_E_CUDA;
-    }
-    for (size_t i = 0; i < nr_max_packets; ++i) g->rw_states[i].store(0, std::memory_order_relaxed);
-    *out = g;
+    g->rw_states.reset(new (std::nothrow) std::atomic<uint8_t>[nr_max_packets]());
+    if (!g->rw_states || palloc(g->buffer, nr_max_packets * g->packet_bytes) != cudaSuccess) return RSPT_E_CUDA;
+    *out = g.release();
     return RSPT_OK;
 }
 
@@ -928,8 +882,6 @@ extern "C" int rspt_gpu_ingest_destroy(rspt_gpu_ingest* g)
     if (!g) return RSPT_E_ARG;
     DeviceGuard dg(g->p->device);
     cudaStreamSynchronize(g->p->stream);
-    if (g->buffer) cudaFreeHost(g->buffer);
-    delete[] g->rw_states;
     delete g;
     return RSPT_OK;
 }
@@ -1045,9 +997,7 @@ extern "C" int rspt_gpu_prefilter_fir(rspt_gpu_packer* p, uint8_t* d_frames, siz
     int rc = ensure_words(p);
     if (rc) return rc;
     if (p->fir_cap < (size_t)kernel_size) {
-        if (p->d_fir) cudaFree(p->d_fir);
-        p->d_fir = nullptr;
-        RSPT_CUDA_CHECK(dalloc(p->d_fir, (size_t)kernel_size));
+        RSPT_CUDA_CHECK(dalloc(p->d_fir, (size_t)kernel_size));  // the smaller buffer stays if this fails
         p->fir_cap = (size_t)kernel_size;
     }
     RSPT_CUDA_CHECK(cudaMemcpyAsync(p->d_fir, kernel, sizeof(double) * (size_t)kernel_size, cudaMemcpyHostToDevice, p->stream));
@@ -1135,47 +1085,27 @@ namespace {
 // offsets copy of the previous chunk while the next chunk is already queued.
 int ensure_host_pipe(rspt_gpu_packer* p)
 {
-    HostPipe& hp = p->pipe;
-    if (hp.chunk) return RSPT_OK;
+    if (p->pipe.chunk) return RSPT_OK;
     size_t c = (size_t)(32u << 20) / p->s.frame_bytes;  // ~32 MB of raw input per chunk
     if (const char* e = getenv("RSPT_HOST_CHUNK_FRAMES")) c = (size_t)atol(e);
     if (c < 1) c = 1;
     if (c > p->max_batch) c = p->max_batch;
-    RSPT_CUDA_CHECK(cudaStreamCreateWithFlags(&hp.s_in, cudaStreamNonBlocking));
-    RSPT_CUDA_CHECK(cudaStreamCreateWithFlags(&hp.s_out, cudaStreamNonBlocking));
+    HostPipe hp;  // the handle takes all of it or, on a failure, none of it
+    RSPT_CUDA_CHECK(create(hp.s_in));
+    RSPT_CUDA_CHECK(create(hp.s_out));
     for (int b = 0; b < 2; ++b) {
-        RSPT_CUDA_CHECK(cudaEventCreateWithFlags(&hp.ev_in[b], cudaEventDisableTiming));
-        RSPT_CUDA_CHECK(cudaEventCreateWithFlags(&hp.ev_comp[b], cudaEventDisableTiming));
-        RSPT_CUDA_CHECK(cudaEventCreateWithFlags(&hp.ev_off[b], cudaEventDisableTiming));
-        RSPT_CUDA_CHECK(cudaEventCreateWithFlags(&hp.ev_out[b], cudaEventDisableTiming));
+        RSPT_CUDA_CHECK(create(hp.ev_in[b]));
+        RSPT_CUDA_CHECK(create(hp.ev_comp[b]));
+        RSPT_CUDA_CHECK(create(hp.ev_off[b]));
+        RSPT_CUDA_CHECK(create(hp.ev_out[b]));
         RSPT_CUDA_CHECK(dalloc(hp.d_src[b], c * (size_t)p->s.frame_bytes));
         RSPT_CUDA_CHECK(dalloc(hp.d_dst[b], c * rspt_gpu_max_compressed_size(p)));
         RSPT_CUDA_CHECK(dalloc(hp.d_off[b], c + 1));
-        RSPT_CUDA_CHECK(cudaMallocHost(reinterpret_cast<void**>(&hp.h_off[b]), (c + 1) * sizeof(uint64_t)));
+        RSPT_CUDA_CHECK(palloc(hp.h_off[b], c + 1));
     }
     hp.chunk = c;
+    p->pipe = std::move(hp);
     return RSPT_OK;
-}
-
-void destroy_host_pipe(rspt_gpu_packer* p)
-{
-    HostPipe& hp = p->pipe;
-    if (!hp.s_in && !hp.s_out) return;
-    if (hp.s_in) cudaStreamSynchronize(hp.s_in);
-    if (hp.s_out) cudaStreamSynchronize(hp.s_out);
-    for (int b = 0; b < 2; ++b) {
-        if (hp.ev_in[b]) cudaEventDestroy(hp.ev_in[b]);
-        if (hp.ev_comp[b]) cudaEventDestroy(hp.ev_comp[b]);
-        if (hp.ev_off[b]) cudaEventDestroy(hp.ev_off[b]);
-        if (hp.ev_out[b]) cudaEventDestroy(hp.ev_out[b]);
-        if (hp.d_src[b]) cudaFree(hp.d_src[b]);
-        if (hp.d_dst[b]) cudaFree(hp.d_dst[b]);
-        if (hp.d_off[b]) cudaFree(hp.d_off[b]);
-        if (hp.h_off[b]) cudaFreeHost(hp.h_off[b]);
-    }
-    if (hp.s_in) cudaStreamDestroy(hp.s_in);
-    if (hp.s_out) cudaStreamDestroy(hp.s_out);
-    memset(&hp, 0, sizeof(hp));
 }
 }  // namespace
 

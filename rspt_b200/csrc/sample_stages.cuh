@@ -213,7 +213,7 @@ inline int launch_forward_transform(rspt_gpu_packer* p, const uint8_t* d_src, si
         const int rc = launch_raw_to_words(p, d_src, F);
         return rc ? rc : spectral_words_forward(p, F);
     }
-    uint32_t* need = p->can_escalate ? p->d_need : nullptr;
+    uint32_t* need = p->can_escalate ? static_cast<uint32_t*>(p->d_need) : nullptr;
     if (need) RSPT_CUDA_CHECK(cudaMemsetAsync(need, 0, F * sizeof(uint32_t), p->stream));
     const bool st = s.kind == RSPT_XDELTA_HZR;
     if (tma_transform_ok(p, d_src)) {
@@ -262,7 +262,7 @@ inline int launch_forward_transform_i32(rspt_gpu_packer* p, const int32_t* d_src
         });
         return rc ? rc : spectral_words_forward(p, F);
     }
-    uint32_t* need = p->can_escalate ? p->d_need : nullptr;
+    uint32_t* need = p->can_escalate ? static_cast<uint32_t*>(p->d_need) : nullptr;
     if (need) RSPT_CUDA_CHECK(cudaMemsetAsync(need, 0, F * sizeof(uint32_t), p->stream));
     const uint32_t chunks = (s.N + kI32Chunk - 1) / kI32Chunk;
     return with_bps(s.bps, [&](auto B) {

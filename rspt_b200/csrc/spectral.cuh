@@ -730,44 +730,47 @@ __global__ void __launch_bounds__(256) k_dct_inv_direct(int32_t* __restrict__ wo
 
 // ---- dct tables (host) ----------------------------------------------------------------------------
 
-// decided once, when the handle is created: non-power-of-two lengths need the direct path,
-// RSPT_DCT_DIRECT=1 requests it
+// the path a handle starts on: non-power-of-two lengths need the direct path, RSPT_DCT_DIRECT=1 requests it
 inline bool dct_choose_direct(uint32_t n)
 {
     const char* e = getenv("RSPT_DCT_DIRECT");
     return (n & (n - 1)) != 0 || (e && e[0] == '1');
 }
 
-inline cudaError_t dct_build_tables(rspt_gpu_packer* p)
+// FFT path (power-of-two n): n/2 twiddles in a buffer of n/2 + 1, and n post-rotations, uploaded on p->stream
+inline cudaError_t dct_build_fft_tables(rspt_gpu_packer* p)
 {
     const uint32_t n = (uint32_t)p->s.ns;
-    const double PI = 3.14159265358979323846;
-    cudaError_t e = cudaSuccess;
-    if ((n & (n - 1)) == 0) {
-        std::vector<double2> tw(n / 2 + 1), post(n);
-        for (uint32_t j = 0; j < n / 2; ++j) {
-            const long double a = -2.0L * 3.14159265358979323846264338327950288L * j / n;
-            tw[j] = make_double2((double)cosl(a), (double)sinl(a));
-        }
-        for (uint32_t k = 0; k < n; ++k) {
-            const long double a = -3.14159265358979323846264338327950288L * k / (2.0L * n);
-            post[k] = make_double2((double)cosl(a), (double)sinl(a));
-        }
-        e = cudaMalloc(&p->d_twiddle, sizeof(double2) * (n / 2 + 1));
-        if (e == cudaSuccess) e = cudaMalloc(&p->d_post, sizeof(double2) * n);
-        if (e == cudaSuccess) e = cudaMemcpy(p->d_twiddle, tw.data(), sizeof(double2) * (n / 2), cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) e = cudaMemcpy(p->d_post, post.data(), sizeof(double2) * n, cudaMemcpyHostToDevice);
+    std::vector<double2> tw(n / 2), post(n);
+    for (uint32_t j = 0; j < n / 2; ++j) {
+        const long double a = -2.0L * 3.14159265358979323846264338327950288L * j / n;
+        tw[j] = make_double2((double)cosl(a), (double)sinl(a));
     }
-    if (e == cudaSuccess && p->dct_direct) {
-        // COSINES[i][j] = (float)cos(((i << 1) * j + j) * PI / (2n))  (dct.cpp:60-68); the same
-        // symmetric-in-role table serves the forward ([x][i]) and inverse ([i][x]) sums
-        std::vector<float> t((size_t)n * n);
-        const double pi_n_2 = PI / (n * 2.0);
-        for (uint32_t i = 0; i < n; ++i)
-            for (uint32_t j = 0; j < n; ++j) t[(size_t)i * n + j] = (float)cos((double)(int)(((int)i << 1) * (int)j + (int)j) * pi_n_2);
-        e = cudaMalloc(&p->d_cos, sizeof(float) * (size_t)n * n);
-        if (e == cudaSuccess) e = cudaMemcpy(p->d_cos, t.data(), sizeof(float) * (size_t)n * n, cudaMemcpyHostToDevice);
+    for (uint32_t k = 0; k < n; ++k) {
+        const long double a = -3.14159265358979323846264338327950288L * k / (2.0L * n);
+        post[k] = make_double2((double)cosl(a), (double)sinl(a));
     }
+    cudaError_t e = dalloc(p->d_twiddle, n / 2 + 1, 0);
+    if (e == cudaSuccess) e = dalloc(p->d_post, n, 0);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(p->d_twiddle, tw.data(), sizeof(double2) * (n / 2), cudaMemcpyHostToDevice, p->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(p->d_post, post.data(), sizeof(double2) * n, cudaMemcpyHostToDevice, p->stream);
+    return e;
+}
+
+// direct path: the n x n cosine table, uploaded on p->stream; p->d_cos is set only once the upload is enqueued
+inline cudaError_t dct_build_cos_table(rspt_gpu_packer* p)
+{
+    const uint32_t n = (uint32_t)p->s.ns;
+    // COSINES[i][j] = (float)cos(((i << 1) * j + j) * PI / (2n))  (dct.cpp:60-68); the same
+    // symmetric-in-role table serves the forward ([x][i]) and inverse ([i][x]) sums
+    std::vector<float> t((size_t)n * n);
+    const double pi_n_2 = 3.14159265358979323846 / (n * 2.0);
+    for (uint32_t i = 0; i < n; ++i)
+        for (uint32_t j = 0; j < n; ++j) t[(size_t)i * n + j] = (float)cos((double)(int)(((int)i << 1) * (int)j + (int)j) * pi_n_2);
+    DeviceBuf<float> c;
+    cudaError_t e = dalloc(c, t.size(), 0);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(c, t.data(), sizeof(float) * t.size(), cudaMemcpyHostToDevice, p->stream);
+    if (e == cudaSuccess) p->d_cos = std::move(c);
     return e;
 }
 
