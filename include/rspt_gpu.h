@@ -174,6 +174,40 @@ int rspt_gpu_decompress_frames_i32(rspt_gpu_packer* p, const uint8_t* d_src, con
                                    const uint8_t* d_frame_nb, const void* d_sidecar, const int64_t* d_frame_ids,
                                    size_t n_frames, int32_t* d_dst, int32_t* d_status);
 
+/* Output element types of the _float calls. */
+enum {
+    RSPT_OUT_F32 = 0,  /* float32 */
+    RSPT_OUT_BF16 = 1  /* bfloat16 */
+};
+
+/* rspt_gpu_decompress_batch_i32 and rspt_gpu_decompress_frames_i32 with the samples in physical units, as float32
+ * or bfloat16 [n_frames][ch][ns] (a training loop's input), dequantized per channel inside the kernels that
+ * produce the samples.  With v the int32 word the _i32 call writes for an element of channel c:
+ *   f32   y = float32((int64) v - (int64) zero_point[c]) * scale[c]   int64 -> float32 rounded to nearest even,
+ *                                                                      then one float32 multiply rounded to nearest
+ *   bf16  y above, rounded to nearest even to bfloat16 (not the exact product rounded once)
+ * which is bit for bit what numpy ((v.astype(int64) - zp).astype(float32) * scale) or torch ((v.long() - zp).float()
+ * * scale, then .to(torch.bfloat16)) computes from the int32 output.  IEEE throughout: subnormal results are kept,
+ * overflow gives +-inf.  Results are specified for finite scales.
+ *   out_type        RSPT_OUT_F32 or RSPT_OUT_BF16
+ *   d_zero_point    int32 [ch] on the device, or NULL = 0 for every channel
+ *   d_scale         float32 [ch] on the device, or NULL = 1.0 for every channel
+ *   d_dst           [n_frames][ch][ns] elements of 4 (f32) or 2 (bf16) bytes, aligned to its element size;
+ *                   16-byte alignment is faster
+ * Everything else (sidecar or none, ids in any order with repeats, RSPT_E_ARG in the status slot of an id outside
+ * [0, n_stored), n_stored not limited by the handle, counters, the PARSE / DECODE / INVERSE stage timers) is as for
+ * the _i32 calls, and so is the call: asynchronous on the handle's stream.  The kernels read d_zero_point and d_scale
+ * while the call runs, so the caller keeps them alive and unchanged until the stream has passed it.  Refused before
+ * anything is launched: an unknown out_type, a NULL d_dst or one not aligned to its element size (RSPT_E_ARG),
+ * n_frames > max_batch_frames (RSPT_E_CAPACITY). */
+int rspt_gpu_decompress_batch_float(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets, size_t n_frames,
+                                    const uint8_t* d_frame_nb, const void* d_sidecar, int out_type,
+                                    const int32_t* d_zero_point, const float* d_scale, void* d_dst, int32_t* d_status);
+int rspt_gpu_decompress_frames_float(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets, size_t n_stored,
+                                     const uint8_t* d_frame_nb, const void* d_sidecar, const int64_t* d_frame_ids,
+                                     size_t n_frames, int out_type, const int32_t* d_zero_point, const float* d_scale,
+                                     void* d_dst, int32_t* d_status);
+
 /* Integrity check without decoding: replaces hzr_verify (lib_hzr/hzr_decode.c:569-624) applied to
  * every hzr stream of `n_frames` frames -- frame / chunk / block headers are walked as in
  * decompress, and the CRC-32C of every block payload is compared with the block header.

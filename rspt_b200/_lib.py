@@ -9,6 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "librspt_gpu.so")
 
 KINDS = {"xdelta_hzr": 0, "hzr": 1, "hadamard": 2, "dct": 3}
+OUT_TYPES = {"float32": 0, "bfloat16": 1}  # RSPT_OUT_F32 / RSPT_OUT_BF16
 STAGES = ["transform", "hist", "tree", "layout", "encode", "parse", "decode", "inverse"]
 ERRORS = {0: "ok", -1: "bad argument / unsupported shape", -2: "CUDA error", -3: "capacity too small",
           -4: "malformed stream", -5: "no CUDA device", -6: "CRC-32C mismatch"}
@@ -20,6 +21,7 @@ EXPORTS = [
     "rspt_gpu_compress_batch_i32", "rspt_gpu_decompress_batch_i32",
     "rspt_gpu_compress_append", "rspt_gpu_compress_append_i32", "rspt_gpu_build_index_frames",
     "rspt_gpu_decompress_frames", "rspt_gpu_decompress_frames_i32",
+    "rspt_gpu_decompress_batch_float", "rspt_gpu_decompress_frames_float",
     "rspt_gpu_sidecar_bytes", "rspt_gpu_sidecar_used_bytes", "rspt_gpu_compress_host", "rspt_gpu_decompress_host",
     "rspt_gpu_compress_batch_host", "rspt_gpu_decompress_batch_host", "rspt_gpu_sync", "rspt_gpu_last_error",
     "rspt_gpu_get_counters", "rspt_gpu_debug_planes", "rspt_gpu_debug_hzr_tables", "rspt_gpu_crc32c",
@@ -83,6 +85,10 @@ def lib() -> C.CDLL:
     for name in ("rspt_gpu_decompress_frames", "rspt_gpu_decompress_frames_i32"):
         getattr(L, name).restype = C.c_int
         getattr(L, name).argtypes = [vp, vp, vp, sz, vp, vp, vp, sz, vp, vp]
+    L.rspt_gpu_decompress_batch_float.restype = C.c_int
+    L.rspt_gpu_decompress_batch_float.argtypes = [vp, vp, vp, sz, vp, vp, C.c_int, vp, vp, vp, vp]
+    L.rspt_gpu_decompress_frames_float.restype = C.c_int
+    L.rspt_gpu_decompress_frames_float.argtypes = [vp, vp, vp, sz, vp, vp, vp, sz, C.c_int, vp, vp, vp, vp]
     dp = C.POINTER(C.c_double)
     L.rspt_gpu_prefilter_iir.restype = C.c_int
     L.rspt_gpu_prefilter_iir.argtypes = [vp, vp, sz, dp, dp, C.c_int, C.c_int]

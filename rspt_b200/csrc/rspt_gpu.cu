@@ -629,11 +629,23 @@ constexpr uint32_t kDecodePairMaxBits = 4;
 
 namespace {
 
-// the decoded samples go to out.raw (interleaved native) or out.words (int32 [ch][ns]); exactly one is set
+// the decoded samples go to out.raw (interleaved native), out.words (int32 [ch][ns]) or out.fdst (float32 / bfloat16
+// [ch][ns] as out_type says, dequantized with dq); exactly one is set
 struct SamplesOut {
     uint8_t* raw;
     int32_t* words;
+    void* fdst = nullptr;
+    int out_type = RSPT_OUT_F32;
+    Dequant dq = {};
 };
+
+// the checks of the _float calls' out_type and d_dst
+bool float_out_ok(int out_type, const void* d_dst)
+{
+    if (out_type != RSPT_OUT_F32 && out_type != RSPT_OUT_BF16) return false;
+    const uintptr_t align = out_type == RSPT_OUT_F32 ? 4 : 2;
+    return d_dst && ((uintptr_t)d_dst & (align - 1)) == 0;
+}
 
 // Slot f of the output decodes stored frame f (ids = NULL: the batch calls) or stored frame ids[f] of the
 // n_stored frames that d_offsets / d_frame_nb / d_sidecar describe (the gather calls).
@@ -683,6 +695,7 @@ int decompress_batch(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d
         if (rc) return rc;
     }
     StageTimer t(p, RSPT_STAGE_INVERSE);
+    if (out.fdst) return launch_inverse_transform_float(p, out.out_type, out.fdst, out.dq, F);
     return out.words ? launch_inverse_transform_i32(p, out.words, F) : launch_inverse_transform(p, out.raw, F);
 }
 
@@ -720,6 +733,26 @@ extern "C" int rspt_gpu_decompress_frames_i32(rspt_gpu_packer* p, const uint8_t*
     if (!p || !d_src || !d_offsets || !d_frame_ids || !d_dst || ((uintptr_t)d_dst & 3)) return RSPT_E_ARG;
     return decompress_batch(p, d_src, d_offsets, n_frames, d_frame_nb, d_sidecar, SamplesOut{nullptr, d_dst}, d_status,
                             d_frame_ids, n_stored);
+}
+
+extern "C" int rspt_gpu_decompress_batch_float(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets,
+                                               size_t n_frames, const uint8_t* d_frame_nb, const void* d_sidecar, int out_type,
+                                               const int32_t* d_zero_point, const float* d_scale, void* d_dst, int32_t* d_status)
+{
+    if (!p || !d_src || !d_offsets || !float_out_ok(out_type, d_dst)) return RSPT_E_ARG;
+    return decompress_batch(p, d_src, d_offsets, n_frames, d_frame_nb, d_sidecar,
+                            SamplesOut{nullptr, nullptr, d_dst, out_type, Dequant{d_zero_point, d_scale}}, d_status);
+}
+
+extern "C" int rspt_gpu_decompress_frames_float(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets,
+                                                size_t n_stored, const uint8_t* d_frame_nb, const void* d_sidecar,
+                                                const int64_t* d_frame_ids, size_t n_frames, int out_type,
+                                                const int32_t* d_zero_point, const float* d_scale, void* d_dst, int32_t* d_status)
+{
+    if (!p || !d_src || !d_offsets || !d_frame_ids || !float_out_ok(out_type, d_dst)) return RSPT_E_ARG;
+    return decompress_batch(p, d_src, d_offsets, n_frames, d_frame_nb, d_sidecar,
+                            SamplesOut{nullptr, nullptr, d_dst, out_type, Dequant{d_zero_point, d_scale}}, d_status, d_frame_ids,
+                            n_stored);
 }
 
 extern "C" int rspt_gpu_verify_batch(rspt_gpu_packer* p, const uint8_t* d_src, const uint64_t* d_offsets, size_t n_frames,

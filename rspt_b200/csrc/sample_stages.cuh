@@ -360,4 +360,46 @@ inline int launch_inverse_transform_i32(rspt_gpu_packer* p, int32_t* d_dst, size
     });
 }
 
+// to float32 / bfloat16 [ch][ns] (rspt_gpu_decompress_*_float, out_type RSPT_OUT_F32 / RSPT_OUT_BF16): the samples
+// launch_inverse_transform_i32 writes, dequantized per channel by the kernel that produces them.  The same
+// eligibility decides between the same kernels with a float store; hadamard needs no word scratch and no second
+// kernel, dct ends in k_words_to_float instead of k_words_sext.  d_dst needs the alignment of its element; 16
+// bytes let the fast sample kernel store it directly.
+inline int launch_inverse_transform_float(rspt_gpu_packer* p, int out_type, void* d_dst, Dequant dq, size_t F)
+{
+    const Shape& s = p->s;
+    auto run = [&](auto* dst) -> int {
+        using OutT = std::remove_pointer_t<decltype(dst)>;
+        const dim3 g2((unsigned)(F * s.ch));
+        if (s.kind == RSPT_HADAMARD) {
+            if (fwht_fast_len(s.ns))
+                return with_flag(s.ns == 4096, [&](auto n4096) {
+                    constexpr int LG = n4096 ? 12 : 13;
+                    return launch(p, k_dq_fwht_fast_inv<LG, OutT>, g2, (1 << LG) / 16, 0, p->d_planes, p->d_headers,
+                                  p->d_dec_nb, s, dst, dq);
+                });
+            return launch(p, k_dq_fwht_inv<OutT>, g2, 256, fwht_smem(s), p->d_planes, p->d_headers, p->d_dec_nb, s, dst, dq);
+        }
+        if (s.kind == RSPT_DCT) {
+            const int rc = spectral_inverse_words(p, F, p->d_words);
+            if (rc) return rc;
+            const size_t n = F * (size_t)s.N;
+            return with_bps(s.bps, [&](auto B) {
+                return launch(p, k_words_to_float<B, OutT>, (unsigned)((n + 1023) / 1024), 256, 0, p->d_words, s, n, dst, dq);
+            });
+        }
+        const bool fast = inv_words_fast_ok(s, dst);
+        return with_bps(s.bps, [&](auto B) {
+            return with_flag(s.kind == RSPT_XDELTA_HZR, [&](auto SC) {
+                if (fast)
+                    return launch(p, k_dq_planes_to_samples_fast<B, SC, OutT>, (unsigned)F, kInvThreads,
+                                  inv_words_fast_smem(s), p->d_planes, s, p->d_dec_nb, dst, dq);
+                return launch(p, k_dq_planes_to_samples<B, SC, OutT>, (unsigned)F, 512, inv_carry_bytes(s), p->d_planes,
+                              s, p->d_dec_nb, dst, dq);
+            });
+        });
+    };
+    return out_type == RSPT_OUT_BF16 ? run(static_cast<__nv_bfloat16*>(d_dst)) : run(static_cast<float*>(d_dst));
+}
+
 }  // namespace rspt

@@ -80,9 +80,20 @@ __global__ void __launch_bounds__(256) k_fwht_fwd(const int32_t* __restrict__ wo
     }
 }
 
-// one CTA per (frame, channel): planes -> q (sign-extended from 24 bits) -> FWHT -> + mean24
-__global__ void __launch_bounds__(256) k_fwht_inv(const uint8_t* __restrict__ planes, const uint8_t* __restrict__ headers,
-                                                   const uint8_t* __restrict__ dec_nb, Shape s, int32_t* __restrict__ words)
+// the float output of a hadamard sample word w (the full 32-bit sum): sign-extended from 8 * bps bits as
+// k_words_sext does, then dequantized
+template <class OutT>
+__device__ __forceinline__ OutT fwht_out(uint32_t w, int sh, const ChanDq& d)
+{
+    return out_elem<OutT>((int32_t)(w << sh) >> sh, d);
+}
+
+// one CTA per (frame, channel): planes -> q (sign-extended from 24 bits) -> FWHT -> + mean24.  The body of
+// k_fwht_inv (OutT = int32_t: the full words) and k_dq_fwht_inv (float / __nv_bfloat16: the samples, dequantized
+// with dq).
+template <class OutT>
+__device__ __forceinline__ void fwht_inv(const uint8_t* __restrict__ planes, const uint8_t* __restrict__ headers,
+                                         const uint8_t* __restrict__ dec_nb, Shape s, OutT* __restrict__ words, Dequant dq)
 {
     extern __shared__ __align__(16) uint32_t a[];
     const uint32_t f = blockIdx.x / s.ch, c = blockIdx.x % s.ch, n = (uint32_t)s.ns;
@@ -97,8 +108,28 @@ __global__ void __launch_bounds__(256) k_fwht_inv(const uint8_t* __restrict__ pl
     __syncthreads();
     fwht_smem(a, n);
     const int32_t mean = load_mean24(headers + (size_t)f * s.hdr_bytes + 3 * c);
-    int32_t* w = words + (size_t)f * s.N + (size_t)c * n;
-    for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) w[i] = (int32_t)(a[i] + (uint32_t)mean);
+    OutT* w = words + (size_t)f * s.N + (size_t)c * n;
+    if constexpr (std::is_same_v<OutT, int32_t>) {
+        for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) w[i] = (int32_t)(a[i] + (uint32_t)mean);
+    } else {
+        const ChanDq d = chan_dq(dq, c);
+        const int osh = 32 - 8 * s.bps;
+        for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) w[i] = fwht_out<OutT>(a[i] + (uint32_t)mean, osh, d);
+    }
+}
+
+__global__ void __launch_bounds__(256) k_fwht_inv(const uint8_t* __restrict__ planes, const uint8_t* __restrict__ headers,
+                                                   const uint8_t* __restrict__ dec_nb, Shape s, int32_t* __restrict__ words)
+{
+    fwht_inv(planes, headers, dec_nb, s, words, Dequant{});
+}
+
+template <class OutT>
+__global__ void __launch_bounds__(256) k_dq_fwht_inv(const uint8_t* __restrict__ planes, const uint8_t* __restrict__ headers,
+                                                      const uint8_t* __restrict__ dec_nb, Shape s, OutT* __restrict__ dst,
+                                                      Dequant dq)
+{
+    fwht_inv(planes, headers, dec_nb, s, dst, dq);
 }
 
 // ---- n = 4096 / 8192 fast path: three radix-16 passes in registers ---------------------------
@@ -190,13 +221,17 @@ __global__ void __launch_bounds__((1 << LG) / 16) k_fwht_fast_fwd(const int32_t*
             *reinterpret_cast<uint4*>(out + (size_t)k * s.plane_stride) = make_uint4(pl[k][0], pl[k][1], pl[k][2], pl[k][3]);
 }
 
-template <int LG>
-__global__ void __launch_bounds__((1 << LG) / 16) k_fwht_fast_inv(const uint8_t* __restrict__ planes, const uint8_t* __restrict__ headers,
-                                                                   const uint8_t* __restrict__ dec_nb, Shape s, int32_t* __restrict__ words)
+// the body of k_fwht_fast_inv and k_dq_fwht_fast_inv; OutT as for fwht_inv.  t = threadIdx.x, read by the kernel:
+// there the compiler knows from __launch_bounds__ that t < N / 16 and keeps the index terms' disjoint bits as
+// ORs and narrow masks, which a read inside this inlined body loses.
+template <int LG, class OutT>
+__device__ __forceinline__ void fwht_fast_inv(const uint8_t* __restrict__ planes, const uint8_t* __restrict__ headers,
+                                              const uint8_t* __restrict__ dec_nb, Shape s, OutT* __restrict__ words, Dequant dq,
+                                              uint32_t t)
 {
     constexpr uint32_t N = 1u << LG, T = N / 16, S2 = N / 256;
     __shared__ uint32_t a[N + N / 32];
-    const uint32_t f = blockIdx.x / s.ch, c = blockIdx.x % s.ch, t = threadIdx.x;
+    const uint32_t f = blockIdx.x / s.ch, c = blockIdx.x % s.ch;
     const uint32_t nb = dec_nb[f];
     const uint8_t* in = planes + (size_t)f * s.nb_alloc * s.plane_stride + (size_t)c * N + 16 * t;
     uint4 pv[4];
@@ -231,9 +266,32 @@ __global__ void __launch_bounds__((1 << LG) / 16) k_fwht_fast_inv(const uint8_t*
     for (int j = 0; j < 16; ++j) r[j] = a[fwht_phys(t + T * j)];
     radix16(r);
     const uint32_t mean = (uint32_t)load_mean24(headers + (size_t)f * s.hdr_bytes + 3 * c);
-    uint32_t* w = reinterpret_cast<uint32_t*>(words) + (size_t)f * s.N + (size_t)c * N;
+    if constexpr (std::is_same_v<OutT, int32_t>) {
+        uint32_t* w = reinterpret_cast<uint32_t*>(words) + (size_t)f * s.N + (size_t)c * N;
 #pragma unroll
-    for (int j = 0; j < 16; ++j) w[t + T * j] = r[j] + mean;
+        for (int j = 0; j < 16; ++j) w[t + T * j] = r[j] + mean;
+    } else {
+        const ChanDq d = chan_dq(dq, c);
+        const int osh = 32 - 8 * s.bps;
+        OutT* w = words + (size_t)f * s.N + (size_t)c * N;
+#pragma unroll
+        for (int j = 0; j < 16; ++j) w[t + T * j] = fwht_out<OutT>(r[j] + mean, osh, d);
+    }
+}
+
+template <int LG>
+__global__ void __launch_bounds__((1 << LG) / 16) k_fwht_fast_inv(const uint8_t* __restrict__ planes, const uint8_t* __restrict__ headers,
+                                                                   const uint8_t* __restrict__ dec_nb, Shape s, int32_t* __restrict__ words)
+{
+    fwht_fast_inv<LG>(planes, headers, dec_nb, s, words, Dequant{}, threadIdx.x);
+}
+
+template <int LG, class OutT>
+__global__ void __launch_bounds__((1 << LG) / 16) k_dq_fwht_fast_inv(const uint8_t* __restrict__ planes, const uint8_t* __restrict__ headers,
+                                                                      const uint8_t* __restrict__ dec_nb, Shape s, OutT* __restrict__ dst,
+                                                                      Dequant dq)
+{
+    fwht_fast_inv<LG>(planes, headers, dec_nb, s, dst, dq, threadIdx.x);
 }
 
 // ---- fused fast path: interleaved samples <-> planes without the int32 word matrix ------------

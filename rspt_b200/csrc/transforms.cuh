@@ -5,6 +5,10 @@
 // signal_packer_base.cpp:40-68 and :122-138.
 #pragma once
 
+#include <cuda_bf16.h>
+
+#include <type_traits>
+
 #include "common.cuh"
 #include "hzr_encode.cuh"
 
@@ -274,6 +278,61 @@ __device__ __forceinline__ uint32_t sext_bps(uint32_t w)
     return (uint32_t)((int32_t)(w << (32 - 8 * BPS)) >> (32 - 8 * BPS));
 }
 
+// ---- float output (rspt_gpu_decompress_*_float) ---------------------------------------------------------------
+// The sample kernels take their output element type as a template argument: int32_t (the sample word itself),
+// float or __nv_bfloat16.  A float output of sample v in channel c is float32((int64)v - zp[c]) * scale[c], each
+// step rounded once to nearest even; bf16 rounds that float32.  The intrinsics keep nvcc from contracting or
+// reordering the two steps, so the result is the one a caller gets from the int32 output in numpy or torch.
+struct Dequant {
+    const int32_t* zp;  // [ch] or NULL = 0
+    const float* scale; // [ch] or NULL = 1.0f
+};
+
+// the zero point and scale of one channel
+struct ChanDq {
+    long long zp;
+    float scale;
+};
+
+__device__ __forceinline__ ChanDq chan_dq(const Dequant& q, uint32_t c)
+{
+    return ChanDq{q.zp ? (long long)__ldg(q.zp + c) : 0ll, q.scale ? __ldg(q.scale + c) : 1.0f};
+}
+
+// the output element of the sign-extended sample v
+template <class OutT>
+__device__ __forceinline__ OutT out_elem(int32_t v, const ChanDq& d)
+{
+    const float y = __fmul_rn(__ll2float_rn((long long)v - d.zp), d.scale);
+    if constexpr (std::is_same_v<OutT, float>)
+        return y;
+    else
+        return __float2bfloat16_rn(y);
+}
+
+// N (4 or 8) consecutive sign-extended samples of one channel -> N output elements at dst, with 8- or 16-byte
+// stores (dst aligned to N elements)
+template <class OutT, int N>
+__device__ __forceinline__ void store_out(OutT* dst, const uint32_t (&y)[N], const ChanDq& d)
+{
+    if constexpr (std::is_same_v<OutT, float>) {
+#pragma unroll
+        for (int k = 0; k < N; k += 4)
+            *reinterpret_cast<float4*>(dst + k) = make_float4(out_elem<float>((int32_t)y[k], d), out_elem<float>((int32_t)y[k + 1], d),
+                                                              out_elem<float>((int32_t)y[k + 2], d), out_elem<float>((int32_t)y[k + 3], d));
+    } else {
+        uint32_t h[N / 2];
+#pragma unroll
+        for (int k = 0; k < N / 2; ++k)
+            h[k] = (uint32_t)__bfloat16_as_ushort(out_elem<OutT>((int32_t)y[2 * k], d)) |
+                   ((uint32_t)__bfloat16_as_ushort(out_elem<OutT>((int32_t)y[2 * k + 1], d)) << 16);
+        if constexpr (N == 8)
+            *reinterpret_cast<uint4*>(dst) = make_uint4(h[0], h[1], h[2], h[3]);
+        else
+            *reinterpret_cast<uint2*>(dst) = make_uint2(h[0], h[1]);
+    }
+}
+
 template <int BPS, bool STENCIL>
 __global__ void __launch_bounds__(256) k_xdelta_planes_i32(const int32_t* __restrict__ src, Shape s, uint32_t chunks,
                                                             uint8_t* __restrict__ planes, uint32_t* __restrict__ need)
@@ -397,10 +456,12 @@ __device__ __forceinline__ void smem_exclusive_scan(uint32_t* a, uint32_t n)
     }
 }
 
-template <int BPS, bool SCAN, bool OUT_RAW>
-__global__ void __launch_bounds__(512) k_planes_to_samples(const uint8_t* __restrict__ planes, Shape s,
-                                                            const uint8_t* __restrict__ dec_nb,
-                                                            uint8_t* __restrict__ dst_raw, int32_t* __restrict__ dst_words)
+// the body of k_planes_to_samples and k_dq_planes_to_samples; OutT (word output only): int32_t, or float /
+// __nv_bfloat16 dequantized with dq
+template <int BPS, bool SCAN, bool OUT_RAW, class OutT>
+__device__ __forceinline__ void planes_to_samples(const uint8_t* __restrict__ planes, Shape s,
+                                                  const uint8_t* __restrict__ dec_nb, uint8_t* __restrict__ dst_raw,
+                                                  OutT* __restrict__ dst_words, Dequant dq)
 {
     extern __shared__ __align__(16) uint32_t sm32[];
     const uint32_t f = blockIdx.x;
@@ -510,12 +571,18 @@ __global__ void __launch_bounds__(512) k_planes_to_samples(const uint8_t* __rest
 #pragma unroll
                         for (int bb = 0; bb < BPS; ++bb) q[bb] = (uint8_t)(y[i] >> (8 * bb));
                     }
-            } else {
+            } else if constexpr (std::is_same_v<OutT, int32_t>) {
                 // sample words are sign-extended from 8*BPS bits (the dct's coefficient words use BPS = 4)
                 int32_t* w = dst_words + (size_t)f * s.N + (size_t)c * ns + s0;
 #pragma unroll
                 for (int i = 0; i < 8; ++i)
                     if ((uint32_t)i < cnt) w[i] = (int32_t)sext_bps<BPS>(y[i]);
+            } else {
+                const ChanDq d = chan_dq(dq, c);
+                OutT* w = dst_words + (size_t)f * s.N + (size_t)c * ns + s0;
+#pragma unroll
+                for (int i = 0; i < 8; ++i)
+                    if ((uint32_t)i < cnt) w[i] = out_elem<OutT>((int32_t)sext_bps<BPS>(y[i]), d);
             }
         }
         if (OUT_RAW) {
@@ -524,6 +591,23 @@ __global__ void __launch_bounds__(512) k_planes_to_samples(const uint8_t* __rest
             __syncthreads();
         }
     }
+}
+
+template <int BPS, bool SCAN, bool OUT_RAW>
+__global__ void __launch_bounds__(512) k_planes_to_samples(const uint8_t* __restrict__ planes, Shape s,
+                                                            const uint8_t* __restrict__ dec_nb,
+                                                            uint8_t* __restrict__ dst_raw, int32_t* __restrict__ dst_words)
+{
+    planes_to_samples<BPS, SCAN, OUT_RAW>(planes, s, dec_nb, dst_raw, dst_words, Dequant{});
+}
+
+// float32 / bfloat16 output of the same body (rspt_gpu_decompress_*_float; "dq": dequantized)
+template <int BPS, bool SCAN, class OutT>
+__global__ void __launch_bounds__(512) k_dq_planes_to_samples(const uint8_t* __restrict__ planes, Shape s,
+                                                               const uint8_t* __restrict__ dec_nb, OutT* __restrict__ dst,
+                                                               Dequant dq)
+{
+    planes_to_samples<BPS, SCAN, false>(planes, s, dec_nb, nullptr, dst, dq);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -578,12 +662,14 @@ __device__ __forceinline__ uint32_t warp_add_inclusive(uint32_t v)
     return v;
 }
 
-template <int BPS, bool SCAN, bool WORDS = false>
-__global__ void __launch_bounds__(1024, 1) k_planes_to_samples_fast(const uint8_t* __restrict__ planes, Shape s,
-                                                                            const uint8_t* __restrict__ dec_nb,
-                                                                            uint32_t tiles_per_group,
-                                                                            uint8_t* __restrict__ dst_raw,
-                                                                            int32_t* __restrict__ dst_words = nullptr)
+// the body of k_planes_to_samples_fast and k_dq_planes_to_samples_fast; OutT (WORDS only): int32_t, or float /
+// __nv_bfloat16 dequantized with dq (the piece's channel is pp / ppc; a lane's 8 values leave as two 16-byte stores
+// for float, one for bf16)
+template <int BPS, bool SCAN, bool WORDS, class OutT>
+__device__ __forceinline__ void planes_to_samples_fast(const uint8_t* __restrict__ planes, Shape s,
+                                                       const uint8_t* __restrict__ dec_nb, uint32_t tiles_per_group,
+                                                       uint8_t* __restrict__ dst_raw, OutT* __restrict__ dst_words,
+                                                       Dequant dq)
 {
     extern __shared__ __align__(16) uint32_t sm32[];
     const uint32_t f = blockIdx.x;
@@ -744,9 +830,15 @@ __global__ void __launch_bounds__(1024, 1) k_planes_to_samples_fast(const uint8_
 #pragma unroll
                     for (int i = 0; i < 8; ++i) y[i] += base;
                 }
-                uint4* w2 = wout + (size_t)(P0 + u) * 64u + 2u * lane;
-                w2[0] = make_uint4(sext_bps<BPS>(y[0]), sext_bps<BPS>(y[1]), sext_bps<BPS>(y[2]), sext_bps<BPS>(y[3]));
-                w2[1] = make_uint4(sext_bps<BPS>(y[4]), sext_bps<BPS>(y[5]), sext_bps<BPS>(y[6]), sext_bps<BPS>(y[7]));
+                if constexpr (std::is_same_v<OutT, int32_t>) {
+                    uint4* w2 = wout + (size_t)(P0 + u) * 64u + 2u * lane;
+                    w2[0] = make_uint4(sext_bps<BPS>(y[0]), sext_bps<BPS>(y[1]), sext_bps<BPS>(y[2]), sext_bps<BPS>(y[3]));
+                    w2[1] = make_uint4(sext_bps<BPS>(y[4]), sext_bps<BPS>(y[5]), sext_bps<BPS>(y[6]), sext_bps<BPS>(y[7]));
+                } else {
+#pragma unroll
+                    for (int i = 0; i < 8; ++i) y[i] = sext_bps<BPS>(y[i]);
+                    store_out(dst_words + (size_t)f * s.N + (size_t)(P0 + u) * 256u + 8u * lane, y, chan_dq(dq, pp / ppc));
+                }
             }
         }
         return;
@@ -906,6 +998,25 @@ __global__ void __launch_bounds__(1024, 1) k_planes_to_samples_fast(const uint8_
         }
         __syncthreads();
     }
+}
+
+template <int BPS, bool SCAN, bool WORDS = false>
+__global__ void __launch_bounds__(1024, 1) k_planes_to_samples_fast(const uint8_t* __restrict__ planes, Shape s,
+                                                                            const uint8_t* __restrict__ dec_nb,
+                                                                            uint32_t tiles_per_group,
+                                                                            uint8_t* __restrict__ dst_raw,
+                                                                            int32_t* __restrict__ dst_words = nullptr)
+{
+    planes_to_samples_fast<BPS, SCAN, WORDS>(planes, s, dec_nb, tiles_per_group, dst_raw, dst_words, Dequant{});
+}
+
+// float32 / bfloat16 output of the same body's word path
+template <int BPS, bool SCAN, class OutT>
+__global__ void __launch_bounds__(1024, 1) k_dq_planes_to_samples_fast(const uint8_t* __restrict__ planes, Shape s,
+                                                                       const uint8_t* __restrict__ dec_nb,
+                                                                       OutT* __restrict__ dst, Dequant dq)
+{
+    planes_to_samples_fast<BPS, SCAN, true>(planes, s, dec_nb, 1, nullptr, dst, dq);
 }
 
 // int32 words [ch][ns] -> interleaved little-endian samples; one CTA per (frame, 256-sample tile)
@@ -1105,6 +1216,36 @@ __global__ void __launch_bounds__(256) k_words_sext(const int32_t* __restrict__ 
 #pragma unroll
         for (int k = 0; k < 4; ++k)
             if ((uint32_t)k < cnt) out[k] = sext_bps<BPS>(__ldg(in + k));
+    }
+}
+
+// decoded word matrix -> float output of rspt_gpu_decompress_*_float (dct): k_words_sext's sample, dequantized
+// with the zero point and scale of its channel ((i / ns) % ch of flat element i) and converted.  4 words per thread.
+template <int BPS, class OutT>
+__global__ void __launch_bounds__(256) k_words_to_float(const int32_t* __restrict__ words, Shape s, size_t n,
+                                                         OutT* __restrict__ dst, Dequant dq)
+{
+    const size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) * 4u;
+    if (i >= n) return;
+    const uint32_t cnt = n - i < 4 ? (uint32_t)(n - i) : 4u;
+    const uint32_t ns = (uint32_t)s.ns, ch = (uint32_t)s.ch;
+    const size_t row = i / ns;
+    uint32_t col = (uint32_t)(i - row * ns), c = (uint32_t)(row % ch);
+    ChanDq d = chan_dq(dq, c);
+    const uint32_t* in = reinterpret_cast<const uint32_t*>(words) + i;
+    if (cnt == 4 && col + 4 <= ns && ((uintptr_t)(dst + i) & (4 * sizeof(OutT) - 1)) == 0) {
+        const uint4 v = __ldg(reinterpret_cast<const uint4*>(in));
+        const uint32_t y[4] = {sext_bps<BPS>(v.x), sext_bps<BPS>(v.y), sext_bps<BPS>(v.z), sext_bps<BPS>(v.w)};
+        store_out(dst + i, y, d);
+    } else {
+        for (uint32_t k = 0; k < cnt; ++k, ++col) {
+            if (col == ns) {  // the next channel row (or channel 0 of the next frame)
+                col = 0;
+                c = c + 1 == ch ? 0 : c + 1;
+                d = chan_dq(dq, c);
+            }
+            dst[i + k] = out_elem<OutT>((int32_t)sext_bps<BPS>(__ldg(in + k)), d);
+        }
     }
 }
 

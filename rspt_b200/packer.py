@@ -350,24 +350,72 @@ class SignalPacker:
         return self._decompress(self.L.rspt_gpu_decompress_batch, batch, out, status, use_sidecar)
 
     def decompress_tensor(self, batch: CompressedBatch, out: torch.Tensor | None = None, status: torch.Tensor | None = None,
-                          use_sidecar: bool = True) -> torch.Tensor:
+                          use_sidecar: bool = True, *, dtype: torch.dtype = torch.int32, zero_point=None,
+                          scale=None) -> torch.Tensor:
         """The batch's samples as an int32 tensor [n, ch, ns]: every word is the sample decompress_batch writes,
         sign-extended from 8 * bps bits.  `out`, when given, must be a contiguous int32 tensor of that shape on the
-        handle's device."""
+        handle's device.
+
+        dtype torch.float32 or torch.bfloat16: the samples in physical units, dequantized per channel c inside the
+        decode kernels (rspt_gpu_decompress_batch_float).  With x the int32 output, the result is bit for bit
+        (x.long() - zero_point).float() * scale, and for bfloat16 that value's .to(torch.bfloat16).  zero_point: an
+        int32 CUDA tensor [ch] on the handle's device or a sequence of ints (None = 0); scale: a float32 CUDA tensor
+        [ch] or a sequence of floats (None = 1.0).  `out` must then have that dtype.  The call is asynchronous and
+        its kernels read zero_point and scale: keep tensors passed for them unchanged until the stream passes it."""
         n = batch.n_frames
+        dq = self._dequant(dtype, zero_point, scale)
+        out = self._samples_out(out, n, dtype)
+        if dq is None:
+            return self._decompress(self.L.rspt_gpu_decompress_batch_i32, batch, out, status, use_sidecar)
+        return self._decompress(self.L.rspt_gpu_decompress_batch_float, batch, out, status, use_sidecar, dq=dq)
+
+    def _samples_out(self, out: torch.Tensor | None, n: int, dtype: torch.dtype) -> torch.Tensor:
         if out is None:
-            out = torch.empty((n, self.ch, self.ns), dtype=torch.int32, device=self._dev())
-        self._check_words(out, n)
-        return self._decompress(self.L.rspt_gpu_decompress_batch_i32, batch, out, status, use_sidecar)
+            out = torch.empty((n, self.ch, self.ns), dtype=dtype, device=self._dev())
+        if dtype == torch.int32:
+            self._check_words(out, n)
+        elif not (isinstance(out, torch.Tensor) and out.dtype == dtype and out.is_cuda and out.device.index == self.device
+                  and tuple(out.shape) == (n, self.ch, self.ns) and out.is_contiguous()):
+            raise ValueError(f"expected a contiguous {dtype} tensor [{n}, {self.ch}, {self.ns}] on cuda:{self.device}")
+        return out
+
+    def _dequant(self, dtype: torch.dtype, zero_point, scale):
+        """(out_type, zero point, scale) of the _float calls, the last two as device tensors or None; None for int32
+        output.  Sequences become tensors allocated on the current stream, which the call runs on: once the caller
+        drops them, the caching allocator hands their memory only to work ordered behind the call."""
+        if dtype == torch.int32:
+            if zero_point is not None or scale is not None:
+                raise ValueError("zero_point and scale apply to float32 / bfloat16 output only")
+            return None
+        out_type = {torch.float32: _lib.OUT_TYPES["float32"], torch.bfloat16: _lib.OUT_TYPES["bfloat16"]}.get(dtype)
+        if out_type is None:
+            raise ValueError(f"dtype must be torch.int32, torch.float32 or torch.bfloat16, not {dtype}")
+
+        def per_channel(v, want: torch.dtype, name: str):
+            if v is None:
+                return None
+            if not isinstance(v, torch.Tensor):
+                v = torch.tensor(list(v), dtype=want, device=self._dev())
+            if not (v.dtype == want and v.is_cuda and v.device.index == self.device and tuple(v.shape) == (self.ch,)
+                    and v.is_contiguous()):
+                raise ValueError(f"{name} must be a contiguous {want} tensor [{self.ch}] on cuda:{self.device}, "
+                                 f"or a sequence of {self.ch} numbers")
+            return v
+
+        zp = per_channel(zero_point, torch.int32, "zero_point")
+        sc = per_channel(scale, torch.float32, "scale")
+        return out_type, zp, sc
 
     def _decompress(self, fn, batch: CompressedBatch, out: torch.Tensor, status: torch.Tensor | None,
-                    use_sidecar: bool, ids: torch.Tensor | None = None) -> torch.Tensor:
-        """The whole batch, or (ids given: the gather calls) its frames ids[0], ids[1], ..."""
+                    use_sidecar: bool, ids: torch.Tensor | None = None, dq: tuple = ()) -> torch.Tensor:
+        """The whole batch, or (ids given: the gather calls) its frames ids[0], ids[1], ...; dq: the _float calls'
+        (out_type, zero point, scale), the tensors held here until the call is enqueued"""
         sc = batch.sidecar.data_ptr() if (use_sidecar and batch.sidecar is not None) else None
         nbp = batch.frame_nb.data_ptr() if batch.frame_nb is not None else None
         sel = () if ids is None else (ids.data_ptr(), ids.numel())
+        fargs = tuple(a.data_ptr() if isinstance(a, torch.Tensor) else a for a in dq)
         self._bind_stream()
-        rc = fn(self.h, batch.stream.data_ptr(), batch.offsets.data_ptr(), batch.n_frames, nbp, sc, *sel,
+        rc = fn(self.h, batch.stream.data_ptr(), batch.offsets.data_ptr(), batch.n_frames, nbp, sc, *sel, *fargs,
                 out.data_ptr(), status.data_ptr() if status is not None else None)
         check(rc, self.h, fn.__name__)
         return out
@@ -387,14 +435,18 @@ class SignalPacker:
         return self._decompress(self.L.rspt_gpu_decompress_frames, batch, out, status, use_sidecar, ids)
 
     def decompress_frames_tensor(self, batch: CompressedBatch, frame_ids, out: torch.Tensor | None = None,
-                                 status: torch.Tensor | None = None, use_sidecar: bool = True) -> torch.Tensor:
-        """decompress_frames with the samples as an int32 tensor [n, ch, ns], as decompress_tensor writes them."""
+                                 status: torch.Tensor | None = None, use_sidecar: bool = True, *,
+                                 dtype: torch.dtype = torch.int32, zero_point=None, scale=None) -> torch.Tensor:
+        """decompress_frames with the samples as an int32 tensor [n, ch, ns], as decompress_tensor writes them; dtype,
+        zero_point and scale as for decompress_tensor (rspt_gpu_decompress_frames_float): a minibatch of stored
+        frames in physical units."""
         ids = self._frame_ids(frame_ids)
         n = ids.numel()
-        if out is None:
-            out = torch.empty((n, self.ch, self.ns), dtype=torch.int32, device=self._dev())
-        self._check_words(out, n)
-        return self._decompress(self.L.rspt_gpu_decompress_frames_i32, batch, out, status, use_sidecar, ids)
+        dq = self._dequant(dtype, zero_point, scale)
+        out = self._samples_out(out, n, dtype)
+        if dq is None:
+            return self._decompress(self.L.rspt_gpu_decompress_frames_i32, batch, out, status, use_sidecar, ids)
+        return self._decompress(self.L.rspt_gpu_decompress_frames_float, batch, out, status, use_sidecar, ids, dq)
 
     def _frame_ids(self, frame_ids) -> torch.Tensor:
         if isinstance(frame_ids, (list, tuple, range)):
