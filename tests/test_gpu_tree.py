@@ -1,6 +1,6 @@
 """The dense and sparse tree builds (k_hzr_tree) against the oracle's MakeTree on chosen histograms:
 code words, code lengths, tree_nbits and n_used through the per-block debug entry, and the serialised
-tree through a one-block hzr frame compared byte for byte with the oracle's stream.  Needs a B200."""
+tree through a one-block hzr frame compared byte for byte with the oracle's stream and decoded back.  Needs a B200."""
 import numpy as np
 import pytest
 
@@ -112,3 +112,12 @@ def test_tree_matches_oracle(R, O, L, kind):
     offs = batch.offsets.cpu().numpy()
     got = batch.stream.cpu().numpy()[offs[0]:offs[1]].tobytes()
     assert got == O.OraclePacker("hzr", 1, 1, block.size, 0).compress(block)
+
+    # and back: with the encoder's decode index and with one rebuilt from the stream
+    bare = R.CompressedBatch(batch.stream, batch.offsets, batch.frame_nb, None, 1)
+    for what, b in (("encoder index", batch), ("rebuilt index", q.build_index(bare))):
+        status = torch.full((1,), 7, dtype=torch.int32, device="cuda")
+        dec = q.decompress_batch(b, status=status)
+        torch.cuda.synchronize()
+        assert status.item() == 0, what
+        assert np.array_equal(dec.cpu().numpy(), block), what
